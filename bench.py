@@ -304,6 +304,25 @@ def config_legs(torch, dev_index, ncores, hbm_peak, fp64_peak, with_cpu=True):
     return out
 
 
+def dump_outputs(outdir, tensors, limit=64 * 10**6):
+    """Per-chain outputs of one step as DIR/<name>.npy (flag as float32, the rest float64), so that two
+    builds can be compared output for output on the same seeded inputs.  Above `limit` bytes in all, the
+    same fixed, seeded sample of chains is kept from every array and its indices go to rows.npy.  Rows
+    whose flag is 0 (failed root search) hold unspecified values."""
+    arrays = {k: t.cpu().numpy().astype(np.float32 if t.dtype.itemsize == 1 else np.float64)
+              for k, t in tensors.items()}
+    nrows = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) / nrows
+    if nrows * row_bytes > limit:
+        keep = int((limit - 4096) // (row_bytes + 8))     # 4096: room for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(nrows, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(outdir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(outdir, k + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -317,7 +336,13 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the C2/C3/C5 legs (run at N=1 only)")
     ap.add_argument("--hmc-traj", type=int, default=100, help="trajectories per chain in the HMC legs")
     ap.add_argument("--da-budget", type=float, default=15.0, help="wall-clock budget of the uncapped DA leg (s)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write U, grad, dsyn and flag of the last timed step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -420,6 +445,8 @@ def main():
     sampler.start()
     l0 = ctx.launches
     ms = timed_steps(args.steps)
+    if args.dump_outputs and rank == 0:       # before profile_eval below overwrites the buffers
+        dump_outputs(args.dump_outputs, {"U": U, "grad": G, "dsyn": D, "flag": Fl})
     launches = ctx.launches - l0
     nev = ctx.read_evals()
     ctx.count_evals(False)

@@ -1,8 +1,9 @@
-"""Golden vectors from the REFERENCE'S OWN Python code, run in the build container:
+"""Golden vectors from the REFERENCE'S OWN Python code:
 
-    python tests/golden/make_reference_golden.py        ->  tests/golden/reference_code.npz
+    RFSURFHMC_REFERENCE=<checkout of the original RfSurfHmc> python tests/golden/make_reference_golden.py
+                                                        ->  tests/golden/reference_code.npz
 
-What runs unmodified from /root/reference (imported, never copied):
+What runs unmodified from that checkout (imported, never copied):
   * model/model_surf.py, model/model_rf.py, model/model_rf_swd_vs_thk.py  -- Brocher relations,
     chain rule, residual contraction, joint weighting, failure convention   (SURVEY rows a1-a3)
   * pyhmc/hmc.py  (HamitonianMC)  and  pyhmc/hmcda.py  (HMCDualAveraging)  -- initial model,
@@ -18,7 +19,7 @@ What is stubbed, because it cannot exist here (gfortran / FFTW3 / h5py absent):
   * `h5py` -> an in-memory stand-in (the samplers only write results through it).
 The fixture pins oracle.surf_* / rf_* (the restated C++ layers), oracle.joint_batch (the restated
 glue) and oracle/hmc_ref.py (the restated samplers) against the reference's real code on top of
-the same numerics; tests never need /root/reference.
+the same numerics; tests never need the checkout.
 """
 import contextlib
 import io
@@ -29,7 +30,9 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
+REF = os.environ.get("RFSURFHMC_REFERENCE")     # a checkout of the original RfSurfHmc project
+if not REF:
+    sys.exit("set RFSURFHMC_REFERENCE to a checkout of the original RfSurfHmc project")
 sys.path.insert(0, ROOT)
 from oracle.oracle import Oracle  # noqa: E402
 
@@ -57,9 +60,10 @@ h5.File = _FakeH5File
 sys.modules["h5py"] = h5
 
 import subprocess  # noqa: E402
-subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], stdout=subprocess.DEVNULL)
+subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref", "REF=" + os.path.abspath(REF)],
+                      stdout=subprocess.DEVNULL)
 sys.path.insert(0, os.path.join(ROOT, "oracle", "_ref"))
-import libsurf  # noqa: E402  (the reference's own pybind11 module, built from /root/reference)
+import libsurf  # noqa: E402  (the reference's own pybind11 module, built from its checkout)
 import librf  # noqa: E402
 lib = types.ModuleType("model.lib")
 lib.__path__ = []

@@ -1,7 +1,7 @@
 """Golden vectors for rfsurfhmc_b200/utils.py from the reference's own src/utils.py, imported
-unmodified from /root/reference (matplotlib, which that module imports but the two functions do not
-use, is replaced by an empty stand-in when absent).  Run in the build container:
-    python tests/golden/make_utils_golden.py        -> tests/golden/utils_resample.npz"""
+unmodified from a checkout of the original RfSurfHmc project (matplotlib, which that module imports but
+the two functions do not use, is replaced by an empty stand-in when absent):
+    RFSURFHMC_REFERENCE=<checkout> python tests/golden/make_utils_golden.py   -> tests/golden/utils_resample.npz"""
 import importlib.util
 import os
 import sys
@@ -15,7 +15,10 @@ except Exception:
     m.pyplot = types.ModuleType("matplotlib.pyplot")
     sys.modules["matplotlib"] = m
     sys.modules["matplotlib.pyplot"] = m.pyplot
-spec = importlib.util.spec_from_file_location("ref_utils", "/root/reference/src/utils.py")
+REF = os.environ.get("RFSURFHMC_REFERENCE")     # a checkout of the original RfSurfHmc project
+if not REF:
+    sys.exit("set RFSURFHMC_REFERENCE to a checkout of the original RfSurfHmc project")
+spec = importlib.util.spec_from_file_location("ref_utils", os.path.join(REF, "src", "utils.py"))
 ref = importlib.util.module_from_spec(spec)
 spec.loader.exec_module(ref)
 

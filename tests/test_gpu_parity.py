@@ -596,3 +596,27 @@ def test_host_pipeline_matches_blocking_api(ctx):
     for (U, g, d, f), (U2, g2, d2, f2) in zip(ref, got):
         assert np.array_equal(U, U2) and np.array_equal(g, g2) and np.array_equal(d, d2)
         assert np.array_equal(f, f2.astype(bool))
+
+
+def test_bench_dump_outputs_is_the_last_timed_step(ctx, tmp_path):
+    """`bench.py --dump-outputs DIR` writes what the last timed step returned.  With 6 timed steps over
+    the 4 rotated input batches that is the second batch (a dump of any other step has other inputs),
+    recomputed here through the blocking host API on the same seeded inputs and observations."""
+    import subprocess, sys
+    import bench
+    B, steps = 256, 6
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3",
+                        "--chains", str(B), "--no-hmc", "--no-configs", "--no-cpu-baseline",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert sorted(os.listdir(tmp_path)) == ["U.npy", "dsyn.npy", "flag.npy", "grad.npy"]
+    cfg, x0, _ = bench.workload(1, 0)
+    _joint_ctx(ctx, np.zeros(197), cfg)
+    ctx.config_obs(bench.make_dobs_gpu(ctx, cfg, x0))
+    U, g, d, f = ctx.misfit_grad_host(bench.workload(B, 1000 + (steps - 1) % 4)[2])
+    got = {k: np.load(tmp_path / f"{k}.npy") for k in ("U", "grad", "dsyn", "flag")}
+    assert got["flag"].dtype == np.float32 and got["U"].dtype == np.float64
+    assert got["U"].shape == (B,) and got["grad"].shape == (B, 14) and got["dsyn"].shape == (B, 197)
+    assert np.array_equal(got["flag"] == 1, f) and f.sum() > B // 2
+    for a, b in ((got["U"], U), (got["grad"], g), (got["dsyn"], d)):
+        assert np.allclose(a[f], b[f], rtol=1e-12, atol=0)
