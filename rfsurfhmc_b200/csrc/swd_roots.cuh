@@ -439,7 +439,6 @@ RFS_DEVINL float gtsolh_dev(float a, float b) {
   return c;
 }
 
-// phases of the flattened getsol/nevill state machine
 // prologue of surfdisp96 (:128-220): water-layer flag, largest S velocity and the float32 start
 // value cc1 = 0.90 * 0.95 * (Rayleigh velocity of the slowest layer as a half space) -- all REAL*4
 template <class MT>
@@ -470,163 +469,164 @@ RFS_DEVINL void swd_start_values(const MT &M, long long mb, int &llw, float &bet
   cc1 = __fmul_rn(0.90f, cc1);
 }
 
+// phases of the flattened getsol/nevill state machine
 enum { PH_SETUP = 0, PH_G_FIRST, PH_G_SCAN, PH_N_TOP, PH_N_OUTSIDE, PH_DONE };
 
-// Solve all modes 1..nmode of sequence `sq` for model b.
+// One column of Neville's table (nevill's x or y).  The caller owns the two columns as objects of their
+// own: they are indexed at run time, so as members they would keep the whole state in local memory
+// instead of registers, and as one object they change the register allocation of the team kernels.
+struct alignas(16) SwdNevCol {
+  double v[12];
+};
+
+// The mode and period loops of surfdisp96, getsol and nevill, flattened into one state machine that
+// solves all modes 1..nmode of sequence `sq` for model b.  It asks for one secular value at a time,
+// Delta(ceval), and never evaluates it itself:
+//   start    once: prologue of surfdisp96 and the job's period range;
+//   advance  while phase == PH_SETUP: next (mode, period) and its start values (PH_G_FIRST), or PH_DONE;
+//   consume  one getsol/nevill step with Delta(ceval); stores an accepted root, cuts a failed mode off.
+// The thread-mapped (swd_solve_sequence) and the team-mapped (swd_solve_team) searches both drive
+// this one machine; they differ only in where and when the secular values are computed, so every
+// mapping returns the same roots and counts the same evaluations.
 //  cout  : [nmode_out][nper][stride] float32-rounded roots (0 where a mode does not exist)
 //  cwork : [nper][stride] unrounded roots of the running mode (chain state), used when nmode > 1
-// returns ierr of this job (1 = fundamental mode not found).
-//
-// The mode loop, the period loop, getsol and nevill are ONE loop whose body performs exactly one
-// secular evaluation: lanes never wait for each other at period or mode boundaries.  The per-period
-// retries of _surfdisp (surfdisp.cpp:93-100) are separate single-period jobs (swd_retry_kernel).
-//
-// Warp-cooperative tail: rare models need 5-10x more evaluations than the rest (upward scans from
-// the floor velocity in the per-period retries).  All 32 lanes of a warp stay in the loop until
-// the last one is done; lanes that are finished evaluate look-ahead scan points c2+j*dc for one
-// scanning lane (same repeated additions, hence bit-identical grid) and hand the values over
-// through shared memory (`wsm`, 32 doubles per warp).  `valid` = this lane owns a sequence.
-// MT: model accessor; mb = this lane's model index for M.ld (the batch index b for the global block,
-// the thread's column for a block staged in shared memory); b always indexes the outputs.
-template <class MT>
-RFS_DEVINL int swd_solve_sequence(const MT &M, long long b, long long mb, const SwdSeq &sq,
-                                  const double *__restrict__ periods, int nmode, int all_modes,
-                                  double *__restrict__ cout, long long cout_mode_stride,
-                                  double *__restrict__ cwork, long long stride,
-                                  unsigned int &n_evals, bool valid, double *wsm, int only_k) {
-  const unsigned FULL = 0xffffffffu;
-  const int lane = threadIdx.x & 31;
-  const int ifunc = sq.ifunc;
-  const int kmax = sq.nper;
-  // ---- prologue of surfdisp96 (:128-220): extremal velocities and float32 start value
+// Neville's table xs/ys is most of the kernels' stack frame: the state is only passed by reference.
+struct SwdRootSearch {
+  static constexpr double dc = (double)0.005f;  // scan step
+  // ---- job and output addressing
+  const SwdSeq &sq;
+  const double *periods;
+  int nmode, all_modes;
+  double *cout;
+  long long cout_mode_stride;
+  double *cwork;
+  long long stride, b;
+  unsigned int &n_evals;  // consumed secular values
+  // ---- prologue of surfdisp96
   int llw;
-  float betmx, cc1;
-  swd_start_values(M, mb, llw, betmx, cc1);
-  const double cc = (double)cc1;
-  const double dc = (double)0.005f;
-  const double one = 1.0e-2, onea = 1.5;
-  const double cm = cc;
-  const double betmxd = (double)betmx;
-  const double twopi = 2.0 * RFS_PI64;
-
+  double cc, betmxd;
   // ---- loop-nest state (job / mode / period)
-  // only_k < 0: the main pass over all periods; only_k >= 0: the single-period job with which
-  // _surfdisp retries a period whose result was zero (surfdisp.cpp:93-100, run by swd_retry_kernel)
-  int kb = (only_k < 0) ? 0 : only_k, jk = (only_k < 0) ? kmax : 1;  // job = periods [kb, kb+jk)
+  int kb, jk;  // job = periods [kb, kb+jk)
   int iq = 1, k = 0, ift = 999, job_ierr = 0;
   double cprev = 0.0, del1st = 0.0;
   // ---- root-search state (getsol / nevill)
   double c1 = 0.0, c2 = 0.0, clow = 0.0, del1 = 0.0, del2 = 0.0, c3 = 0.0, del3 = 0.0, omega = 0.0,
          iomega = 0.0;
-  double xs[12], ys[12];
+  double *xs, *ys;  // Neville's table, SwdNevCol::v of the caller
   int idir = 1, nev = 1, nctrl = 1, mm = 1, ifirst = 0;
-  int phase = valid ? PH_SETUP : PH_DONE;
+  int phase = PH_SETUP;
   double ceval = 0.0;
 
-  for (;;) {
-    if (phase == PH_SETUP) {
-      // ---- advance the (job, mode, period) nest until a root search starts or all is done
-      for (;;) {
-        if (iq <= nmode && k < jk && (k + 1 >= ift)) {
-          // label 1700/1750 reached through `if(k.ge.ift)`: this mode is cut off from k on
-          double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
-          if (iq <= 1) job_ierr = 1;
-          ift = k + 1;
-          for (int i = k; i < jk; i++) cq[(long long)(sq.out_off + kb + i) * stride + b] = 0.0;
-          iq++;
-          k = 0;
-          continue;
-        }
-        if (iq <= nmode && k >= jk) {  // mode finished normally
-          iq++;
-          k = 0;
-          continue;
-        }
-        if (iq > nmode) {  // job finished
-          phase = PH_DONE;
-          break;
-        }
-        // ---- start values of (iq, k) (surfdisp96.f:257-276)
-        const double t1 = __ldg(periods + sq.per_off + kb + k) * sq.scale;
-        omega = twopi / t1;
-        iomega = 1.0 / omega;
-        if (k == 0 && iq == 1) {
-          c1 = cc;
-          clow = cc;
-          ifirst = 1;
-        } else if (k == 0 && iq > 1) {
-          c1 = RFS_ADD(cwork[(long long)(sq.out_off + kb + 0) * stride + b], RFS_MUL(one, dc));
-          clow = c1;
-          ifirst = 1;
-        } else if (k > 0 && iq > 1) {
-          ifirst = 0;
-          clow = RFS_ADD(cwork[(long long)(sq.out_off + kb + k) * stride + b], RFS_MUL(one, dc));
-          c1 = cprev;
-          if (c1 < clow) c1 = clow;
-        } else {
-          ifirst = 0;
-          c1 = RFS_SUB(cprev, RFS_MUL(onea, dc));
-          clow = cm;
-        }
-        ceval = c1;
-        phase = PH_G_FIRST;
-        break;
-      }
-    }
-    // ---- warp bookkeeping: who is finished, who is scanning upward
-    const unsigned done_mask = __ballot_sync(FULL, phase == PH_DONE);
-    if (done_mask == FULL) break;
-    const unsigned want_mask = __ballot_sync(FULL, phase == PH_G_SCAN && idir > 0);
-    int nhelp = 0, hsrc = 0, hj = 0;
-    bool helper = false;
-    double e_c = ceval, e_om = omega, e_iom = iomega;
-    long long e_b = mb;
-    int e_llw = llw, e_if = ifunc;
-    if (done_mask != 0u && want_mask != 0u) {
-      hsrc = __ffs(want_mask) - 1;
-      nhelp = __popc(done_mask);
-      const double c_h = __shfl_sync(FULL, ceval, hsrc);
-      const double om_h = __shfl_sync(FULL, omega, hsrc);
-      const double iom_h = __shfl_sync(FULL, iomega, hsrc);
-      const long long b_h = __shfl_sync(FULL, mb, hsrc);
-      const int llw_h = __shfl_sync(FULL, llw, hsrc);
-      const int if_h = __shfl_sync(FULL, ifunc, hsrc);
-      if (phase == PH_DONE) {
-        helper = true;
-        hj = __popc(done_mask & ((1u << lane) - 1u)) + 1;  // look-ahead index 1..nhelp
-        double c = c_h;
-        for (int t = 0; t < hj; t++) c = c + dc;           // same additions as the scanning lane
-        e_c = c;
-        e_om = om_h;
-        e_iom = iom_h;
-        e_b = b_h;
-        e_llw = llw_h;
-        e_if = if_h;
-      }
-    }
+  RFS_DEVINL SwdRootSearch(SwdNevCol &xs_, SwdNevCol &ys_, const SwdSeq &sq_, const double *periods_,
+                           int nmode_, int all_modes_, double *cout_, long long cout_mode_stride_,
+                           double *cwork_, long long stride_, long long b_, unsigned int &n_evals_)
+      : sq(sq_), periods(periods_), nmode(nmode_), all_modes(all_modes_), cout(cout_),
+        cout_mode_stride(cout_mode_stride_), cwork(cwork_), stride(stride_), b(b_),
+        n_evals(n_evals_), xs(xs_.v), ys(ys_.v) {}
 
-    // ---- the single secular-function evaluation site
-    double val = 0.0;
-    if (phase != PH_DONE || helper) {
-      const double wv = e_om / e_c;
-      val = (e_if == 1) ? dltar1_dev(wv, e_om, M, e_b, e_llw)
-                        : dltar4_dev(wv, e_om, e_iom, M, e_b, e_llw);
+  // mb = the model's index for M.ld.  only_k < 0: the main pass over all periods; only_k >= 0: the
+  // single-period job with which _surfdisp retries a period whose result was zero
+  // (surfdisp.cpp:93-100, run by swd_retry_kernel)
+  template <class MT>
+  RFS_DEVINL void start(const MT &M, long long mb, int only_k) {
+    float betmx, cc1;
+    swd_start_values(M, mb, llw, betmx, cc1);
+    cc = (double)cc1;
+    betmxd = (double)betmx;
+    kb = (only_k < 0) ? 0 : only_k;
+    jk = (only_k < 0) ? sq.nper : 1;
+  }
+
+  // output index of period i of the job; the output block of mode iq
+  RFS_DEVINL long long at(int i) const { return (long long)(sq.out_off + kb + i) * stride + b; }
+  RFS_DEVINL double *mode_out() const {
+    return cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
+  }
+
+  // label 1700/1750: mode iq is cut off from period k on (its results are 0), next mode
+  RFS_DEVINL void cut_mode() {
+    double *cq = mode_out();
+    if (iq <= 1) job_ierr = 1;
+    ift = k + 1;
+    for (int i = k; i < jk; i++) cq[at(i)] = 0.0;
+    iq++;
+    k = 0;
+  }
+
+  // advance the (job, mode, period) nest until a root search starts or all is done
+  RFS_DEVINL void advance() {
+    for (;;) {
+      if (iq <= nmode && k < jk && (k + 1 >= ift)) {  // reached through `if(k.ge.ift)`
+        cut_mode();
+        continue;
+      }
+      if (iq <= nmode && k >= jk) {  // mode finished normally
+        iq++;
+        k = 0;
+        continue;
+      }
+      if (iq > nmode) {  // job finished
+        phase = PH_DONE;
+        return;
+      }
+      // ---- start values of (iq, k) (surfdisp96.f:257-276); surfdisp96's cm is cc
+      const double one = 1.0e-2, onea = 1.5;
+      const double twopi = 2.0 * RFS_PI64;
+      const double t1 = __ldg(periods + sq.per_off + kb + k) * sq.scale;
+      omega = twopi / t1;
+      iomega = 1.0 / omega;
+      if (k == 0 && iq == 1) {
+        c1 = cc;
+        clow = cc;
+        ifirst = 1;
+      } else if (k == 0 && iq > 1) {
+        c1 = RFS_ADD(cwork[at(0)], RFS_MUL(one, dc));
+        clow = c1;
+        ifirst = 1;
+      } else if (k > 0 && iq > 1) {
+        ifirst = 0;
+        clow = RFS_ADD(cwork[at(k)], RFS_MUL(one, dc));
+        c1 = cprev;
+        if (c1 < clow) c1 = clow;
+      } else {
+        ifirst = 0;
+        c1 = RFS_SUB(cprev, RFS_MUL(onea, dc));
+        clow = cc;
+      }
+      ceval = c1;
+      phase = PH_G_FIRST;
+      return;
     }
-    if (nhelp) {
-      if (helper) wsm[hj] = val;
-      __syncwarp();
+  }
+
+  // label 1000 (getsol :457-470): the next scan point c2 = c1 +- dc, turned upward at clow
+  RFS_DEVINL void next_scan_point() {
+    for (;;) {
+      c2 = (idir > 0) ? c1 + dc : c1 - dc;
+      if (c2 <= clow) {
+        idir = +1;
+        c1 = clow;
+        continue;
+      }
+      break;
     }
-    if (phase == PH_DONE) {
-      if (nhelp) __syncwarp();
-      continue;
-    }
+    ceval = c2;
+  }
+
+  // one step of getsol / nevill with val = Delta(ceval)
+  RFS_DEVINL void consume(double val) {
     n_evals++;
-
-    int iret = 0;  // 0 running, 1 root accepted, -1 failed
+    int iret = 0;  // 0 running, 1 root accepted, -1 failed, 2 nevill done
     bool body = false;
-    // one upward/downward scan step given Delta(c2) (getsol :457-479)
-    auto scan_step = [&](double v) {
-      del2 = v;
+    if (phase == PH_G_FIRST) {
+      del1 = val;
+      if (ifirst == 1) del1st = del1;
+      // plmn = dsign(1, del1st) * dsign(1, del1) >= 0 (:452-456)
+      idir = (ifirst == 1 || neg1(del1st) == neg1(del1)) ? +1 : -1;
+      next_scan_point();
+      phase = PH_G_SCAN;
+    } else if (phase == PH_G_SCAN) {  // one upward/downward scan step (getsol :457-479)
+      del2 = val;
       if (neg1(del1) != neg1(del2)) {
         c3 = 0.5 * (c1 + c2);  // bracketed -> nevill: initial half
         ceval = c3;
@@ -636,46 +636,10 @@ RFS_DEVINL int swd_solve_sequence(const MT &M, long long b, long long mb, const 
       } else {
         c1 = c2;
         del1 = del2;
-        if (c1 < cm || c1 >= (betmxd + dc)) {
+        if (c1 < cc || c1 >= (betmxd + dc)) {
           iret = -1;
         } else {
-          for (;;) {
-            c2 = (idir > 0) ? c1 + dc : c1 - dc;
-            if (c2 <= clow) {
-              idir = +1;
-              c1 = clow;
-              continue;
-            }
-            break;
-          }
-          ceval = c2;
-        }
-      }
-    };
-    if (phase == PH_G_FIRST) {
-      del1 = val;
-      if (ifirst == 1) del1st = del1;
-      // plmn = dsign(1, del1st) * dsign(1, del1) >= 0 (:452-456)
-      idir = (ifirst == 1 || neg1(del1st) == neg1(del1)) ? +1 : -1;
-      for (;;) {  // label 1000 (:457-470)
-        c2 = (idir > 0) ? c1 + dc : c1 - dc;
-        if (c2 <= clow) {
-          idir = +1;
-          c1 = clow;
-          continue;
-        }
-        break;
-      }
-      ceval = c2;
-      phase = PH_G_SCAN;
-    } else if (phase == PH_G_SCAN) {
-      scan_step(val);
-      if (nhelp && lane == hsrc) {
-        // consume the look-ahead values while the scan simply slides upward
-        for (int j = 1; j <= nhelp; j++) {
-          if (!(phase == PH_G_SCAN && idir > 0 && iret == 0)) break;
-          n_evals++;
-          scan_step(wsm[j]);
+          next_scan_point();
         }
       }
     } else if (phase == PH_N_TOP) {
@@ -756,24 +720,105 @@ RFS_DEVINL int swd_solve_sequence(const MT &M, long long b, long long mb, const 
       iret = (c1 > betmxd) ? -1 : 1;
     }
     if (iret == 1) {
-      double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
       cprev = c1;
-      if (nmode > 1) cwork[(long long)(sq.out_off + kb + k) * stride + b] = c1;
-      cq[(long long)(sq.out_off + kb + k) * stride + b] = (double)(float)c1;  // cg(k)=sngl(c(k))
+      if (nmode > 1) cwork[at(k)] = c1;
+      mode_out()[at(k)] = (double)(float)c1;  // cg(k)=sngl(c(k))
       k++;
       phase = PH_SETUP;
     } else if (iret == -1) {
-      double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
-      if (iq <= 1) job_ierr = 1;
-      ift = k + 1;
-      for (int i = k; i < jk; i++) cq[(long long)(sq.out_off + kb + i) * stride + b] = 0.0;
-      iq++;
-      k = 0;
+      cut_mode();
       phase = PH_SETUP;
     }
+  }
+};
+
+// K1: one thread per (model, sequence) drives SwdRootSearch; returns ierr of this job (1 =
+// fundamental mode not found).
+//
+// The mode loop, the period loop, getsol and nevill are ONE loop whose body performs exactly one
+// secular evaluation: lanes never wait for each other at period or mode boundaries.  The per-period
+// retries of _surfdisp (surfdisp.cpp:93-100) are separate single-period jobs (swd_retry_kernel).
+//
+// Warp-cooperative tail: rare models need 5-10x more evaluations than the rest (upward scans from
+// the floor velocity in the per-period retries).  All 32 lanes of a warp stay in the loop until
+// the last one is done; lanes that are finished evaluate look-ahead scan points c2+j*dc for one
+// scanning lane (same repeated additions, hence bit-identical grid) and hand the values over
+// through shared memory (`wsm`, 32 doubles per warp).  `valid` = this lane owns a sequence.
+// MT: model accessor; mb = this lane's model index for M.ld (the batch index b for the global block,
+// the thread's column for a block staged in shared memory); b always indexes the outputs.
+template <class MT>
+RFS_DEVINL int swd_solve_sequence(const MT &M, long long b, long long mb, const SwdSeq &sq,
+                                  const double *__restrict__ periods, int nmode, int all_modes,
+                                  double *__restrict__ cout, long long cout_mode_stride,
+                                  double *__restrict__ cwork, long long stride,
+                                  unsigned int &n_evals, bool valid, double *wsm, int only_k) {
+  const unsigned FULL = 0xffffffffu;
+  const int lane = threadIdx.x & 31;
+  const int ifunc = sq.ifunc;
+  SwdNevCol xs, ys;
+  SwdRootSearch rs(xs, ys, sq, periods, nmode, all_modes, cout, cout_mode_stride, cwork, stride, b,
+                   n_evals);
+  rs.start(M, mb, only_k);
+  if (!valid) rs.phase = PH_DONE;
+
+  for (;;) {
+    if (rs.phase == PH_SETUP) rs.advance();
+    // ---- warp bookkeeping: who is finished, who is scanning upward
+    const unsigned done_mask = __ballot_sync(FULL, rs.phase == PH_DONE);
+    if (done_mask == FULL) break;
+    const unsigned want_mask = __ballot_sync(FULL, rs.phase == PH_G_SCAN && rs.idir > 0);
+    int nhelp = 0, hsrc = 0, hj = 0;
+    bool helper = false;
+    double e_c = rs.ceval, e_om = rs.omega, e_iom = rs.iomega;
+    long long e_b = mb;
+    int e_llw = rs.llw, e_if = ifunc;
+    if (done_mask != 0u && want_mask != 0u) {
+      hsrc = __ffs(want_mask) - 1;
+      nhelp = __popc(done_mask);
+      const double c_h = __shfl_sync(FULL, rs.ceval, hsrc);
+      const double om_h = __shfl_sync(FULL, rs.omega, hsrc);
+      const double iom_h = __shfl_sync(FULL, rs.iomega, hsrc);
+      const long long b_h = __shfl_sync(FULL, mb, hsrc);
+      const int llw_h = __shfl_sync(FULL, rs.llw, hsrc);
+      const int if_h = __shfl_sync(FULL, ifunc, hsrc);
+      if (rs.phase == PH_DONE) {
+        helper = true;
+        hj = __popc(done_mask & ((1u << lane) - 1u)) + 1;  // look-ahead index 1..nhelp
+        double c = c_h;
+        for (int t = 0; t < hj; t++) c = c + SwdRootSearch::dc;  // same additions as the scanning lane
+        e_c = c;
+        e_om = om_h;
+        e_iom = iom_h;
+        e_b = b_h;
+        e_llw = llw_h;
+        e_if = if_h;
+      }
+    }
+
+    // ---- the single secular-function evaluation site
+    double val = 0.0;
+    if (rs.phase != PH_DONE || helper) {
+      const double wv = e_om / e_c;
+      val = (e_if == 1) ? dltar1_dev(wv, e_om, M, e_b, e_llw)
+                        : dltar4_dev(wv, e_om, e_iom, M, e_b, e_llw);
+    }
+    if (nhelp) {
+      if (helper) wsm[hj] = val;
+      __syncwarp();
+    }
+    if (rs.phase == PH_DONE) {
+      if (nhelp) __syncwarp();
+      continue;
+    }
+    rs.consume(val);
+    // the lane being helped consumes the look-ahead values while its scan simply slides upward (a
+    // bracket or a failed scan leaves PH_G_SCAN).  A call site of its own keeps the common path
+    // straight-line: one shared loop over val, wsm[1..] is 2 % slower (B200 at 1000 W).
+    if (nhelp && lane == hsrc)
+      for (int j = 1; j <= nhelp && rs.phase == PH_G_SCAN && rs.idir > 0; j++) rs.consume(wsm[j]);
     if (nhelp) __syncwarp();  // wsm may be rewritten in the next trip
   }
-  return job_ierr;
+  return rs.job_ierr;
 }
 
 }  // namespace rfs

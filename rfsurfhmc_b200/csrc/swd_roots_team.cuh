@@ -5,8 +5,9 @@
 //
 // Same algorithm, same operations, same bits (surfdisp96.f: surfdisp96 :54-368, getsol :398-491,
 // nevill :568-687, dltar1 :727-787, dltar4 :791-891): the returned roots are bit-identical to the
-// thread-mapped kernel (GPU test), because every secular value is produced by the same inlined
-// functions in the same order.  What changes is the schedule:
+// thread-mapped kernel (GPU test), because both mappings drive the one getsol/nevill state machine
+// (SwdRootSearch, swd_roots.cuh) and every secular value is produced by the same inlined functions in
+// the same order.  What changes is the schedule:
 //
 //  * layer parallelism.  A team evaluates the secular function cooperatively.  The Dunkin 5x5 layer
 //    matrices (resp. the Love layer terms) — ~4/5 of the arithmetic, independent from layer to layer
@@ -143,10 +144,10 @@ RFS_DEVINL double team_secular(const SmemModel &M, int ifunc, int llw, double om
   return e0;
 }
 
-// The flattened surfdisp96/getsol/nevill state machine of swd_solve_sequence (swd_roots.cuh), run
-// by a team.  Every lane of the team executes it with identical values.  Global results are written
-// by every lane (same address, same value: one transaction), so each lane later reads back its own
-// store of the chain values in `cwork`.
+// A team drives the state machine that the thread mapping drives too (SwdRootSearch, swd_roots.cuh).
+// Every lane of the team runs it with identical values.  Global results are written by every lane
+// (same address, same value: one transaction), so each lane later reads back its own store of the
+// chain values in `cwork`.
 template <int T, int S>
 RFS_DEVINL int swd_solve_team(const SmemModel &M, long long b, const SwdSeq &sq,
                               const double *__restrict__ periods, int nmode, int all_modes,
@@ -154,255 +155,23 @@ RFS_DEVINL int swd_solve_team(const SmemModel &M, long long b, const SwdSeq &sq,
                               double *__restrict__ cwork, long long stride, unsigned int &n_evals,
                               unsigned tmask, int tl, int only_k, double2 *park, int lane) {
   constexpr int GL = T / S;
-  const int mmax = M.n;
-  const int ifunc = sq.ifunc;
-  const int kmax = sq.nper;
-  // ---- prologue of surfdisp96 (:128-220): extremal velocities and float32 start value
-  const int llw = (M.ld(F_B, 0, 0) <= 0.0) ? 2 : 1;
-  int jmn = 0, jsol = 1;
-  float betmx = -1.e20f, betmn = 1.e20f;
-  for (int i = 0; i < mmax; i++) {
-    const float bi = (float)M.ld(F_B, i, 0), ai = (float)M.ld(F_A, i, 0);
-    if (bi > 0.01f && bi < betmn) {
-      betmn = bi;
-      jmn = i;
-      jsol = 1;
-    } else if (bi <= 0.01f && ai < betmn) {
-      betmn = ai;
-      jmn = i;
-      jsol = 0;
-    }
-    if (bi > betmx) betmx = bi;
-  }
-  float cc1;
-  if (jsol == 0)
-    cc1 = betmn;
-  else
-    cc1 = gtsolh_dev((float)M.ld(F_A, jmn, 0), (float)M.ld(F_B, jmn, 0));
-  cc1 = __fmul_rn(0.95f, cc1);
-  cc1 = __fmul_rn(0.90f, cc1);
-  const double cc = (double)cc1;
-  const double dc = (double)0.005f;
-  const double one = 1.0e-2, onea = 1.5;
-  const double cm = cc;
-  const double betmxd = (double)betmx;
-  const double twopi = 2.0 * RFS_PI64;
-
-  // ---- loop-nest state (job / mode / period); see swd_solve_sequence for the meaning of only_k
-  const int kb = (only_k < 0) ? 0 : only_k, jk = (only_k < 0) ? kmax : 1;
-  int iq = 1, k = 0, ift = 999, job_ierr = 0;
-  double cprev = 0.0, del1st = 0.0;
-  // ---- root-search state (getsol / nevill)
-  double c1 = 0.0, c2 = 0.0, clow = 0.0, del1 = 0.0, del2 = 0.0, c3 = 0.0, del3 = 0.0, omega = 0.0,
-         iomega = 0.0;
-  double xs[12], ys[12];
-  int idir = 1, nev = 1, nctrl = 1, mm = 1, ifirst = 0;
-  int phase = PH_SETUP;
-  double ceval = 0.0;
-
-  // consume Delta(ceval) = val: one step of the getsol / nevill state machine
-  auto consume = [&](double val) {
-    n_evals++;
-    int iret = 0;  // 0 running, 1 root accepted, -1 failed
-    bool body = false;
-    if (phase == PH_G_FIRST) {
-      del1 = val;
-      if (ifirst == 1) del1st = del1;
-      const double plmn = sgn1(del1st) * sgn1(del1);
-      idir = (ifirst == 1 || plmn >= 0.0) ? +1 : -1;
-      for (;;) {  // label 1000 (:457-470)
-        c2 = (idir > 0) ? c1 + dc : c1 - dc;
-        if (c2 <= clow) {
-          idir = +1;
-          c1 = clow;
-          continue;
-        }
-        break;
-      }
-      ceval = c2;
-      phase = PH_G_SCAN;
-    } else if (phase == PH_G_SCAN) {
-      // one upward/downward scan step given Delta(c2) (getsol :457-479)
-      del2 = val;
-      if (sgn1(del1) != sgn1(del2)) {
-        c3 = 0.5 * (c1 + c2);  // bracketed -> nevill: initial half
-        ceval = c3;
-        nev = 1;
-        nctrl = 1;
-        phase = PH_N_TOP;
-      } else {
-        c1 = c2;
-        del1 = del2;
-        if (c1 < cm || c1 >= (betmxd + dc)) {
-          iret = -1;
-        } else {
-          for (;;) {
-            c2 = (idir > 0) ? c1 + dc : c1 - dc;
-            if (c2 <= clow) {
-              idir = +1;
-              c1 = clow;
-              continue;
-            }
-            break;
-          }
-          ceval = c2;
-        }
-      }
-    } else if (phase == PH_N_TOP) {
-      del3 = val;
-      nctrl = nctrl + 1;
-      if (nctrl >= 100) {
-        iret = 2;  // nevill exit by iteration cap -> cc = c3
-      } else if (c3 < fmin(c1, c2) || c3 > fmax(c1, c2)) {
-        nev = 0;
-        c3 = 0.5 * (c1 + c2);
-        ceval = c3;
-        phase = PH_N_OUTSIDE;
-      } else {
-        body = true;
-      }
-    } else {  // PH_N_OUTSIDE
-      del3 = val;
-      body = true;
-    }
-    if (body) {
-      const double s13 = del1 - del3;
-      const double s32 = del3 - del2;
-      if (sgn1(del3) * sgn1(del1) < 0.0) {
-        c2 = c3;
-        del2 = del3;
-      } else {
-        c1 = c3;
-        del1 = del3;
-      }
-      if (fabs(c1 - c2) <= 1.e-6 * c1) {
-        iret = 2;
-      } else {
-        if (sgn1(s13) != sgn1(s32)) nev = 0;
-        const double ss1 = fabs(del1), ss2 = fabs(del2);
-        const double s1 = (double)0.01f * ss1, s2 = (double)0.01f * ss2;
-        bool do_half = (s1 > ss2 || s2 > ss1 || nev == 0);
-        if (!do_half) {
-          if (nev == 2) {
-            xs[mm] = c3;
-            ys[mm] = del3;
-          } else {
-            xs[0] = c1;
-            ys[0] = del1;
-            xs[1] = c2;
-            ys[1] = del2;
-            mm = 1;
-          }
-          bool bad = false;
-          for (int kk = 1; kk <= mm; kk++) {
-            const int j = mm - kk;  // 0-based index of x(j)
-            const double denom = ys[mm] - ys[j];
-            if (fabs(denom) < 1.0e-10 * fabs(ys[mm])) {
-              bad = true;
-              break;
-            }
-            xs[j] = RFS_FMA(ys[mm], xs[j], RFS_MUL(-ys[j], xs[j + 1])) / denom;
-          }
-          if (!bad) {
-            c3 = xs[0];
-            nev = 2;
-            mm = mm + 1;
-            if (mm > 10) mm = 10;
-          } else {
-            do_half = true;
-          }
-        }
-        if (do_half) {
-          c3 = 0.5 * (c1 + c2);
-          nev = 1;
-          mm = 1;
-        }
-        ceval = c3;
-        phase = PH_N_TOP;
-      }
-    }
-    if (iret == 2) {
-      c1 = c3;  // back in getsol (:483-487)
-      iret = (c1 > betmxd) ? -1 : 1;
-    }
-    if (iret == 1) {
-      double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
-      cprev = c1;
-      if (nmode > 1) cwork[(long long)(sq.out_off + kb + k) * stride + b] = c1;
-      cq[(long long)(sq.out_off + kb + k) * stride + b] = (double)(float)c1;  // cg(k)=sngl(c(k))
-      k++;
-      phase = PH_SETUP;
-    } else if (iret == -1) {
-      double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
-      if (iq <= 1) job_ierr = 1;
-      ift = k + 1;
-      for (int i = k; i < jk; i++) cq[(long long)(sq.out_off + kb + i) * stride + b] = 0.0;
-      iq++;
-      k = 0;
-      phase = PH_SETUP;
-    }
-  };
+  SwdNevCol xs, ys;
+  SwdRootSearch rs(xs, ys, sq, periods, nmode, all_modes, cout, cout_mode_stride, cwork, stride, b,
+                   n_evals);
+  rs.start(M, 0, only_k);
 
   for (;;) {
-    if (phase == PH_SETUP) {
-      // ---- advance the (job, mode, period) nest until a root search starts or all is done
-      for (;;) {
-        if (iq <= nmode && k < jk && (k + 1 >= ift)) {
-          // label 1700/1750 reached through `if(k.ge.ift)`: this mode is cut off from k on
-          double *cq = cout + (all_modes ? (long long)(iq - 1) * cout_mode_stride : 0);
-          if (iq <= 1) job_ierr = 1;
-          ift = k + 1;
-          for (int i = k; i < jk; i++) cq[(long long)(sq.out_off + kb + i) * stride + b] = 0.0;
-          iq++;
-          k = 0;
-          continue;
-        }
-        if (iq <= nmode && k >= jk) {  // mode finished normally
-          iq++;
-          k = 0;
-          continue;
-        }
-        if (iq > nmode) {  // job finished
-          phase = PH_DONE;
-          break;
-        }
-        // ---- start values of (iq, k) (surfdisp96.f:257-276)
-        const double t1 = __ldg(periods + sq.per_off + kb + k) * sq.scale;
-        omega = twopi / t1;
-        iomega = 1.0 / omega;
-        if (k == 0 && iq == 1) {
-          c1 = cc;
-          clow = cc;
-          ifirst = 1;
-        } else if (k == 0 && iq > 1) {
-          c1 = RFS_ADD(cwork[(long long)(sq.out_off + kb + 0) * stride + b], RFS_MUL(one, dc));
-          clow = c1;
-          ifirst = 1;
-        } else if (k > 0 && iq > 1) {
-          ifirst = 0;
-          clow = RFS_ADD(cwork[(long long)(sq.out_off + kb + k) * stride + b], RFS_MUL(one, dc));
-          c1 = cprev;
-          if (c1 < clow) c1 = clow;
-        } else {
-          ifirst = 0;
-          c1 = RFS_SUB(cprev, RFS_MUL(onea, dc));
-          clow = cm;
-        }
-        ceval = c1;
-        phase = PH_G_FIRST;
-        break;
-      }
-    }
-    if (phase == PH_DONE) break;
+    if (rs.phase == PH_SETUP) rs.advance();
+    if (rs.phase == PH_DONE) break;
 
     // ---- candidate grid points of this round: ceval, ceval +- dc, ... (same additions as the scan)
     double cand[S];
-    cand[0] = ceval;
-    double myc = ceval;
+    cand[0] = rs.ceval;
+    double myc = rs.ceval;
     if (S > 1) {
-      const bool down = (phase == PH_G_SCAN) && (idir < 0);
-      const double stepc = down ? -dc : dc;  // c + (-dc) == c - dc exactly
-      const bool spec = (phase == PH_G_FIRST || phase == PH_G_SCAN);
+      const bool down = (rs.phase == PH_G_SCAN) && (rs.idir < 0);
+      const double stepc = down ? -SwdRootSearch::dc : SwdRootSearch::dc;  // c + (-dc) == c - dc exactly
+      const bool spec = (rs.phase == PH_G_FIRST || rs.phase == PH_G_SCAN);
       const int slot = tl / GL;
 #pragma unroll
       for (int j = 1; j < S; j++) {
@@ -410,24 +179,25 @@ RFS_DEVINL int swd_solve_team(const SmemModel &M, long long b, const SwdSeq &sq,
         if (spec && slot == j) myc = cand[j];
       }
     }
-    const double myval = team_secular<T, S>(M, ifunc, llw, omega, iomega, myc, tmask, tl, park, lane);
+    const double myval =
+        team_secular<T, S>(M, sq.ifunc, rs.llw, rs.omega, rs.iomega, myc, tmask, tl, park, lane);
     double vals[S];
     vals[0] = myval;
     if (S > 1) {
 #pragma unroll
       for (int j = 0; j < S; j++) vals[j] = __shfl_sync(tmask, myval, j * GL, T);
     }
-    consume(vals[0]);
+    rs.consume(vals[0]);
     if (S > 1) {
 #pragma unroll
       for (int j = 1; j < S; j++) {
         // consumed only if the scan really asks for this grid point next (bitwise the same double)
-        if (!(phase == PH_G_SCAN && ceval == cand[j])) break;
-        consume(vals[j]);
+        if (!(rs.phase == PH_G_SCAN && rs.ceval == cand[j])) break;
+        rs.consume(vals[j]);
       }
     }
   }
-  return job_ierr;
+  return rs.job_ierr;
 }
 
 // ---- K1t: T lanes per (model, sequence); blockDim.x / T teams per block
