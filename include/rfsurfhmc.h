@@ -70,6 +70,14 @@ int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, 
                        double gauss, double time_shift, double water, int rf_type, int method);
 /* dobs (host pointer): [nt_rf + n_swd] joint, or the matching sub-vector for which=1/2 */
 int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dobs, int ndobs);
+/* S observation sets ("stations", no reference counterpart: the reference inverts one station per run):
+ * dobs [S][ndobs], sigma1/sigma2 [S] (host pointers).  Every set shares the forward configuration above
+ * (layer count, periods, modes, ray parameters, RF sampling); each has its own data vector and its own
+ * joint weight (sigma1[s]/sigma2[s])^2 n_rf/n_swd.  rfs_config_obs is this call with S = 1.
+ * On a context holding S > 1 sets, every call without a set array (rfs_misfit_grad_dev/_host,
+ * rfs_hmc_run) returns RFS_E_CONFIG. */
+int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
+                        const double *dobs, int ndobs);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)
@@ -78,6 +86,17 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
                         double *grad, double *dsyn, unsigned char *flag, void *stream);
 int rfs_misfit_grad_host(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
                          double *grad, double *dsyn, unsigned char *flag);
+/* The same over several observation sets: row b is compared with set[b]'s data vector (and weighted
+ * with its sigma1/sigma2).  set [B] int32: a DEVICE pointer for _dev, a HOST pointer for _host; NULL
+ * only when the context holds one set (then these are the two calls above).  The failure convention
+ * (U 0, grad 0, dsyn = dobs, flag 0) returns the row's own set's dobs.
+ * _host rejects an index outside [0, S) with RFS_E_ARG.  _dev cannot check without synchronising: a
+ * row whose index is outside [0, S) reads no observation and gets flag 0, U 0, grad 0 and NaN dsyn;
+ * every other row is unaffected. */
+int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
+                             double *U, double *grad, double *dsyn, unsigned char *flag, void *stream);
+int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
+                              double *U, double *grad, double *dsyn, unsigned char *flag);
 
 /* ---- libsurf drop-ins, batched over B models (host pointers) --------------------------------
  * thk,vp,vs,rho [B][n] (cast to float32 inside, as src/SWD/main.cpp:9);  period [nT]
@@ -130,6 +149,18 @@ int rfs_hmc_run(rfs_ctx *ctx, int sampler, int which, long long C, const long lo
                 double *misfit, double *syn, double *initmodel, long long *n_iter,
                 long long *n_acc, double *dt_final, signed char *accept_seq,
                 long long max_iter_log);
+/* The same over several observation sets: chain c samples set chain_set[c]'s objective (host pointer
+ * [C]; NULL only when the context holds one set) inside its box, bounds [nb][2n][2] with nb = 1 (one
+ * box for all chains) or S (one box per set).  An index outside [0, S) returns RFS_E_ARG.  Chain ids
+ * may repeat across sets: chain c is seeded seed + chain_id[c] and the id is used for nothing else, so
+ * set s's chains 0..K-1 give exactly what a one-set run of chains 0..K-1 on set s gives.
+ * rfs_hmc_run is this call with chain_set = NULL and nb = 1. */
+int rfs_hmc_run_sets(rfs_ctx *ctx, int sampler, int which, long long C, const long long *chain_id,
+                     const int *chain_set, const double *bounds, int nb, double dt, int Lmin, int Lmax,
+                     int L0, double target_ratio, long long seed, int nsamples, int ndraws,
+                     long long max_iters, double *samples, double *misfit, double *syn, double *initmodel,
+                     long long *n_iter, long long *n_acc, double *dt_final, signed char *accept_seq,
+                     long long max_iter_log);
 /* number of misfit_and_grad evaluations / of global steps (one batched evaluation each) performed by
  * the last rfs_hmc_run */
 long long rfs_hmc_last_evals(rfs_ctx *ctx);

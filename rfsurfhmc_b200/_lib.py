@@ -11,6 +11,7 @@ _dp = C.POINTER(C.c_double)
 _u8p = C.POINTER(C.c_ubyte)
 _i8p = C.POINTER(C.c_byte)
 _llp = C.POINTER(C.c_longlong)
+_ip = C.POINTER(C.c_int)
 _vp = C.c_void_p
 
 WAVETYPES = {"Rc": 0, "Rg": 1, "Lc": 2, "Lg": 3}
@@ -65,6 +66,12 @@ def load_library():
         L.rfs_misfit_grad_dev.argtypes = [_vp, C.c_longlong, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_host.restype = C.c_int
         L.rfs_misfit_grad_host.argtypes = [_vp, C.c_longlong, _dp, C.c_int, _dp, _dp, _dp, _u8p]
+        L.rfs_config_obs_sets.restype = C.c_int
+        L.rfs_config_obs_sets.argtypes = [_vp, C.c_int, _dp, _dp, _dp, C.c_int]
+        L.rfs_misfit_grad_sets_dev.restype = C.c_int
+        L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
+        L.rfs_misfit_grad_sets_host.restype = C.c_int
+        L.rfs_misfit_grad_sets_host.argtypes = [_vp, C.c_longlong, _dp, _ip, C.c_int, _dp, _dp, _dp, _u8p]
         surf_in = [_vp, C.c_longlong, C.c_int, _dp, _dp, _dp, _dp, C.c_int, _dp, C.c_int, C.c_int]
         L.rfs_surf_forward.restype = C.c_int
         L.rfs_surf_forward.argtypes = surf_in + [C.c_int, _dp, _u8p]
@@ -84,6 +91,10 @@ def load_library():
         L.rfs_hmc_run.argtypes = [_vp, C.c_int, C.c_int, C.c_longlong, _llp, _dp, C.c_double, C.c_int, C.c_int, C.c_int,
                                   C.c_double, C.c_longlong, C.c_int, C.c_int, C.c_longlong, _dp, _dp, _dp, _dp,
                                   _llp, _llp, _dp, _i8p, C.c_longlong]
+        L.rfs_hmc_run_sets.restype = C.c_int
+        L.rfs_hmc_run_sets.argtypes = [_vp, C.c_int, C.c_int, C.c_longlong, _llp, _ip, _dp, C.c_int, C.c_double,
+                                       C.c_int, C.c_int, C.c_int, C.c_double, C.c_longlong, C.c_int, C.c_int,
+                                       C.c_longlong, _dp, _dp, _dp, _dp, _llp, _llp, _dp, _i8p, C.c_longlong]
         L.rfs_hmc_last_evals.restype = C.c_longlong
         L.rfs_hmc_last_evals.argtypes = [_vp]
         L.rfs_hmc_last_steps.restype = C.c_longlong
@@ -126,7 +137,8 @@ def exported_symbols():
             "rfs_measure_fp64_peak", "rfs_read_eval_stats", "rfs_selftest_math",
             "rfs_set_roots_team", "rfs_last_roots_team", "rfs_set_roots_sched",
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
-            "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options"]
+            "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
+            "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets"]
 
 
 def _f64(a):
@@ -135,6 +147,16 @@ def _f64(a):
 
 def _p(a):
     return a.ctypes.data_as(_dp) if a is not None else None
+
+
+def _sets(sets, rows):
+    """Observation-set index per row (int32, host) or None."""
+    if sets is None:
+        return None
+    s = np.ascontiguousarray(np.asarray(sets), dtype=np.int32)
+    if s.shape != (rows,):
+        raise ValueError(f"sets must have shape ({rows},), got {s.shape}")
+    return s
 
 
 class Context:
@@ -151,6 +173,7 @@ class Context:
         self.n = None
         self.nt_rf = 0
         self.n_swd_data = 0
+        self.nsets = 0
 
     def close(self):
         if getattr(self, "h", None):
@@ -240,28 +263,40 @@ class Context:
         self.nt_rf = int(nt) * rays.size
 
     def config_obs(self, dobs, sigma1=1.0, sigma2=1.0):
+        """dobs [ndata]: one data vector.  dobs [S, ndata]: S observation sets (stations) sharing the
+        forward configuration, with sigma1 / sigma2 scalars or [S] arrays; the evaluations and the HMC
+        then take a set index per row / per chain."""
         d = _f64(dobs)
-        self._ck(self.L.rfs_config_obs(self.h, float(sigma1), float(sigma2), _p(d), d.size))
+        if d.ndim not in (1, 2) or d.size == 0:
+            raise ValueError(f"dobs must be [ndata] or [S, ndata], got shape {d.shape}")
+        S = 1 if d.ndim == 1 else d.shape[0]
+        s1 = _f64(np.broadcast_to(np.asarray(sigma1, dtype=np.float64), (S,)))
+        s2 = _f64(np.broadcast_to(np.asarray(sigma2, dtype=np.float64), (S,)))
+        self._ck(self.L.rfs_config_obs_sets(self.h, S, _p(s1), _p(s2), _p(d), d.shape[-1]))
+        self.nsets = S
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)
 
     # ---- hot path
-    def misfit_grad_host(self, x, which=0):
+    def misfit_grad_host(self, x, which=0, sets=None):
+        """sets [B]: observation set of each row (required when the context holds several)."""
         x = _f64(x)
         B, n2 = x.shape
+        s = _sets(sets, B)
         nd = self.ndata(which)
         U = np.empty(B)
         g = np.empty((B, n2))
         d = np.empty((B, nd))
         f = np.empty(B, dtype=np.uint8)
-        self._ck(self.L.rfs_misfit_grad_host(self.h, B, _p(x), int(which), _p(U), _p(g), _p(d),
-                                             f.ctypes.data_as(_u8p)))
+        self._ck(self.L.rfs_misfit_grad_sets_host(self.h, B, _p(x), s.ctypes.data_as(_ip) if s is not None else None,
+                                                  int(which), _p(U), _p(g), _p(d), f.ctypes.data_as(_u8p)))
         return U, g, d, f.astype(bool)
 
-    def misfit_grad_dev(self, B, x_ptr, which, U_ptr, g_ptr, d_ptr, f_ptr, stream_ptr):
-        self._ck(self.L.rfs_misfit_grad_dev(self.h, int(B), _vp(x_ptr), int(which), _vp(U_ptr), _vp(g_ptr),
-                                            _vp(d_ptr), _vp(f_ptr), _vp(stream_ptr)))
+    def misfit_grad_dev(self, B, x_ptr, which, U_ptr, g_ptr, d_ptr, f_ptr, stream_ptr, sets_ptr=0):
+        """sets_ptr: device int32 [B] observation set of each row, 0 = none (one set)."""
+        self._ck(self.L.rfs_misfit_grad_sets_dev(self.h, int(B), _vp(x_ptr), _vp(sets_ptr or None), int(which),
+                                                 _vp(U_ptr), _vp(g_ptr), _vp(d_ptr), _vp(f_ptr), _vp(stream_ptr)))
 
     PROF_NK = 10
 
@@ -351,11 +386,17 @@ class Context:
 
     def hmc_run(self, sampler, chain_ids, bounds, dt, Lrange=(5, 20), L0=10, target_ratio=0.65,
                 seed=0, nsamples=800, ndraws=200, max_iters=0, want_samples=True, want_syn=False,
-                log_accepts=0, which=0):
+                log_accepts=0, which=0, sets=None):
+        """bounds [2n, 2] (one box) or [S, 2n, 2] (one box per observation set); sets [C]: observation
+        set of each chain (required when the context holds several)."""
         ids = np.ascontiguousarray(np.asarray(chain_ids, dtype=np.int64))
         Cn = ids.size
+        s = _sets(sets, Cn)
         b = _f64(bounds)
-        n2 = b.shape[0]
+        if b.ndim not in (2, 3) or b.shape[-1] != 2:
+            raise ValueError(f"bounds must be [2n, 2] or [S, 2n, 2], got shape {b.shape}")
+        nb = 1 if b.ndim == 2 else b.shape[0]
+        n2 = b.shape[-2]
         nd = self.ndata(which)
         out = {
             "misfit": np.zeros((Cn, nsamples)),
@@ -370,8 +411,9 @@ class Context:
         if Cn == 0:   # a rank without chains (nchains < world size): empty results, nothing to run
             out.update(evals=0, warning="")
             return out
-        rc = self.L.rfs_hmc_run(
-            self.h, int(sampler), int(which), Cn, ids.ctypes.data_as(_llp), _p(b), float(dt), int(Lrange[0]),
+        rc = self.L.rfs_hmc_run_sets(
+            self.h, int(sampler), int(which), Cn, ids.ctypes.data_as(_llp),
+            s.ctypes.data_as(_ip) if s is not None else None, _p(b), nb, float(dt), int(Lrange[0]),
             int(Lrange[1]), int(L0), float(target_ratio), int(seed), int(nsamples), int(ndraws),
             int(max_iters), _p(out["samples"]), _p(out["misfit"]), _p(out["syn"]), _p(out["initmodel"]),
             out["n_iter"].ctypes.data_as(_llp), out["n_acc"].ctypes.data_as(_llp), _p(out["dt"]),

@@ -5,7 +5,9 @@ from ._lib import Context
 
 
 class JointEvaluator:
-    """Many-chains Joint_RF_SWD.misfit_and_grad on one GPU with resident inputs/outputs."""
+    """Many-chains Joint_RF_SWD.misfit_and_grad on one GPU with resident inputs/outputs.  dobs [ndata]
+    or [S, ndata]: S observation sets (stations) sharing `cfg`; cfg's sigma1 / sigma2 may then be
+    [S] arrays."""
 
     def __init__(self, cfg, dobs, nlayer, device=0, which=0):
         self.ctx = Context(device)
@@ -23,10 +25,13 @@ class JointEvaluator:
         self.ndata = self.ctx.ndata(which)
         self._out = None
 
-    def __call__(self, x):
-        """x: float64 CUDA tensor [B, 2n] -> (U [B], grad [B,2n], dsyn [B,ndata], flag [B] uint8)."""
+    def __call__(self, x, sets=None):
+        """x: float64 CUDA tensor [B, 2n] -> (U [B], grad [B,2n], dsyn [B,ndata], flag [B] uint8).
+        sets: int32 CUDA tensor [B], the observation set of each row (required with several sets)."""
         assert x.is_cuda and x.dtype == torch.float64 and x.is_contiguous()
         B = x.shape[0]
+        if sets is not None:
+            assert sets.is_cuda and sets.dtype == torch.int32 and sets.is_contiguous() and sets.shape == (B,)
         if self._out is None or self._out[0].shape[0] != B:
             self._out = (torch.empty(B, dtype=torch.float64, device=self.device),
                          torch.empty(B, 2 * self.n, dtype=torch.float64, device=self.device),
@@ -34,7 +39,8 @@ class JointEvaluator:
                          torch.empty(B, dtype=torch.uint8, device=self.device))
         U, G, D, F = self._out
         self.ctx.misfit_grad_dev(B, x.data_ptr(), self.which, U.data_ptr(), G.data_ptr(), D.data_ptr(),
-                                 F.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream)
+                                 F.data_ptr(), torch.cuda.current_stream(self.device).cuda_stream,
+                                 sets.data_ptr() if sets is not None else 0)
         return U, G, D, F
 
 

@@ -82,11 +82,16 @@ struct rfs_ctx {
   bool has_rf = false;
   RfCfg rf;
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
-  // ---- observations
+  // ---- observations: nsets data vectors ("stations") of ndobs values each
   bool has_obs = false;
-  double sigma1 = 1.0, sigma2 = 1.0;
-  std::vector<double> dobs;
-  Buf d_dobs;
+  int nsets = 0, ndobs = 0;
+  std::vector<double> sigma1, sigma2;  // [nsets]
+  Buf d_dobs;                          // [nsets][ndobs]
+  // SWD weight of the joint objective per set, (sigma1/sigma2)^2 n1/nsw: computed on the host for the
+  // data lengths (wt_n1, wt_nsw) of the last joint call and uploaded again when they change
+  std::vector<double> wt;
+  Buf d_wt;
+  int wt_n1 = -1, wt_nsw = -1;
   // ---- workspace (grown on demand, never shrunk)
   std::vector<std::unique_ptr<Front>> fronts;  // one per chunk; fronts[0] always exists (drop-ins use it)
   cudaStream_t stream_front[3] = {nullptr, nullptr, nullptr};  // root searches (high priority)
@@ -94,7 +99,7 @@ struct rfs_ctx {
   Buf d_tw;   // FFT twiddle factors exp(-i pi j/(nft/2)), j < nft/2, of transform length tw_nft
   int tw_nft = 0;
   Buf w_ugr, w_kern, w_spec, w_dspec, w_urf, w_grf, w_rftr;
-  Buf io_x, io_U, io_grad, io_dsyn, io_flag, io_a, io_b, io_c, io_d, io_e, io_f;
+  Buf io_x, io_U, io_grad, io_dsyn, io_flag, io_set, io_a, io_b, io_c, io_d, io_e, io_f;
   // ---- HMC
   long long hmc_evals = 0, hmc_steps = 0;
   long long hmc_resident = 0;    // resident chain slots of rfs_hmc_run (0 = all chains at once)
@@ -481,9 +486,9 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, double ray_p, const double *d
 size_t decon_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 6 * (size_t)n2 + 64); }
 int decon_threads(int nft) { return std::max(64, std::min(512, nft / 2)); }
 
-int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const double *d_dobs,
-                 double *d_rf, long long ldrf, double *d_U, double *d_grad, double sigma, double tshift,
-                 cudaStream_t st, int accumulate = 0) {
+int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs,
+                 double *d_rf, long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag,
+                 double sigma, double tshift, cudaStream_t st, int accumulate = 0) {
   const size_t sm = decon_smem(cfg.nft, cfg.n2);
   if (sm > 48 * 1024) {
     CK(cudaFuncSetAttribute(rf_decon_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
@@ -492,7 +497,7 @@ int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const do
   }
   LAUNCH(rf_decon_kernel, (unsigned)B, decon_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, cfg.gauss, tshift, cfg.water, sigma, d_dobs, d_rf, ldrf, d_U, d_grad,
+         cfg.logn, cfg.dt, cfg.gauss, tshift, cfg.water, sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
          (const double2 *)ctx->d_tw.p, accumulate);
   return RFS_OK;
 }
@@ -712,21 +717,29 @@ int rfs_config_rf(rfs_ctx *ctx, int nlayer, double ray_p, int nt, double dt, dou
                             method);
 }
 
-int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dobs, int ndobs) {
-  if (!ctx || !dobs || ndobs <= 0) return RFS_E_ARG;
+int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
+                        const double *dobs, int ndobs) {
+  if (!ctx || S < 1 || !sigma1 || !sigma2 || !dobs || ndobs <= 0) return RFS_E_ARG;
   CK(cudaSetDevice(ctx->device));
-  ctx->sigma1 = sigma1;
-  ctx->sigma2 = sigma2;
-  ctx->dobs.assign(dobs, dobs + ndobs);
-  int rc = ensure(ctx, ctx->d_dobs, sizeof(double) * ndobs);
+  const size_t bytes = sizeof(double) * (size_t)S * ndobs;
+  int rc = ensure(ctx, ctx->d_dobs, bytes);
   if (rc) return rc;
-  CK(cudaMemcpy(ctx->d_dobs.p, dobs, sizeof(double) * ndobs, cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(ctx->d_dobs.p, dobs, bytes, cudaMemcpyHostToDevice));
+  ctx->sigma1.assign(sigma1, sigma1 + S);
+  ctx->sigma2.assign(sigma2, sigma2 + S);
+  ctx->nsets = S;
+  ctx->ndobs = ndobs;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
   ctx->has_obs = true;
   return RFS_OK;
 }
 
-int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
-                        double *grad, double *dsyn, unsigned char *flag, void *stream) {
+int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dobs, int ndobs) {
+  return rfs_config_obs_sets(ctx, 1, &sigma1, &sigma2, dobs, ndobs);
+}
+
+int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
+                             double *U, double *grad, double *dsyn, unsigned char *flag, void *stream) {
   if (!ctx) return RFS_E_ARG;
   if (B <= 0) return RFS_OK;
   if (which < 0 || which > 2) return fail(ctx, RFS_E_ARG, "which must be 0,1,2");
@@ -735,13 +748,17 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
     return fail(ctx, RFS_E_CONFIG, "context not configured (rfs_config_swd/rf/obs)");
   if (use_swd && use_rf && ctx->n_swd != ctx->rf.n)
     return fail(ctx, RFS_E_CONFIG, "SWD and RF layer counts differ");
+  if (!set && ctx->nsets > 1)
+    return fail(ctx, RFS_E_CONFIG,
+                "the context holds " + std::to_string(ctx->nsets) +
+                    " observation sets: evaluate with rfs_misfit_grad_sets_dev/_host and a set index per row");
   const RfCfg &rf = ctx->rf;
   const int n = use_swd ? ctx->n_swd : rf.n;
   const int nray = use_rf ? (int)ctx->ray_ps.size() : 0;
   const int nmsel = use_swd ? (int)ctx->modes.size() : 0;
   const int n1 = use_rf ? rf.nt * nray : 0, nsw = use_swd ? ctx->plan.ndata * nmsel : 0;
   const int ndata = n1 + nsw;
-  if ((int)ctx->dobs.size() != ndata) return fail(ctx, RFS_E_CONFIG, "dobs length != ndata");
+  if (ctx->ndobs != ndata) return fail(ctx, RFS_E_CONFIG, "dobs length != ndata");
   CK(cudaSetDevice(ctx->device));
   cudaStream_t st = (cudaStream_t)stream;
   // chunking: the front buffers (model blocks, roots) are kept for the whole batch, the eigen / RF
@@ -754,13 +771,23 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
   Bmax = std::min(Bmax, 2147483647LL / ((long long)SWD_NF * n));  // 32-bit offsets in SwdModel::ld
   const int nch = (int)((B + Bmax - 1) / Bmax);
   const long long Bch = (B + nch - 1) / nch;
-  const double *d_dobs = (const double *)ctx->d_dobs.p;
+  const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata};
   double tshift = rf.tshift;
   if (rf.rf_type == 2) tshift = -tshift;  // src/RF/main.cpp:35
   const bool rf_time = use_rf && rf.method == 0;
   const double sigma = rf_time ? 0.0 : 1.0 / rf.dt / rf.nft * 4.;
-  const double q = ctx->sigma1 / ctx->sigma2;
-  const double wt = (which == 0) ? q * q * n1 / nsw : 1.0;
+  if (which == 0 && (ctx->wt_n1 != n1 || ctx->wt_nsw != nsw)) {
+    ctx->wt.resize(ctx->nsets);
+    for (int k = 0; k < ctx->nsets; k++) {
+      const double q = ctx->sigma1[k] / ctx->sigma2[k];
+      ctx->wt[k] = q * q * n1 / nsw;
+    }
+    int rc;
+    if ((rc = ensure(ctx, ctx->d_wt, sizeof(double) * ctx->nsets))) return rc;
+    CK(cudaMemcpyAsync(ctx->d_wt.p, ctx->wt.data(), sizeof(double) * ctx->nsets, cudaMemcpyHostToDevice, st));
+    ctx->wt_n1 = n1;
+    ctx->wt_nsw = nsw;
+  }
   // several modes in one objective: solve all modes 0..max in one chained pass and pick the listed ones
   const bool multi_mode = use_swd && nmsel > 1;
   ModeSel msel;
@@ -811,6 +838,8 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
     Front &F = *ctx->fronts[k];
     int rc;
     const size_t nB = (size_t)n * Bc;
+    ObsSets obs_k = obs;  // the set indices of this chunk's rows
+    if (set) obs_k.set = set + off;
     if (use_rf) {
       // the RF branch only needs the chunk's model blocks: it runs on a second stream, beside the
       // (latency-bound, < 1 wave) root search and the eigen solves
@@ -833,6 +862,9 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
       if ((rc = ensure(ctx, ctx->w_grf, sizeof(double) * 2 * nB))) return rc;
       double *Uo = (which == 1) ? U + off : (double *)ctx->w_urf.p;
       double *go = (which == 1) ? grad + off * 2 * n : (double *)ctx->w_grf.p;
+      // RF only: every row succeeds except one whose set index is out of range (the RF kernels write its 0)
+      unsigned char *fo = (which == 1) ? flag + off : nullptr;
+      if (fo) CK(cudaMemsetAsync(fo, 1, Bc, sr));
       // one pass per ray parameter; misfit and gradient accumulate over the passes (the reference's
       // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3)
       for (int ir = 0; ir < nray; ir++) {
@@ -841,19 +873,19 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
                                  sr, rf_time ? RFS_PI64 : RFS_PI32)))
           return rc;
         double *dsyn_r = dsyn + off * ndata + (size_t)ir * rf.nt;
-        const double *dobs_r = d_dobs + (size_t)ir * rf.nt;
+        ObsSets obs_r = obs_k;
+        obs_r.dobs += (size_t)ir * rf.nt;
         if (!rf_time) {
-          if ((rc = run_rf_decon(ctx, rf, Bc, 2 * n, dobs_r, dsyn_r, ndata, Uo, go, sigma, tshift, sr, ir > 0)))
+          if ((rc = run_rf_decon(ctx, rf, Bc, 2 * n, obs_r, dsyn_r, ndata, Uo, go, fo, sigma, tshift, sr, ir > 0)))
             return rc;
         } else {
           // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces
           if ((rc = run_rf_time(ctx, rf, Bc, 4 * n, dsyn_r, ndata, tshift, sr))) return rc;
           LAUNCH(rf_trace_grad_kernel, gridFor(Bc * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
-                 (const double *)F.w_chain.p, (const double *)dsyn_r, (long long)ndata, dobs_r, Bc, n, rf.nt,
-                 Uo, go, ir > 0);
+                 (const double *)F.w_chain.p, dsyn_r, (long long)ndata, obs_r, Bc, n, rf.nt, Uo, go, fo,
+                 ir > 0);
         }
       }
-      if (which == 1) CK(cudaMemsetAsync(flag + off, 1, Bc, sr));
       if (sr != st) CK(cudaEventRecord(ctx->ev_join, sr));
     }
     if (use_swd) {
@@ -873,7 +905,8 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
       if (use_rf && ctx->overlap) CK(cudaStreamWaitEvent(st, ctx->ev_join, 0));
       LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, ctx->plan, V,
              (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, which, n1,
-             d_dobs, (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, wt, U + off,
+             obs_k, (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p,
+             U + off,
              grad + off * 2 * n, dsyn + off * ndata, flag + off, msel);
       CK(cudaEventRecord(ctx->ev_asm, st));
     }
@@ -881,14 +914,24 @@ int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, d
   return RFS_OK;
 }
 
-int rfs_misfit_grad_host(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
-                         double *grad, double *dsyn, unsigned char *flag) {
+int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
+                        double *grad, double *dsyn, unsigned char *flag, void *stream) {
+  return rfs_misfit_grad_sets_dev(ctx, B, x, nullptr, which, U, grad, dsyn, flag, stream);
+}
+
+int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
+                              double *U, double *grad, double *dsyn, unsigned char *flag) {
   if (!ctx) return RFS_E_ARG;
   if (B <= 0) return RFS_OK;
   if (which < 0 || which > 2) return fail(ctx, RFS_E_ARG, "which must be 0,1,2");
   const bool use_swd = which != 1, use_rf = which != 2;
   if ((use_swd && !ctx->has_swd) || (use_rf && !ctx->has_rf))
     return fail(ctx, RFS_E_CONFIG, "context not configured (rfs_config_swd/rf/obs)");
+  if (set)
+    for (long long b = 0; b < B; b++)
+      if (set[b] < 0 || set[b] >= ctx->nsets)
+        return fail(ctx, RFS_E_ARG, "set index " + std::to_string(set[b]) + " of row " + std::to_string(b) +
+                                        " outside [0, " + std::to_string(ctx->nsets) + ")");
   const int n = use_swd ? ctx->n_swd : ctx->rf.n;
   const int ndata = (use_rf ? ctx->rf.nt * (int)ctx->ray_ps.size() : 0) +
                     (use_swd ? ctx->plan.ndata * (int)ctx->modes.size() : 0);
@@ -899,11 +942,13 @@ int rfs_misfit_grad_host(rfs_ctx *ctx, long long B, const double *x, int which, 
   if ((rc = ensure(ctx, ctx->io_grad, sizeof(double) * B * 2 * n))) return rc;
   if ((rc = ensure(ctx, ctx->io_dsyn, sizeof(double) * B * ndata))) return rc;
   if ((rc = ensure(ctx, ctx->io_flag, B))) return rc;
+  if (set && (rc = ensure(ctx, ctx->io_set, sizeof(int) * B))) return rc;
   cudaStream_t st = ctx->stream;
   CK(cudaMemcpyAsync(ctx->io_x.p, x, sizeof(double) * B * 2 * n, cudaMemcpyHostToDevice, st));
-  rc = rfs_misfit_grad_dev(ctx, B, (const double *)ctx->io_x.p, which, (double *)ctx->io_U.p,
-                           (double *)ctx->io_grad.p, (double *)ctx->io_dsyn.p,
-                           (unsigned char *)ctx->io_flag.p, st);
+  if (set) CK(cudaMemcpyAsync(ctx->io_set.p, set, sizeof(int) * B, cudaMemcpyHostToDevice, st));
+  rc = rfs_misfit_grad_sets_dev(ctx, B, (const double *)ctx->io_x.p, set ? (const int *)ctx->io_set.p : nullptr,
+                                which, (double *)ctx->io_U.p, (double *)ctx->io_grad.p, (double *)ctx->io_dsyn.p,
+                                (unsigned char *)ctx->io_flag.p, st);
   if (rc) return rc;
   if (U) CK(cudaMemcpyAsync(U, ctx->io_U.p, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
   if (grad)
@@ -913,6 +958,11 @@ int rfs_misfit_grad_host(rfs_ctx *ctx, long long B, const double *x, int which, 
   if (flag) CK(cudaMemcpyAsync(flag, ctx->io_flag.p, B, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   return RFS_OK;
+}
+
+int rfs_misfit_grad_host(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
+                         double *grad, double *dsyn, unsigned char *flag) {
+  return rfs_misfit_grad_sets_host(ctx, B, x, nullptr, which, U, grad, dsyn, flag);
 }
 
 // ------------------------------------------------------------------------------ libsurf drop-ins
@@ -1103,8 +1153,8 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
     if ((rc = run_rf_time(ctx, cfg, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, tshift, st)))
       return rc;
   } else {
-    if ((rc = run_rf_decon(ctx, cfg, B, 0, nullptr, (double *)ctx->io_b.p, nt, nullptr, nullptr, sigma,
-                           tshift, st)))
+    if ((rc = run_rf_decon(ctx, cfg, B, 0, ObsSets{nullptr, nullptr, 1, 0}, (double *)ctx->io_b.p, nt, nullptr,
+                           nullptr, nullptr, sigma, tshift, st)))
       return rc;
   }
   CK(cudaMemcpyAsync(rf, ctx->io_b.p, sizeof(double) * B * nt, cudaMemcpyDeviceToHost, st));

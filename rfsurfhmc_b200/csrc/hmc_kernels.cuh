@@ -60,7 +60,12 @@ struct HmcDev {
   // outputs (may be null)
   double *samples, *misfit, *syn, *initmodel;
   signed char *alog;
-  const double *bounds;  // [n2][2]
+  const double *bounds;  // [nb][n2][2]: one box for all chains (box_ld 0) or one per set (box_ld 2 n2)
+  long long box_ld;
+  // observation sets: set [C] of each chain (NULL: one set), rowset [R] = set of the chain a slot runs,
+  // setg [Ba] = rowset gathered for the packed batch (evaluated with the rows' own observations)
+  const int *set;
+  int *rowset, *setg;
   int *n_active;         // [0] slots still running after the last advance, [1] compaction counter
   // compaction of the evaluation batch once slots have run dry: slot[s] = row of slot s in the
   // evaluated batch (-1: finished), idx[j] = slot of row j, xg = gathered positions [Ba][n2]
@@ -173,12 +178,14 @@ RFS_DEVINL void rng_store(const HmcDev &D, const Rng &r) {
   D.gauss[r.c] = r.gauss;
 }
 
-// _mirror (hmc.py:121-137) applied to (xnew, pnew) of chain c; returns false if x is not finite
+// _mirror (hmc.py:121-137) applied to (xnew, pnew) of slot c, in the box of the chain it runs; returns
+// false if x is not finite
 RFS_DEVINL bool hmc_mirror(const HmcDev &D, const HmcCfg &cfg, long long c) {
   bool fin = true;
+  const double *box = D.bounds + D.rowset[c] * D.box_ld;
   for (int j = 0; j < cfg.n2; j++) {
     double x = D.xnew[c * cfg.n2 + j], p = D.pnew[c * cfg.n2 + j];
-    const double lo = D.bounds[2 * j], hi = D.bounds[2 * j + 1];
+    const double lo = box[2 * j], hi = box[2 * j + 1];
     int it = 0;
     while (x > hi || x < lo) {
       if (x > hi) {
@@ -218,9 +225,13 @@ RFS_DEVINL bool hmc_mirror(const HmcDev &D, const HmcCfg &cfg, long long c) {
 }
 
 // chain initialisation: seed, set_initial_model until in bounds (hmc.py:74-99,231-235).
-// Starts chain `ch` in slot `c` (R = number of slots: the stride of the MT19937 state).
+// Starts chain `ch` in slot `c` (R = number of slots: the stride of the MT19937 state).  The chain id
+// only offsets the seed: chains of different sets may share an id and then draw the same stream.
 RFS_DEVINL void hmc_chain_start(const HmcDev &D, const HmcCfg &cfg, long long R, long long c,
                                 long long ch) {
+  const int set = D.set ? D.set[ch] : 0;
+  const double *box = D.bounds + set * D.box_ld;
+  D.rowset[c] = set;
   Rng r;
   r.mt = D.mt;
   r.C = R;
@@ -230,7 +241,7 @@ RFS_DEVINL void hmc_chain_start(const HmcDev &D, const HmcCfg &cfg, long long R,
   double *x = D.xcur + c * n2;
   for (;;) {
     for (int i = 0; i < n2; i++) {
-      const double lo = D.bounds[2 * i], hi = D.bounds[2 * i + 1];
+      const double lo = box[2 * i], hi = box[2 * i + 1];
       x[i] = lo + (hi - lo) * r.rand();
     }
     // sort vs ascending, permute thk alike (insertion sort; values are distinct a.s.)
@@ -247,7 +258,7 @@ RFS_DEVINL void hmc_chain_start(const HmcDev &D, const HmcCfg &cfg, long long R,
     }
     bool ok = true;
     for (int i = 0; i < n2 - 1; i++)
-      if (x[i] < D.bounds[2 * i] || x[i] > D.bounds[2 * i + 1]) ok = false;
+      if (x[i] < box[2 * i] || x[i] > box[2 * i + 1]) ok = false;
     if (ok) break;
   }
   for (int i = 0; i < n2; i++) {
@@ -300,6 +311,7 @@ __global__ void hmc_gather_kernel(HmcDev D, int n2, long long Ba) {
   const long long j = t / n2;
   const int i = (int)(t % n2);
   D.xg[t] = D.xeval[(long long)D.idx[j] * n2 + i];
+  if (D.setg && i == 0) D.setg[j] = D.rowset[D.idx[j]];
 }
 
 // Wall-clock budget exhausted (rfs_set_hmc_options): stop every running slot where it stands and mark

@@ -27,13 +27,14 @@ struct ModeSel {
 // global loads: four times the threads cut its latency (0.30 -> ~0.1 ms at C1).
 // Layout of outputs (row-major per model, as the Python API):
 //   U[B], grad[B][2n] (vs then thk), dsyn[B][ndata] with ndata = nt_rf + nsw (joint),
-//   flag[B] (1 ok, 0 failed SWD root search)
+//   flag[B] (1 ok, 0 failed SWD root search or observation-set index out of range)
+// Row b is compared with observation set obs.row_set(b); wt[S] is each set's SWD weight
+// (sigma1/sigma2)^2 n1/nsw of the joint objective.
 #define RFS_ASM_Q 4
 __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__restrict__ ierr,
                                       const double *__restrict__ chain, int stale, int which,
-                                      int nt_rf, const double *__restrict__ dobs,
-                                      const double *__restrict__ U_rf,
-                                      const double *__restrict__ g_rf, double wt,
+                                      int nt_rf, ObsSets obs, const double *__restrict__ U_rf,
+                                      const double *__restrict__ g_rf, const double *__restrict__ wt,
                                       double *__restrict__ U, double *__restrict__ grad,
                                       double *__restrict__ dsyn, unsigned char *__restrict__ flag,
                                       ModeSel ms) {
@@ -48,7 +49,9 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__rest
   const int nsw = (which == 1) ? 0 : plan.ndata * ms.n;
   const int n1 = (which == 2) ? 0 : nt_rf;
   const int ndata = n1 + nsw;
-  bool ok = true;
+  const int set = live ? obs.row_set(b) : 0;
+  const double *dobs = obs.row(set < 0 ? 0 : set);
+  bool ok = set >= 0;
   if (which != 1 && live)
     for (int s = 0; s < plan.nseq; s++) ok = ok && (ierr[(long long)s * B + b] == 0);
   double gv = 0.0, gh = 0.0, us = 0.0;
@@ -94,7 +97,7 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__rest
     us += red[2][j][bl];
   }
   if (ok) {
-    const double w = (which == 0) ? wt : 1.0;
+    const double w = (which == 0) ? wt[set] : 1.0;
     double g0 = w * gv, g1 = w * gh;
     if (which != 2) {
       g0 += g_rf[b * 2 * n + m];
@@ -109,10 +112,11 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__rest
       flag[b] = 1;
     }
   } else {
-    // model_rf_swd_vs_thk.py:73-74: (0.0, zeros, dobs, False)
+    // model_rf_swd_vs_thk.py:73-74: (0.0, zeros, dobs, False), dobs of the row's own set
     grad[b * 2 * n + m] = 0.0;
     grad[b * 2 * n + n + m] = 0.0;
-    for (int j = m; j < ndata; j += n) dsyn[b * ndata + j] = (which == 2) ? 0.0 : dobs[j];
+    const double fill = (set < 0) ? nan("") : 0.0;
+    for (int j = m; j < ndata; j += n) dsyn[b * ndata + j] = (which == 2 || set < 0) ? fill : dobs[j];
     if (m == 0) {
       U[b] = 0.0;
       flag[b] = 0;

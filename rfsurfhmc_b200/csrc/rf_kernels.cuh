@@ -570,14 +570,14 @@ RFS_DEVINL double block_reduce(double v, double *red, bool is_max) {
 
 // ---- K4: one block per model: water-level deconvolution, c2r FFT, trace, misfit and (optional)
 // adjoint gradient.   dynamic smem: cd buf[nft] + cd s21[n2] + cd s22[n2] + cd wt[n2] + 32 doubles
-//   rf   : [B][ldrf>=nt]  dobs: [nt] or NULL       U: [B]       grad: [B][nrow] (nrow = NQ*n)
+//   rf   : [B][ldrf>=nt]  obs.dobs: [nsets][ld >= nt] or NULL   U: [B]   grad: [B][nrow] (nrow = NQ*n)
+//   flag : [B] or NULL; only written (0) for a row whose observation-set index is out of range
 __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 *__restrict__ dspec,
                                 long long B, int nrow, int nt, int nft, int logn, double dt,
-                                double f0, double t0, double water, double sigma,
-                                const double *__restrict__ dobs, double *__restrict__ rf,
-                                long long ldrf, double *__restrict__ U,
-                                double *__restrict__ grad, const double2 *__restrict__ tw,
-                                int accumulate) {
+                                double f0, double t0, double water, double sigma, ObsSets obs,
+                                double *__restrict__ rf, long long ldrf, double *__restrict__ U,
+                                double *__restrict__ grad, unsigned char *__restrict__ flag,
+                                const double2 *__restrict__ tw, int accumulate) {
   // accumulate != 0: U and grad are added to (second and later ray parameters of one objective)
   extern __shared__ double smem[];
   const int n2 = nft / 2 + 1;
@@ -588,6 +588,18 @@ __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 
   double *red = reinterpret_cast<double *>(wt + n2);
   const long long b = blockIdx.x;
   const int tid = threadIdx.x, nth = blockDim.x;
+  const int set = obs.row_set(b);
+  if (set < 0) {
+    for (int it = tid; it < nt; it += nth) rf[b * ldrf + it] = nan("");
+    if (grad)
+      for (int rr = tid; rr < nrow; rr += nth) grad[b * nrow + rr] = 0.0;
+    if (tid == 0) {
+      U[b] = 0.0;
+      if (flag) flag[b] = 0;
+    }
+    return;
+  }
+  const double *dobs = obs.dobs ? obs.row(set) : nullptr;
 
   double lmax = 0.0;
   for (int k = tid; k < n2; k += nth) {

@@ -157,15 +157,28 @@ __global__ void __launch_bounds__(256, 3) rf_time_kernel(const double2 *__restri
 // misfit and gradient from materialised Frechet traces (time-domain method, where the adjoint
 // shortcut does not apply because deconit is nonlinear).  One thread per (model, layer).
 //   traces [B][4][n][nt] (rho, vp, vs, h);  chain [2][n][B];  rf [B][ldrf];  grad [B][2n]
+//   flag [B] or NULL: only written (0) for a row whose observation-set index is out of range; such a
+//   row gets U 0, grad 0 and a NaN trace
 __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const double *__restrict__ chain,
-                                     const double *__restrict__ rf, long long ldrf,
-                                     const double *__restrict__ dobs, long long B, int n, int nt,
-                                     double *__restrict__ U, double *__restrict__ grad,
-                                     int accumulate) {
+                                     double *__restrict__ rf, long long ldrf, ObsSets obs, long long B,
+                                     int n, int nt, double *__restrict__ U, double *__restrict__ grad,
+                                     unsigned char *__restrict__ flag, int accumulate) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= B * n) return;
   const long long b = i % B;
   const int m = (int)(i / B);
+  const int set = obs.row_set(b);
+  if (set < 0) {
+    grad[b * 2 * n + m] = 0.0;
+    grad[b * 2 * n + n + m] = 0.0;
+    if (m == 0) {
+      for (int t = 0; t < nt; t++) rf[b * ldrf + t] = nan("");
+      U[b] = 0.0;
+      if (flag) flag[b] = 0;
+    }
+    return;
+  }
+  const double *dobs = obs.row(set);
   const long long nB = (long long)n * B;
   const double dadb = chain[0 * nB + m * B + b], drda = chain[1 * nB + m * B + b];
   const double *kr = traces + ((b * 4 + 0) * n + m) * (long long)nt;

@@ -26,6 +26,15 @@ def shard_chains(nchains, rank=None, world_size=None):
     return np.arange(lo, hi, dtype=np.int64)
 
 
+def shard_station_chains(nstations, nchains, rank=None, world_size=None):
+    """(station [m], chain id [m]) of the (station, chain) pairs owned by `rank`: the S*K pairs are
+    sharded as S*K chains by shard_chains; global index g is chain g % K of station g // K, so
+    gather_chains(..., S*K) returns them station-major.  Chain ids repeat across stations: station s's
+    chain k is seeded seed + k, as in a one-station run."""
+    g = shard_chains(int(nstations) * int(nchains), rank, world_size)
+    return g // int(nchains), g % int(nchains)
+
+
 def _dev():
     if dist.is_initialized() and dist.get_backend() == "nccl":
         return torch.device("cuda", torch.cuda.current_device())

@@ -5,7 +5,13 @@ write `real_syn.npy`, per-chain result files and `misfit.npy [nchains, nsamples]
     python -m rfsurfhmc_b200.driver --param param.yaml --sampler base --chains 4
     torchrun --nproc-per-node 8 -m rfsurfhmc_b200.driver --sampler da --chains 16384
 
-`mpiexec -n N` of the reference becomes `--chains N`: all chains of a rank run at once on its GPU."""
+`mpiexec -n N` of the reference becomes `--chains N`: all chains of a rank run at once on its GPU.
+
+    python -m rfsurfhmc_b200.driver --param param.yaml --stations stations.npz --chains K
+
+inverts a station array instead: the observations of S stations come from the file (see
+model/stations.py: load_stations), K chains run per station, all S*K in one device run (sharded over
+ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
 import argparse
 import os
 import time
@@ -15,13 +21,16 @@ import yaml
 from .model.model_rf import ReceiverFunc
 from .model.model_surf import SurfWD
 from .model.model_rf_swd_vs_thk import Joint_RF_SWD
+from .model.stations import StationArray, load_stations
 from .pyhmc.hmc import HamitonianMC
 from .pyhmc.hmcda import HMCDualAveraging
 from .fixtures import driver_bounds
 from . import distributed as D
 
 
-def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0):
+def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0, stations=None):
+    """stations: None (observations synthesised from `true_model`, as the reference) or a stations file
+    / mapping (load_stations): then `nchains` chains run per station."""
     import torch
     import torch.distributed as dist
     rank = int(os.environ.get("RANK", "0"))
@@ -41,24 +50,32 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
     outdir = param['hmc']['OUTPUT_DIR']
     os.makedirs(outdir, exist_ok=True)
     x = np.hstack((vs, thk))
-    dobs = np.zeros(model.ndata)
-    if rank == 0:
-        drsyn, dssyn, _ = model.forward(x)
-        dobs[:model.rfmodel.nt] = drsyn
-        dobs[model.rfmodel.nt:] = dssyn
-        np.save(f"{outdir}/real_syn.npy", dobs)
-    dobs = D.bcast_array(dobs)
-    nt = model.rfmodel.nt
-    model.set_obsdata(dobs[:nt], dobs[nt:])
-    boundaries = driver_bounds(x)
+    if stations is None:
+        dobs = np.zeros(model.ndata)
+        if rank == 0:
+            drsyn, dssyn, _ = model.forward(x)
+            dobs[:model.rfmodel.nt] = drsyn
+            dobs[model.rfmodel.nt:] = dssyn
+            np.save(f"{outdir}/real_syn.npy", dobs)
+        dobs = D.bcast_array(dobs)
+        nt = model.rfmodel.nt
+        model.set_obsdata(dobs[:nt], dobs[nt:])
+        boundaries = driver_bounds(x)
+        npairs = nchains
+        ids, sidx = D.shard_chains(nchains), None
+    else:
+        st = load_stations(stations, model.ndata, x.size, driver_bounds(x))
+        model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"])
+        boundaries = st["bounds"]
+        npairs = model.nstations * nchains
+        sidx, ids = D.shard_station_chains(model.nstations, nchains)
     cls = HamitonianMC if sampler == "base" else HMCDualAveraging
     chain = cls.init(model, boundaries, 0, **param['hmc'])
     chain.max_iters = int(max_iters)  # 0 = unbounded, as the reference's `while True` loops
     if sampler == "da":
         chain.max_L = int(max_L)      # 0 = the reference's uncapped L = int(lambda/dt)
-    ids = D.shard_chains(nchains)
-    if nchains < ws:
-        raise ValueError("need at least one chain per rank (chains %d < world size %d)" % (nchains, ws))
+    if npairs < ws:
+        raise ValueError("need at least one chain per rank (chains %d < world size %d)" % (npairs, ws))
     if save_chains:
         # per-chain files need every accepted sample's synthetics on the host: [chains, nsamples, ndata];
         # the decision is collective (max over ranks) so that no rank leaves the others in a gather
@@ -66,18 +83,23 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
         if need > 8e9:
             raise MemoryError("per-chain result files for %d chains need %.1f GB of synthetics per rank; "
                               "run with --no-chain-files (misfit.npy is still written)" % (len(ids), need / 1e9))
-    out = chain.sample_chains(ids, want_syn=save_chains, save=save_chains)
+    out = chain.sample_chains(ids, want_syn=save_chains, save=save_chains, stations=sidx)
     # end-of-run gathers (replace comm.Gather at main_base.py:90): misfit history + per-chain counters
     t0 = time.perf_counter()
-    misfit = D.gather_chains(out["misfit"], nchains)
-    n_iter = D.gather_chains(out["n_iter"], nchains)
-    n_acc = D.gather_chains(out["n_acc"], nchains)
-    complete = D.gather_chains(out["complete"].astype(np.int64), nchains).astype(bool)
+    misfit = D.gather_chains(out["misfit"], npairs)
+    n_iter = D.gather_chains(out["n_iter"], npairs)
+    n_acc = D.gather_chains(out["n_acc"], npairs)
+    complete = D.gather_chains(out["complete"].astype(np.int64), npairs).astype(bool)
     out["gather_ms"] = 1e3 * (time.perf_counter() - t0)
     out["n_acc_all"], out["complete_all"] = n_acc, complete
     if rank == 0:
         # rows an incomplete chain never filled are NaN (never 0.0: argsort would pick them as "best")
-        np.save(f"{outdir}/misfit.npy", misfit)
+        if sidx is None:
+            np.save(f"{outdir}/misfit.npy", misfit)
+        else:
+            for s, name in enumerate(model.names):
+                os.makedirs(f"{outdir}/{name}", exist_ok=True)
+                np.save(f"{outdir}/{name}/misfit.npy", misfit[s * nchains:(s + 1) * nchains])
     return misfit, n_iter, out
 
 
@@ -85,7 +107,10 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--param", default="param.yaml")
     ap.add_argument("--sampler", default="base", choices=["base", "da"])
-    ap.add_argument("--chains", type=int, default=4)
+    ap.add_argument("--chains", type=int, default=4, help="chains (per station with --stations)")
+    ap.add_argument("--stations", default=None,
+                    help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2]): "
+                         "invert every station instead of observations synthesised from true_model")
     ap.add_argument("--no-chain-files", action="store_true")
     ap.add_argument("--outdir", default=None, help="override hmc.OUTPUT_DIR of the parameter file")
     ap.add_argument("--nsamples", type=int, default=None, help="override hmc.nsamples")
@@ -101,7 +126,8 @@ def main():
         if val is not None:
             param['hmc'][key] = val
     tic = time.time()
-    misfit, n_iter, out = run(param, a.sampler, a.chains, not a.no_chain_files, a.max_iters, a.max_L)
+    misfit, n_iter, out = run(param, a.sampler, a.chains, not a.no_chain_files, a.max_iters, a.max_L,
+                              a.stations)
     if int(os.environ.get("RANK", "0")) == 0:
         comp = out["complete_all"]
         print("chains %d (%d complete), kept samples %d, accept ratio %.3f" %

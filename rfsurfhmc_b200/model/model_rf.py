@@ -71,11 +71,14 @@ class ReceiverFunc:
             self._ctx = Context(self._device)
         key = self._config_key(n)
         if self._ctx_key != key:
-            self._ctx.config_rf(n, self.ray_p, self.nt_trace, self.dt, self.gauss, self.time_shift,
-                                self.water_level, self.rf_type, self.method)
+            self._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs)
             self._ctx_key = key
         return self._ctx
+
+    def _config_forward(self, ctx, n):
+        ctx.config_rf(n, self.ray_p, self.nt_trace, self.dt, self.gauss, self.time_shift, self.water_level,
+                      self.rf_type, self.method)
 
     _context = device_context
 

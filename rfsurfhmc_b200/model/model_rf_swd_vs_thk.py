@@ -45,17 +45,20 @@ class Joint_RF_SWD:
         the two sub-models, the observations): model_rf_swd_vs_thk.py:66-86."""
         if self._ctx is None:
             self._ctx = Context(self._device)
-        r, s = self.rfmodel, self.swdmodel
-        key = (self.sigma1, self.sigma2, r._config_fields(n), s._config_fields(n),
-               np.asarray(self.dobs, dtype=np.float64).tobytes())
+        key = (self.sigma1, self.sigma2) + self._config_fields(n) + (
+            np.asarray(self.dobs, dtype=np.float64).tobytes(),)
         if self._ctx_key != key:
-            tRc, tRg, tLc, tLg = s._grad_periods()
-            self._ctx.config_swd(n, tRc, tRg, tLc, tLg, mode=s.mode, sphere=s.sphere)
-            self._ctx.config_rf(n, r.ray_p, r.nt_trace, r.dt, r.gauss, r.time_shift, r.water_level,
-                                r.rf_type, r.method)
+            self._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
             self._ctx_key = key
         return self._ctx
+
+    def _config_fields(self, n):
+        return (self.rfmodel._config_fields(n), self.swdmodel._config_fields(n))
+
+    def _config_forward(self, ctx, n):
+        self.swdmodel._config_forward(ctx, n)
+        self.rfmodel._config_forward(ctx, n)
 
     def forward(self, x: np.ndarray):
         drf = self.rfmodel.forward(x)

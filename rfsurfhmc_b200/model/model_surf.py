@@ -96,11 +96,14 @@ class SurfWD:
             self._ctx = Context(self._device)
         key = self._config_key(n)
         if self._ctx_key != key:
-            tRc, tRg, tLc, tLg = self._grad_periods()
-            self._ctx.config_swd(n, tRc, tRg, tLc, tLg, mode=self.mode, sphere=self.sphere)
+            self._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs)
             self._ctx_key = key
         return self._ctx
+
+    def _config_forward(self, ctx, n):
+        tRc, tRg, tLc, tLg = self._grad_periods()
+        ctx.config_swd(n, tRc, tRg, tLc, tLg, mode=self.mode, sphere=self.sphere)
 
     _context = device_context
 

@@ -1,0 +1,134 @@
+"""StationArray — many stations (observation sets) that share one forward configuration.
+
+A station array is inverted station by station: each station has its own data vector (receiver
+function and dispersion curves) and its own sigma1 / sigma2, while the layer count, period lists,
+modes, ray parameter(s) and RF sampling are shared.  The reference runs one job per station; here one
+context holds every station's observations and each evaluated row, or each HMC chain, names its
+station, so one device run fills the GPU with all of them (include/rfsurfhmc.h: rfs_config_obs_sets).
+
+    stations = StationArray(joint_model, dobs)            # dobs [S, ndata]
+    HamitonianMC(stations, bounds, ...).sample_chains(ids, stations=station_of_each_chain)
+"""
+import copy
+import numpy as np
+from .._lib import Context
+from .model_rf_swd_vs_thk import Joint_RF_SWD
+
+
+def _fresh_copy(m):
+    """Shallow copy of a model object without its device context."""
+    c = copy.copy(m)
+    c._ctx = None
+    c._ctx_key = None
+    return c
+
+
+class StationArray:
+    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None):
+        """model: a configured Joint_RF_SWD, ReceiverFunc or SurfWD; only its forward configuration is
+        used (its own observations are ignored).  dobs [S, ndata] in the model's data layout.
+        sigma1 / sigma2: scalars or [S] (default: the joint model's own, 1.0 for the others; they only
+        weight the joint objective).  names [S]: output sub-directories (default station0000, ...)."""
+        if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
+            raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
+        self.template = model
+        self.which = model.which
+        self.dobs = np.array(dobs, dtype=np.float64, ndmin=2)
+        if self.dobs.ndim != 2:
+            raise ValueError(f"dobs must be [S, ndata], got shape {self.dobs.shape}")
+        S, nd = self.dobs.shape
+        want = model.ndata if isinstance(model, Joint_RF_SWD) else model.nt
+        if nd != want:
+            raise ValueError(f"dobs has {nd} values per station, the model's data vector has {want}")
+        self.nstations = S
+        self.ndata = nd
+        s1 = getattr(model, "sigma1", 1.0) if sigma1 is None else sigma1
+        s2 = getattr(model, "sigma2", 1.0) if sigma2 is None else sigma2
+        self.sigma1 = np.broadcast_to(np.asarray(s1, dtype=np.float64), (S,)).copy()
+        self.sigma2 = np.broadcast_to(np.asarray(s2, dtype=np.float64), (S,)).copy()
+        self.names = [f"station{s:04d}" for s in range(S)] if names is None else [str(v) for v in names]
+        if len(self.names) != S:
+            raise ValueError(f"names has {len(self.names)} entries for {S} stations")
+        self._ctx = None
+        self._ctx_key = None
+
+    @property
+    def _device(self):
+        return self.template._device
+
+    def device_context(self, n):
+        """Configured rfs context (the template's forward configuration + every station's observations)
+        for n layers; re-configured whenever a template field, a sigma or an observation has changed."""
+        if self._ctx is None or self._ctx.device != self._device:
+            self._ctx = Context(self._device)
+            self._ctx_key = None
+        key = (type(self.template), self.template._config_fields(n), self.sigma1.tobytes(),
+               self.sigma2.tobytes(), self.dobs.tobytes())
+        if self._ctx_key != key:
+            self.template._config_forward(self._ctx, n)
+            self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
+            self._ctx_key = key
+        return self._ctx
+
+    def misfit_and_grad_batch(self, X, stations):
+        """X [B, 2n], stations [B] -> (U[B], grad[B,2n], dsyn[B,ndata], flag[B]): row b against station
+        stations[b], all rows in one fused GPU evaluation."""
+        X = np.atleast_2d(np.asarray(X, dtype=np.float64))
+        return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=self.which, sets=stations)
+
+    def station_model(self, s):
+        """Single-station copy of the template holding station s's observations (and sigmas)."""
+        s = int(s)
+        if not 0 <= s < self.nstations:
+            raise IndexError(f"station {s} outside [0, {self.nstations})")
+        d = self.dobs[s].copy()
+        t = self.template
+        if isinstance(t, Joint_RF_SWD):
+            m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), _fresh_copy(t.rfmodel),
+                             _fresh_copy(t.swdmodel))
+            m._device = t._device
+            nt = t.rfmodel.nt
+            m.set_obsdata(d[:nt], d[nt:])
+            return m
+        m = _fresh_copy(t)
+        m.set_obsdata(d)
+        return m
+
+
+def load_stations(src, ndata, nparam, default_bounds):
+    """Validated content of a stations file (.npz path or a mapping with the same keys):
+    dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0) and bounds [S, nparam, 2]
+    (default: default_bounds [nparam, 2] for every station).  Raises ValueError naming the bad key."""
+    if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
+        with np.load(src, allow_pickle=False) as f:
+            src = {k: f[k] for k in f.files}
+    if "dobs" not in src:
+        raise ValueError("stations file: key 'dobs' [S, ndata] is required")
+    dobs = np.asarray(src["dobs"], dtype=np.float64)
+    if dobs.ndim != 2 or dobs.shape[0] < 1 or dobs.shape[1] != ndata:
+        raise ValueError(f"stations file: 'dobs' must have shape [S, {ndata}], got {dobs.shape}")
+    S = dobs.shape[0]
+    out = {"dobs": dobs}
+    names = np.asarray(src["names"]) if "names" in src else np.array([f"station{s:04d}" for s in range(S)])
+    if names.shape != (S,):
+        raise ValueError(f"stations file: 'names' must have shape [{S}], got {names.shape}")
+    out["names"] = [str(v) for v in names]
+    if len(set(out["names"])) != S or any(not v or "/" in v or v in (".", "..") for v in out["names"]):
+        raise ValueError("stations file: 'names' must be distinct, non-empty and free of '/'")
+    for key in ("sigma1", "sigma2"):
+        v = np.asarray(src[key], dtype=np.float64) if key in src else np.ones(S)
+        if v.shape != (S,):
+            raise ValueError(f"stations file: '{key}' must have shape [{S}], got {v.shape}")
+        if not np.all(np.isfinite(v) & (v > 0)):
+            raise ValueError(f"stations file: '{key}' must be finite and positive")
+        out[key] = v
+    if "bounds" in src:
+        b = np.asarray(src["bounds"], dtype=np.float64)
+        if b.shape != (S, nparam, 2):
+            raise ValueError(f"stations file: 'bounds' must have shape [{S}, {nparam}, 2], got {b.shape}")
+        if not np.all(b[..., 0] <= b[..., 1]):
+            raise ValueError("stations file: 'bounds' needs low <= high in every row")
+    else:
+        b = np.broadcast_to(np.asarray(default_bounds, dtype=np.float64), (S, nparam, 2)).copy()
+    out["bounds"] = b
+    return out

@@ -25,6 +25,38 @@ def finish_run(out, nsamples, ndraws):
     return out
 
 
+def station_run_args(model, boundaries, chain_ids, stations):
+    """(n, sets) for Context.hmc_run: the layer count from `boundaries` ([2n,2] or [S,2n,2]) and the
+    station of each chain (None without a StationArray).  Chain i samples station stations[i]."""
+    b = np.asarray(boundaries)
+    if b.ndim not in (2, 3) or b.shape[-1] != 2:
+        raise ValueError(f"boundaries must be [2n, 2] or [S, 2n, 2], got shape {b.shape}")
+    if stations is None:
+        return b.shape[-2] // 2, None
+    if not hasattr(model, "station_model"):
+        raise ValueError("stations= needs a StationArray model")
+    st = np.asarray(stations, dtype=np.int64)
+    if st.shape != np.shape(np.atleast_1d(chain_ids)):
+        raise ValueError("stations must give one station per chain id")
+    if b.ndim == 3 and b.shape[0] != model.nstations:
+        raise ValueError(f"boundaries has {b.shape[0]} boxes for {model.nstations} stations")
+    return b.shape[-2] // 2, st
+
+
+def save_chains(model, out, chain_ids, stations, outdir, name, nbest, nsamples):
+    """Write every chain of a run: {outdir}/{name}.{cid}.npz, or {outdir}/{station name}/{name}.{cid}.npz
+    with the station's observations and synthetics when the chains sample a StationArray."""
+    single = {}
+    for i, cid in enumerate(np.atleast_1d(chain_ids)):
+        if stations is None:
+            save_chain(f"{outdir}/{name}.{int(cid)}.npz", model, out, i, nbest, nsamples)
+            continue
+        s = int(stations[i])
+        if s not in single:
+            single[s] = model.station_model(s)
+        save_chain(f"{outdir}/{model.names[s]}/{name}.{int(cid)}.npz", single[s], out, i, nbest, nsamples)
+
+
 def save_chain(path, model, out, i, nbest, nsamples):
     """Write chain i of a device run.  Only the rows the chain really produced are stored; incomplete
     chains are flagged (`complete` = False)."""

@@ -7,7 +7,7 @@ hmc_kernels.cuh; chain `myrank` is seeded with `seed + myrank` exactly like one 
 reference (hmc.py:43,61), so `sample()` reproduces that rank's accept/reject sequence, and
 `sample_chains(ids)` runs any number of ranks at once on one GPU."""
 import numpy as np
-from ._common import require_device_model, finish_run, save_chain
+from ._common import require_device_model, finish_run, save_chains, station_run_args
 
 
 class HamitonianMC:
@@ -34,20 +34,19 @@ class HamitonianMC:
                             kargs['seed'], kargs['nsamples'], kargs['ndraws'], rank, kargs['name'],
                             kargs['OUTPUT_DIR'])
 
-    def sample_chains(self, chain_ids, want_syn=True, log_accepts=0, save=False):
+    def sample_chains(self, chain_ids, want_syn=True, log_accepts=0, save=False, stations=None):
         """Run the chains `chain_ids` (the reference's MPI ranks) at once; returns the result dict of
         Context.hmc_run (misfit [C,nsamples], samples, syn, initmodel, n_iter, n_acc, ...)."""
-        n = self.boundaries.shape[0] // 2
+        n, sets = station_run_args(self.model, self.boundaries, chain_ids, stations)
         ctx = self.model.device_context(n)
         out = ctx.hmc_run(0, chain_ids, self.boundaries, self.dt, Lrange=self.Lrange, seed=self._base_seed,
                           nsamples=self.nsamples, ndraws=self.ndraws, max_iters=self.max_iters,
                           want_samples=True, want_syn=want_syn, log_accepts=log_accepts,
-                          which=self.model.which)
+                          which=self.model.which, sets=sets)
         finish_run(out, self.nsamples, self.ndraws)
+        out["station"] = sets
         if save:
-            for i, cid in enumerate(np.atleast_1d(chain_ids)):
-                save_chain(f"{self.outdir}/{self.name}.{int(cid)}.npz", self.model, out, i, self.nbest_model,
-                           self.nsamples)
+            save_chains(self.model, out, chain_ids, sets, self.outdir, self.name, self.nbest_model, self.nsamples)
         self.last = out
         return out
 

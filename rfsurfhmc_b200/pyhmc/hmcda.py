@@ -3,7 +3,7 @@
 sampler (rfs_hmc_run, sampler=1): `_find_initial_dt`, L = max(1, int(lambda/dt)), always-drawn u and
 the Hoffman-Gelman dual-averaging recursion run per chain on the GPU (hmc_kernels.cuh)."""
 import numpy as np
-from ._common import require_device_model, finish_run, save_chain
+from ._common import require_device_model, finish_run, save_chains, station_run_args
 
 
 class HMCDualAveraging:
@@ -36,19 +36,19 @@ class HMCDualAveraging:
                                 kargs['target_ratio'], kargs['seed'], kargs['nsamples'], kargs['ndraws'],
                                 rank, kargs['name'], kargs['OUTPUT_DIR'])
 
-    def sample_chains(self, chain_ids, want_syn=True, log_accepts=0, save=False):
-        n = self.boundaries.shape[0] // 2
+    def sample_chains(self, chain_ids, want_syn=True, log_accepts=0, save=False, stations=None):
+        n, sets = station_run_args(self.model, self.boundaries, chain_ids, stations)
         ctx = self.model.device_context(n)
         out = ctx.hmc_run(1, chain_ids, self.boundaries, self.dt, Lrange=(1, self.max_L), L0=self.L,
                           target_ratio=self.delta,
                           seed=self._base_seed, nsamples=self.nsamples, ndraws=self.ndraws,
                           max_iters=self.max_iters, want_samples=True, want_syn=want_syn,
-                          log_accepts=log_accepts, which=self.model.which)
+                          log_accepts=log_accepts, which=self.model.which, sets=sets)
         finish_run(out, self.nsamples, self.ndraws)
+        out["station"] = sets
         if save:
-            for i, cid in enumerate(np.atleast_1d(chain_ids)):
-                # nbests hard-coded to 10 in the reference (hmcda.py:359)
-                save_chain(f"{self.outdir}/{self.name}.{int(cid)}.npz", self.model, out, i, 10, self.nsamples)
+            # nbests hard-coded to 10 in the reference (hmcda.py:359)
+            save_chains(self.model, out, chain_ids, sets, self.outdir, self.name, 10, self.nsamples)
         self.last = out
         return out
 
