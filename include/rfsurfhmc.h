@@ -78,6 +78,22 @@ int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dob
  * rfs_hmc_run) returns RFS_E_CONFIG. */
 int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
                         const double *dobs, int ndobs);
+/* Per-set ray parameters of the RF objective (each station's stack has its own mean slowness; the
+ * reference's ReceiverFunc.ray_p is per station): ray_p [S][nray] (host pointer, copied to the device
+ * here, never during an evaluation).  Row b's pass ir then uses ray_p[set[b]][ir] in place of the
+ * shared list of rfs_config_rf / rfs_config_rf_rays; everything else (nt, dt, gauss, time shift, water
+ * level, RF type, method, layers, periods, modes) stays shared.  The evaluations and the HMC use the
+ * table whenever it is present; their signatures do not change.  The librf drop-ins keep their own
+ * ray_p argument.
+ * Returns RFS_E_CONFIG without an RF configuration or when S differs from the number of observation
+ * sets held, RFS_E_ARG when nray differs from the configured ray count or a value is not finite and > 0.
+ * The table belongs to the current sets and the current RF configuration: rfs_config_obs_sets,
+ * rfs_config_obs, rfs_config_rf and rfs_config_rf_rays drop it, and the context uses the shared list
+ * again; so does a call of this function that fails.  A row whose device set index lies outside [0, S)
+ * reads no table entry; it computes with the shared value and is failed as described below.
+ * Like every rfs_config_* call, this one copies synchronously into the context's device buffers: an
+ * evaluation still running on a caller's stream must have finished before the context is reconfigured. */
+int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)

@@ -68,6 +68,8 @@ def load_library():
         L.rfs_misfit_grad_host.argtypes = [_vp, C.c_longlong, _dp, C.c_int, _dp, _dp, _dp, _u8p]
         L.rfs_config_obs_sets.restype = C.c_int
         L.rfs_config_obs_sets.argtypes = [_vp, C.c_int, _dp, _dp, _dp, C.c_int]
+        L.rfs_config_obs_rays.restype = C.c_int
+        L.rfs_config_obs_rays.argtypes = [_vp, C.c_int, C.c_int, _dp]
         L.rfs_misfit_grad_sets_dev.restype = C.c_int
         L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_sets_host.restype = C.c_int
@@ -138,7 +140,8 @@ def exported_symbols():
             "rfs_set_roots_team", "rfs_last_roots_team", "rfs_set_roots_sched",
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
-            "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets"]
+            "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
+            "rfs_config_obs_rays"]
 
 
 def _f64(a):
@@ -174,6 +177,7 @@ class Context:
         self.nt_rf = 0
         self.n_swd_data = 0
         self.nsets = 0
+        self.nray = 0
 
     def close(self):
         if getattr(self, "h", None):
@@ -261,6 +265,7 @@ class Context:
                                            rf_type_code(rf_type), method_code(method)))
         self.n = int(nlayer)
         self.nt_rf = int(nt) * rays.size
+        self.nray = rays.size
 
     def config_obs(self, dobs, sigma1=1.0, sigma2=1.0):
         """dobs [ndata]: one data vector.  dobs [S, ndata]: S observation sets (stations) sharing the
@@ -274,6 +279,16 @@ class Context:
         s2 = _f64(np.broadcast_to(np.asarray(sigma2, dtype=np.float64), (S,)))
         self._ck(self.L.rfs_config_obs_sets(self.h, S, _p(s1), _p(s2), _p(d), d.shape[-1]))
         self.nsets = S
+
+    def config_obs_rays(self, ray_p):
+        """Per-station ray parameters: ray_p [S] (one ray parameter per objective) or [S, nray], for the S
+        observation sets held now.  Row b then uses ray_p[set[b]] in place of config_rf's shared list.
+        config_obs and config_rf drop the table again."""
+        r = _f64(ray_p)
+        if r.ndim not in (1, 2) or r.shape[0] == 0:
+            raise ValueError(f"ray_p must be [S] or [S, nray], got shape {r.shape}")
+        nray = 1 if r.ndim == 1 else r.shape[1]
+        self._ck(self.L.rfs_config_obs_rays(self.h, r.shape[0], nray, _p(r)))
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)

@@ -4,6 +4,7 @@
 #include "../../include/rfsurfhmc.h"
 
 #include <cuda_runtime.h>
+#include <math.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -38,7 +39,8 @@ struct Buf {
 };
 
 // settings of one receiver-function run: the fused objective's (rfs_config_rf*) or one drop-in call's.
-// The ray parameter is passed on its own: the fused objective has a list of them.
+// The ray parameter is passed on its own (RayView): the fused objective has a list of them, and may have
+// one list per observation set.
 struct RfCfg {
   int n = 0, nt = 0, nft = 0, logn = 0, n2 = 0, rf_type = 1, method = 1;
   double dt = 0, gauss = 0, tshift = 0, water = 0.001;
@@ -82,6 +84,10 @@ struct rfs_ctx {
   bool has_rf = false;
   RfCfg rf;
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
+  // per-set ray parameters [nsets][nray] (rfs_config_obs_rays), used in place of ray_ps when present.
+  // Every call that changes the sets or the RF configuration drops the table.
+  bool has_set_rays = false;
+  Buf d_set_rays;
   // ---- observations: nsets data vectors ("stations") of ndobs values each
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
@@ -442,7 +448,7 @@ int run_swd(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, c
 // ---- RF pipeline on a prepared model block (freq method)
 // nq: 0 forward only, 2 chain-rule rows (vs, thk), 4 all parameters.  Brings the twiddle table that the
 // FFTs of run_rf_decon / run_rf_time read to cfg.nft, in order on `st`.
-int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, double ray_p, const double *d_rfm,
+int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const double *d_rfm,
                    const double *d_chain, const double *d_qa, const double *d_qb, long long B, int n,
                    int nq, double sigma, cudaStream_t st, double pi_used = RFS_PI32) {
   int rc;
@@ -458,12 +464,12 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, double ray_p, const double *d
   double2 *dsp = nq > 0 ? (double2 *)ctx->w_dspec.p : nullptr;
   // frequency-independent layer constants, once per (model, layer)
   if ((rc = ensure(ctx, ctx->w_rfl, sizeof(RfLayer) * (size_t)B * n))) return rc;
-  LAUNCH(rf_layer_kernel, gridFor(B * n, 128), 128, 0, st, d_rfm, d_qa, d_qb, B, n, ray_p,
+  LAUNCH(rf_layer_kernel, gridFor(B * n, 128), 128, 0, st, d_rfm, d_qa, d_qb, B, n, ray,
          (RfLayer *)ctx->w_rfl.p);
   const long long tot = B * n2;
 #define PROP(NM, NQ)                                                                             \
   LAUNCH((rf_propagate_kernel<NM, NQ>), gridFor(tot, 128), 128, 0, st,                           \
-         (const RfLayer *)ctx->w_rfl.p, d_chain, B, n, n2, cfg.nft, cfg.dt, ray_p, sigma,        \
+         (const RfLayer *)ctx->w_rfl.p, d_chain, B, n, n2, cfg.nft, cfg.dt, ray, sigma,          \
          pi_used, cfg.rf_type, (double2 *)ctx->w_spec.p, dsp)
 #define PROPQ(NM)    \
   if (nq == 2) {     \
@@ -707,6 +713,7 @@ int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, 
   int rc = make_rf_cfg(ctx, ctx->rf, nlayer, nt, dt, gauss, time_shift, water, rf_type, method);
   if (rc) return rc;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
+  ctx->has_set_rays = false;
   ctx->has_rf = true;
   return RFS_OK;
 }
@@ -730,12 +737,37 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
   ctx->nsets = S;
   ctx->ndobs = ndobs;
   ctx->wt_n1 = ctx->wt_nsw = -1;
+  ctx->has_set_rays = false;
   ctx->has_obs = true;
   return RFS_OK;
 }
 
 int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dobs, int ndobs) {
   return rfs_config_obs_sets(ctx, 1, &sigma1, &sigma2, dobs, ndobs);
+}
+
+int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p) {
+  if (!ctx) return RFS_E_ARG;
+  if (!ctx->has_rf) return fail(ctx, RFS_E_CONFIG, "per-set ray parameters need an RF configuration (rfs_config_rf)");
+  if (!ctx->has_obs || S != ctx->nsets)
+    return fail(ctx, RFS_E_CONFIG, "ray-parameter table for " + std::to_string(S) + " sets, the context holds " +
+                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
+  if (nray != (int)ctx->ray_ps.size())
+    return fail(ctx, RFS_E_ARG, "ray-parameter table has " + std::to_string(nray) + " rays per set, the RF " +
+                                    "objective has " + std::to_string(ctx->ray_ps.size()));
+  if (!ray_p) return fail(ctx, RFS_E_ARG, "no ray-parameter table");
+  const size_t cnt = (size_t)S * nray;
+  for (size_t i = 0; i < cnt; i++)
+    if (!(isfinite(ray_p[i]) && ray_p[i] > 0.0))
+      return fail(ctx, RFS_E_ARG, "ray parameters must be finite and > 0");
+  CK(cudaSetDevice(ctx->device));
+  // a failed upload leaves no table: the context then uses the shared list, as after rfs_config_obs_sets
+  ctx->has_set_rays = false;
+  int rc = ensure(ctx, ctx->d_set_rays, sizeof(double) * cnt);
+  if (rc) return rc;
+  CK(cudaMemcpy(ctx->d_set_rays.p, ray_p, sizeof(double) * cnt, cudaMemcpyHostToDevice));
+  ctx->has_set_rays = true;
+  return RFS_OK;
 }
 
 int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
@@ -868,7 +900,10 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       // one pass per ray parameter; misfit and gradient accumulate over the passes (the reference's
       // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3)
       for (int ir = 0; ir < nray; ir++) {
-        if ((rc = run_rf_spectra(ctx, rf, ctx->ray_ps[ir], (const double *)F.w_rfm.p,
+        // obs_k.set: this chunk's rows, as the residual kernels read them
+        const RayView ray{ctx->has_set_rays ? (const double *)ctx->d_set_rays.p : nullptr, obs_k.set, ctx->nsets,
+                          nray, ir, ctx->ray_ps[ir]};
+        if ((rc = run_rf_spectra(ctx, rf, ray, (const double *)F.w_rfm.p,
                                  (const double *)F.w_chain.p, nullptr, nullptr, Bc, n, rf_time ? 4 : 2, sigma,
                                  sr, rf_time ? RFS_PI64 : RFS_PI32)))
           return rc;
@@ -1143,7 +1178,7 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
   double tshift = time_shift;
   if (rf_type == 2) tshift = -tshift;
   const double sigma = (method == 0) ? 0.0 : 1.0 / dt / cfg.nft * 4.;
-  if ((rc = run_rf_spectra(ctx, cfg, ray_p, d_rfm, nullptr, d_rfm + 4 * nB, d_rfm + 5 * nB, B, n,
+  if ((rc = run_rf_spectra(ctx, cfg, RayView{nullptr, nullptr, 0, 1, 0, ray_p}, d_rfm, nullptr, d_rfm + 4 * nB, d_rfm + 5 * nB, B, n,
                            nq > 0 ? 4 : 0, sigma, st,
                            (method == 0 && nq == 4) ? RFS_PI64 : RFS_PI32)))
     return rc;

@@ -87,18 +87,42 @@ RFS_DEVINL RfLayer rf_layer(double thick, double rho, double vp, double vs, doub
   L.avp = L.alpha / vp;
   return L;
 }
+// Ray parameter of each row in pass `ir` of an RF objective: ray_p[set[b]][ir] of a per-set table, or
+// the shared value.  set points at the rows of this launch (NULL: every row is set 0).  A row whose set
+// index lies outside [0, nsets) reads nothing from the table and computes with the shared value; the
+// residual kernels fail that row (ObsSets::row_set), so no NaN spectrum reaches the spike picking.
+struct RayView {
+  const double *tab;  // [nsets][nray] or NULL (every row uses `shared`)
+  const int *set;     // [B] or NULL
+  int nsets, nray, ir;
+  double shared;
+  RFS_DEVINL double row_p(long long b) const {
+    if (!tab) return shared;
+    const int s = set ? set[b] : 0;
+    return (s >= 0 && s < nsets) ? tab[s * nray + ir] : shared;
+  }
+};
+
+// Layer constants of row b, layer m, for ray parameter p.  Not inlined, so that p reaches rf_layer as a
+// function parameter, as the ray parameter did when it was a kernel argument: inlined next to the table
+// lookup, the compiler shares rf_layer's products between their uses and contracts multiply-add pairs
+// differently (rf_layer_kernel: 172 instead of 173 DFMA), which changes the last bits of every RF result.
+__device__ __noinline__ void rf_layer_row(const double *__restrict__ rfm, const double *__restrict__ qa,
+                                          const double *__restrict__ qb, long long B, int n, long long b, int m,
+                                          double p, RfLayer *__restrict__ tab) {
+  const long long nB = (long long)n * B;
+  const double qam = qa ? qa[m * B + b] : 9999.0, qbm = qb ? qb[m * B + b] : 9999.0;
+  tab[b * n + m] = rf_layer(rfm[0 * nB + m * B + b], rfm[1 * nB + m * B + b],
+                            rfm[2 * nB + m * B + b], rfm[3 * nB + m * B + b], qam, qbm, p);
+}
 // one thread per (model, layer): rfm [4][n][B] thk, rho, vp, vs -> tab [B][n] RfLayer
 __global__ void rf_layer_kernel(const double *__restrict__ rfm, const double *__restrict__ qa,
-                                const double *__restrict__ qb, long long B, int n, double ray_p,
+                                const double *__restrict__ qb, long long B, int n, RayView ray,
                                 RfLayer *__restrict__ tab) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= B * n) return;
   const long long b = i % B;
-  const int m = (int)(i / B);
-  const long long nB = (long long)n * B;
-  const double qam = qa ? qa[m * B + b] : 9999.0, qbm = qb ? qb[m * B + b] : 9999.0;
-  tab[b * n + m] = rf_layer(rfm[0 * nB + m * B + b], rfm[1 * nB + m * B + b],
-                            rfm[2 * nB + m * B + b], rfm[3 * nB + m * B + b], qam, qbm, ray_p);
+  rf_layer_row(rfm, qa, qb, B, n, b, (int)(i / B), ray.row_p(b), tab);
 }
 RFS_DEVINL RfLayer rf_layer_ld(const RfLayer *__restrict__ tab, long long idx) {
   RfLayer L;
@@ -255,7 +279,7 @@ RFS_DEVINL cd nan0(cd z) { return (isnan(z.x) || isnan(z.y)) ? cd(0.0, 0.0) : z;
 template <int NMAX, int NQ>
 __global__ void __launch_bounds__(128, RFS_RF_MINBLOCKS)
     rf_propagate_kernel(const RfLayer *__restrict__ tab, const double *__restrict__ chain,
-                        long long B, int n, int n2, int nft, double dt, double ray_p, double sigma,
+                        long long B, int n, int n2, int nft, double dt, RayView ray, double sigma,
                         double pi_used, int rf_type, double2 *__restrict__ spec,
                         double2 *__restrict__ dspec) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -266,7 +290,7 @@ __global__ void __launch_bounds__(128, RFS_RF_MINBLOCKS)
   // pi_used: float32 pi everywhere except cal_rf_par_time_all (RFModule.f90:94 uses atan(1.0_dp))
   const double w = 1.0 / nft / dt * kf * 2.0 * pi_used;
   const cd omega(w, -sigma);
-  const double p = ray_p;
+  const double p = ray.row_p(b);
   const int row = (rf_type == 1) ? 1 : 0;
 
   cd Ls[NMAX * 4];       // suffix rows l_j

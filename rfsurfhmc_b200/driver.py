@@ -10,8 +10,9 @@ write `real_syn.npy`, per-chain result files and `misfit.npy [nchains, nsamples]
     python -m rfsurfhmc_b200.driver --param param.yaml --stations stations.npz --chains K
 
 inverts a station array instead: the observations of S stations come from the file (see
-model/stations.py: load_stations), K chains run per station, all S*K in one device run (sharded over
-ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
+model/stations.py: load_stations; the optional key ray_p [S] or [S, nray] gives each station its own
+ray parameter(s) in place of rf.ray_p), K chains run per station, all S*K in one device run (sharded
+over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
 import argparse
 import os
 import time
@@ -64,8 +65,8 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
         npairs = nchains
         ids, sidx = D.shard_chains(nchains), None
     else:
-        st = load_stations(stations, model.ndata, x.size, driver_bounds(x))
-        model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"])
+        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray)
+        model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"], st["ray_p"])
         boundaries = st["bounds"]
         npairs = model.nstations * nchains
         sidx, ids = D.shard_station_chains(model.nstations, nchains)
@@ -109,8 +110,9 @@ def main():
     ap.add_argument("--sampler", default="base", choices=["base", "da"])
     ap.add_argument("--chains", type=int, default=4, help="chains (per station with --stations)")
     ap.add_argument("--stations", default=None,
-                    help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2]): "
-                         "invert every station instead of observations synthesised from true_model")
+                    help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2], "
+                         "ray_p [S] or [S,nray] in place of rf.ray_p): invert every station instead of "
+                         "observations synthesised from true_model")
     ap.add_argument("--no-chain-files", action="store_true")
     ap.add_argument("--outdir", default=None, help="override hmc.OUTPUT_DIR of the parameter file")
     ap.add_argument("--nsamples", type=int, default=None, help="override hmc.nsamples")

@@ -1,18 +1,23 @@
 """StationArray — many stations (observation sets) that share one forward configuration.
 
 A station array is inverted station by station: each station has its own data vector (receiver
-function and dispersion curves) and its own sigma1 / sigma2, while the layer count, period lists,
-modes, ray parameter(s) and RF sampling are shared.  The reference runs one job per station; here one
-context holds every station's observations and each evaluated row, or each HMC chain, names its
-station, so one device run fills the GPU with all of them (include/rfsurfhmc.h: rfs_config_obs_sets).
+function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s), while
+the layer count, period lists, modes and RF sampling are shared.  The reference runs one job per
+station; here one context holds every station's observations and each evaluated row, or each HMC chain,
+names its station, so one device run fills the GPU with all of them (include/rfsurfhmc.h:
+rfs_config_obs_sets, rfs_config_obs_rays).
 
-    stations = StationArray(joint_model, dobs)            # dobs [S, ndata]
+    stations = StationArray(joint_model, dobs, ray_p=p)   # dobs [S, ndata], p [S] or [S, nray]
     HamitonianMC(stations, bounds, ...).sample_chains(ids, stations=station_of_each_chain)
+
+A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
+keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2] and ray_p [S] or [S, nray].
 """
 import copy
 import numpy as np
 from .._lib import Context
 from .model_rf_swd_vs_thk import Joint_RF_SWD
+from .model_rf import ReceiverFunc
 
 
 def _fresh_copy(m):
@@ -24,11 +29,13 @@ def _fresh_copy(m):
 
 
 class StationArray:
-    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None):
+    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None):
         """model: a configured Joint_RF_SWD, ReceiverFunc or SurfWD; only its forward configuration is
         used (its own observations are ignored).  dobs [S, ndata] in the model's data layout.
         sigma1 / sigma2: scalars or [S] (default: the joint model's own, 1.0 for the others; they only
-        weight the joint objective).  names [S]: output sub-directories (default station0000, ...)."""
+        weight the joint objective).  names [S]: output sub-directories (default station0000, ...).
+        ray_p: None (every station uses the template's ray parameter(s)) or each station's own, [S] or
+        [S, nray] with the template's ray count; not for a SurfWD template."""
         if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
             raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
         self.template = model
@@ -49,6 +56,12 @@ class StationArray:
         self.names = [f"station{s:04d}" for s in range(S)] if names is None else [str(v) for v in names]
         if len(self.names) != S:
             raise ValueError(f"names has {len(self.names)} entries for {S} stations")
+        self.ray_p = None
+        if ray_p is not None:
+            rf = model.rfmodel if isinstance(model, Joint_RF_SWD) else model
+            if not isinstance(rf, ReceiverFunc):
+                raise TypeError("ray_p needs a receiver-function template (Joint_RF_SWD or ReceiverFunc)")
+            self.ray_p = station_rays(ray_p, S, rf.nray)
         self._ctx = None
         self._ctx_key = None
 
@@ -63,10 +76,12 @@ class StationArray:
             self._ctx = Context(self._device)
             self._ctx_key = None
         key = (type(self.template), self.template._config_fields(n), self.sigma1.tobytes(),
-               self.sigma2.tobytes(), self.dobs.tobytes())
+               self.sigma2.tobytes(), self.dobs.tobytes(), None if self.ray_p is None else self.ray_p.tobytes())
         if self._ctx_key != key:
             self.template._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
+            if self.ray_p is not None:
+                self._ctx.config_obs_rays(self.ray_p)
             self._ctx_key = key
         return self._ctx
 
@@ -77,28 +92,49 @@ class StationArray:
         return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=self.which, sets=stations)
 
     def station_model(self, s):
-        """Single-station copy of the template holding station s's observations (and sigmas)."""
+        """Single-station copy of the template holding station s's observations (and sigmas, and ray
+        parameter(s): a scalar for one ray, a list otherwise)."""
         s = int(s)
         if not 0 <= s < self.nstations:
             raise IndexError(f"station {s} outside [0, {self.nstations})")
         d = self.dobs[s].copy()
         t = self.template
         if isinstance(t, Joint_RF_SWD):
-            m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), _fresh_copy(t.rfmodel),
-                             _fresh_copy(t.swdmodel))
+            rf = self._station_rf(t.rfmodel, s)
+            m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), rf, _fresh_copy(t.swdmodel))
             m._device = t._device
             nt = t.rfmodel.nt
             m.set_obsdata(d[:nt], d[nt:])
             return m
-        m = _fresh_copy(t)
+        m = self._station_rf(t, s) if isinstance(t, ReceiverFunc) else _fresh_copy(t)
         m.set_obsdata(d)
         return m
 
+    def _station_rf(self, rf, s):
+        c = _fresh_copy(rf)
+        if self.ray_p is not None:
+            r = self.ray_p[s]
+            c.ray_p = float(r[0]) if r.size == 1 else r.tolist()
+        return c
 
-def load_stations(src, ndata, nparam, default_bounds):
+
+def station_rays(ray_p, S, nray, where=""):
+    """ray_p [S] (nray = 1) or [S, nray] -> float64 [S, nray], finite and > 0; the ValueError names the
+    key 'ray_p' (after `where`)."""
+    r = np.asarray(ray_p, dtype=np.float64)
+    if not (r.shape == (S, nray) or (nray == 1 and r.shape == (S,))):
+        want = f"[{S}] or [{S}, 1]" if nray == 1 else f"[{S}, {nray}]"
+        raise ValueError(f"{where}'ray_p' must have shape {want}, got {r.shape}")
+    if not np.all(np.isfinite(r) & (r > 0)):
+        raise ValueError(f"{where}'ray_p' must be finite and positive")
+    return np.ascontiguousarray(r.reshape(S, nray))
+
+
+def load_stations(src, ndata, nparam, default_bounds, nray=1):
     """Validated content of a stations file (.npz path or a mapping with the same keys):
-    dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0) and bounds [S, nparam, 2]
-    (default: default_bounds [nparam, 2] for every station).  Raises ValueError naming the bad key."""
+    dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0), bounds [S, nparam, 2]
+    (default: default_bounds [nparam, 2] for every station) and ray_p [S] or [S, nray] (default None: the
+    ray parameter(s) of the forward configuration).  Raises ValueError naming the bad key."""
     if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
         with np.load(src, allow_pickle=False) as f:
             src = {k: f[k] for k in f.files}
@@ -131,4 +167,5 @@ def load_stations(src, ndata, nparam, default_bounds):
     else:
         b = np.broadcast_to(np.asarray(default_bounds, dtype=np.float64), (S, nparam, 2)).copy()
     out["bounds"] = b
+    out["ray_p"] = station_rays(src["ray_p"], S, nray, "stations file: ") if "ray_p" in src else None
     return out

@@ -10,6 +10,16 @@ models per station K) = (256, 64), (64, 256), (1024, 16):
   (c) one set : the same 16 384 models against one observation vector (the cost of the set lookup).
 HMC: 16 stations x 64 chains, base sampler, fixed max_iters: one hmc_run over all stations vs 16
 sequential single-station runs.
+Leg "rays" (per-station ray parameters, rfs_config_obs_rays), every station with its own ray parameter:
+  (d) F1 (S, K) = (256, 64), (1024, 16): the grouped call with a ray table vs the same grouped call with
+      the shared ray parameter (two contexts, timed alternately, --inner calls per timing);
+  (e) RF only, C3-like: n = 40, nt = 2048, three ray parameters per station, 65 536 models over 256
+      stations, with a [256, 3] table vs the shared list (the propagate kernel dominates there).  The two
+      contexts live side by side, so each gets a 48 GB workspace budget (RFS_WS_BUDGET_MB): both run the
+      batch in the same two chunks;
+  (f) HMC, 16 stations x 64 chains, distinct ray parameters: one grouped run vs 16 single-station runs,
+      each in a context configured with its station's ray parameter.
+--legs sets,rays selects the legs; the legs run replace their keys in --out and keep the others.
 Every shape is warmed up first; each timing is repeated --reps times (median, min, max reported), with a
 host clock around work that ends in a device synchronise.  Station observations are the forward model
 of seeded perturbations of the F1 true model plus seeded noise.  Prints one JSON line and writes it to
@@ -46,7 +56,10 @@ def main():
     ap.add_argument("--total", type=int, default=16384)
     ap.add_argument("--hmc-iters", type=int, default=20)
     ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "stations_bench.json"))
+    ap.add_argument("--legs", default="sets,rays")
+    ap.add_argument("--inner", type=int, default=20, help="calls per timing in the rays leg")
     a = ap.parse_args()
+    legs = set(a.legs.split(","))
     import torch
     if not torch.cuda.is_available():
         raise SystemExit("stations_bench.py measures on a CUDA device; none is available")
@@ -90,7 +103,16 @@ def main():
             ts.append(time.perf_counter() - t0)
         return spread(ts)
 
-    res = {"tool": "stations_bench", **gpu_info(), "forward_config": "F1", "rows": B, "eval": []}
+    res = {}
+    if os.path.exists(a.out):
+        with open(a.out) as f:
+            res = json.loads(f.read())
+    if "rays" in legs:
+        res["rays"] = rays_leg(a, torch, station_obs, X, nd)
+    if "sets" not in legs:
+        c.close()
+        return write(a, res)
+    res.update({"tool": "stations_bench", **gpu_info(), "forward_config": "F1", "rows": B, "eval": []})
     one = station_obs(1, 99)[0]
     c.config_obs(one)
     single = timed(lambda: call(0, B))
@@ -140,11 +162,128 @@ def main():
     hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
     res["hmc"] = hmc
     c.close()
+    write(a, res)
+
+
+def write(a, res):
     line = json.dumps(res)
     print(line, flush=True)
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, "w") as f:
         f.write(line + "\n")
+
+
+def rays_leg(a, torch, station_obs, X, nd):
+    """Per-station ray parameters against the shared one, same grouped call (see the module docstring)."""
+    from rfsurfhmc_b200._lib import Context
+    from rfsurfhmc_b200.fixtures import f1_config, f1_true_model, driver_bounds, perturbed_models
+    from bench import layered_models
+    cfg, x0 = f1_config(), f1_true_model()
+    dev = torch.device("cuda", 0)
+    st = torch.cuda.current_stream(dev)
+    out = {**gpu_info(), "inner_calls": a.inner, "eval": []}
+
+    def contexts(which, n, rays, nt, dt, gauss, dobs, table):
+        """(shared, table): two contexts on the same stations, without and with the ray table"""
+        cs = []
+        for with_table in (False, True):
+            c = Context(0)
+            if which != 1:
+                c.config_swd(n, tRc=cfg["tRc"], tRg=cfg["tRg"])
+            c.config_rf(n, rays, nt, dt, gauss, cfg["time_shift"], cfg["water"], "P", "freq")
+            c.config_obs(dobs)
+            if with_table:
+                c.config_obs_rays(table)
+            cs.append(c)
+        return cs
+
+    def alternate(cs, which, Xd, sets):
+        B = Xd.shape[0]
+        U = torch.empty(B, dtype=torch.float64, device=dev)
+        G = torch.empty(Xd.shape, dtype=torch.float64, device=dev)
+        D = torch.empty(B, cs[0].ndata(which), dtype=torch.float64, device=dev)
+        F = torch.empty(B, dtype=torch.uint8, device=dev)
+
+        def call(c):
+            for _ in range(a.inner):
+                c.misfit_grad_dev(B, Xd.data_ptr(), which, U.data_ptr(), G.data_ptr(), D.data_ptr(), F.data_ptr(),
+                                  st.cuda_stream, sets_ptr=sets.data_ptr())
+        ts = ([], [])
+        for c in cs:
+            call(c)
+        torch.cuda.synchronize()
+        for _ in range(a.reps):
+            for k, c in enumerate(cs):
+                t0 = time.perf_counter()
+                call(c)
+                torch.cuda.synchronize()
+                ts[k].append((time.perf_counter() - t0) / a.inner)
+        for c in cs:
+            c.close()
+        shared, table = spread(ts[0]), spread(ts[1])
+        return {"shared_ray": shared, "ray_table": table, "table_cost": table["median_ms"] / shared["median_ms"] - 1.0}
+
+    rng = np.random.default_rng(17)
+    for S, K in ((256, 64), (1024, 16)):
+        dobs = station_obs(S, 100 + S)
+        table = rng.uniform(0.04, 0.08, S)
+        sets = torch.from_numpy(np.repeat(np.arange(S, dtype=np.int32), K)).to(dev)
+        cs = contexts(0, x0.size // 2, cfg["ray_p"], cfg["nt"], cfg["dt"], cfg["gauss"], dobs, table)
+        out["eval"].append({"workload": "F1 joint, %d stations x %d models" % (S, K), "S": S, "K": K,
+                            **alternate(cs, 0, X, sets)})
+    # RF only, C3-like
+    n, nt, S, K = 40, 2048, 256, 256
+    rays = [0.04, 0.06, 0.08]
+    Xc = torch.from_numpy(layered_models(S * K, n, 2)).to(dev)
+    table = np.sort(rng.uniform(0.035, 0.085, (S, 3)), axis=1)
+    dobs = 0.01 * np.random.default_rng(3).standard_normal((S, 3 * nt))
+    sets = torch.from_numpy(np.repeat(np.arange(S, dtype=np.int32), K)).to(dev)
+    old = os.environ.get("RFS_WS_BUDGET_MB")
+    os.environ["RFS_WS_BUDGET_MB"] = "48000"
+    try:
+        cs = contexts(1, n, rays, nt, 0.05, 2.5, dobs, table)
+    finally:
+        if old is None:
+            del os.environ["RFS_WS_BUDGET_MB"]
+        else:
+            os.environ["RFS_WS_BUDGET_MB"] = old
+    out["rf_c3"] = {"workload": "RF only (freq), n=40, nt=2048, dt=0.05, a=2.5, three ray parameters per station, "
+                                "%d stations x %d models" % (S, K), "S": S, "K": K, **alternate(cs, 1, Xc, sets)}
+    # HMC, 16 stations x 64 chains, distinct ray parameters
+    Sh, Kh = 16, 64
+    dobs = station_obs(Sh, 7)
+    table = np.linspace(0.04, 0.08, Sh)
+    bounds = driver_bounds(x0)
+    kw = dict(dt=0.1, Lrange=(5, 20), seed=991206, nsamples=a.hmc_iters + 1, ndraws=0, max_iters=a.hmc_iters,
+              want_samples=False)
+    n = x0.size // 2
+    grouped = contexts(0, n, cfg["ray_p"], cfg["nt"], cfg["dt"], cfg["gauss"], dobs, table)
+    grouped[0].close()
+    single = []
+    for s in range(Sh):
+        c = Context(0)
+        c.config_swd(n, tRc=cfg["tRc"], tRg=cfg["tRg"])
+        c.config_rf(n, float(table[s]), cfg["nt"], cfg["dt"], cfg["gauss"], cfg["time_shift"], cfg["water"], "P", "freq")
+        c.config_obs(dobs[s])
+        single.append(c)
+    ids, hsets = np.tile(np.arange(Kh), Sh), np.repeat(np.arange(Sh), Kh)
+    runs = {"grouped": lambda: grouped[1].hmc_run(0, ids, bounds, sets=hsets, **kw)["evals"],
+            "per_station": lambda: sum(single[s].hmc_run(0, np.arange(Kh), bounds, **kw)["evals"] for s in range(Sh))}
+    hmc = {"S": Sh, "K": Kh, "max_iters": a.hmc_iters}
+    for name, fn in runs.items():
+        fn()
+        ts, evs = [], 0
+        for _ in range(max(1, a.reps // 2)):
+            t0 = time.perf_counter()
+            evs = fn()
+            ts.append(time.perf_counter() - t0)
+        hmc[name] = {**spread(ts), "evals": int(evs), "evals_per_s": float(evs / np.median(ts))}
+    hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
+    out["hmc"] = hmc
+    grouped[1].close()
+    for c in single:
+        c.close()
+    return out
 
 
 if __name__ == "__main__":
