@@ -94,6 +94,23 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
  * Like every rfs_config_* call, this one copies synchronously into the context's device buffers: an
  * evaluation still running on a caller's stream must have finished before the context is reconfigured. */
 int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
+/* Per-set SWD period lists (dispersion curves are rarely measured on the same periods at every
+ * station): the four lists of rfs_config_swd[_modes] form a common period grid, and use [S][nper]
+ * (host pointer, values 0 or 1, nper = ntRc + ntRg + ntLc + ntLg, one mode block of the data vector in
+ * its order) marks the grid periods each set observes.  The same mask applies to every mode block.
+ * Row b of set s then gives exactly U, grad and flag of a one-set context configured with
+ * rfs_config_swd[_modes] on set s's subset lists (everything else unchanged): every root search runs
+ * the set's own compact period list.  dsyn keeps the grid layout: the subset context's values at the
+ * observed positions, NaN at the others in every mode block; a failed row returns dobs as before.  The
+ * joint weight of set s is (sigma1[s]/sigma2[s])^2 n_rf/(nmodes * observed periods of s).  RF-only
+ * evaluations (which = 1) ignore the table; the libsurf drop-ins are not affected.
+ * Returns RFS_E_CONFIG without an SWD configuration or when S differs from the number of observation
+ * sets held, RFS_E_ARG when nper is wrong, a value is not 0 or 1, or a set observes no period.
+ * The table belongs to the current sets and the current SWD configuration: rfs_config_obs_sets,
+ * rfs_config_obs, rfs_config_swd and rfs_config_swd_modes drop it, and so does a call of this function
+ * that fails; rfs_config_rf* keep it.  A row whose device set index lies outside [0, S) runs the grid
+ * lists and is failed as described below.  Copies synchronously, like rfs_config_obs_rays. */
+int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)

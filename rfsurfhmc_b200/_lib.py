@@ -70,6 +70,8 @@ def load_library():
         L.rfs_config_obs_sets.argtypes = [_vp, C.c_int, _dp, _dp, _dp, C.c_int]
         L.rfs_config_obs_rays.restype = C.c_int
         L.rfs_config_obs_rays.argtypes = [_vp, C.c_int, C.c_int, _dp]
+        L.rfs_config_obs_periods.restype = C.c_int
+        L.rfs_config_obs_periods.argtypes = [_vp, C.c_int, C.c_int, _u8p]
         L.rfs_misfit_grad_sets_dev.restype = C.c_int
         L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_sets_host.restype = C.c_int
@@ -141,7 +143,7 @@ def exported_symbols():
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
             "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
-            "rfs_config_obs_rays"]
+            "rfs_config_obs_rays", "rfs_config_obs_periods"]
 
 
 def _f64(a):
@@ -289,6 +291,20 @@ class Context:
             raise ValueError(f"ray_p must be [S] or [S, nray], got shape {r.shape}")
         nray = 1 if r.ndim == 1 else r.shape[1]
         self._ck(self.L.rfs_config_obs_rays(self.h, r.shape[0], nray, _p(r)))
+
+    def config_obs_periods(self, use):
+        """Per-station SWD period lists: use [S, nper] (bool or 0/1) marks the periods of config_swd's
+        lists (the common grid, nper = len(tRc) + len(tRg) + len(tLc) + len(tLg), in the data vector's
+        order; the same mask for every mode block) that each of the S observation sets held now observes.
+        Row b then equals a one-station context configured on set[b]'s subset lists; dsyn is NaN at the
+        periods it does not observe.  config_obs and config_swd drop the table again."""
+        u = np.asarray(use)
+        if u.ndim != 2 or u.shape[0] == 0:
+            raise ValueError(f"use must be [S, nper], got shape {u.shape}")
+        if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
+            raise ValueError("use must hold booleans or 0/1")
+        u8 = np.ascontiguousarray(u, dtype=np.uint8)
+        self._ck(self.L.rfs_config_obs_periods(self.h, u8.shape[0], u8.shape[1], u8.ctypes.data_as(_u8p)))
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)

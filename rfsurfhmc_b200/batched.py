@@ -7,9 +7,10 @@ from ._lib import Context
 class JointEvaluator:
     """Many-chains Joint_RF_SWD.misfit_and_grad on one GPU with resident inputs/outputs.  dobs [ndata]
     or [S, ndata]: S observation sets (stations) sharing `cfg`; cfg's sigma1 / sigma2 may then be
-    [S] arrays.  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's ray_p."""
+    [S] arrays.  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's ray_p.
+    obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set observes."""
 
-    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None):
+    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None):
         self.ctx = Context(device)
         self.which = which
         self.n = nlayer
@@ -23,6 +24,8 @@ class JointEvaluator:
         self.ctx.config_obs(dobs, cfg.get("sigma1", 1.0), cfg.get("sigma2", 1.0))
         if obs_ray_p is not None:
             self.ctx.config_obs_rays(obs_ray_p)
+        if obs_swd_use is not None:
+            self.ctx.config_obs_periods(obs_swd_use)
         self.device = torch.device("cuda", device)
         self.ndata = self.ctx.ndata(which)
         self._out = None

@@ -78,8 +78,16 @@ struct rfs_ctx {
   int n_swd = 0, mode = 0, stale = 1, sphere = 0;
   std::vector<int> modes;  // modes of the fused SWD objective (reference: one mode)
   SwdPlan plan;
-  std::vector<double> periods;
+  std::vector<double> periods;  // the four grid lists (d_periods holds the per-set compact lists after them)
   Buf d_periods;
+  int swd_nts[4] = {0, 0, 0, 0};  // lengths of the grid lists tRc, tRg, tLc, tLg
+  // per-set period lists (rfs_config_obs_periods): SwdSetView table [nsets][set_per_ld] and each set's
+  // observed count per mode block.  plan_unshared: the plan was rebuilt without the Rc/Rg sequence
+  // sharing for the table's lifetime.  rfs_config_obs_sets / rfs_config_obs / rfs_config_swd* drop it.
+  bool has_set_periods = false, plan_unshared = false;
+  Buf d_set_per;
+  int set_per_ld = 0;
+  std::vector<int> set_nobs;
   // ---- RF configuration
   bool has_rf = false;
   RfCfg rf;
@@ -207,8 +215,9 @@ bool same_periods(const double *a, int na, const double *b, int nb) {
 
 // Build the sequence / row plan for the requested wave types (see swd_kernels.cuh).
 // want_kernels: group-velocity rows need the 1.05 T / 0.95 T sequences (surfdisp.cpp:234-241).
+// share: a group-velocity row on the same periods as the phase-velocity row reuses its T sequence
 int build_plan(rfs_ctx *ctx, SwdPlan &P, std::vector<double> &periods, const int nts[4],
-               const double *ts[4], int mode, bool want_kernels) {
+               const double *ts[4], int mode, bool want_kernels, bool share = true) {
   memset(&P, 0, sizeof(P));
   periods.clear();
   P.nmode = mode + 1;
@@ -250,7 +259,7 @@ int build_plan(rfs_ctx *ctx, SwdPlan &P, std::vector<double> &periods, const int
     }
     if (nts[wg] > 0) {
       int s0;
-      if (sc >= 0 && same_periods(ts[wc], nts[wc], ts[wg], nts[wg]))
+      if (share && sc >= 0 && same_periods(ts[wc], nts[wc], ts[wg], nts[wg]))
         s0 = sc;  // the reference recomputes these roots (surfdisp.cpp:239); they are identical
       else
         s0 = add_seq(ifunc, per_off[wg], nts[wg], 1.0);
@@ -350,8 +359,8 @@ static inline void release_rf_branch(Front &F, cudaStream_t st) {
 #ifndef RFS_SCHED_MIN_JOBS
 #define RFS_SCHED_MIN_JOBS 32768
 #endif
-int launch_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, const SwdBlocks &d_swd,
-                 long long B, int n, int all_modes, cudaStream_t st) {
+int launch_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const SwdSetView &sv, const double *d_periods,
+                 const SwdBlocks &d_swd, long long B, int n, int all_modes, cudaStream_t st) {
   unsigned long long *cnt = ctx->count_evals ? (unsigned long long *)ctx->d_counter.p : nullptr;
   int T, S;
   const long long jobs = B * P.nseq;
@@ -370,7 +379,7 @@ int launch_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_perio
       if ((rc = ensure(ctx, F.w_key, sizeof(unsigned int) * (size_t)jobs))) return rc;
       if ((rc = ensure(ctx, F.w_perm, sizeof(int) * (size_t)jobs))) return rc;
       LAUNCH_TU("swd_roots_sched_key_kernel",
-                launch_sched_keys(P, d_swd, B, n, d_periods, (unsigned int *)F.w_key.p, st));
+                launch_sched_keys(P, d_swd, sv, B, n, d_periods, (unsigned int *)F.w_key.p, st));
       LAUNCH_TU("swd_roots_sched_sort_kernel",
                 launch_sched_sort(P, B, (const unsigned int *)F.w_key.p, (int *)F.w_perm.p, st));
       perm = (const int *)F.w_perm.p;
@@ -378,22 +387,23 @@ int launch_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_perio
     }
     release_rf_branch(F, st);
     LAUNCH_TU("swd_roots_kernel",
-              launch_roots_thread(P, d_swd, B, n, d_periods, all_modes, (double *)F.w_croot.p,
+              launch_roots_thread(P, d_swd, sv, B, n, d_periods, all_modes, (double *)F.w_croot.p,
                                   (double *)F.w_cwork.p, (int *)F.w_ierr.p, cnt, perm, ctx->nsm, st));
     return RFS_OK;
   }
   if (!team_shape_supported(T, S)) return fail(ctx, RFS_E_ARG, "unsupported root-search team shape");
   release_rf_branch(F, st);
   LAUNCH_TU("swd_roots_team_kernel",
-            launch_roots_team(T, S, P, d_swd, B, n, d_periods, all_modes, (double *)F.w_croot.p,
+            launch_roots_team(T, S, P, d_swd, sv, B, n, d_periods, all_modes, (double *)F.w_croot.p,
                               (double *)F.w_cwork.p, (int *)F.w_ierr.p, cnt, st));
   return RFS_OK;
 }
 
 // ---- SWD pipeline on a prepared model block: roots + eigen solves
 // roots (+ retries) into the front set F, then (run_swd_eigen) the eigen solves
-int run_swd_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, const SwdBlocks &d_swd,
-                  long long B, int n, bool all_modes, cudaStream_t st) {
+// sv: each row's own period lists (SwdSetView; tab NULL for the plan's)
+int run_swd_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const SwdSetView &sv, const double *d_periods,
+                  const SwdBlocks &d_swd, long long B, int n, bool all_modes, cudaStream_t st) {
   const int nmo = all_modes ? P.nmode : 1;
   int rc;
   // the kernels index the model block with 32-bit element offsets (SwdModel::ld)
@@ -402,19 +412,19 @@ int run_swd_roots(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_peri
   if ((rc = ensure(ctx, F.w_croot, sizeof(double) * (size_t)nmo * P.nsolve * B))) return rc;
   if ((rc = ensure(ctx, F.w_cwork, sizeof(double) * (size_t)P.nsolve * B))) return rc;
   if ((rc = ensure(ctx, F.w_ierr, sizeof(int) * (size_t)P.nseq * B))) return rc;
-  if ((rc = launch_roots(ctx, F, P, d_periods, d_swd, B, n, all_modes ? 1 : 0, st))) return rc;
+  if ((rc = launch_roots(ctx, F, P, sv, d_periods, d_swd, B, n, all_modes ? 1 : 0, st))) return rc;
   // per-period retries of failed fundamental-mode searches (rare; idle warps exit at once)
   if ((rc = ensure(ctx, F.w_rstat, sizeof(int) * (size_t)P.nsolve * B))) return rc;
   LAUNCH_TU("swd_retry_kernel",
-            launch_roots_retry(P, d_swd, B, n, d_periods, all_modes ? 1 : 0, (double *)F.w_croot.p,
+            launch_roots_retry(P, d_swd, sv, B, n, d_periods, all_modes ? 1 : 0, (double *)F.w_croot.p,
                                (double *)F.w_cwork.p, (const int *)F.w_ierr.p, (int *)F.w_rstat.p,
                                ctx->count_evals ? (unsigned long long *)ctx->d_counter.p : nullptr, st));
-  LAUNCH(swd_retry_finish_kernel, gridFor(B * P.nseq, 128), 128, 0, st, P, B, all_modes ? 1 : 0,
+  LAUNCH(swd_retry_finish_kernel, gridFor(B * P.nseq, 128), 128, 0, st, P, sv, B, all_modes ? 1 : 0,
          (double *)F.w_croot.p, (int *)F.w_ierr.p, (const int *)F.w_rstat.p);
   return RFS_OK;
 }
 
-int run_swd_eigen(rfs_ctx *ctx, const Front &F, const SwdPlan &P, const double *d_periods,
+int run_swd_eigen(rfs_ctx *ctx, const Front &F, const SwdPlan &P, const SwdSetView &sv, const double *d_periods,
                   const SwdBlocks &d_swd, long long B, int n, bool all_modes, cudaStream_t st) {
   const int nmo = all_modes ? P.nmode : 1;
   int rc;
@@ -425,7 +435,7 @@ int run_swd_eigen(rfs_ctx *ctx, const Front &F, const SwdPlan &P, const double *
   // NMAX = 8: the Rayleigh up-sweep vectors live in shared memory ([48][128] doubles per block)
 #define EIG(NM)                                                                                 \
   LAUNCH(swd_eigen_kernel<NM>, gridFor(tot, 128), 128, (NM <= 8 ? 128 * NM * 6 * sizeof(double) : 0), st, \
-         P, d_swd, B, n, d_periods, nmo, (const double *)F.w_croot.p, (double *)ctx->w_ugr.p,             \
+         P, d_swd, sv, B, n, d_periods, nmo, (const double *)F.w_croot.p, (double *)ctx->w_ugr.p,         \
          (double *)ctx->w_kern.p)
   switch (nmax_for(n)) {
     case 8: EIG(8); break;
@@ -440,9 +450,10 @@ int run_swd_eigen(rfs_ctx *ctx, const Front &F, const SwdPlan &P, const double *
 
 int run_swd(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, const SwdBlocks &d_swd,
             long long B, int n, bool all_modes, bool want_eigen, cudaStream_t st) {
-  int rc = run_swd_roots(ctx, F, P, d_periods, d_swd, B, n, all_modes, st);
+  const SwdSetView sv{nullptr, nullptr, 0, 0};  // the drop-ins: one period list for every model
+  int rc = run_swd_roots(ctx, F, P, sv, d_periods, d_swd, B, n, all_modes, st);
   if (rc || !want_eigen) return rc;
-  return run_swd_eigen(ctx, F, P, d_periods, d_swd, B, n, all_modes, st);
+  return run_swd_eigen(ctx, F, P, sv, d_periods, d_swd, B, n, all_modes, st);
 }
 
 // ---- RF pipeline on a prepared model block (freq method)
@@ -590,6 +601,30 @@ size_t per_model_bytes(const rfs_ctx *ctx, int which) {
   return s + 64;
 }
 
+// Builds ctx->plan on the context's grid lists (ctx->periods, swd_nts entries per wave type) and uploads
+// the period table.  share = false: no Rc/Rg sequence sharing (see rfs_config_obs_periods).
+int rebuild_grid_plan(rfs_ctx *ctx, bool share) {
+  const std::vector<double> grid = ctx->periods;  // build_plan refills ctx->periods
+  const double *ts[4];
+  for (int w = 0, o = 0; w < 4; o += ctx->swd_nts[w], w++) ts[w] = grid.data() + o;
+  int rc = build_plan(ctx, ctx->plan, ctx->periods, ctx->swd_nts, ts, ctx->mode, true, share);
+  if (rc) return rc;
+  if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * ctx->periods.size()))) return rc;
+  CK(cudaMemcpy(ctx->d_periods.p, ctx->periods.data(), sizeof(double) * ctx->periods.size(),
+                cudaMemcpyHostToDevice));
+  return RFS_OK;
+}
+
+// drops the per-set period table; the plan shares the Rc/Rg sequence again where the grid allows
+int drop_set_periods(rfs_ctx *ctx) {
+  if (!ctx->has_set_periods) return RFS_OK;
+  ctx->has_set_periods = false;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
+  if (!ctx->plan_unshared) return RFS_OK;
+  ctx->plan_unshared = false;
+  return rebuild_grid_plan(ctx, true);
+}
+
 }  // namespace
 
 extern "C" {
@@ -684,9 +719,13 @@ int rfs_config_swd_modes(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, 
   }
   const int nts[4] = {ntRc, ntRg, ntLc, ntLg};
   const double *ts[4] = {tRc, tRg, tLc, tLg};
+  // the per-set period table belongs to the previous grid (the plan below is built with sharing)
+  ctx->has_set_periods = ctx->plan_unshared = false;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
   int rc = build_plan(ctx, ctx->plan, ctx->periods, nts, ts, mode, true);
   if (rc) return rc;
   if (ctx->plan.ndata == 0) return fail(ctx, RFS_E_ARG, "no periods given");
+  for (int w = 0; w < 4; w++) ctx->swd_nts[w] = nts[w];
   if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * ctx->periods.size()))) return rc;
   CK(cudaMemcpy(ctx->d_periods.p, ctx->periods.data(), sizeof(double) * ctx->periods.size(),
                 cudaMemcpyHostToDevice));
@@ -728,8 +767,10 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
                         const double *dobs, int ndobs) {
   if (!ctx || S < 1 || !sigma1 || !sigma2 || !dobs || ndobs <= 0) return RFS_E_ARG;
   CK(cudaSetDevice(ctx->device));
+  int rc = drop_set_periods(ctx);
+  if (rc) return rc;
   const size_t bytes = sizeof(double) * (size_t)S * ndobs;
-  int rc = ensure(ctx, ctx->d_dobs, bytes);
+  rc = ensure(ctx, ctx->d_dobs, bytes);
   if (rc) return rc;
   CK(cudaMemcpy(ctx->d_dobs.p, dobs, bytes, cudaMemcpyHostToDevice));
   ctx->sigma1.assign(sigma1, sigma1 + S);
@@ -770,6 +811,96 @@ int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p) {
   return RFS_OK;
 }
 
+int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use) {
+  if (!ctx) return RFS_E_ARG;
+  if (!ctx->has_swd)
+    return fail(ctx, RFS_E_CONFIG, "per-set period lists need an SWD configuration (rfs_config_swd)");
+  if (!ctx->has_obs || S != ctx->nsets)
+    return fail(ctx, RFS_E_CONFIG, "period table for " + std::to_string(S) + " sets, the context holds " +
+                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
+  CK(cudaSetDevice(ctx->device));
+  // a failed call leaves no table: the context then evaluates every set on the grid lists
+  int rc = drop_set_periods(ctx);
+  if (rc) return rc;
+  const int ng = ctx->plan.ndata;  // one mode block of the data vector
+  if (nper != ng)
+    return fail(ctx, RFS_E_ARG, "period mask has " + std::to_string(nper) + " entries per set, the SWD " +
+                                    "configuration has " + std::to_string(ng) + " periods");
+  if (!use) return fail(ctx, RFS_E_ARG, "no period mask");
+  std::vector<int> nobs(S, 0);
+  for (int st = 0; st < S; st++) {
+    for (int j = 0; j < ng; j++) {
+      const unsigned char u = use[(size_t)st * ng + j];
+      if (u > 1) return fail(ctx, RFS_E_ARG, "period mask values must be 0 or 1");
+      nobs[st] += u;
+    }
+    if (nobs[st] == 0)
+      return fail(ctx, RFS_E_ARG, "set " + std::to_string(st) + " observes no period (no periods given)");
+  }
+  // the T sequence of Rc may serve Rg only where every set observes the same Rc and Rg periods
+  bool share = true;
+  for (int fam = 0; fam < 2; fam++) {
+    const SwdPlan &P = ctx->plan;
+    int rc_row = -1, rg_row = -1;
+    for (int r = 0; r < P.nrow; r++) {
+      if (P.row[r].type == 2 * fam) rc_row = r;
+      if (P.row[r].type == 2 * fam + 1) rg_row = r;
+    }
+    if (rc_row < 0 || rg_row < 0 || P.row[rc_row].s0 != P.row[rg_row].s0) continue;
+    const SwdRow &a = P.row[rc_row], &g = P.row[rg_row];
+    for (int st = 0; st < S && share; st++)
+      share = memcmp(use + (size_t)st * ng + a.d_off, use + (size_t)st * ng + g.d_off, a.nper) == 0;
+  }
+  // from here on a failure restores the shared plan (drop_set_periods) and leaves no table
+  auto abandon = [&](int code) {
+    ctx->has_set_periods = true;
+    drop_set_periods(ctx);
+    return code;
+  };
+  ctx->plan_unshared = !share;
+  if (!share && (rc = rebuild_grid_plan(ctx, false))) return abandon(rc);
+  const SwdPlan &P = ctx->plan;
+  const int ld = 2 * P.nseq + 2 * ng;
+  std::vector<int> tab((size_t)S * ld, 0);
+  std::vector<double> per = ctx->periods;  // the grid lists, then each set's compact lists
+  for (int st = 0; st < S; st++) {
+    const unsigned char *u = use + (size_t)st * ng;
+    int *t = tab.data() + (size_t)st * ld;
+    for (int r = 0; r < P.nrow; r++) {
+      const SwdRow &rw = P.row[r];
+      const int off = (int)per.size();
+      int nk = 0;
+      for (int g = 0; g < rw.nper; g++)
+        if (u[rw.d_off + g]) {
+          per.push_back(ctx->periods[rw.per_off + g]);
+          t[2 * P.nseq + rw.d_off + nk++] = g;
+        }
+      for (int q : {rw.s0, rw.s1, rw.s2})
+        if (q >= 0) {
+          t[q] = off;
+          t[P.nseq + q] = nk;
+        }
+    }
+    for (int j = 0; j < ng; j++) t[2 * P.nseq + ng + j] = u[j];
+  }
+  if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * per.size())) ||
+      (rc = ensure(ctx, ctx->d_set_per, sizeof(int) * tab.size())))
+    return abandon(rc);
+  // the grid lists stay in front: without the table every kernel reads them as before
+  cudaError_t e = cudaMemcpy(ctx->d_periods.p, per.data(), sizeof(double) * per.size(), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess)
+    e = cudaMemcpy(ctx->d_set_per.p, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) {
+    ctx->err = std::string("rfs_config_obs_periods: ") + cudaGetErrorString(e);
+    return abandon(RFS_E_CUDA);
+  }
+  ctx->set_per_ld = ld;
+  ctx->set_nobs = nobs;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
+  ctx->has_set_periods = true;
+  return RFS_OK;
+}
+
 int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
                              double *U, double *grad, double *dsyn, unsigned char *flag, void *stream) {
   if (!ctx) return RFS_E_ARG;
@@ -804,6 +935,11 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
   const int nch = (int)((B + Bmax - 1) / Bmax);
   const long long Bch = (B + nch - 1) / nch;
   const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata};
+  // each row's own SWD period lists (rfs_config_obs_periods) for the rows of one chunk
+  auto set_view = [&](const int *chunk_set) {
+    return SwdSetView{ctx->has_set_periods ? (const int *)ctx->d_set_per.p : nullptr, chunk_set, ctx->nsets,
+                      ctx->set_per_ld};
+  };
   double tshift = rf.tshift;
   if (rf.rf_type == 2) tshift = -tshift;  // src/RF/main.cpp:35
   const bool rf_time = use_rf && rf.method == 0;
@@ -812,7 +948,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     ctx->wt.resize(ctx->nsets);
     for (int k = 0; k < ctx->nsets; k++) {
       const double q = ctx->sigma1[k] / ctx->sigma2[k];
-      ctx->wt[k] = q * q * n1 / nsw;
+      // with per-set period lists: the data count of set k's own lists, as a one-set context has it
+      const int nsw_k = ctx->has_set_periods ? nmsel * ctx->set_nobs[k] : nsw;
+      ctx->wt[k] = q * q * n1 / nsw_k;
     }
     int rc;
     if ((rc = ensure(ctx, ctx->d_wt, sizeof(double) * ctx->nsets))) return rc;
@@ -856,8 +994,8 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     if (!use_swd) release_rf_branch(F, sk);
     if (use_swd) {
       if ((rc = make_blocks(ctx, F, (const double *)F.w_swd.p, Bc, n, ctx->sphere, blks[k], sk))) return rc;
-      if ((rc = run_swd_roots(ctx, F, ctx->plan, (const double *)ctx->d_periods.p, blks[k], Bc, n, multi_mode,
-                              sk)))
+      if ((rc = run_swd_roots(ctx, F, ctx->plan, set_view(set ? set + off : nullptr),
+                              (const double *)ctx->d_periods.p, blks[k], Bc, n, multi_mode, sk)))
         return rc;
     }
     release_rf_branch(F, sk);
@@ -925,8 +1063,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     }
     if (use_swd) {
       CK(cudaStreamWaitEvent(st, F.ev_ready, 0));
-      if ((rc = run_swd_eigen(ctx, F, ctx->plan, (const double *)ctx->d_periods.p, blks[k], Bc, n, multi_mode,
-                              st)))
+      const SwdSetView sv = set_view(obs_k.set);
+      if ((rc = run_swd_eigen(ctx, F, ctx->plan, sv, (const double *)ctx->d_periods.p, blks[k], Bc, n,
+                              multi_mode, st)))
         return rc;
       SwdView V;
       V.blk = blks[k];
@@ -938,7 +1077,7 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       V.B = Bc;
       V.n = n;
       if (use_rf && ctx->overlap) CK(cudaStreamWaitEvent(st, ctx->ev_join, 0));
-      LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, ctx->plan, V,
+      LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, ctx->plan, V, sv,
              (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, which, n1,
              obs_k, (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p,
              U + off,

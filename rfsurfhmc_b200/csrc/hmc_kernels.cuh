@@ -66,6 +66,11 @@ struct HmcDev {
   // setg [Ba] = rowset gathered for the packed batch (evaluated with the rows' own observations)
   const int *set;
   int *rowset, *setg;
+  // per-set period lists (rfs_config_obs_periods): obs_use + rowset[c] * use_ld is the grid mask of the
+  // slot's set over one SWD mode block (data values use_n1 + k * use_ng + j); the synthetics at the
+  // periods a set does not observe are NaN and are not a failure.  NULL: every value is checked.
+  const int *obs_use;
+  int use_ld, use_n1, use_ng;
   int *n_active;         // [0] slots still running after the last advance, [1] compaction counter
   // compaction of the evaluation batch once slots have run dry: slot[s] = row of slot s in the
   // evaluated batch (-1: finished), idx[j] = slot of row j, xg = gathered positions [Ba][n2]
@@ -342,6 +347,15 @@ RFS_DEVINL bool any_nan(const double *v, int n) {
   return f;
 }
 
+// NaN in the data values slot c's set observes (a failed forward model)
+RFS_DEVINL bool any_nan_obs(const HmcDev &D, long long c, const double *v, int n) {
+  if (!D.obs_use) return any_nan(v, n);
+  const int *u = D.obs_use + (long long)D.rowset[c] * D.use_ld;
+  bool f = false;
+  for (int i = 0; i < n; i++) f = f || (isnan(v[i]) && (i < D.use_n1 || u[(i - D.use_n1) % D.use_ng]));
+  return f;
+}
+
 // One global step of every slot (c = slot, ch = the chain it currently runs; C = number of slots).
 __global__ void hmc_advance_kernel(HmcDev D, HmcCfg cfg, long long C) {
   const long long c = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -370,7 +384,7 @@ __global__ void hmc_advance_kernel(HmcDev D, HmcCfg cfg, long long C) {
     D.Ucur[c] = Ue;
     for (int j = 0; j < n2; j++) gcur[j] = ge[j];
     for (int j = 0; j < nd; j++) dcur[j] = de[j];
-    D.okcur[c] = (fe && !any_nan(de, nd)) ? 1 : 0;
+    D.okcur[c] = (fe && !any_nan_obs(D, c, de, nd)) ? 1 : 0;
     if (cfg.sampler == 1) {
       // ---- _find_initial_dt prologue (hmcda.py:170-184)
       if (!D.okcur[c]) {
@@ -441,7 +455,7 @@ __global__ void hmc_advance_kernel(HmcDev D, HmcCfg cfg, long long C) {
   } else {  // HP_LEAP
     const int L = D.L[c];
     int istep = D.istep[c];
-    if (any_nan(ge, n2) || !fe || any_nan(de, nd)) {
+    if (any_nan(ge, n2) || !fe || any_nan_obs(D, c, de, nd)) {
       traj_end = true;
       failed = true;
     } else if (istep < L - 1) {

@@ -29,9 +29,11 @@ struct ModeSel {
 //   U[B], grad[B][2n] (vs then thk), dsyn[B][ndata] with ndata = nt_rf + nsw (joint),
 //   flag[B] (1 ok, 0 failed SWD root search or observation-set index out of range)
 // Row b is compared with observation set obs.row_set(b); wt[S] is each set's SWD weight
-// (sigma1/sigma2)^2 n1/nsw of the joint objective.
+// (sigma1/sigma2)^2 n1/nsw of the joint objective.  With per-set period lists (sv) slice q contracts the
+// set's compact periods k = q, q + Q, ... (the sums of a one-set context on those lists), dsyn holds
+// them at their grid positions and NaN at the grid positions the set does not observe.
 #define RFS_ASM_Q 4
-__global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__restrict__ ierr,
+__global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, const int *__restrict__ ierr,
                                       const double *__restrict__ chain, int stale, int which,
                                       int nt_rf, ObsSets obs, const double *__restrict__ U_rf,
                                       const double *__restrict__ g_rf, const double *__restrict__ wt,
@@ -66,10 +68,12 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__rest
       Vm.kern = V.kern + mo * plan.nsolve * 4 * nB;
       const int doff = n1 + im * plan.ndata;
       for (int r = 0; r < plan.nrow; r++) {
-        const SwdRow rw = plan.row[r];
+        const int *c2g;
+        const SwdRow rw = sv.row(plan, r, b, &c2g);
         for (int k = q; k < rw.nper; k += RFS_ASM_Q) {
+          const int j = doff + rw.d_off + (c2g ? c2g[k] : k);  // grid position of compact period k
           const double d = swd_row_value(plan, Vm, rw, k, b);
-          const double res = d - dobs[doff + rw.d_off + k];
+          const double res = d - dobs[j];
           double K[4];
           swd_row_kernels(plan, Vm, rw, k, m, b, stale, K);
           const double kv = K[1] + K[0] * dadb + K[2] * drda * dadb;
@@ -77,8 +81,14 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, const int *__rest
           gh += res * K[3];
           if (m == 0) {
             us += res * res;
-            dsyn[b * ndata + doff + rw.d_off + k] = d;
+            dsyn[b * ndata + j] = d;
           }
+        }
+        if (c2g && m == 0) {
+          const int *use = c2g - rw.d_off + plan.ndata;  // the set's grid mask
+          const int ng = plan.row[r].nper;
+          for (int g = q; g < ng; g += RFS_ASM_Q)
+            if (!use[rw.d_off + g]) dsyn[b * ndata + doff + rw.d_off + g] = nan("");
         }
       }
     }

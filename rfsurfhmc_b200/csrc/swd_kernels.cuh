@@ -145,7 +145,7 @@ __global__ void prep_sphere_kernel(const double *__restrict__ flat, long long B,
 
 // sequential stop rule of the retry loop: `if(ierr !=0) return ierr;` leaves the later periods
 // un-retried (zero) and reports failure; otherwise ierr is that of the last retry (0).
-__global__ void swd_retry_finish_kernel(SwdPlan plan, long long B, int all_modes,
+__global__ void swd_retry_finish_kernel(SwdPlan plan, SwdSetView sv, long long B, int all_modes,
                                         double *__restrict__ croot, int *__restrict__ ierr,
                                         const int *__restrict__ rstat) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
@@ -153,7 +153,7 @@ __global__ void swd_retry_finish_kernel(SwdPlan plan, long long B, int all_modes
   const long long b = i % B;
   const int s = (int)(i / B);
   if (ierr[(long long)s * B + b] == 0) return;
-  const SwdSeq sq = plan.seq[s];
+  const SwdSeq sq = sv.seq(plan, s, b);  // only row b's own periods were searched
   double *clast = croot + (all_modes ? (long long)(plan.nmode - 1) * plan.nsolve * B : 0);
   int e = 1;  // ierr stays 1 if nothing was retried (cannot happen: a failed period is zero)
   bool stopped = false;
@@ -178,7 +178,7 @@ __global__ void swd_retry_finish_kernel(SwdPlan plan, long long B, int all_modes
 #endif
 template <int NMAX>
 __global__ void __launch_bounds__(128, RFS_EIGEN_MINBLOCKS)
-    swd_eigen_kernel(SwdPlan plan, SwdBlocks blk, long long B, int n,
+    swd_eigen_kernel(SwdPlan plan, SwdBlocks blk, SwdSetView setv, long long B, int n,
                      const double *__restrict__ periods, int nmode_out,
                      const double *__restrict__ croot, double *__restrict__ ugr,
                      double *__restrict__ kern) {
@@ -192,8 +192,9 @@ __global__ void __launch_bounds__(128, RFS_EIGEN_MINBLOCKS)
   int s = 0;
   for (int q = 0; q < plan.nseq; q++)
     if (solve >= plan.seq[q].out_off && solve < plan.seq[q].out_off + plan.seq[q].nper) s = q;
-  const SwdSeq sq = plan.seq[s];
+  const SwdSeq sq = setv.seq(plan, s, b);
   const int k = solve - sq.out_off;
+  if (k >= sq.nper) return;  // beyond row b's own period list: no root, nothing reads this solve
   const double T = __ldg(periods + sq.per_off + k) * sq.scale;
   const double c = croot[sv * B + b];
   double *kp = kern + sv * 4 * (long long)n * B + b;

@@ -27,4 +27,46 @@ struct SwdPlan {
   SwdRow row[RFS_MAX_ROWS];
 };
 
+// Per-set period lists (rfs_config_obs_periods): observation set s observes a subset of the plan's
+// period grid, and every (model, sequence) job of a row of set s runs set s's compact list.  Results
+// keep the plan's capacity layout: compact period k of sequence q is solve plan.seq[q].out_off + k.
+// tab [nsets][ld] ints, ld = 2 nseq + 2 ndata, per set:
+//   [0, nseq)              per_off of sequence q's compact list in the period table
+//   [nseq, 2 nseq)         its length (0: the set observes none of the sequence's periods)
+//   [2 nseq + d_off + k]   row r's compact period k -> grid position (d_off = plan.row[r].d_off)
+//   [2 nseq + ndata + j]   grid position j of the data vector observed (1) or not (0)
+// tab == NULL, or a row whose set index lies outside [0, nsets): the plan's own lists (such a row is
+// failed by the residual kernels).  One code path for both is what makes an all-ones table give the
+// bits of no table.
+struct SwdSetView {
+  const int *tab;
+  const int *set;  // [B] set index of each row of the launch, or NULL (set 0)
+  int nsets, ld;
+  RFS_DEVINL const int *of(long long b) const {
+    if (!tab) return nullptr;
+    const int s = set ? set[b] : 0;
+    return (s >= 0 && s < nsets) ? tab + (long long)s * ld : nullptr;
+  }
+  // sequence q of row b's job
+  RFS_DEVINL SwdSeq seq(const SwdPlan &P, int q, long long b) const {
+    SwdSeq sq = P.seq[q];
+    if (const int *t = of(b)) {
+      sq.per_off = t[q];
+      sq.nper = t[P.nseq + q];
+    }
+    return sq;
+  }
+  // data row r of row b: its compact length and period offset; *c2g = compact -> grid map (NULL: identity)
+  RFS_DEVINL SwdRow row(const SwdPlan &P, int r, long long b, const int **c2g) const {
+    SwdRow rw = P.row[r];
+    *c2g = nullptr;
+    if (const int *t = of(b)) {
+      rw.per_off = t[rw.s0];
+      rw.nper = t[P.nseq + rw.s0];
+      *c2g = t + 2 * P.nseq + rw.d_off;
+    }
+    return rw;
+  }
+};
+
 }  // namespace rfs

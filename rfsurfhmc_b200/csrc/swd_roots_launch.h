@@ -19,23 +19,24 @@ namespace rfs {
 
 // one thread per (model, sequence); perm != NULL: jobs taken in the length-sorted order of
 // launch_sched_sort (nsm = SMs of the device, for the block-to-SM composition)
-cudaError_t launch_roots_thread(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_roots_thread(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                                 const double *periods, int all_modes, double *croot, double *cwork,
                                 int *ierr, unsigned long long *counter, const int *perm, int nsm,
                                 cudaStream_t st);
 // length-sorted job order: key[nseq*B] = predicted scan length of every job (bisection estimate of
 // c at the longest period); perm[nseq*B] = job ids, longest first, Rayleigh before Love
-cudaError_t launch_sched_keys(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_sched_keys(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                               const double *periods, unsigned int *key, cudaStream_t st);
 cudaError_t launch_sched_sort(const SwdPlan &P, long long B, const unsigned int *key, int *perm,
                               cudaStream_t st);
 // T lanes per (model, sequence), S speculative scan points; false if (T,S) is not instantiated
 bool team_shape_supported(int T, int S);
-cudaError_t launch_roots_team(int T, int S, const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_roots_team(int T, int S, const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                               const double *periods, int all_modes, double *croot, double *cwork,
                               int *ierr, unsigned long long *counter, cudaStream_t st);
 // per-period retries of failed fundamental-mode searches (surfdisp.cpp:93-100)
-cudaError_t launch_roots_retry(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+// sv: every launcher runs each row's job on that row's own period list (SwdSetView)
+cudaError_t launch_roots_retry(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                                const double *periods, int all_modes, double *croot, double *cwork,
                                const int *ierr, int *rstat, unsigned long long *counter,
                                cudaStream_t st);

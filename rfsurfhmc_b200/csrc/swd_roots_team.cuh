@@ -205,7 +205,7 @@ RFS_DEVINL int swd_solve_team(const SmemModel &M, long long b, const SwdSeq &sq,
 //                        + (blockDim.x / 32) * RFS_TEAM_NP * 32 double2 (parked layer terms)
 template <int T, int S>
 __global__ void __launch_bounds__(128)
-    swd_roots_team_kernel(SwdPlan plan, SwdBlocks blk, long long B, int n,
+    swd_roots_team_kernel(SwdPlan plan, SwdBlocks blk, SwdSetView sv, long long B, int n,
                           const double *__restrict__ periods, int all_modes,
                           double *__restrict__ croot, double *__restrict__ cwork,
                           int *__restrict__ ierr, unsigned long long *__restrict__ neval_total) {
@@ -216,10 +216,11 @@ __global__ void __launch_bounds__(128)
   const bool valid = job < B * plan.nseq;
   const long long b = valid ? job % B : 0;
   const int s = valid ? (int)(job / B) : 0;
+  const SwdSeq sq = sv.seq(plan, s, b);  // row b's own period list
   // ---- stage the layer parameters of this team's model
   double *lp = team_sm + (size_t)team * RFS_TEAM_NF * n;
   {
-    const double *src = blk.root[plan.seq[s].ifunc == 2 ? 0 : 1];
+    const double *src = blk.root[sq.ifunc == 2 ? 0 : 1];
     const long long nB = (long long)n * B;
     for (int idx = tl; idx < RFS_TEAM_NF * n; idx += T) {
       const int f = idx / n, m = idx - f * n;
@@ -236,7 +237,7 @@ __global__ void __launch_bounds__(128)
                 (size_t)(threadIdx.x >> 5) * RFS_TEAM_NP * 32;
   SmemModel M{lp, n};
   unsigned int nev = 0;
-  const int e = swd_solve_team<T, S>(M, b, plan.seq[s], periods, plan.nmode, all_modes, croot,
+  const int e = swd_solve_team<T, S>(M, b, sq, periods, plan.nmode, all_modes, croot,
                                      (long long)plan.nsolve * B, cwork, B, nev, tmask, tl, -1, cm, lane);
   if (tl == 0) {
     ierr[(long long)s * B + b] = e;

@@ -19,7 +19,7 @@ namespace rfs {
 // (one LDS with an immediate offset per value instead of index arithmetic + a global load).
 template <bool STAGED>
 __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
-    swd_roots_kernel(SwdPlan plan, SwdBlocks blk, long long B, int n,
+    swd_roots_kernel(SwdPlan plan, SwdBlocks blk, SwdSetView sv, long long B, int n,
                      const double *__restrict__ periods, int all_modes,
                      double *__restrict__ croot, double *__restrict__ cwork,
                      int *__restrict__ ierr, unsigned long long *__restrict__ neval_total,
@@ -43,7 +43,8 @@ __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
   }
   const long long b = valid ? i % B : 0;
   const int s = valid ? (int)(i / B) : 0;
-  SwdModel M(blk.root[plan.seq[s].ifunc == 2 ? 0 : 1], B, n);
+  const SwdSeq sq = sv.seq(plan, s, b);  // row b's own period list
+  SwdModel M(blk.root[sq.ifunc == 2 ? 0 : 1], B, n);
   unsigned int nev = 0;
   int e;
   if (STAGED) {
@@ -53,11 +54,11 @@ __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
         stage[(m * RFS_ROOT_NF + f) * RFS_ROOTS_BLOCK + threadIdx.x] = M.ld(f, m, b);
     __syncwarp();  // a lane only ever reads columns of its own warp (its own, or the lane it helps)
     SmemColModel<RFS_ROOTS_BLOCK> Ms{stage, n};
-    e = swd_solve_sequence(Ms, b, (long long)threadIdx.x, plan.seq[s], periods, plan.nmode, all_modes,
+    e = swd_solve_sequence(Ms, b, (long long)threadIdx.x, sq, periods, plan.nmode, all_modes,
                            croot, (long long)plan.nsolve * B, cwork, B, nev, valid,
                            wsm_all[threadIdx.x >> 5], -1);
   } else {
-    e = swd_solve_sequence(M, b, b, plan.seq[s], periods, plan.nmode, all_modes, croot,
+    e = swd_solve_sequence(M, b, b, sq, periods, plan.nmode, all_modes, croot,
                            (long long)plan.nsolve * B, cwork, B, nev, valid,
                            wsm_all[threadIdx.x >> 5], -1);
   }
@@ -86,12 +87,12 @@ __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
 #define RFS_SCHED_BISECT 6
 #define RFS_SCHED_BINS 1024
 __global__ void __launch_bounds__(128)
-    swd_sched_key_kernel(SwdPlan plan, SwdBlocks blk, long long B, int n,
+    swd_sched_key_kernel(SwdPlan plan, SwdBlocks blk, SwdSetView sv, long long B, int n,
                          const double *__restrict__ periods, unsigned int *__restrict__ key) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= B * plan.nseq) return;
   const long long b = i % B;
-  const SwdSeq sq = plan.seq[(int)(i / B)];
+  const SwdSeq sq = sv.seq(plan, (int)(i / B), b);
   SwdModel M(blk.root[sq.ifunc == 2 ? 0 : 1], B, n);
   int llw;
   float betmx, cc1;
@@ -193,7 +194,7 @@ __global__ void __launch_bounds__(RFS_SCHED_BINS)
 // swd_retry_finish_kernel re-imposes the sequential stop rule.
 //   rstat [nsolve][B] int: -1 not retried, 0 retried ok, 1 retried and failed again
 __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
-    swd_retry_kernel(SwdPlan plan, SwdBlocks blk, long long B, int n,
+    swd_retry_kernel(SwdPlan plan, SwdBlocks blk, SwdSetView sv, long long B, int n,
                      const double *__restrict__ periods, int all_modes,
                      double *__restrict__ croot, double *__restrict__ cwork,
                      const int *__restrict__ ierr, int *__restrict__ rstat,
@@ -207,8 +208,10 @@ __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
   for (int q = 0; q < plan.nseq; q++)
     if (solve >= plan.seq[q].out_off && solve < plan.seq[q].out_off + plan.seq[q].nper) s = q;
   const int k = solve - plan.seq[s].out_off;
+  const SwdSeq sq = sv.seq(plan, s, b);
   bool valid = false;
-  if (inrange && ierr[(long long)s * B + b] != 0) {
+  // a solve beyond row b's own list (k >= sq.nper) was never written by the search
+  if (inrange && k < sq.nper && ierr[(long long)s * B + b] != 0) {
     const double *clast = croot + (all_modes ? (long long)(plan.nmode - 1) * plan.nsolve * B : 0);
     const double v = clast[(long long)solve * B + b];
     valid = (v == 0.0 || isnan(v));
@@ -218,9 +221,9 @@ __global__ void __launch_bounds__(RFS_ROOTS_BLOCK, RFS_ROOTS_MINBLOCKS)
     if (inrange) rstat[(long long)solve * B + b] = -1;
     return;
   }
-  SwdModel M(blk.root[plan.seq[s].ifunc == 2 ? 0 : 1], B, n);
+  SwdModel M(blk.root[sq.ifunc == 2 ? 0 : 1], B, n);
   unsigned int nev = 0;
-  const int e = swd_solve_sequence(M, b, b, plan.seq[s], periods, plan.nmode, all_modes, croot,
+  const int e = swd_solve_sequence(M, b, b, sq, periods, plan.nmode, all_modes, croot,
                                    (long long)plan.nsolve * B, cwork, B, nev, valid,
                                    wsm_all[threadIdx.x >> 5], k);
   if (inrange) rstat[(long long)solve * B + b] = valid ? e : -1;
@@ -236,7 +239,7 @@ static inline unsigned grid_for(long long total, int block) {
   return (unsigned)((total + block - 1) / block);
 }
 
-cudaError_t launch_roots_thread(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_roots_thread(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                                 const double *periods, int all_modes, double *croot, double *cwork,
                                 int *ierr, unsigned long long *counter, const int *perm, int nsm,
                                 cudaStream_t st) {
@@ -248,17 +251,17 @@ cudaError_t launch_roots_thread(const SwdPlan &P, const SwdBlocks &blk, long lon
       if (e != cudaSuccess) return e;
     }
     swd_roots_kernel<true><<<grid_for(B * P.nseq, RFS_ROOTS_BLOCK), RFS_ROOTS_BLOCK, sm, st>>>(
-        P, blk, B, n, periods, all_modes, croot, cwork, ierr, counter, perm, nsm);
+        P, blk, sv, B, n, periods, all_modes, croot, cwork, ierr, counter, perm, nsm);
   } else {
     swd_roots_kernel<false><<<grid_for(B * P.nseq, RFS_ROOTS_BLOCK), RFS_ROOTS_BLOCK, 0, st>>>(
-        P, blk, B, n, periods, all_modes, croot, cwork, ierr, counter, perm, nsm);
+        P, blk, sv, B, n, periods, all_modes, croot, cwork, ierr, counter, perm, nsm);
   }
   return cudaGetLastError();
 }
 
-cudaError_t launch_sched_keys(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_sched_keys(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                               const double *periods, unsigned int *key, cudaStream_t st) {
-  swd_sched_key_kernel<<<grid_for(B * P.nseq, 128), 128, 0, st>>>(P, blk, B, n, periods, key);
+  swd_sched_key_kernel<<<grid_for(B * P.nseq, 128), 128, 0, st>>>(P, blk, sv, B, n, periods, key);
   return cudaGetLastError();
 }
 
@@ -268,12 +271,12 @@ cudaError_t launch_sched_sort(const SwdPlan &P, long long B, const unsigned int 
   return cudaGetLastError();
 }
 
-cudaError_t launch_roots_retry(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_roots_retry(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                                const double *periods, int all_modes, double *croot, double *cwork,
                                const int *ierr, int *rstat, unsigned long long *counter,
                                cudaStream_t st) {
   swd_retry_kernel<<<grid_for(B * P.nsolve, RFS_ROOTS_BLOCK), RFS_ROOTS_BLOCK, 0, st>>>(
-      P, blk, B, n, periods, all_modes, croot, cwork, ierr, rstat, counter);
+      P, blk, sv, B, n, periods, all_modes, croot, cwork, ierr, rstat, counter);
   return cudaGetLastError();
 }
 
@@ -286,7 +289,7 @@ bool team_shape_supported(int T, int S) {
 }
 
 template <int T, int S>
-static cudaError_t launch_team(const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+static cudaError_t launch_team(const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                                const double *periods, int all_modes, double *croot, double *cwork,
                                int *ierr, unsigned long long *counter, cudaStream_t st) {
   // threads per block: as many teams as fit ~64 KB of staged layer parameters
@@ -301,15 +304,15 @@ static cudaError_t launch_team(const SwdPlan &P, const SwdBlocks &blk, long long
     if (e != cudaSuccess) return e;
   }
   swd_roots_team_kernel<T, S><<<grid_for(B * P.nseq, threads / T), threads, sm, st>>>(
-      P, blk, B, n, periods, all_modes, croot, cwork, ierr, counter);
+      P, blk, sv, B, n, periods, all_modes, croot, cwork, ierr, counter);
   return cudaGetLastError();
 }
 
-cudaError_t launch_roots_team(int T, int S, const SwdPlan &P, const SwdBlocks &blk, long long B, int n,
+cudaError_t launch_roots_team(int T, int S, const SwdPlan &P, const SwdBlocks &blk, const SwdSetView &sv, long long B, int n,
                               const double *periods, int all_modes, double *croot, double *cwork,
                               int *ierr, unsigned long long *counter, cudaStream_t st) {
 #define RFS_TEAM(TT, SS) \
-  if (T == TT && S == SS) return launch_team<TT, SS>(P, blk, B, n, periods, all_modes, croot, cwork, ierr, counter, st);
+  if (T == TT && S == SS) return launch_team<TT, SS>(P, blk, sv, B, n, periods, all_modes, croot, cwork, ierr, counter, st);
   RFS_TEAM(2, 2) RFS_TEAM(4, 1) RFS_TEAM(4, 4) RFS_TEAM(8, 1) RFS_TEAM(8, 2) RFS_TEAM(8, 8) RFS_TEAM(16, 1)
   RFS_TEAM(16, 2)
   RFS_TEAM(32, 1) RFS_TEAM(32, 2) RFS_TEAM(32, 4)

@@ -1,23 +1,29 @@
 """StationArray — many stations (observation sets) that share one forward configuration.
 
 A station array is inverted station by station: each station has its own data vector (receiver
-function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s), while
-the layer count, period lists, modes and RF sampling are shared.  The reference runs one job per
-station; here one context holds every station's observations and each evaluated row, or each HMC chain,
-names its station, so one device run fills the GPU with all of them (include/rfsurfhmc.h:
-rfs_config_obs_sets, rfs_config_obs_rays).
+function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s) and
+its own subset of the dispersion periods, while the layer count, the period grid, modes and RF sampling
+are shared.  The reference runs one job per station; here one context holds every station's
+observations and each evaluated row, or each HMC chain, names its station, so one device run fills the
+GPU with all of them (include/rfsurfhmc.h: rfs_config_obs_sets, rfs_config_obs_rays,
+rfs_config_obs_periods).
 
     stations = StationArray(joint_model, dobs, ray_p=p)   # dobs [S, ndata], p [S] or [S, nray]
     HamitonianMC(stations, bounds, ...).sample_chains(ids, stations=station_of_each_chain)
 
+With swd_use [S, nper] the template's four period lists are a common grid (nper = len(tRc) + len(tRg) +
+len(tLc) + len(tLg)) and station s observes the grid periods where swd_use[s] is true: dobs keeps the grid
+layout (its values at unobserved periods are ignored), synthetics are NaN there.
+
 A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
-keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2] and ray_p [S] or [S, nray].
+keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray] and swd_use [S, nper].
 """
 import copy
 import numpy as np
 from .._lib import Context
 from .model_rf_swd_vs_thk import Joint_RF_SWD
 from .model_rf import ReceiverFunc
+from .model_surf import SurfWD
 
 
 def _fresh_copy(m):
@@ -29,13 +35,15 @@ def _fresh_copy(m):
 
 
 class StationArray:
-    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None):
+    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None, swd_use=None):
         """model: a configured Joint_RF_SWD, ReceiverFunc or SurfWD; only its forward configuration is
         used (its own observations are ignored).  dobs [S, ndata] in the model's data layout.
         sigma1 / sigma2: scalars or [S] (default: the joint model's own, 1.0 for the others; they only
         weight the joint objective).  names [S]: output sub-directories (default station0000, ...).
         ray_p: None (every station uses the template's ray parameter(s)) or each station's own, [S] or
-        [S, nray] with the template's ray count; not for a SurfWD template."""
+        [S, nray] with the template's ray count; not for a SurfWD template.
+        swd_use: None (every station observes every period) or [S, nper] bool / 0-1, the grid periods
+        each station observes; for a Joint_RF_SWD or SurfWD template."""
         if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
             raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
         self.template = model
@@ -62,6 +70,12 @@ class StationArray:
             if not isinstance(rf, ReceiverFunc):
                 raise TypeError("ray_p needs a receiver-function template (Joint_RF_SWD or ReceiverFunc)")
             self.ray_p = station_rays(ray_p, S, rf.nray)
+        self.swd_use = None
+        if swd_use is not None:
+            swd = model.swdmodel if isinstance(model, Joint_RF_SWD) else model
+            if not isinstance(swd, SurfWD):
+                raise TypeError("swd_use needs a dispersion template (Joint_RF_SWD or SurfWD)")
+            self.swd_use = station_periods(swd_use, S, swd)
         self._ctx = None
         self._ctx_key = None
 
@@ -76,12 +90,15 @@ class StationArray:
             self._ctx = Context(self._device)
             self._ctx_key = None
         key = (type(self.template), self.template._config_fields(n), self.sigma1.tobytes(),
-               self.sigma2.tobytes(), self.dobs.tobytes(), None if self.ray_p is None else self.ray_p.tobytes())
+               self.sigma2.tobytes(), self.dobs.tobytes(), None if self.ray_p is None else self.ray_p.tobytes(),
+               None if self.swd_use is None else self.swd_use.tobytes())
         if self._ctx_key != key:
             self.template._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
             if self.ray_p is not None:
                 self._ctx.config_obs_rays(self.ray_p)
+            if self.swd_use is not None:
+                self._ctx.config_obs_periods(self.swd_use)
             self._ctx_key = key
         return self._ctx
 
@@ -93,7 +110,8 @@ class StationArray:
 
     def station_model(self, s):
         """Single-station copy of the template holding station s's observations (and sigmas, and ray
-        parameter(s): a scalar for one ray, a list otherwise)."""
+        parameter(s): a scalar for one ray, a list otherwise).  With swd_use its SurfWD holds the
+        station's subset period lists and its dispersion data only the observed values."""
         s = int(s)
         if not 0 <= s < self.nstations:
             raise IndexError(f"station {s} outside [0, {self.nstations})")
@@ -101,14 +119,47 @@ class StationArray:
         t = self.template
         if isinstance(t, Joint_RF_SWD):
             rf = self._station_rf(t.rfmodel, s)
-            m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), rf, _fresh_copy(t.swdmodel))
+            m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), rf, self._station_swd(t.swdmodel, s))
             m._device = t._device
             nt = t.rfmodel.nt
-            m.set_obsdata(d[:nt], d[nt:])
+            m.set_obsdata(d[:nt], self._compact(d[nt:], s))
             return m
-        m = self._station_rf(t, s) if isinstance(t, ReceiverFunc) else _fresh_copy(t)
+        if isinstance(t, ReceiverFunc):
+            m = self._station_rf(t, s)
+        else:
+            m = self._station_swd(t, s)
+            d = self._compact(d, s)
         m.set_obsdata(d)
         return m
+
+    def station_view(self, s):
+        """Station s in the array's own data layout: .dobs [ndata] and .misfit_and_grad(x) through the
+        grouped context (dsyn NaN at the periods the station does not observe)."""
+        return _StationView(self, int(s))
+
+    def _compact(self, dswd, s):
+        if self.swd_use is None:
+            return dswd
+        nmode = dswd.size // self.swd_use.shape[1]
+        return dswd[np.tile(self.swd_use[s], nmode)]
+
+    def _station_swd(self, swd, s):
+        c = _fresh_copy(swd)
+        if self.swd_use is None:
+            return c
+        u = self.swd_use[s]
+        o = 0
+        nt = 0
+        for w in ("Rc", "Rg", "Lc", "Lg"):
+            k = getattr(swd, "nt" + w)
+            if k:
+                t = np.asarray(getattr(swd, "t" + w))[u[o:o + k]]
+                setattr(c, "t" + w, t if t.size else None)
+                setattr(c, "nt" + w, int(t.size))
+                nt += t.size
+                o += k
+        c.nt = nt * swd.nmode
+        return c
 
     def _station_rf(self, rf, s):
         c = _fresh_copy(rf)
@@ -116,6 +167,42 @@ class StationArray:
             r = self.ray_p[s]
             c.ray_p = float(r[0]) if r.size == 1 else r.tolist()
         return c
+
+
+class _StationView:
+    def __init__(self, array, s):
+        self._array, self._s = array, s
+        self.dobs = array.dobs[s]
+
+    def misfit_and_grad(self, x):
+        U, g, d, f = self._array.misfit_and_grad_batch(np.asarray(x, dtype=np.float64)[None, :], [self._s])
+        return U[0], g[0], d[0], bool(f[0])
+
+
+def station_periods(use, S, swd, where=""):
+    """swd_use [S, nper] (bool or 0/1) of a SurfWD template's period grid -> bool [S, nper]; the
+    ValueError names the key 'swd_use' (after `where`)."""
+    nper = swd.ntRc + swd.ntRg + swd.ntLc + swd.ntLg
+    u = np.asarray(use)
+    if u.shape != (S, nper):
+        raise ValueError(f"{where}'swd_use' must have shape [{S}, {nper}], got {u.shape}")
+    if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
+        raise ValueError(f"{where}'swd_use' must hold booleans or 0/1")
+    u = np.ascontiguousarray(u, dtype=bool)
+    empty = np.flatnonzero(~u.any(axis=1))
+    if empty.size:
+        raise ValueError(f"{where}'swd_use': station {int(empty[0])} observes no period")
+    # SurfWD evaluates Love waves on tRc (model_surf.py _grad_periods): a station whose Lc / Lg periods
+    # differ from its Rc periods has no single-station SurfWD
+    rc = u[:, :swd.ntRc]
+    o = swd.ntRc + swd.ntRg
+    for w, k in (("Lc", swd.ntLc), ("Lg", swd.ntLg)):
+        if k and not np.array_equal(u[:, o:o + k], rc):
+            bad = int(np.flatnonzero(np.any(u[:, o:o + k] != rc, axis=1))[0])
+            raise ValueError(f"{where}'swd_use': station {bad} observes other {w} than Rc periods; SurfWD "
+                             f"evaluates Love waves on tRc, so the {w} mask must equal the Rc mask")
+        o += k
+    return u
 
 
 def station_rays(ray_p, S, nray, where=""):
@@ -130,11 +217,12 @@ def station_rays(ray_p, S, nray, where=""):
     return np.ascontiguousarray(r.reshape(S, nray))
 
 
-def load_stations(src, ndata, nparam, default_bounds, nray=1):
+def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None):
     """Validated content of a stations file (.npz path or a mapping with the same keys):
     dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0), bounds [S, nparam, 2]
-    (default: default_bounds [nparam, 2] for every station) and ray_p [S] or [S, nray] (default None: the
-    ray parameter(s) of the forward configuration).  Raises ValueError naming the bad key."""
+    (default: default_bounds [nparam, 2] for every station), ray_p [S] or [S, nray] (default None: the
+    ray parameter(s) of the forward configuration) and swd_use [S, nper] (default None: every period;
+    swd = the SurfWD whose period grid it marks).  Raises ValueError naming the bad key."""
     if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
         with np.load(src, allow_pickle=False) as f:
             src = {k: f[k] for k in f.files}
@@ -168,4 +256,9 @@ def load_stations(src, ndata, nparam, default_bounds, nray=1):
         b = np.broadcast_to(np.asarray(default_bounds, dtype=np.float64), (S, nparam, 2)).copy()
     out["bounds"] = b
     out["ray_p"] = station_rays(src["ray_p"], S, nray, "stations file: ") if "ray_p" in src else None
+    out["swd_use"] = None
+    if "swd_use" in src:
+        if swd is None:
+            raise ValueError("stations file: 'swd_use' needs a dispersion configuration")
+        out["swd_use"] = station_periods(src["swd_use"], S, swd, "stations file: ")
     return out

@@ -53,7 +53,8 @@ def save_chains(model, out, chain_ids, stations, outdir, name, nbest, nsamples):
             continue
         s = int(stations[i])
         if s not in single:
-            single[s] = model.station_model(s)
+            # with per-station periods the file keeps the array's grid layout, as the chain's syn rows do
+            single[s] = model.station_model(s) if model.swd_use is None else model.station_view(s)
         save_chain(f"{outdir}/{model.names[s]}/{name}.{int(cid)}.npz", single[s], out, i, nbest, nsamples)
 
 

@@ -19,7 +19,16 @@ Leg "rays" (per-station ray parameters, rfs_config_obs_rays), every station with
       batch in the same two chunks;
   (f) HMC, 16 stations x 64 chains, distinct ray parameters: one grouped run vs 16 single-station runs,
       each in a context configured with its station's ray parameter.
---legs sets,rays selects the legs; the legs run replace their keys in --out and keep the others.
+Leg "periods" (per-station SWD period lists, rfs_config_obs_periods), every station observing a seeded
+random contiguous window of 60-100 % of each of the lists tRc and tRg (chosen independently):
+  (g) F1 joint, (S, K) = (256, 64), (1024, 16): the grouped call with the mask vs the same grouped call
+      on the full grid (two contexts, timed alternately, --inner calls per timing) vs one context
+      reconfigured for each station in turn (config_swd on its subset lists, config_obs, its K rows);
+  (h) SWD only, n = 40, modes 0-2, 24 Rc and 18 Rg periods, 64 stations x 64 models: the same three;
+  (i) HMC, 16 stations x 64 chains: one grouped run with the mask vs 16 single-station runs, each in a
+      context configured on its station's subset lists.
+--legs sets,rays,periods selects the legs (default sets,rays); the legs run replace their keys in --out
+and keep the others.
 Every shape is warmed up first; each timing is repeated --reps times (median, min, max reported), with a
 host clock around work that ends in a device synchronise.  Station observations are the forward model
 of seeded perturbations of the F1 true model plus seeded noise.  Prints one JSON line and writes it to
@@ -109,6 +118,8 @@ def main():
             res = json.loads(f.read())
     if "rays" in legs:
         res["rays"] = rays_leg(a, torch, station_obs, X, nd)
+    if "periods" in legs:
+        res["periods"] = periods_leg(a, torch, X)
     if "sets" not in legs:
         c.close()
         return write(a, res)
@@ -281,6 +292,167 @@ def rays_leg(a, torch, station_obs, X, nd):
     hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
     out["hmc"] = hmc
     grouped[1].close()
+    for c in single:
+        c.close()
+    return out
+
+
+def periods_leg(a, torch, X):
+    """Per-station period lists against the full grid and against one context per station (see the
+    module docstring)."""
+    from rfsurfhmc_b200._lib import Context
+    from rfsurfhmc_b200.fixtures import f1_config, f1_true_model, driver_bounds, perturbed_models
+    cfg, x0 = f1_config(), f1_true_model()
+    dev = torch.device("cuda", 0)
+    st = torch.cuda.current_stream(dev)
+    out = {**gpu_info(), "inner_calls": a.inner, "mask": "contiguous window of 60-100 % of each list", "eval": []}
+    rng = np.random.default_rng(23)
+
+    def masks(S, lists):
+        rows = []
+        for _ in range(S):
+            parts = []
+            for t in lists:
+                k = int(rng.integers(int(np.ceil(0.6 * len(t))), len(t) + 1))
+                o = int(rng.integers(0, len(t) - k + 1))
+                m = np.zeros(len(t), dtype=bool)
+                m[o:o + k] = True
+                parts.append(m)
+            rows.append(np.concatenate(parts))
+        return np.array(rows)
+
+    def configure(c, which, n, lists, modes):
+        if which != 1:
+            c.config_swd(n, *lists, mode=modes)
+        if which != 2:
+            c.config_rf(n, cfg["ray_p"], cfg["nt"], cfg["dt"], cfg["gauss"], cfg["time_shift"], cfg["water"],
+                        cfg["rf_type"], cfg["method"])
+
+    def subset(lists, u):
+        r, o = [], 0
+        for t in lists:
+            r.append(np.asarray(t)[u[o:o + len(t)]])
+            o += len(t)
+        return r
+
+    def observations(which, n, lists, modes, x_true, S, seed):
+        c = Context(0)
+        configure(c, which, n, lists, modes)
+        c.config_obs(np.zeros((S, c.ndata(which))))
+        _, _, d, _ = c.misfit_grad_host(perturbed_models(x_true, S, seed=seed, rel=0.05), which, sets=np.arange(S))
+        c.close()
+        d = np.where(np.isfinite(d), d, 0.0)
+        return d + 0.01 * np.random.default_rng(seed).standard_normal(d.shape)
+
+    def compare(which, n, lists, modes, Xd, S, K, dobs, use):
+        nt = cfg["nt"] if which == 0 else 0
+        nm = int(np.size(modes))
+        B = Xd.shape[0]
+        sets = torch.from_numpy(np.repeat(np.arange(S, dtype=np.int32), K)).to(dev)
+        cs = []
+        for with_mask in (True, False):
+            c = Context(0)
+            configure(c, which, n, lists, modes)
+            c.config_obs(dobs)
+            if with_mask:
+                c.config_obs_periods(use)
+            cs.append(c)
+        U = torch.empty(B, dtype=torch.float64, device=dev)
+        G = torch.empty(Xd.shape, dtype=torch.float64, device=dev)
+        D = torch.empty(B, cs[0].ndata(which), dtype=torch.float64, device=dev)
+        F = torch.empty(B, dtype=torch.uint8, device=dev)
+
+        def call(c):
+            for _ in range(a.inner):
+                c.misfit_grad_dev(B, Xd.data_ptr(), which, U.data_ptr(), G.data_ptr(), D.data_ptr(), F.data_ptr(),
+                                  st.cuda_stream, sets_ptr=sets.data_ptr())
+        ts = ([], [])
+        for c in cs:
+            call(c)
+        torch.cuda.synchronize()
+        for _ in range(a.reps):
+            for k, c in enumerate(cs):
+                t0 = time.perf_counter()
+                call(c)
+                torch.cuda.synchronize()
+                ts[k].append((time.perf_counter() - t0) / a.inner)
+        for c in cs:
+            c.close()
+        # what a user does without the table: one context, reconfigured for each station in turn
+        one = Context(0)
+        configure(one, which, n, lists, modes)
+        compact = [np.concatenate([dobs[s, :nt], dobs[s, nt:][np.tile(use[s], nm)]]) for s in range(S)]
+        subs = [subset(lists, use[s]) for s in range(S)]
+
+        def per_station():
+            for s in range(S):
+                one.config_swd(n, *subs[s], mode=modes)
+                one.config_obs(compact[s])
+                one.misfit_grad_dev(K, Xd[s * K].data_ptr(), which, U[s * K].data_ptr(), G[s * K].data_ptr(),
+                                    D[s * K].data_ptr(), F[s * K].data_ptr(), st.cuda_stream)
+        per_station()
+        torch.cuda.synchronize()
+        tp = []
+        for _ in range(a.reps):
+            t0 = time.perf_counter()
+            per_station()
+            torch.cuda.synchronize()
+            tp.append(time.perf_counter() - t0)
+        one.close()
+        masked, grid, seq = spread(ts[0]), spread(ts[1]), spread(tp)
+        return {"masked": masked, "full_grid": grid, "per_station": seq,
+                "observed_share": float(use.mean()),
+                "masked_over_full_grid": masked["median_ms"] / grid["median_ms"],
+                "speedup_per_station_over_masked": seq["median_ms"] / masked["median_ms"]}
+
+    n = x0.size // 2
+    f1 = (cfg["tRc"], cfg["tRg"], [], [])
+    for S, K in ((256, 64), (1024, 16)):
+        dobs = observations(0, n, f1, 0, x0, S, 100 + S)
+        use = masks(S, f1[:2])
+        out["eval"].append({"workload": "F1 joint, %d stations x %d models" % (S, K), "S": S, "K": K,
+                            **compare(0, n, f1, 0, X[:S * K], S, K, dobs, use)})
+    # SWD only, n = 40, modes 0-2
+    n40, S, K = 40, 64, 64
+    lists = (np.geomspace(2, 100, 24), np.geomspace(3, 80, 18), [], [])
+    i = np.arange(n40)
+    x40 = np.hstack((2.0 + 2.7 * (i / (n40 - 1.0)) ** 0.7, np.hstack((0.5 + 0.1 * i[:-1], [0.0]))))
+    X40 = torch.from_numpy(perturbed_models(x40, S * K, seed=31, rel=0.05)).to(dev)
+    dobs = observations(2, n40, lists, [0, 1, 2], x40, S, 41)
+    out["n40"] = {"workload": "SWD only, n=40, modes 0-2, 24 Rc + 18 Rg periods, %d stations x %d models" % (S, K),
+                  "S": S, "K": K, **compare(2, n40, lists, [0, 1, 2], X40, S, K, dobs, masks(S, lists[:2]))}
+    # HMC, 16 stations x 64 chains
+    Sh, Kh = 16, 64
+    dobs = observations(0, n, f1, 0, x0, Sh, 7)
+    use = masks(Sh, f1[:2])
+    bounds = driver_bounds(x0)
+    kw = dict(dt=0.1, Lrange=(5, 20), seed=991206, nsamples=a.hmc_iters + 1, ndraws=0, max_iters=a.hmc_iters,
+              want_samples=False)
+    grouped = Context(0)
+    configure(grouped, 0, n, f1, 0)
+    grouped.config_obs(dobs)
+    grouped.config_obs_periods(use)
+    single = []
+    for s in range(Sh):
+        c = Context(0)
+        configure(c, 0, n, subset(f1, use[s]), 0)
+        c.config_obs(np.concatenate([dobs[s, :cfg["nt"]], dobs[s, cfg["nt"]:][use[s]]]))
+        single.append(c)
+    ids, hsets = np.tile(np.arange(Kh), Sh), np.repeat(np.arange(Sh), Kh)
+    runs = {"grouped": lambda: grouped.hmc_run(0, ids, bounds, sets=hsets, **kw)["evals"],
+            "per_station": lambda: sum(single[s].hmc_run(0, np.arange(Kh), bounds, **kw)["evals"] for s in range(Sh))}
+    hmc = {"S": Sh, "K": Kh, "max_iters": a.hmc_iters}
+    for name, fn in runs.items():
+        fn()
+        ts, evs = [], 0
+        for _ in range(max(1, a.reps // 2)):
+            t0 = time.perf_counter()
+            evs = fn()
+            ts.append(time.perf_counter() - t0)
+        hmc[name] = {**spread(ts), "evals": int(evs), "evals_per_s": float(evs / np.median(ts))}
+    hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
+    out["hmc"] = hmc
+    grouped.close()
     for c in single:
         c.close()
     return out
