@@ -111,6 +111,23 @@ int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
  * that fails; rfs_config_rf* keep it.  A row whose device set index lies outside [0, S) runs the grid
  * lists and is failed as described below.  Copies synchronously, like rfs_config_obs_rays. */
 int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use);
+/* Per-set receiver-function samples (missing ray-parameter bins, station-dependent fitting windows):
+ * use [S][nrf] (host pointer, values 0 or 1, nrf = nray * nt, the RF block of the data vector in its
+ * order [ray][sample]) marks the samples each set fits.  For a row of set s the RF misfit is
+ * 0.5 sum over observed samples (d - dobs)^2 and the adjoint source is zero at the others: the residual
+ * there is selected as 0, never formed, so dobs may hold anything at unobserved samples (missing data
+ * may be stored as NaN).  dsyn keeps the full synthetic trace at every sample; a failed row returns
+ * dobs as before.  A set whose mask keeps whole traces gives exactly U, grad and flag of a one-set
+ * context configured with rfs_config_rf_rays on its observed rays.  The joint weight of set s is
+ * (sigma1[s]/sigma2[s])^2 n1_s/nsw_s with n1_s = sum of use[s].  SWD-only evaluations (which = 2) ignore
+ * the table; the librf drop-ins are not affected.
+ * Returns RFS_E_CONFIG without an RF configuration or when S differs from the number of observation
+ * sets held, RFS_E_ARG when nrf is wrong, use is NULL, a value is not 0 or 1, or a set observes no
+ * sample (its joint weight would be zero).  A call that fails leaves no table.  rfs_config_obs_sets,
+ * rfs_config_obs, rfs_config_rf and rfs_config_rf_rays drop it; rfs_config_swd*, rfs_config_obs_rays and
+ * rfs_config_obs_periods keep it.  A row whose device set index lies outside [0, S) reads no mask entry
+ * and is failed as described below.  Copies synchronously, like rfs_config_obs_rays. */
+int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char *use);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)

@@ -72,6 +72,8 @@ def load_library():
         L.rfs_config_obs_rays.argtypes = [_vp, C.c_int, C.c_int, _dp]
         L.rfs_config_obs_periods.restype = C.c_int
         L.rfs_config_obs_periods.argtypes = [_vp, C.c_int, C.c_int, _u8p]
+        L.rfs_config_obs_rf_samples.restype = C.c_int
+        L.rfs_config_obs_rf_samples.argtypes = [_vp, C.c_int, C.c_int, _u8p]
         L.rfs_misfit_grad_sets_dev.restype = C.c_int
         L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_sets_host.restype = C.c_int
@@ -143,7 +145,7 @@ def exported_symbols():
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
             "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
-            "rfs_config_obs_rays", "rfs_config_obs_periods"]
+            "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples"]
 
 
 def _f64(a):
@@ -305,6 +307,20 @@ class Context:
             raise ValueError("use must hold booleans or 0/1")
         u8 = np.ascontiguousarray(u, dtype=np.uint8)
         self._ck(self.L.rfs_config_obs_periods(self.h, u8.shape[0], u8.shape[1], u8.ctypes.data_as(_u8p)))
+
+    def config_obs_rf_samples(self, use):
+        """Per-station receiver-function samples: use [S, nray * nt] or [S, nray, nt] (bool or 0/1) marks
+        the samples of the RF block of the data vector (order [ray][sample]) that each of the S
+        observation sets held now fits.  The misfit sums over the observed samples only and dobs is never
+        read at the others (NaN there is harmless); dsyn keeps the full traces.  config_obs and config_rf
+        drop the table again."""
+        u = np.asarray(use)
+        if u.ndim not in (2, 3) or u.shape[0] == 0:
+            raise ValueError(f"use must be [S, nray * nt] or [S, nray, nt], got shape {u.shape}")
+        if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
+            raise ValueError("use must hold booleans or 0/1")
+        u8 = np.ascontiguousarray(u.reshape(u.shape[0], -1), dtype=np.uint8)
+        self._ck(self.L.rfs_config_obs_rf_samples(self.h, u8.shape[0], u8.shape[1], u8.ctypes.data_as(_u8p)))
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)

@@ -8,9 +8,10 @@ class JointEvaluator:
     """Many-chains Joint_RF_SWD.misfit_and_grad on one GPU with resident inputs/outputs.  dobs [ndata]
     or [S, ndata]: S observation sets (stations) sharing `cfg`; cfg's sigma1 / sigma2 may then be
     [S] arrays.  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's ray_p.
-    obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set observes."""
+    obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set observes.
+    obs_rf_use [S, nray * nt] or [S, nray, nt]: the receiver-function samples each set fits."""
 
-    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None):
+    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None, obs_rf_use=None):
         self.ctx = Context(device)
         self.which = which
         self.n = nlayer
@@ -26,6 +27,8 @@ class JointEvaluator:
             self.ctx.config_obs_rays(obs_ray_p)
         if obs_swd_use is not None:
             self.ctx.config_obs_periods(obs_swd_use)
+        if obs_rf_use is not None:
+            self.ctx.config_obs_rf_samples(obs_rf_use)
         self.device = torch.device("cuda", device)
         self.ndata = self.ctx.ndata(which)
         self._out = None

@@ -96,6 +96,11 @@ struct rfs_ctx {
   // Every call that changes the sets or the RF configuration drops the table.
   bool has_set_rays = false;
   Buf d_set_rays;
+  // per-set RF sample mask [nsets][nray * nt] (rfs_config_obs_rf_samples, read through ObsSets::observed)
+  // and each set's observed sample count; dropped by the same calls as the ray table
+  bool has_set_rf = false;
+  Buf d_set_rf;
+  std::vector<int> set_n1;
   // ---- observations: nsets data vectors ("stations") of ndobs values each
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
@@ -753,6 +758,8 @@ int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, 
   if (rc) return rc;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
   ctx->has_set_rays = false;
+  ctx->has_set_rf = false;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
   ctx->has_rf = true;
   return RFS_OK;
 }
@@ -779,6 +786,7 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
   ctx->ndobs = ndobs;
   ctx->wt_n1 = ctx->wt_nsw = -1;
   ctx->has_set_rays = false;
+  ctx->has_set_rf = false;
   ctx->has_obs = true;
   return RFS_OK;
 }
@@ -901,6 +909,42 @@ int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *u
   return RFS_OK;
 }
 
+int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char *use) {
+  if (!ctx) return RFS_E_ARG;
+  // a failed call leaves no table: every set then fits every sample.  The joint weights follow the
+  // table, with or without it.
+  ctx->has_set_rf = false;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
+  if (!ctx->has_rf)
+    return fail(ctx, RFS_E_CONFIG, "per-set RF samples need an RF configuration (rfs_config_rf)");
+  if (!ctx->has_obs || S != ctx->nsets)
+    return fail(ctx, RFS_E_CONFIG, "RF sample mask for " + std::to_string(S) + " sets, the context holds " +
+                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
+  const int n1 = ctx->rf.nt * (int)ctx->ray_ps.size();
+  if (nrf != n1)
+    return fail(ctx, RFS_E_ARG, "RF sample mask has " + std::to_string(nrf) + " entries per set, the RF " +
+                                    "objective has " + std::to_string(n1) + " samples (nray * nt)");
+  if (!use) return fail(ctx, RFS_E_ARG, "no RF sample mask");
+  std::vector<int> cnt(S, 0);
+  for (int st = 0; st < S; st++) {
+    for (int j = 0; j < n1; j++) {
+      const unsigned char u = use[(size_t)st * n1 + j];
+      if (u > 1) return fail(ctx, RFS_E_ARG, "RF sample mask values must be 0 or 1");
+      cnt[st] += u;
+    }
+    // no RF sample would give the set a zero joint weight, silently dropping its dispersion data
+    if (cnt[st] == 0) return fail(ctx, RFS_E_ARG, "set " + std::to_string(st) + " observes no RF sample");
+  }
+  CK(cudaSetDevice(ctx->device));
+  const size_t bytes = (size_t)S * n1;
+  int rc = ensure(ctx, ctx->d_set_rf, bytes);
+  if (rc) return rc;
+  CK(cudaMemcpy(ctx->d_set_rf.p, use, bytes, cudaMemcpyHostToDevice));
+  ctx->set_n1 = cnt;
+  ctx->has_set_rf = true;
+  return RFS_OK;
+}
+
 int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
                              double *U, double *grad, double *dsyn, unsigned char *flag, void *stream) {
   if (!ctx) return RFS_E_ARG;
@@ -934,7 +978,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
   Bmax = std::min(Bmax, 2147483647LL / ((long long)SWD_NF * n));  // 32-bit offsets in SwdModel::ld
   const int nch = (int)((B + Bmax - 1) / Bmax);
   const long long Bch = (B + nch - 1) / nch;
-  const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata};
+  // the RF sample mask rides along for the RF residual kernels (ld n1: one set's RF block)
+  const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata,
+                    use_rf && ctx->has_set_rf ? (const unsigned char *)ctx->d_set_rf.p : nullptr, n1};
   // each row's own SWD period lists (rfs_config_obs_periods) for the rows of one chunk
   auto set_view = [&](const int *chunk_set) {
     return SwdSetView{ctx->has_set_periods ? (const int *)ctx->d_set_per.p : nullptr, chunk_set, ctx->nsets,
@@ -950,7 +996,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       const double q = ctx->sigma1[k] / ctx->sigma2[k];
       // with per-set period lists: the data count of set k's own lists, as a one-set context has it
       const int nsw_k = ctx->has_set_periods ? nmsel * ctx->set_nobs[k] : nsw;
-      ctx->wt[k] = q * q * n1 / nsw_k;
+      // likewise the set's own observed RF samples (rfs_config_obs_rf_samples)
+      const int n1_k = ctx->has_set_rf ? ctx->set_n1[k] : n1;
+      ctx->wt[k] = q * q * n1_k / nsw_k;
     }
     int rc;
     if ((rc = ensure(ctx, ctx->d_wt, sizeof(double) * ctx->nsets))) return rc;
@@ -1048,6 +1096,7 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
         double *dsyn_r = dsyn + off * ndata + (size_t)ir * rf.nt;
         ObsSets obs_r = obs_k;
         obs_r.dobs += (size_t)ir * rf.nt;
+        if (obs_r.use) obs_r.use += (size_t)ir * rf.nt;
         if (!rf_time) {
           if ((rc = run_rf_decon(ctx, rf, Bc, 2 * n, obs_r, dsyn_r, ndata, Uo, go, fo, sigma, tshift, sr, ir > 0)))
             return rc;

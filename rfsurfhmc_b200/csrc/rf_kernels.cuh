@@ -595,6 +595,7 @@ RFS_DEVINL double block_reduce(double v, double *red, bool is_max) {
 // ---- K4: one block per model: water-level deconvolution, c2r FFT, trace, misfit and (optional)
 // adjoint gradient.   dynamic smem: cd buf[nft] + cd s21[n2] + cd s22[n2] + cd wt[n2] + 32 doubles
 //   rf   : [B][ldrf>=nt]  obs.dobs: [nsets][ld >= nt] or NULL   U: [B]   grad: [B][nrow] (nrow = NQ*n)
+//   the residual is 0 at the samples the row's set does not fit (ObsSets::observed); rf is written whole
 //   flag : [B] or NULL; only written (0) for a row whose observation-set index is out of range
 __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 *__restrict__ dspec,
                                 long long B, int nrow, int nt, int nft, int logn, double dt,
@@ -655,7 +656,7 @@ __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 
       const double v = irfft_at(z, it) / nft / dt * e;
       rf[b * ldrf + it] = v;
       if (dobs) {
-        const double r = v - dobs[it];
+        const double r = obs.observed(set, it) ? v - dobs[it] : 0.0;
         lsum += r * r;
         rt = r * e / dt;
       }

@@ -158,7 +158,8 @@ __global__ void __launch_bounds__(256, 3) rf_time_kernel(const double2 *__restri
 // shortcut does not apply because deconit is nonlinear).  One thread per (model, layer).
 //   traces [B][4][n][nt] (rho, vp, vs, h);  chain [2][n][B];  rf [B][ldrf];  grad [B][2n]
 //   flag [B] or NULL: only written (0) for a row whose observation-set index is out of range; such a
-//   row gets U 0, grad 0 and a NaN trace
+//   row gets U 0, grad 0 and a NaN trace.  The residual is 0 at the samples the row's set does not fit
+//   (ObsSets::observed).
 __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const double *__restrict__ chain,
                                      double *__restrict__ rf, long long ldrf, ObsSets obs, long long B,
                                      int n, int nt, double *__restrict__ U, double *__restrict__ grad,
@@ -187,7 +188,7 @@ __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const do
   const double *kh = traces + ((b * 4 + 3) * n + m) * (long long)nt;
   double g0 = 0.0, g1 = 0.0, us = 0.0;
   for (int t = 0; t < nt; t++) {
-    const double res = rf[b * ldrf + t] - dobs[t];
+    const double res = obs.observed(set, t) ? rf[b * ldrf + t] - dobs[t] : 0.0;
     g0 += (kb[t] + dadb * ka[t] + drda * dadb * kr[t]) * res;
     g1 += kh[t] * res;
     us += res * res;

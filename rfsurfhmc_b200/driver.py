@@ -11,8 +11,9 @@ write `real_syn.npy`, per-chain result files and `misfit.npy [nchains, nsamples]
 
 inverts a station array instead: the observations of S stations come from the file (see
 model/stations.py: load_stations; the optional key ray_p [S] or [S, nray] gives each station its own
-ray parameter(s) in place of rf.ray_p, and swd_use [S, nper] the periods of the swd lists it observes),
-K chains run per station, all S*K in one device run (sharded
+ray parameter(s) in place of rf.ray_p, swd_use [S, nper] the periods of the swd lists it observes and
+rf_use [S, nray*nt] or [S, nray, nt] the receiver-function samples it fits: missing ray bins, fitting
+windows), K chains run per station, all S*K in one device run (sharded
 over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
 import argparse
 import os
@@ -66,9 +67,9 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
         npairs = nchains
         ids, sidx = D.shard_chains(nchains), None
     else:
-        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray, model_swd)
+        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray, model_swd, model_rf)
         model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"], st["ray_p"],
-                             st["swd_use"])
+                             st["swd_use"], st["rf_use"])
         boundaries = st["bounds"]
         npairs = model.nstations * nchains
         sidx, ids = D.shard_station_chains(model.nstations, nchains)
@@ -114,7 +115,8 @@ def main():
     ap.add_argument("--stations", default=None,
                     help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2], "
                          "ray_p [S] or [S,nray] in place of rf.ray_p, swd_use [S,nper] observed periods of the "
-                         "swd lists): invert every station instead of "
+                         "swd lists, rf_use [S,nray*nt] or [S,nray,nt] fitted RF samples): invert every station "
+                         "instead of "
                          "observations synthesised from true_model")
     ap.add_argument("--no-chain-files", action="store_true")
     ap.add_argument("--outdir", default=None, help="override hmc.OUTPUT_DIR of the parameter file")

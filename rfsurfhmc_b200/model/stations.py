@@ -1,12 +1,12 @@
 """StationArray — many stations (observation sets) that share one forward configuration.
 
 A station array is inverted station by station: each station has its own data vector (receiver
-function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s) and
-its own subset of the dispersion periods, while the layer count, the period grid, modes and RF sampling
-are shared.  The reference runs one job per station; here one context holds every station's
+function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s), its
+own subset of the dispersion periods and its own receiver-function samples, while the layer count, the
+period grid, modes and RF sampling are shared.  The reference runs one job per station; here one context holds every station's
 observations and each evaluated row, or each HMC chain, names its station, so one device run fills the
 GPU with all of them (include/rfsurfhmc.h: rfs_config_obs_sets, rfs_config_obs_rays,
-rfs_config_obs_periods).
+rfs_config_obs_periods, rfs_config_obs_rf_samples).
 
     stations = StationArray(joint_model, dobs, ray_p=p)   # dobs [S, ndata], p [S] or [S, nray]
     HamitonianMC(stations, bounds, ...).sample_chains(ids, stations=station_of_each_chain)
@@ -15,8 +15,14 @@ With swd_use [S, nper] the template's four period lists are a common grid (nper 
 len(tLc) + len(tLg)) and station s observes the grid periods where swd_use[s] is true: dobs keeps the grid
 layout (its values at unobserved periods are ignored), synthetics are NaN there.
 
+With rf_use [S, nray * nt] (or [S, nray, nt]) station s fits the receiver-function samples where
+rf_use[s] is true: a missing ray-parameter bin is a ray whose trace is all false, a fitting window a run
+of true samples.  dobs keeps the full layout (its values at unobserved samples are never read, NaN is
+fine) and the synthetics keep the full traces.  rf_time_window builds the mask from bounds in seconds.
+
 A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
-keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray] and swd_use [S, nper].
+keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray], swd_use [S, nper] and
+rf_use [S, nray * nt] or [S, nray, nt].
 """
 import copy
 import numpy as np
@@ -35,7 +41,8 @@ def _fresh_copy(m):
 
 
 class StationArray:
-    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None, swd_use=None):
+    def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None, swd_use=None,
+                 rf_use=None):
         """model: a configured Joint_RF_SWD, ReceiverFunc or SurfWD; only its forward configuration is
         used (its own observations are ignored).  dobs [S, ndata] in the model's data layout.
         sigma1 / sigma2: scalars or [S] (default: the joint model's own, 1.0 for the others; they only
@@ -43,7 +50,10 @@ class StationArray:
         ray_p: None (every station uses the template's ray parameter(s)) or each station's own, [S] or
         [S, nray] with the template's ray count; not for a SurfWD template.
         swd_use: None (every station observes every period) or [S, nper] bool / 0-1, the grid periods
-        each station observes; for a Joint_RF_SWD or SurfWD template."""
+        each station observes; for a Joint_RF_SWD or SurfWD template.
+        rf_use: None (every station fits every RF sample) or [S, nray * nt] / [S, nray, nt] bool / 0-1,
+        the receiver-function samples each station fits (see rf_time_window); for a Joint_RF_SWD or
+        ReceiverFunc template."""
         if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
             raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
         self.template = model
@@ -76,6 +86,12 @@ class StationArray:
             if not isinstance(swd, SurfWD):
                 raise TypeError("swd_use needs a dispersion template (Joint_RF_SWD or SurfWD)")
             self.swd_use = station_periods(swd_use, S, swd)
+        self.rf_use = None
+        if rf_use is not None:
+            rf = model.rfmodel if isinstance(model, Joint_RF_SWD) else model
+            if not isinstance(rf, ReceiverFunc):
+                raise TypeError("rf_use needs a receiver-function template (Joint_RF_SWD or ReceiverFunc)")
+            self.rf_use = station_rf_samples(rf_use, S, rf)
         self._ctx = None
         self._ctx_key = None
 
@@ -91,7 +107,8 @@ class StationArray:
             self._ctx_key = None
         key = (type(self.template), self.template._config_fields(n), self.sigma1.tobytes(),
                self.sigma2.tobytes(), self.dobs.tobytes(), None if self.ray_p is None else self.ray_p.tobytes(),
-               None if self.swd_use is None else self.swd_use.tobytes())
+               None if self.swd_use is None else self.swd_use.tobytes(),
+               None if self.rf_use is None else self.rf_use.tobytes())
         if self._ctx_key != key:
             self.template._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
@@ -99,6 +116,8 @@ class StationArray:
                 self._ctx.config_obs_rays(self.ray_p)
             if self.swd_use is not None:
                 self._ctx.config_obs_periods(self.swd_use)
+            if self.rf_use is not None:
+                self._ctx.config_obs_rf_samples(self.rf_use)
             self._ctx_key = key
         return self._ctx
 
@@ -111,21 +130,24 @@ class StationArray:
     def station_model(self, s):
         """Single-station copy of the template holding station s's observations (and sigmas, and ray
         parameter(s): a scalar for one ray, a list otherwise).  With swd_use its SurfWD holds the
-        station's subset period lists and its dispersion data only the observed values."""
+        station's subset period lists and its dispersion data only the observed values.  With rf_use its
+        ReceiverFunc holds only the station's observed rays (ray parameters and traces); a station that
+        fits part of a trace has no single-station model (ValueError)."""
         s = int(s)
         if not 0 <= s < self.nstations:
             raise IndexError(f"station {s} outside [0, {self.nstations})")
         d = self.dobs[s].copy()
         t = self.template
         if isinstance(t, Joint_RF_SWD):
-            rf = self._station_rf(t.rfmodel, s)
+            rf, keep = self._station_rf(t.rfmodel, s)
             m = Joint_RF_SWD(float(self.sigma1[s]), float(self.sigma2[s]), rf, self._station_swd(t.swdmodel, s))
             m._device = t._device
             nt = t.rfmodel.nt
-            m.set_obsdata(d[:nt], self._compact(d[nt:], s))
+            m.set_obsdata(d[:nt][keep], self._compact(d[nt:], s))
             return m
         if isinstance(t, ReceiverFunc):
-            m = self._station_rf(t, s)
+            m, keep = self._station_rf(t, s)
+            d = d[keep]
         else:
             m = self._station_swd(t, s)
             d = self._compact(d, s)
@@ -162,11 +184,23 @@ class StationArray:
         return c
 
     def _station_rf(self, rf, s):
+        """Station s's ReceiverFunc and the data positions of its observed rays' traces."""
         c = _fresh_copy(rf)
-        if self.ray_p is not None:
-            r = self.ray_p[s]
+        r = self.ray_p[s] if self.ray_p is not None else np.atleast_1d(np.asarray(rf.ray_p, dtype=np.float64))
+        keep = np.ones(rf.nt, dtype=bool)
+        if self.rf_use is not None:
+            u = self.rf_use[s].reshape(rf.nray, rf.nt_trace)
+            obs = u.all(axis=1)
+            if not np.array_equal(obs, u.any(axis=1)):
+                raise ValueError(f"station {s} ({self.names[s]}) fits part of a receiver-function trace: no "
+                                 "single-station ReceiverFunc fits a window, use station_view")
+            r = r[obs]
+            keep = u.reshape(-1)
+            c.nray = int(r.size)
+            c.nt = c.nt_trace * c.nray
+        if self.ray_p is not None or self.rf_use is not None:
             c.ray_p = float(r[0]) if r.size == 1 else r.tolist()
-        return c
+        return c, keep
 
 
 class _StationView:
@@ -205,6 +239,42 @@ def station_periods(use, S, swd, where=""):
     return u
 
 
+def station_rf_samples(use, S, rf, where=""):
+    """rf_use [S, nray * nt] or [S, nray, nt] (bool or 0/1) of a ReceiverFunc template's data vector ->
+    bool [S, nray * nt]; the ValueError names the key 'rf_use' (after `where`)."""
+    u = np.asarray(use)
+    if u.shape not in ((S, rf.nt), (S, rf.nray, rf.nt_trace)):
+        raise ValueError(f"{where}'rf_use' must have shape [{S}, {rf.nt}] or [{S}, {rf.nray}, {rf.nt_trace}], "
+                         f"got {u.shape}")
+    if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
+        raise ValueError(f"{where}'rf_use' must hold booleans or 0/1")
+    u = np.ascontiguousarray(u.reshape(S, rf.nt), dtype=bool)
+    empty = np.flatnonzero(~u.any(axis=1))
+    if empty.size:
+        # a station without RF data would get a zero joint weight and lose its dispersion data silently
+        raise ValueError(f"{where}'rf_use': station {int(empty[0])} observes no receiver-function sample")
+    return u
+
+
+def rf_time_window(rf, lo, hi):
+    """RF sample mask (rf_use) of the time windows lo <= t <= hi on a ReceiverFunc's trace axis
+    t = arange(nt) * dt - time_shift (rf.t), in seconds.  lo, hi: [S] (every ray) or [S, nray]; a NaN
+    bound marks a ray the station does not observe.  A bound equal to a sample time, up to rounding
+    (1e-9 of dt), includes that sample.  Returns bool [S, nray * nt]."""
+    lo = np.asarray(lo, dtype=np.float64)
+    hi = np.asarray(hi, dtype=np.float64)
+    if lo.shape != hi.shape or lo.ndim not in (1, 2) or (lo.ndim == 2 and lo.shape[1] != rf.nray):
+        raise ValueError(f"lo and hi must both be [S] or [S, {rf.nray}], got {lo.shape} and {hi.shape}")
+    S = lo.shape[0]
+    lo = np.broadcast_to(lo.reshape(S, -1), (S, rf.nray))
+    hi = np.broadcast_to(hi.reshape(S, -1), (S, rf.nray))
+    eps = 1e-9 * rf.dt
+    t = np.asarray(rf.t, dtype=np.float64)
+    # comparisons with NaN are false: a NaN bound leaves its ray without samples
+    u = (t >= lo[..., None] - eps) & (t <= hi[..., None] + eps)
+    return u.reshape(S, rf.nray * rf.nt_trace)
+
+
 def station_rays(ray_p, S, nray, where=""):
     """ray_p [S] (nray = 1) or [S, nray] -> float64 [S, nray], finite and > 0; the ValueError names the
     key 'ray_p' (after `where`)."""
@@ -217,12 +287,14 @@ def station_rays(ray_p, S, nray, where=""):
     return np.ascontiguousarray(r.reshape(S, nray))
 
 
-def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None):
+def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None, rf=None):
     """Validated content of a stations file (.npz path or a mapping with the same keys):
     dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0), bounds [S, nparam, 2]
     (default: default_bounds [nparam, 2] for every station), ray_p [S] or [S, nray] (default None: the
-    ray parameter(s) of the forward configuration) and swd_use [S, nper] (default None: every period;
-    swd = the SurfWD whose period grid it marks).  Raises ValueError naming the bad key."""
+    ray parameter(s) of the forward configuration), swd_use [S, nper] (default None: every period;
+    swd = the SurfWD whose period grid it marks) and rf_use [S, nray * nt] or [S, nray, nt] (default
+    None: every RF sample; rf = the ReceiverFunc whose data it marks).  Raises ValueError naming the
+    bad key."""
     if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
         with np.load(src, allow_pickle=False) as f:
             src = {k: f[k] for k in f.files}
@@ -261,4 +333,9 @@ def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None):
         if swd is None:
             raise ValueError("stations file: 'swd_use' needs a dispersion configuration")
         out["swd_use"] = station_periods(src["swd_use"], S, swd, "stations file: ")
+    out["rf_use"] = None
+    if "rf_use" in src:
+        if rf is None:
+            raise ValueError("stations file: 'rf_use' needs a receiver-function configuration")
+        out["rf_use"] = station_rf_samples(src["rf_use"], S, rf, "stations file: ")
     return out

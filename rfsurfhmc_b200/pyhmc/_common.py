@@ -53,8 +53,10 @@ def save_chains(model, out, chain_ids, stations, outdir, name, nbest, nsamples):
             continue
         s = int(stations[i])
         if s not in single:
-            # with per-station periods the file keeps the array's grid layout, as the chain's syn rows do
-            single[s] = model.station_model(s) if model.swd_use is None else model.station_view(s)
+            # with per-station periods or RF samples the file keeps the array's data layout, as the chain's
+            # syn rows do
+            masked = model.swd_use is not None or model.rf_use is not None
+            single[s] = model.station_view(s) if masked else model.station_model(s)
         save_chain(f"{outdir}/{model.names[s]}/{name}.{int(cid)}.npz", single[s], out, i, nbest, nsamples)
 
 

@@ -27,8 +27,18 @@ random contiguous window of 60-100 % of each of the lists tRc and tRg (chosen in
   (h) SWD only, n = 40, modes 0-2, 24 Rc and 18 Rg periods, 64 stations x 64 models: the same three;
   (i) HMC, 16 stations x 64 chains: one grouped run with the mask vs 16 single-station runs, each in a
       context configured on its station's subset lists.
---legs sets,rays,periods selects the legs (default sets,rays); the legs run replace their keys in --out
-and keep the others.
+Leg "rfwin" (per-station receiver-function samples, rfs_config_obs_rf_samples), every station fitting a
+seeded window of 40-100 % of each trace, about a quarter of the stations missing one ray bin (three ray
+parameters 0.045, 0.06, 0.075 in place of F1's one, so that a bin can be missing):
+  (j) F1 joint, (S, K) = (256, 64), (1024, 16): the grouped call with the mask vs the same grouped call
+      without a table (two contexts, timed alternately, --inner calls per timing);
+  (k) RF only, frequency method, n = 40, nt = 2048, three rays, 256 stations x 256 models: the same two
+      (48 GB workspace budget each, as in (e));
+  (l) RF only, time method, F1 layers and sampling, 64 stations x 16 models: the same two;
+  (m) HMC, 16 stations x 64 chains with whole-trace masks (missing bins only): one grouped run vs 16
+      single-station runs, each in a context configured on its station's observed rays.
+--legs sets,rays,periods,rfwin selects the legs (default sets,rays); the legs run replace their keys in
+--out and keep the others.
 Every shape is warmed up first; each timing is repeated --reps times (median, min, max reported), with a
 host clock around work that ends in a device synchronise.  Station observations are the forward model
 of seeded perturbations of the F1 true model plus seeded noise.  Prints one JSON line and writes it to
@@ -120,6 +130,8 @@ def main():
         res["rays"] = rays_leg(a, torch, station_obs, X, nd)
     if "periods" in legs:
         res["periods"] = periods_leg(a, torch, X)
+    if "rfwin" in legs:
+        res["rfwin"] = rfwin_leg(a, torch, X)
     if "sets" not in legs:
         c.close()
         return write(a, res)
@@ -456,6 +468,155 @@ def periods_leg(a, torch, X):
     for c in single:
         c.close()
     return out
+
+
+def rfwin_leg(a, torch, X):
+    """Per-station RF samples against the same grouped call without a table, and the HMC against one
+    context per station on its observed rays (see the module docstring)."""
+    from rfsurfhmc_b200._lib import Context
+    from rfsurfhmc_b200.fixtures import f1_config, f1_true_model, driver_bounds, perturbed_models
+    from bench import layered_models
+    cfg, x0 = f1_config(), f1_true_model()
+    dev = torch.device("cuda", 0)
+    st = torch.cuda.current_stream(dev)
+    rays = [0.045, 0.06, 0.075]
+    out = {**gpu_info(), "inner_calls": a.inner, "rays": rays,
+           "mask": "window of 40-100 % of each trace, a quarter of the stations miss one ray bin", "eval": []}
+    rng = np.random.default_rng(29)
+
+    def masks(S, nt, whole=False):
+        u = np.zeros((S, len(rays), nt), dtype=bool)
+        for s in range(S):
+            for r in range(len(rays)):
+                k = nt if whole else int(rng.integers(int(np.ceil(0.4 * nt)), nt + 1))
+                o = int(rng.integers(0, nt - k + 1))
+                u[s, r, o:o + k] = True
+            if rng.random() < 0.25:
+                u[s, int(rng.integers(0, len(rays)))] = False
+        return u.reshape(S, -1)
+
+    def configure(c, which, n, nt, dt, gauss, method, rp=rays):
+        if which != 1:
+            c.config_swd(n, tRc=cfg["tRc"], tRg=cfg["tRg"])
+        c.config_rf(n, rp, nt, dt, gauss, cfg["time_shift"], cfg["water"], "P", method)
+
+    def observations(which, n, nt, dt, gauss, method, Xs):
+        c = Context(0)
+        configure(c, which, n, nt, dt, gauss, method)
+        S = Xs.shape[0]
+        c.config_obs(np.zeros((S, c.ndata(which))))
+        _, _, d, _ = c.misfit_grad_host(Xs, which, sets=np.arange(S))
+        c.close()
+        d = np.where(np.isfinite(d), d, 0.0)
+        return d + 0.01 * np.random.default_rng(S).standard_normal(d.shape)
+
+    def compare(which, n, nt, dt, gauss, method, Xd, S, K, dobs, use):
+        B = Xd.shape[0]
+        sets = torch.from_numpy(np.repeat(np.arange(S, dtype=np.int32), K)).to(dev)
+        cs = []
+        for with_mask in (True, False):
+            c = Context(0)
+            configure(c, which, n, nt, dt, gauss, method)
+            c.config_obs(dobs)
+            if with_mask:
+                c.config_obs_rf_samples(use)
+            cs.append(c)
+        U = torch.empty(B, dtype=torch.float64, device=dev)
+        G = torch.empty(Xd.shape, dtype=torch.float64, device=dev)
+        D = torch.empty(B, cs[0].ndata(which), dtype=torch.float64, device=dev)
+        F = torch.empty(B, dtype=torch.uint8, device=dev)
+
+        def call(c):
+            for _ in range(a.inner):
+                c.misfit_grad_dev(B, Xd.data_ptr(), which, U.data_ptr(), G.data_ptr(), D.data_ptr(), F.data_ptr(),
+                                  st.cuda_stream, sets_ptr=sets.data_ptr())
+        ts = ([], [])
+        for c in cs:
+            call(c)
+        torch.cuda.synchronize()
+        for _ in range(a.reps):
+            for k, c in enumerate(cs):
+                t0 = time.perf_counter()
+                call(c)
+                torch.cuda.synchronize()
+                ts[k].append((time.perf_counter() - t0) / a.inner)
+        for c in cs:
+            c.close()
+        masked, plain = spread(ts[0]), spread(ts[1])
+        return {"masked": masked, "no_table": plain, "observed_share": float(use.mean()),
+                "mask_cost": masked["median_ms"] / plain["median_ms"] - 1.0}
+
+    n = x0.size // 2
+    f1 = (n, cfg["nt"], cfg["dt"], cfg["gauss"])
+    for S, K in ((256, 64), (1024, 16)):
+        dobs = observations(0, *f1, "freq", perturbed_models(x0, S, seed=100 + S, rel=0.05))
+        out["eval"].append({"workload": "F1 joint, three rays, %d stations x %d models" % (S, K), "S": S, "K": K,
+                            **compare(0, *f1, "freq", X[:S * K], S, K, dobs, masks(S, cfg["nt"]))})
+        progress(out["eval"][-1])
+    # RF only, frequency method, C3-like
+    nc, ntc, S, K = 40, 2048, 256, 256
+    Xc = torch.from_numpy(layered_models(S * K, nc, 2)).to(dev)
+    dobs = 0.01 * np.random.default_rng(3).standard_normal((S, 3 * ntc))
+    old = os.environ.get("RFS_WS_BUDGET_MB")
+    os.environ["RFS_WS_BUDGET_MB"] = "48000"
+    try:
+        out["rf_c3"] = {"workload": "RF only (freq), n=40, nt=2048, dt=0.05, a=2.5, three rays, "
+                                    "%d stations x %d models" % (S, K), "S": S, "K": K,
+                        **compare(1, nc, ntc, 0.05, 2.5, "freq", Xc, S, K, dobs, masks(S, ntc))}
+    finally:
+        if old is None:
+            del os.environ["RFS_WS_BUDGET_MB"]
+        else:
+            os.environ["RFS_WS_BUDGET_MB"] = old
+    progress(out["rf_c3"])
+    # RF only, time method
+    S, K = 64, 16
+    dobs = observations(1, *f1, "time", perturbed_models(x0, S, seed=43, rel=0.05))
+    out["rf_time"] = {"workload": "RF only (time), F1 layers and sampling, three rays, %d stations x %d models"
+                                  % (S, K), "S": S, "K": K,
+                      **compare(1, *f1, "time", X[:S * K], S, K, dobs, masks(S, cfg["nt"]))}
+    progress(out["rf_time"])
+    # HMC, 16 stations x 64 chains, whole-trace masks
+    Sh, Kh = 16, 64
+    dobs = observations(0, *f1, "freq", perturbed_models(x0, Sh, seed=7, rel=0.05))
+    use = masks(Sh, cfg["nt"], whole=True)
+    bounds = driver_bounds(x0)
+    kw = dict(dt=0.1, Lrange=(5, 20), seed=991206, nsamples=a.hmc_iters + 1, ndraws=0, max_iters=a.hmc_iters,
+              want_samples=False)
+    grouped = Context(0)
+    configure(grouped, 0, *f1, "freq")
+    grouped.config_obs(dobs)
+    grouped.config_obs_rf_samples(use)
+    single = []
+    for s in range(Sh):
+        obs = use[s].reshape(len(rays), -1).all(axis=1)
+        c = Context(0)
+        configure(c, 0, *f1, "freq", np.asarray(rays)[obs].tolist())
+        c.config_obs(np.concatenate([dobs[s, :use.shape[1]][use[s]], dobs[s, use.shape[1]:]]))
+        single.append(c)
+    ids, hsets = np.tile(np.arange(Kh), Sh), np.repeat(np.arange(Sh), Kh)
+    runs = {"grouped": lambda: grouped.hmc_run(0, ids, bounds, sets=hsets, **kw)["evals"],
+            "per_station": lambda: sum(single[s].hmc_run(0, np.arange(Kh), bounds, **kw)["evals"] for s in range(Sh))}
+    hmc = {"S": Sh, "K": Kh, "max_iters": a.hmc_iters, "stations_missing_a_bin": int((~use.all(axis=1)).sum())}
+    for name, fn in runs.items():
+        fn()
+        ts, evs = [], 0
+        for _ in range(max(1, a.reps // 2)):
+            t0 = time.perf_counter()
+            evs = fn()
+            ts.append(time.perf_counter() - t0)
+        hmc[name] = {**spread(ts), "evals": int(evs), "evals_per_s": float(evs / np.median(ts))}
+    hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
+    out["hmc"] = hmc
+    grouped.close()
+    for c in single:
+        c.close()
+    return out
+
+
+def progress(r):
+    """One finished workload of a leg on stderr (the RF C3 workloads take minutes)."""
+    print(json.dumps(r), file=sys.stderr, flush=True)
 
 
 if __name__ == "__main__":
