@@ -78,21 +78,31 @@ int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dob
  * rfs_hmc_run) returns RFS_E_CONFIG. */
 int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
                         const double *dobs, int ndobs);
+/* Per-set tables.  The three calls below give each of the S observation sets held its own ray
+ * parameters, SWD period lists or receiver-function samples.  Each table belongs to the sets held and to
+ * the configuration it refines, and its lifetime follows one rule:
+ *   - rfs_config_obs_sets and rfs_config_obs drop all three tables;
+ *   - a successful rfs_config_rf or rfs_config_rf_rays drops the ray table and the RF-sample table, and
+ *     keeps the period table;
+ *   - a successful rfs_config_swd or rfs_config_swd_modes drops the period table, and keeps the other two;
+ *   - each of the three calls below drops its own table first, so a call of it that fails leaves no such
+ *     table, and it keeps the other two;
+ *   - a failed rfs_config_swd* or rfs_config_rf* changes nothing: the configuration and every table stay.
+ * Without a table the context evaluates every set on the shared configuration.  Each call returns
+ * RFS_E_CONFIG without the configuration its table refines or when S differs from the number of
+ * observation sets held.  A row whose device set index lies outside [0, S) reads no table entry; it is
+ * failed as described below.  Like every rfs_config_* call, these copy synchronously into the context's
+ * device buffers: an evaluation still running on a caller's stream must have finished before the
+ * context is reconfigured. */
 /* Per-set ray parameters of the RF objective (each station's stack has its own mean slowness; the
  * reference's ReceiverFunc.ray_p is per station): ray_p [S][nray] (host pointer, copied to the device
  * here, never during an evaluation).  Row b's pass ir then uses ray_p[set[b]][ir] in place of the
  * shared list of rfs_config_rf / rfs_config_rf_rays; everything else (nt, dt, gauss, time shift, water
  * level, RF type, method, layers, periods, modes) stays shared.  The evaluations and the HMC use the
  * table whenever it is present; their signatures do not change.  The librf drop-ins keep their own
- * ray_p argument.
- * Returns RFS_E_CONFIG without an RF configuration or when S differs from the number of observation
- * sets held, RFS_E_ARG when nray differs from the configured ray count or a value is not finite and > 0.
- * The table belongs to the current sets and the current RF configuration: rfs_config_obs_sets,
- * rfs_config_obs, rfs_config_rf and rfs_config_rf_rays drop it, and the context uses the shared list
- * again; so does a call of this function that fails.  A row whose device set index lies outside [0, S)
- * reads no table entry; it computes with the shared value and is failed as described below.
- * Like every rfs_config_* call, this one copies synchronously into the context's device buffers: an
- * evaluation still running on a caller's stream must have finished before the context is reconfigured. */
+ * ray_p argument.  A row with an out-of-range set index computes with the shared value.
+ * Returns RFS_E_ARG when nray differs from the configured ray count, ray_p is NULL or a value is not
+ * finite and > 0.  Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
 /* Per-set SWD period lists (dispersion curves are rarely measured on the same periods at every
  * station): the four lists of rfs_config_swd[_modes] form a common period grid, and use [S][nper]
@@ -103,13 +113,10 @@ int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
  * the set's own compact period list.  dsyn keeps the grid layout: the subset context's values at the
  * observed positions, NaN at the others in every mode block; a failed row returns dobs as before.  The
  * joint weight of set s is (sigma1[s]/sigma2[s])^2 n_rf/(nmodes * observed periods of s).  RF-only
- * evaluations (which = 1) ignore the table; the libsurf drop-ins are not affected.
- * Returns RFS_E_CONFIG without an SWD configuration or when S differs from the number of observation
- * sets held, RFS_E_ARG when nper is wrong, a value is not 0 or 1, or a set observes no period.
- * The table belongs to the current sets and the current SWD configuration: rfs_config_obs_sets,
- * rfs_config_obs, rfs_config_swd and rfs_config_swd_modes drop it, and so does a call of this function
- * that fails; rfs_config_rf* keep it.  A row whose device set index lies outside [0, S) runs the grid
- * lists and is failed as described below.  Copies synchronously, like rfs_config_obs_rays. */
+ * evaluations (which = 1) ignore the table; the libsurf drop-ins are not affected.  A row with an
+ * out-of-range set index runs the grid lists.
+ * Returns RFS_E_ARG when nper is wrong, use is NULL, a value is not 0 or 1, or a set observes no period.
+ * Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use);
 /* Per-set receiver-function samples (missing ray-parameter bins, station-dependent fitting windows):
  * use [S][nrf] (host pointer, values 0 or 1, nrf = nray * nt, the RF block of the data vector in its
@@ -121,12 +128,8 @@ int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *u
  * context configured with rfs_config_rf_rays on its observed rays.  The joint weight of set s is
  * (sigma1[s]/sigma2[s])^2 n1_s/nsw_s with n1_s = sum of use[s].  SWD-only evaluations (which = 2) ignore
  * the table; the librf drop-ins are not affected.
- * Returns RFS_E_CONFIG without an RF configuration or when S differs from the number of observation
- * sets held, RFS_E_ARG when nrf is wrong, use is NULL, a value is not 0 or 1, or a set observes no
- * sample (its joint weight would be zero).  A call that fails leaves no table.  rfs_config_obs_sets,
- * rfs_config_obs, rfs_config_rf and rfs_config_rf_rays drop it; rfs_config_swd*, rfs_config_obs_rays and
- * rfs_config_obs_periods keep it.  A row whose device set index lies outside [0, S) reads no mask entry
- * and is failed as described below.  Copies synchronously, like rfs_config_obs_rays. */
+ * Returns RFS_E_ARG when nrf is wrong, use is NULL, a value is not 0 or 1, or a set observes no sample
+ * (its joint weight would be zero).  Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char *use);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------

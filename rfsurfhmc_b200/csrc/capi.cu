@@ -46,6 +46,27 @@ struct RfCfg {
   double dt = 0, gauss = 0, tshift = 0, water = 0.001;
 };
 
+// Per-set observation tables of the sets held (rfs_config_obs_rays / _periods / _rf_samples).  Each one
+// belongs to the sets and to one configuration; drop_tables is the only code that clears one.
+struct ObsTables {
+  // ray parameters [nsets][nray], used in place of the shared list
+  bool has_rays = false;
+  Buf d_rays;
+  // period lists: the plan the table was built for (the grid's, or the grid's without the Rc/Rg sequence
+  // sharing when a set observes other Rg than Rc periods), its period table (the grid lists, then each
+  // set's compact lists) and the SwdSetView table [nsets][ld], whose column use_col starts the observed
+  // flags; nobs: each set's observed periods per mode block
+  bool has_periods = false;
+  SwdPlan plan;
+  Buf d_periods, d_tab;
+  int ld = 0, use_col = 0;
+  std::vector<int> nobs;
+  // RF samples: the mask [nsets][nray * nt] (read through ObsSets::observed) and each set's sample count
+  bool has_rf = false;
+  Buf d_rf;
+  std::vector<int> n1;
+};
+
 }  // namespace
 
 // "Front" buffers of one chunk of a batch: model blocks and everything the root search produces.  They
@@ -77,37 +98,25 @@ struct rfs_ctx {
   bool has_swd = false;
   int n_swd = 0, mode = 0, stale = 1, sphere = 0;
   std::vector<int> modes;  // modes of the fused SWD objective (reference: one mode)
+  // the period grid (plan, its four lists and their lengths tRc, tRg, tLc, tLg): written only by a
+  // successful rfs_config_swd*
   SwdPlan plan;
-  std::vector<double> periods;  // the four grid lists (d_periods holds the per-set compact lists after them)
+  std::vector<double> periods;
   Buf d_periods;
-  int swd_nts[4] = {0, 0, 0, 0};  // lengths of the grid lists tRc, tRg, tLc, tLg
-  // per-set period lists (rfs_config_obs_periods): SwdSetView table [nsets][set_per_ld] and each set's
-  // observed count per mode block.  plan_unshared: the plan was rebuilt without the Rc/Rg sequence
-  // sharing for the table's lifetime.  rfs_config_obs_sets / rfs_config_obs / rfs_config_swd* drop it.
-  bool has_set_periods = false, plan_unshared = false;
-  Buf d_set_per;
-  int set_per_ld = 0;
-  std::vector<int> set_nobs;
+  int swd_nts[4] = {0, 0, 0, 0};
   // ---- RF configuration
   bool has_rf = false;
   RfCfg rf;
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
-  // per-set ray parameters [nsets][nray] (rfs_config_obs_rays), used in place of ray_ps when present.
-  // Every call that changes the sets or the RF configuration drops the table.
-  bool has_set_rays = false;
-  Buf d_set_rays;
-  // per-set RF sample mask [nsets][nray * nt] (rfs_config_obs_rf_samples, read through ObsSets::observed)
-  // and each set's observed sample count; dropped by the same calls as the ray table
-  bool has_set_rf = false;
-  Buf d_set_rf;
-  std::vector<int> set_n1;
-  // ---- observations: nsets data vectors ("stations") of ndobs values each
+  // ---- observations: nsets data vectors ("stations") of ndobs values each, and their per-set tables
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
   std::vector<double> sigma1, sigma2;  // [nsets]
   Buf d_dobs;                          // [nsets][ndobs]
+  ObsTables tables;
   // SWD weight of the joint objective per set, (sigma1/sigma2)^2 n1/nsw: computed on the host for the
-  // data lengths (wt_n1, wt_nsw) of the last joint call and uploaded again when they change
+  // data lengths (wt_n1, wt_nsw) of the last joint call and uploaded again when they change or when
+  // drop_tables resets them
   std::vector<double> wt;
   Buf d_wt;
   int wt_n1 = -1, wt_nsw = -1;
@@ -199,6 +208,66 @@ int ensure(rfs_ctx *ctx, Buf &b, size_t bytes) {
 int fail(rfs_ctx *ctx, int code, const std::string &msg) {
   if (ctx) ctx->err = msg;
   return code;
+}
+
+enum { TAB_RAYS = 1, TAB_PERIODS = 2, TAB_RF = 4, TAB_ALL = 7 };
+
+// The only code that clears a per-set table.  The joint weights follow the period and RF-sample tables,
+// so their cache goes with any table.
+void drop_tables(rfs_ctx *ctx, int which) {
+  ObsTables &ot = ctx->tables;
+  if (which & TAB_RAYS) ot.has_rays = false;
+  if (which & TAB_PERIODS) ot.has_periods = false;
+  if (which & TAB_RF) ot.has_rf = false;
+  ctx->wt_n1 = ctx->wt_nsw = -1;
+}
+
+// Prologue of the three table setters.  It drops the table first, so that a call that fails leaves none.
+int begin_table(rfs_ctx *ctx, int table, const std::string &name, bool configured, const char *config, int S) {
+  drop_tables(ctx, table);
+  if (!configured) return fail(ctx, RFS_E_CONFIG, name + " needs " + config);
+  if (!ctx->has_obs || S != ctx->nsets)
+    return fail(ctx, RFS_E_CONFIG, name + " for " + std::to_string(S) + " sets, the context holds " +
+                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
+  return RFS_OK;
+}
+
+// A per-set 0/1 mask use [S][width] over the `want` entries of one data block, in which every set keeps
+// at least one entry ("set s observes no <what>"); cnt: each set's count of ones.
+int check_mask(rfs_ctx *ctx, const std::string &name, const char *what, const unsigned char *use, int S,
+               int width, int want, std::vector<int> &cnt) {
+  if (width != want)
+    return fail(ctx, RFS_E_ARG, name + " has " + std::to_string(width) + " entries per set, the configuration has " +
+                                    std::to_string(want));
+  if (!use) return fail(ctx, RFS_E_ARG, "no " + name);
+  cnt.assign(S, 0);
+  for (int s = 0; s < S; s++) {
+    for (int j = 0; j < width; j++) {
+      const unsigned char u = use[(size_t)s * width + j];
+      if (u > 1) return fail(ctx, RFS_E_ARG, name + " values must be 0 or 1");
+      cnt[s] += u;
+    }
+    if (cnt[s] == 0) return fail(ctx, RFS_E_ARG, "set " + std::to_string(s) + " observes no " + what);
+  }
+  return RFS_OK;
+}
+
+// Length of one set's data vector for `which` (0 joint, 1 RF, 2 SWD): the RF block [ray][nt], then the
+// SWD block [mode][grid periods].
+int ndata_of(const rfs_ctx *ctx, int which) {
+  return (which != 2 ? ctx->rf.nt * (int)ctx->ray_ps.size() : 0) +
+         (which != 1 ? ctx->plan.ndata * (int)ctx->modes.size() : 0);
+}
+
+// The plan and device period table the SWD stage runs: the period table's when present, else the grid's.
+struct SwdGrid {
+  const SwdPlan &plan;
+  const double *periods;
+};
+SwdGrid swd_grid(const rfs_ctx *ctx) {
+  const ObsTables &ot = ctx->tables;
+  if (ot.has_periods) return {ot.plan, (const double *)ot.d_periods.p};
+  return {ctx->plan, (const double *)ctx->d_periods.p};
 }
 
 inline unsigned gridFor(long long total, int block) { return (unsigned)((total + block - 1) / block); }
@@ -581,7 +650,7 @@ size_t per_model_front_bytes(const rfs_ctx *ctx, int which) {
   size_t s = 0;
   const int n = (which != 1) ? ctx->n_swd : ctx->rf.n;
   if (which != 1 && ctx->has_swd) {
-    const SwdPlan &P = ctx->plan;
+    const SwdPlan &P = swd_grid(ctx).plan;
     const size_t nmo = ctx->modes.size() > 1 ? (size_t)P.nmode : 1;
     s += sizeof(double) * ((size_t)SWD_NF * n * (ctx->sphere ? 5 : 1) + (1 + nmo) * (size_t)P.nsolve) +
          sizeof(int) * ((size_t)3 * P.nseq + P.nsolve);  // ierr, sched key + perm, rstat
@@ -592,7 +661,7 @@ size_t per_model_front_bytes(const rfs_ctx *ctx, int which) {
 size_t per_model_bytes(const rfs_ctx *ctx, int which) {
   size_t s = 0;
   if (which != 1 && ctx->has_swd) {
-    const SwdPlan &P = ctx->plan;
+    const SwdPlan &P = swd_grid(ctx).plan;
     const size_t nmo = ctx->modes.size() > 1 ? (size_t)P.nmode : 1;
     s += sizeof(double) * (nmo * (size_t)P.nsolve + nmo * (size_t)P.nsolve * 4 * ctx->n_swd);
   }
@@ -604,30 +673,6 @@ size_t per_model_bytes(const rfs_ctx *ctx, int which) {
       s += sizeof(double2) * ((size_t)2 * rf.n * rf.n2) + sizeof(double) * ((size_t)4 * rf.n * rf.nt);
   }
   return s + 64;
-}
-
-// Builds ctx->plan on the context's grid lists (ctx->periods, swd_nts entries per wave type) and uploads
-// the period table.  share = false: no Rc/Rg sequence sharing (see rfs_config_obs_periods).
-int rebuild_grid_plan(rfs_ctx *ctx, bool share) {
-  const std::vector<double> grid = ctx->periods;  // build_plan refills ctx->periods
-  const double *ts[4];
-  for (int w = 0, o = 0; w < 4; o += ctx->swd_nts[w], w++) ts[w] = grid.data() + o;
-  int rc = build_plan(ctx, ctx->plan, ctx->periods, ctx->swd_nts, ts, ctx->mode, true, share);
-  if (rc) return rc;
-  if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * ctx->periods.size()))) return rc;
-  CK(cudaMemcpy(ctx->d_periods.p, ctx->periods.data(), sizeof(double) * ctx->periods.size(),
-                cudaMemcpyHostToDevice));
-  return RFS_OK;
-}
-
-// drops the per-set period table; the plan shares the Rc/Rg sequence again where the grid allows
-int drop_set_periods(rfs_ctx *ctx) {
-  if (!ctx->has_set_periods) return RFS_OK;
-  ctx->has_set_periods = false;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
-  if (!ctx->plan_unshared) return RFS_OK;
-  ctx->plan_unshared = false;
-  return rebuild_grid_plan(ctx, true);
 }
 
 }  // namespace
@@ -724,22 +769,32 @@ int rfs_config_swd_modes(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, 
   }
   const int nts[4] = {ntRc, ntRg, ntLc, ntLg};
   const double *ts[4] = {tRc, tRg, tLc, tLg};
-  // the per-set period table belongs to the previous grid (the plan below is built with sharing)
-  ctx->has_set_periods = ctx->plan_unshared = false;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
-  int rc = build_plan(ctx, ctx->plan, ctx->periods, nts, ts, mode, true);
+  // the new grid is built aside, and a larger period table is uploaded into a new buffer before the old
+  // one is released: a call that fails leaves the context as it was
+  SwdPlan plan;
+  std::vector<double> periods;
+  int rc = build_plan(ctx, plan, periods, nts, ts, mode, true);
   if (rc) return rc;
-  if (ctx->plan.ndata == 0) return fail(ctx, RFS_E_ARG, "no periods given");
+  if (plan.ndata == 0) return fail(ctx, RFS_E_ARG, "no periods given");
+  const size_t bytes = sizeof(double) * periods.size();
+  Buf grown;
+  Buf &dst = bytes <= ctx->d_periods.cap ? ctx->d_periods : grown;
+  if ((rc = ensure(ctx, dst, bytes))) return rc;
+  CK(cudaMemcpy(dst.p, periods.data(), bytes, cudaMemcpyHostToDevice));
+  if (grown.p) {
+    std::swap(ctx->d_periods.p, grown.p);
+    std::swap(ctx->d_periods.cap, grown.cap);
+  }
+  ctx->plan = plan;
+  ctx->periods.swap(periods);
   for (int w = 0; w < 4; w++) ctx->swd_nts[w] = nts[w];
-  if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * ctx->periods.size()))) return rc;
-  CK(cudaMemcpy(ctx->d_periods.p, ctx->periods.data(), sizeof(double) * ctx->periods.size(),
-                cudaMemcpyHostToDevice));
   ctx->n_swd = nlayer;
   ctx->mode = mode;
   ctx->modes.assign(modes, modes + nmodes);
   ctx->stale = stale ? 1 : 0;
   ctx->sphere = sphere ? 1 : 0;
   ctx->has_swd = true;
+  drop_tables(ctx, TAB_PERIODS);  // it marks periods of the previous grid
   return RFS_OK;
 }
 
@@ -754,13 +809,13 @@ int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, 
                        double gauss, double time_shift, double water, int rf_type, int method) {
   if (!ctx) return RFS_E_ARG;
   if (nray < 1 || nray > 64 || !ray_p) return fail(ctx, RFS_E_ARG, "bad ray-parameter list");
-  int rc = make_rf_cfg(ctx, ctx->rf, nlayer, nt, dt, gauss, time_shift, water, rf_type, method);
+  RfCfg cfg;
+  int rc = make_rf_cfg(ctx, cfg, nlayer, nt, dt, gauss, time_shift, water, rf_type, method);
   if (rc) return rc;
+  ctx->rf = cfg;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
-  ctx->has_set_rays = false;
-  ctx->has_set_rf = false;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
   ctx->has_rf = true;
+  drop_tables(ctx, TAB_RAYS | TAB_RF);  // both are laid out by the previous ray list and nt
   return RFS_OK;
 }
 
@@ -773,20 +828,16 @@ int rfs_config_rf(rfs_ctx *ctx, int nlayer, double ray_p, int nt, double dt, dou
 int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
                         const double *dobs, int ndobs) {
   if (!ctx || S < 1 || !sigma1 || !sigma2 || !dobs || ndobs <= 0) return RFS_E_ARG;
+  drop_tables(ctx, TAB_ALL);  // every table belongs to the sets held
   CK(cudaSetDevice(ctx->device));
-  int rc = drop_set_periods(ctx);
-  if (rc) return rc;
   const size_t bytes = sizeof(double) * (size_t)S * ndobs;
-  rc = ensure(ctx, ctx->d_dobs, bytes);
+  int rc = ensure(ctx, ctx->d_dobs, bytes);
   if (rc) return rc;
   CK(cudaMemcpy(ctx->d_dobs.p, dobs, bytes, cudaMemcpyHostToDevice));
   ctx->sigma1.assign(sigma1, sigma1 + S);
   ctx->sigma2.assign(sigma2, sigma2 + S);
   ctx->nsets = S;
   ctx->ndobs = ndobs;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
-  ctx->has_set_rays = false;
-  ctx->has_set_rf = false;
   ctx->has_obs = true;
   return RFS_OK;
 }
@@ -797,10 +848,8 @@ int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dob
 
 int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p) {
   if (!ctx) return RFS_E_ARG;
-  if (!ctx->has_rf) return fail(ctx, RFS_E_CONFIG, "per-set ray parameters need an RF configuration (rfs_config_rf)");
-  if (!ctx->has_obs || S != ctx->nsets)
-    return fail(ctx, RFS_E_CONFIG, "ray-parameter table for " + std::to_string(S) + " sets, the context holds " +
-                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
+  int rc = begin_table(ctx, TAB_RAYS, "ray-parameter table", ctx->has_rf, "an RF configuration (rfs_config_rf)", S);
+  if (rc) return rc;
   if (nray != (int)ctx->ray_ps.size())
     return fail(ctx, RFS_E_ARG, "ray-parameter table has " + std::to_string(nray) + " rays per set, the RF " +
                                     "objective has " + std::to_string(ctx->ray_ps.size()));
@@ -810,67 +859,42 @@ int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p) {
     if (!(isfinite(ray_p[i]) && ray_p[i] > 0.0))
       return fail(ctx, RFS_E_ARG, "ray parameters must be finite and > 0");
   CK(cudaSetDevice(ctx->device));
-  // a failed upload leaves no table: the context then uses the shared list, as after rfs_config_obs_sets
-  ctx->has_set_rays = false;
-  int rc = ensure(ctx, ctx->d_set_rays, sizeof(double) * cnt);
-  if (rc) return rc;
-  CK(cudaMemcpy(ctx->d_set_rays.p, ray_p, sizeof(double) * cnt, cudaMemcpyHostToDevice));
-  ctx->has_set_rays = true;
+  ObsTables &ot = ctx->tables;
+  if ((rc = ensure(ctx, ot.d_rays, sizeof(double) * cnt))) return rc;
+  CK(cudaMemcpy(ot.d_rays.p, ray_p, sizeof(double) * cnt, cudaMemcpyHostToDevice));
+  ot.has_rays = true;
   return RFS_OK;
 }
 
 int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use) {
   if (!ctx) return RFS_E_ARG;
-  if (!ctx->has_swd)
-    return fail(ctx, RFS_E_CONFIG, "per-set period lists need an SWD configuration (rfs_config_swd)");
-  if (!ctx->has_obs || S != ctx->nsets)
-    return fail(ctx, RFS_E_CONFIG, "period table for " + std::to_string(S) + " sets, the context holds " +
-                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
-  CK(cudaSetDevice(ctx->device));
-  // a failed call leaves no table: the context then evaluates every set on the grid lists
-  int rc = drop_set_periods(ctx);
+  int rc = begin_table(ctx, TAB_PERIODS, "period table", ctx->has_swd, "an SWD configuration (rfs_config_swd)", S);
   if (rc) return rc;
-  const int ng = ctx->plan.ndata;  // one mode block of the data vector
-  if (nper != ng)
-    return fail(ctx, RFS_E_ARG, "period mask has " + std::to_string(nper) + " entries per set, the SWD " +
-                                    "configuration has " + std::to_string(ng) + " periods");
-  if (!use) return fail(ctx, RFS_E_ARG, "no period mask");
-  std::vector<int> nobs(S, 0);
-  for (int st = 0; st < S; st++) {
-    for (int j = 0; j < ng; j++) {
-      const unsigned char u = use[(size_t)st * ng + j];
-      if (u > 1) return fail(ctx, RFS_E_ARG, "period mask values must be 0 or 1");
-      nobs[st] += u;
-    }
-    if (nobs[st] == 0)
-      return fail(ctx, RFS_E_ARG, "set " + std::to_string(st) + " observes no period (no periods given)");
-  }
+  ObsTables &ot = ctx->tables;
+  const SwdPlan &G = ctx->plan;
+  const int ng = G.ndata;  // one mode block of the data vector
+  if ((rc = check_mask(ctx, "period mask", "period", use, S, nper, ng, ot.nobs))) return rc;
   // the T sequence of Rc may serve Rg only where every set observes the same Rc and Rg periods
   bool share = true;
   for (int fam = 0; fam < 2; fam++) {
-    const SwdPlan &P = ctx->plan;
     int rc_row = -1, rg_row = -1;
-    for (int r = 0; r < P.nrow; r++) {
-      if (P.row[r].type == 2 * fam) rc_row = r;
-      if (P.row[r].type == 2 * fam + 1) rg_row = r;
+    for (int r = 0; r < G.nrow; r++) {
+      if (G.row[r].type == 2 * fam) rc_row = r;
+      if (G.row[r].type == 2 * fam + 1) rg_row = r;
     }
-    if (rc_row < 0 || rg_row < 0 || P.row[rc_row].s0 != P.row[rg_row].s0) continue;
-    const SwdRow &a = P.row[rc_row], &g = P.row[rg_row];
+    if (rc_row < 0 || rg_row < 0 || G.row[rc_row].s0 != G.row[rg_row].s0) continue;
+    const SwdRow &a = G.row[rc_row], &g = G.row[rg_row];
     for (int st = 0; st < S && share; st++)
       share = memcmp(use + (size_t)st * ng + a.d_off, use + (size_t)st * ng + g.d_off, a.nper) == 0;
   }
-  // from here on a failure restores the shared plan (drop_set_periods) and leaves no table
-  auto abandon = [&](int code) {
-    ctx->has_set_periods = true;
-    drop_set_periods(ctx);
-    return code;
-  };
-  ctx->plan_unshared = !share;
-  if (!share && (rc = rebuild_grid_plan(ctx, false))) return abandon(rc);
-  const SwdPlan &P = ctx->plan;
+  // the table's plan on the grid lists (the grid plan itself when sharing stays)
+  const double *ts[4];
+  for (int w = 0, o = 0; w < 4; o += ctx->swd_nts[w], w++) ts[w] = ctx->periods.data() + o;
+  std::vector<double> per;  // the grid lists, then each set's compact lists
+  if ((rc = build_plan(ctx, ot.plan, per, ctx->swd_nts, ts, ctx->mode, true, share))) return rc;
+  const SwdPlan &P = ot.plan;
   const int ld = 2 * P.nseq + 2 * ng;
   std::vector<int> tab((size_t)S * ld, 0);
-  std::vector<double> per = ctx->periods;  // the grid lists, then each set's compact lists
   for (int st = 0; st < S; st++) {
     const unsigned char *u = use + (size_t)st * ng;
     int *t = tab.data() + (size_t)st * ld;
@@ -891,57 +915,30 @@ int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *u
     }
     for (int j = 0; j < ng; j++) t[2 * P.nseq + ng + j] = u[j];
   }
-  if ((rc = ensure(ctx, ctx->d_periods, sizeof(double) * per.size())) ||
-      (rc = ensure(ctx, ctx->d_set_per, sizeof(int) * tab.size())))
-    return abandon(rc);
-  // the grid lists stay in front: without the table every kernel reads them as before
-  cudaError_t e = cudaMemcpy(ctx->d_periods.p, per.data(), sizeof(double) * per.size(), cudaMemcpyHostToDevice);
-  if (e == cudaSuccess)
-    e = cudaMemcpy(ctx->d_set_per.p, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice);
-  if (e != cudaSuccess) {
-    ctx->err = std::string("rfs_config_obs_periods: ") + cudaGetErrorString(e);
-    return abandon(RFS_E_CUDA);
-  }
-  ctx->set_per_ld = ld;
-  ctx->set_nobs = nobs;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
-  ctx->has_set_periods = true;
+  CK(cudaSetDevice(ctx->device));
+  if ((rc = ensure(ctx, ot.d_periods, sizeof(double) * per.size())) ||
+      (rc = ensure(ctx, ot.d_tab, sizeof(int) * tab.size())))
+    return rc;
+  CK(cudaMemcpy(ot.d_periods.p, per.data(), sizeof(double) * per.size(), cudaMemcpyHostToDevice));
+  CK(cudaMemcpy(ot.d_tab.p, tab.data(), sizeof(int) * tab.size(), cudaMemcpyHostToDevice));
+  ot.ld = ld;
+  ot.use_col = 2 * P.nseq + ng;
+  ot.has_periods = true;
   return RFS_OK;
 }
 
 int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char *use) {
   if (!ctx) return RFS_E_ARG;
-  // a failed call leaves no table: every set then fits every sample.  The joint weights follow the
-  // table, with or without it.
-  ctx->has_set_rf = false;
-  ctx->wt_n1 = ctx->wt_nsw = -1;
-  if (!ctx->has_rf)
-    return fail(ctx, RFS_E_CONFIG, "per-set RF samples need an RF configuration (rfs_config_rf)");
-  if (!ctx->has_obs || S != ctx->nsets)
-    return fail(ctx, RFS_E_CONFIG, "RF sample mask for " + std::to_string(S) + " sets, the context holds " +
-                                       std::to_string(ctx->has_obs ? ctx->nsets : 0));
-  const int n1 = ctx->rf.nt * (int)ctx->ray_ps.size();
-  if (nrf != n1)
-    return fail(ctx, RFS_E_ARG, "RF sample mask has " + std::to_string(nrf) + " entries per set, the RF " +
-                                    "objective has " + std::to_string(n1) + " samples (nray * nt)");
-  if (!use) return fail(ctx, RFS_E_ARG, "no RF sample mask");
-  std::vector<int> cnt(S, 0);
-  for (int st = 0; st < S; st++) {
-    for (int j = 0; j < n1; j++) {
-      const unsigned char u = use[(size_t)st * n1 + j];
-      if (u > 1) return fail(ctx, RFS_E_ARG, "RF sample mask values must be 0 or 1");
-      cnt[st] += u;
-    }
-    // no RF sample would give the set a zero joint weight, silently dropping its dispersion data
-    if (cnt[st] == 0) return fail(ctx, RFS_E_ARG, "set " + std::to_string(st) + " observes no RF sample");
-  }
-  CK(cudaSetDevice(ctx->device));
-  const size_t bytes = (size_t)S * n1;
-  int rc = ensure(ctx, ctx->d_set_rf, bytes);
+  int rc = begin_table(ctx, TAB_RF, "RF sample mask", ctx->has_rf, "an RF configuration (rfs_config_rf)", S);
   if (rc) return rc;
-  CK(cudaMemcpy(ctx->d_set_rf.p, use, bytes, cudaMemcpyHostToDevice));
-  ctx->set_n1 = cnt;
-  ctx->has_set_rf = true;
+  ObsTables &ot = ctx->tables;
+  // a set without RF samples would get a zero joint weight, silently dropping its dispersion data
+  if ((rc = check_mask(ctx, "RF sample mask", "RF sample", use, S, nrf, ndata_of(ctx, 1), ot.n1))) return rc;
+  CK(cudaSetDevice(ctx->device));
+  const size_t bytes = (size_t)S * nrf;
+  if ((rc = ensure(ctx, ot.d_rf, bytes))) return rc;
+  CK(cudaMemcpy(ot.d_rf.p, use, bytes, cudaMemcpyHostToDevice));
+  ot.has_rf = true;
   return RFS_OK;
 }
 
@@ -963,7 +960,7 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
   const int n = use_swd ? ctx->n_swd : rf.n;
   const int nray = use_rf ? (int)ctx->ray_ps.size() : 0;
   const int nmsel = use_swd ? (int)ctx->modes.size() : 0;
-  const int n1 = use_rf ? rf.nt * nray : 0, nsw = use_swd ? ctx->plan.ndata * nmsel : 0;
+  const int n1 = use_rf ? ndata_of(ctx, 1) : 0, nsw = use_swd ? ndata_of(ctx, 2) : 0;
   const int ndata = n1 + nsw;
   if (ctx->ndobs != ndata) return fail(ctx, RFS_E_CONFIG, "dobs length != ndata");
   CK(cudaSetDevice(ctx->device));
@@ -978,13 +975,15 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
   Bmax = std::min(Bmax, 2147483647LL / ((long long)SWD_NF * n));  // 32-bit offsets in SwdModel::ld
   const int nch = (int)((B + Bmax - 1) / Bmax);
   const long long Bch = (B + nch - 1) / nch;
+  const ObsTables &ot = ctx->tables;
   // the RF sample mask rides along for the RF residual kernels (ld n1: one set's RF block)
   const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata,
-                    use_rf && ctx->has_set_rf ? (const unsigned char *)ctx->d_set_rf.p : nullptr, n1};
-  // each row's own SWD period lists (rfs_config_obs_periods) for the rows of one chunk
+                    use_rf && ot.has_rf ? (const unsigned char *)ot.d_rf.p : nullptr, n1};
+  // the SWD stage runs the period table's plan when there is one, and each row's own period lists
+  // (rfs_config_obs_periods) for the rows of one chunk
+  const SwdGrid grid = swd_grid(ctx);
   auto set_view = [&](const int *chunk_set) {
-    return SwdSetView{ctx->has_set_periods ? (const int *)ctx->d_set_per.p : nullptr, chunk_set, ctx->nsets,
-                      ctx->set_per_ld};
+    return SwdSetView{ot.has_periods ? (const int *)ot.d_tab.p : nullptr, chunk_set, ctx->nsets, ot.ld};
   };
   double tshift = rf.tshift;
   if (rf.rf_type == 2) tshift = -tshift;  // src/RF/main.cpp:35
@@ -995,9 +994,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     for (int k = 0; k < ctx->nsets; k++) {
       const double q = ctx->sigma1[k] / ctx->sigma2[k];
       // with per-set period lists: the data count of set k's own lists, as a one-set context has it
-      const int nsw_k = ctx->has_set_periods ? nmsel * ctx->set_nobs[k] : nsw;
+      const int nsw_k = ot.has_periods ? nmsel * ot.nobs[k] : nsw;
       // likewise the set's own observed RF samples (rfs_config_obs_rf_samples)
-      const int n1_k = ctx->has_set_rf ? ctx->set_n1[k] : n1;
+      const int n1_k = ot.has_rf ? ot.n1[k] : n1;
       ctx->wt[k] = q * q * n1_k / nsw_k;
     }
     int rc;
@@ -1042,8 +1041,8 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     if (!use_swd) release_rf_branch(F, sk);
     if (use_swd) {
       if ((rc = make_blocks(ctx, F, (const double *)F.w_swd.p, Bc, n, ctx->sphere, blks[k], sk))) return rc;
-      if ((rc = run_swd_roots(ctx, F, ctx->plan, set_view(set ? set + off : nullptr),
-                              (const double *)ctx->d_periods.p, blks[k], Bc, n, multi_mode, sk)))
+      if ((rc = run_swd_roots(ctx, F, grid.plan, set_view(set ? set + off : nullptr), grid.periods, blks[k], Bc,
+                              n, multi_mode, sk)))
         return rc;
     }
     release_rf_branch(F, sk);
@@ -1087,8 +1086,8 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3)
       for (int ir = 0; ir < nray; ir++) {
         // obs_k.set: this chunk's rows, as the residual kernels read them
-        const RayView ray{ctx->has_set_rays ? (const double *)ctx->d_set_rays.p : nullptr, obs_k.set, ctx->nsets,
-                          nray, ir, ctx->ray_ps[ir]};
+        const RayView ray{ot.has_rays ? (const double *)ot.d_rays.p : nullptr, obs_k.set, ctx->nsets, nray, ir,
+                          ctx->ray_ps[ir]};
         if ((rc = run_rf_spectra(ctx, rf, ray, (const double *)F.w_rfm.p,
                                  (const double *)F.w_chain.p, nullptr, nullptr, Bc, n, rf_time ? 4 : 2, sigma,
                                  sr, rf_time ? RFS_PI64 : RFS_PI32)))
@@ -1113,8 +1112,7 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
     if (use_swd) {
       CK(cudaStreamWaitEvent(st, F.ev_ready, 0));
       const SwdSetView sv = set_view(obs_k.set);
-      if ((rc = run_swd_eigen(ctx, F, ctx->plan, sv, (const double *)ctx->d_periods.p, blks[k], Bc, n,
-                              multi_mode, st)))
+      if ((rc = run_swd_eigen(ctx, F, grid.plan, sv, grid.periods, blks[k], Bc, n, multi_mode, st)))
         return rc;
       SwdView V;
       V.blk = blks[k];
@@ -1122,11 +1120,11 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       V.croot = (const double *)F.w_croot.p;
       V.ugr = (const double *)ctx->w_ugr.p;
       V.kern = (const double *)ctx->w_kern.p;
-      V.periods = (const double *)ctx->d_periods.p;
+      V.periods = grid.periods;
       V.B = Bc;
       V.n = n;
       if (use_rf && ctx->overlap) CK(cudaStreamWaitEvent(st, ctx->ev_join, 0));
-      LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, ctx->plan, V, sv,
+      LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, grid.plan, V, sv,
              (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, which, n1,
              obs_k, (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p,
              U + off,
@@ -1156,8 +1154,7 @@ int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const 
         return fail(ctx, RFS_E_ARG, "set index " + std::to_string(set[b]) + " of row " + std::to_string(b) +
                                         " outside [0, " + std::to_string(ctx->nsets) + ")");
   const int n = use_swd ? ctx->n_swd : ctx->rf.n;
-  const int ndata = (use_rf ? ctx->rf.nt * (int)ctx->ray_ps.size() : 0) +
-                    (use_swd ? ctx->plan.ndata * (int)ctx->modes.size() : 0);
+  const int ndata = ndata_of(ctx, which);
   CK(cudaSetDevice(ctx->device));
   int rc;
   if ((rc = ensure(ctx, ctx->io_x, sizeof(double) * B * 2 * n))) return rc;
