@@ -68,6 +68,20 @@ int rfs_config_swd_modes(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, 
                          int nmodes, const int *modes, int sphere, int stale_group_kernel);
 int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int nt, double dt,
                        double gauss, double time_shift, double water, int rf_type, int method);
+/* Receiver functions at several Gaussian widths in one objective (RFs are usually inverted at two or
+ * three widths together, e.g. gauss = 1.0, 2.5, 5.0: low widths give stable traces, high widths resolve
+ * thin layers; the reference's ReceiverFunc holds one `gauss`).  gauss [ngauss] (host pointer), 1 <= ngauss
+ * <= 16, every width finite and > 0.  The RF data vector becomes [ray parameter][gauss][nt], so
+ * n_rf = nray * ngauss * nt (also in the joint weight); misfit and gradient are the sums over all (ray,
+ * width) traces.  nt, dt, time shift, water level, RF type and method are shared by every width.  Each
+ * trace equals the trace of a one-width configuration; the frequency method deconvolves every width of a
+ * ray on the same spectra and contracts the summed adjoint weights with the derivative spectra once.
+ * rfs_config_rf_rays is this call with ngauss = 1 (and, as before, no check of its one width).
+ * Returns RFS_E_ARG for a bad width list, and for everything rfs_config_rf_rays rejects.  Lifetime: see
+ * "Per-set tables" below (an rfs_config_rf* call). */
+int rfs_config_rf_gauss(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int ngauss,
+                        const double *gauss, int nt, double dt, double time_shift, double water,
+                        int rf_type, int method);
 /* dobs (host pointer): [nt_rf + n_swd] joint, or the matching sub-vector for which=1/2 */
 int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dobs, int ndobs);
 /* S observation sets ("stations", no reference counterpart: the reference inverts one station per run):
@@ -82,8 +96,8 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
  * parameters, SWD period lists or receiver-function samples.  Each table belongs to the sets held and to
  * the configuration it refines, and its lifetime follows one rule:
  *   - rfs_config_obs_sets and rfs_config_obs drop all three tables;
- *   - a successful rfs_config_rf or rfs_config_rf_rays drops the ray table and the RF-sample table, and
- *     keeps the period table;
+ *   - a successful rfs_config_rf, rfs_config_rf_rays or rfs_config_rf_gauss drops the ray table and the
+ *     RF-sample table, and keeps the period table;
  *   - a successful rfs_config_swd or rfs_config_swd_modes drops the period table, and keeps the other two;
  *   - each of the three calls below drops its own table first, so a call of it that fails leaves no such
  *     table, and it keeps the other two;
@@ -97,7 +111,7 @@ int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double 
 /* Per-set ray parameters of the RF objective (each station's stack has its own mean slowness; the
  * reference's ReceiverFunc.ray_p is per station): ray_p [S][nray] (host pointer, copied to the device
  * here, never during an evaluation).  Row b's pass ir then uses ray_p[set[b]][ir] in place of the
- * shared list of rfs_config_rf / rfs_config_rf_rays; everything else (nt, dt, gauss, time shift, water
+ * shared list of rfs_config_rf*, for every Gaussian width of that ray; everything else (nt, dt, gauss, time shift, water
  * level, RF type, method, layers, periods, modes) stays shared.  The evaluations and the HMC use the
  * table whenever it is present; their signatures do not change.  The librf drop-ins keep their own
  * ray_p argument.  A row with an out-of-range set index computes with the shared value.
@@ -119,8 +133,8 @@ int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p);
  * Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *use);
 /* Per-set receiver-function samples (missing ray-parameter bins, station-dependent fitting windows):
- * use [S][nrf] (host pointer, values 0 or 1, nrf = nray * nt, the RF block of the data vector in its
- * order [ray][sample]) marks the samples each set fits.  For a row of set s the RF misfit is
+ * use [S][nrf] (host pointer, values 0 or 1, nrf = nray * ngauss * nt, the RF block of the data vector in
+ * its order [ray][gauss][sample]) marks the samples each set fits.  For a row of set s the RF misfit is
  * 0.5 sum over observed samples (d - dobs)^2 and the adjoint source is zero at the others: the residual
  * there is selected as 0, never formed, so dobs may hold anything at unobserved samples (missing data
  * may be stored as NaN).  dsyn keeps the full synthetic trace at every sample; a failed row returns

@@ -60,6 +60,9 @@ def load_library():
         L.rfs_config_rf_rays.restype = C.c_int
         L.rfs_config_rf_rays.argtypes = [_vp, C.c_int, C.c_int, _dp, C.c_int, C.c_double, C.c_double,
                                          C.c_double, C.c_double, C.c_int, C.c_int]
+        L.rfs_config_rf_gauss.restype = C.c_int
+        L.rfs_config_rf_gauss.argtypes = [_vp, C.c_int, C.c_int, _dp, C.c_int, _dp, C.c_int, C.c_double,
+                                          C.c_double, C.c_double, C.c_int, C.c_int]
         L.rfs_config_obs.restype = C.c_int
         L.rfs_config_obs.argtypes = [_vp, C.c_double, C.c_double, _dp, C.c_int]
         L.rfs_misfit_grad_dev.restype = C.c_int
@@ -145,7 +148,7 @@ def exported_symbols():
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
             "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
-            "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples"]
+            "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples", "rfs_config_rf_gauss"]
 
 
 def _f64(a):
@@ -182,6 +185,7 @@ class Context:
         self.n_swd_data = 0
         self.nsets = 0
         self.nray = 0
+        self.ngauss = 0
 
     def close(self):
         if getattr(self, "h", None):
@@ -262,14 +266,26 @@ class Context:
 
     def config_rf(self, nlayer, ray_p, nt, dt, gauss, time_shift, water=0.001, rf_type="P", method="freq"):
         """ray_p: float (the reference's ReceiverFunc.ray_p) or a list (one objective over several ray
-        parameters; data vector [ray parameter][nt])."""
+        parameters; data vector [ray parameter][nt]).  gauss: float (the reference's ReceiverFunc.gauss)
+        or a list of Gaussian widths (one objective over all of them; data vector [ray][gauss][nt])."""
         rays = _f64(np.atleast_1d(ray_p))
-        self._ck(self.L.rfs_config_rf_rays(self.h, int(nlayer), rays.size, _p(rays), int(nt), float(dt),
-                                           float(gauss), float(time_shift), float(water),
-                                           rf_type_code(rf_type), method_code(method)))
+        if np.ndim(gauss) == 0:
+            self._ck(self.L.rfs_config_rf_rays(self.h, int(nlayer), rays.size, _p(rays), int(nt), float(dt),
+                                               float(gauss), float(time_shift), float(water),
+                                               rf_type_code(rf_type), method_code(method)))
+            ng = 1
+        else:
+            g = _f64(gauss)
+            if g.ndim != 1:
+                raise ValueError(f"gauss must be a number or a list of widths, got shape {g.shape}")
+            self._ck(self.L.rfs_config_rf_gauss(self.h, int(nlayer), rays.size, _p(rays), g.size, _p(g), int(nt),
+                                                float(dt), float(time_shift), float(water),
+                                                rf_type_code(rf_type), method_code(method)))
+            ng = g.size
         self.n = int(nlayer)
-        self.nt_rf = int(nt) * rays.size
+        self.nt_rf = int(nt) * rays.size * ng
         self.nray = rays.size
+        self.ngauss = ng
 
     def config_obs(self, dobs, sigma1=1.0, sigma2=1.0):
         """dobs [ndata]: one data vector.  dobs [S, ndata]: S observation sets (stations) sharing the
@@ -309,14 +325,16 @@ class Context:
         self._ck(self.L.rfs_config_obs_periods(self.h, u8.shape[0], u8.shape[1], u8.ctypes.data_as(_u8p)))
 
     def config_obs_rf_samples(self, use):
-        """Per-station receiver-function samples: use [S, nray * nt] or [S, nray, nt] (bool or 0/1) marks
-        the samples of the RF block of the data vector (order [ray][sample]) that each of the S
+        """Per-station receiver-function samples: use [S, nray * ngauss * nt], [S, nray, nt] or
+        [S, nray, ngauss, nt] (bool or 0/1) marks the samples of the RF block of the data vector (order
+        [ray][gauss][sample]) that each of the S
         observation sets held now fits.  The misfit sums over the observed samples only and dobs is never
         read at the others (NaN there is harmless); dsyn keeps the full traces.  config_obs and config_rf
         drop the table again."""
         u = np.asarray(use)
-        if u.ndim not in (2, 3) or u.shape[0] == 0:
-            raise ValueError(f"use must be [S, nray * nt] or [S, nray, nt], got shape {u.shape}")
+        if u.ndim not in (2, 3, 4) or u.shape[0] == 0:
+            raise ValueError(f"use must be [S, nray * ngauss * nt], [S, nray, nt] or [S, nray, ngauss, nt], "
+                             f"got shape {u.shape}")
         if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
             raise ValueError("use must hold booleans or 0/1")
         u8 = np.ascontiguousarray(u.reshape(u.shape[0], -1), dtype=np.uint8)

@@ -7,9 +7,11 @@ from ._lib import Context
 class JointEvaluator:
     """Many-chains Joint_RF_SWD.misfit_and_grad on one GPU with resident inputs/outputs.  dobs [ndata]
     or [S, ndata]: S observation sets (stations) sharing `cfg`; cfg's sigma1 / sigma2 may then be
-    [S] arrays.  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's ray_p.
-    obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set observes.
-    obs_rf_use [S, nray * nt] or [S, nray, nt]: the receiver-function samples each set fits."""
+    [S] arrays.  cfg's gauss may be a list of Gaussian widths: the RF block of the data vector is then
+    [ray][gauss][nt].  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's
+    ray_p (for every width).  obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set
+    observes.  obs_rf_use [S, nray * ngauss * nt], [S, nray, ngauss, nt] or [S, nray, nt]: the
+    receiver-function samples each set fits."""
 
     def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None, obs_rf_use=None):
         self.ctx = Context(device)

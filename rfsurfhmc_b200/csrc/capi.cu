@@ -108,6 +108,7 @@ struct rfs_ctx {
   bool has_rf = false;
   RfCfg rf;
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
+  GaussList gauss{1, {0.0}};   // its Gaussian widths (reference: one, rf.gauss)
   // ---- observations: nsets data vectors ("stations") of ndobs values each, and their per-set tables
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
@@ -252,10 +253,10 @@ int check_mask(rfs_ctx *ctx, const std::string &name, const char *what, const un
   return RFS_OK;
 }
 
-// Length of one set's data vector for `which` (0 joint, 1 RF, 2 SWD): the RF block [ray][nt], then the
-// SWD block [mode][grid periods].
+// Length of one set's data vector for `which` (0 joint, 1 RF, 2 SWD): the RF block [ray][gauss][nt],
+// then the SWD block [mode][grid periods].
 int ndata_of(const rfs_ctx *ctx, int which) {
-  return (which != 2 ? ctx->rf.nt * (int)ctx->ray_ps.size() : 0) +
+  return (which != 2 ? ctx->rf.nt * (int)ctx->ray_ps.size() * ctx->gauss.n : 0) +
          (which != 1 ? ctx->plan.ndata * (int)ctx->modes.size() : 0);
 }
 
@@ -574,23 +575,37 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const dou
   return RFS_OK;
 }
 
-size_t decon_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 6 * (size_t)n2 + 64); }
+// rf_decon_kernel's layout; more than one Gaussian width adds the weight accumulator (n2 complex)
+size_t decon_smem(int nft, int n2, int ngauss = 1) {
+  return sizeof(double) * (2 * (size_t)nft + (ngauss > 1 ? 8 : 6) * (size_t)n2 + 64);
+}
 int decon_threads(int nft) { return std::max(64, std::min(512, nft / 2)); }
 
-int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs,
-                 double *d_rf, long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag,
-                 double sigma, double tshift, cudaStream_t st, int accumulate = 0) {
-  const size_t sm = decon_smem(cfg.nft, cfg.n2);
+template <bool MULTI>
+int launch_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussList &gauss, long long B, int nrow,
+                    const ObsSets &obs, double *d_rf, long long ldrf, double *d_U, double *d_grad,
+                    unsigned char *d_flag, double sigma, double tshift, cudaStream_t st, int accumulate) {
+  const size_t sm = decon_smem(cfg.nft, cfg.n2, gauss.n);
   if (sm > 48 * 1024) {
-    CK(cudaFuncSetAttribute(rf_decon_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    CK(cudaFuncSetAttribute(rf_decon_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
+    CK(cudaFuncSetAttribute(rf_decon_kernel<MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
+    CK(cudaFuncSetAttribute(rf_decon_kernel<MULTI>, cudaFuncAttributePreferredSharedMemoryCarveout,
                             cudaSharedmemCarveoutMaxShared));
   }
-  LAUNCH(rf_decon_kernel, (unsigned)B, decon_threads(cfg.nft), sm, st,
+  LAUNCH(rf_decon_kernel<MULTI>, (unsigned)B, decon_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, cfg.gauss, tshift, cfg.water, sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
+         cfg.logn, cfg.dt, gauss, tshift, cfg.water, sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
          (const double2 *)ctx->d_tw.p, accumulate);
   return RFS_OK;
+}
+// gauss: the widths, each one trace of d_rf / obs (cfg.gauss is not read)
+int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussList &gauss, long long B, int nrow,
+                 const ObsSets &obs, double *d_rf, long long ldrf, double *d_U, double *d_grad,
+                 unsigned char *d_flag, double sigma, double tshift, cudaStream_t st, int accumulate = 0) {
+  if (gauss.n > 1)
+    return launch_rf_decon<true>(ctx, cfg, gauss, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, sigma, tshift,
+                                 st, accumulate);
+  return launch_rf_decon<false>(ctx, cfg, gauss, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, sigma, tshift,
+                                st, accumulate);
 }
 
 size_t time_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 5 * (size_t)n2 + 64); }
@@ -599,9 +614,10 @@ size_t time_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 5
 int time_threads(int nft) { return std::max(64, std::min(256, nft / 8)); }
 
 // time-domain method: iterative deconvolution of the spectra in w_spec / w_dspec (sigma = 0)
-// nrow = 0 (receiver function only) or 4n (plus all Frechet traces -> w_rftr [B][4n][nt])
-int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, double *d_rf, long long ldrf,
-                double tshift, cudaStream_t st) {
+// nrow = 0 (receiver function only) or 4n (plus all Frechet traces -> w_rftr [B][4n][nt]); gauss: the
+// Gaussian width of this pass (cfg.gauss is not read)
+int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, double gauss, long long B, int nrow, double *d_rf,
+                long long ldrf, double tshift, cudaStream_t st) {
   int rc;
   if (nrow > 0)
     if ((rc = ensure(ctx, ctx->w_rftr, sizeof(double) * (size_t)B * nrow * cfg.nt))) return rc;
@@ -614,14 +630,15 @@ int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, double *d
   }
   LAUNCH(rf_time_kernel, (unsigned)(B * (nrow + 1)), time_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, cfg.gauss, tshift, d_rf, ldrf, (double *)ctx->w_rftr.p,
+         cfg.logn, cfg.dt, gauss, tshift, d_rf, ldrf, (double *)ctx->w_rftr.p,
          (const double2 *)ctx->d_tw.p);
   return RFS_OK;
 }
 
-// validated RF settings with the transform length derived from nt; ctx only receives the error message
+// validated RF settings with the transform length derived from nt; ctx only receives the error message.
+// ngauss: the number of Gaussian widths the frequency method deconvolves per block
 int make_rf_cfg(rfs_ctx *ctx, RfCfg &cfg, int n, int nt, double dt, double gauss, double time_shift,
-                double water, int rf_type, int method) {
+                double water, int rf_type, int method, int ngauss = 1) {
   if (rf_type != 1 && rf_type != 2) return fail(ctx, RFS_E_ARG, "rf_type should be one of [P,p,S,s]");
   if (method != 0 && method != 1) return fail(ctx, RFS_E_ARG, "method should be time or freq");
   if (nt < 1 || !(dt > 0.0) || n < 2) return fail(ctx, RFS_E_ARG, "bad nt/dt/nlayer");
@@ -636,8 +653,9 @@ int make_rf_cfg(rfs_ctx *ctx, RfCfg &cfg, int n, int nt, double dt, double gauss
     lg = 1;
   }
   const int n2 = nft / 2 + 1;
-  // this cap also bounds the twiddle table allocated in rfs_create (nft / 2 <= 2048 entries)
-  if (std::max(decon_smem(nft, n2), time_smem(nft, n2)) > 220 * 1024)
+  // this cap also bounds the twiddle table allocated in rfs_create (nft / 2 <= 2048 entries); at nft = 4096
+  // rf_decon_kernel takes 197 184 bytes with several widths, so the cap is the same for every width count
+  if (std::max(decon_smem(nft, n2, ngauss), time_smem(nft, n2)) > 220 * 1024)
     return fail(ctx, RFS_E_ARG, "nt too large (max 4096 samples after padding)");
   cfg = RfCfg{n, nt, nft, lg, n2, rf_type, method, dt, gauss, time_shift, water};
   return RFS_OK;
@@ -805,18 +823,38 @@ int rfs_config_swd(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, int nt
                               sphere, stale);
 }
 
-int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int nt, double dt,
-                       double gauss, double time_shift, double water, int rf_type, int method) {
-  if (!ctx) return RFS_E_ARG;
+// The one implementation of the rfs_config_rf* calls; the width list is checked by rfs_config_rf_gauss
+// (rfs_config_rf and rfs_config_rf_rays accept any one width, as they always have).
+static int config_rf(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int ngauss, const double *gauss,
+                     int nt, double dt, double time_shift, double water, int rf_type, int method) {
   if (nray < 1 || nray > 64 || !ray_p) return fail(ctx, RFS_E_ARG, "bad ray-parameter list");
   RfCfg cfg;
-  int rc = make_rf_cfg(ctx, cfg, nlayer, nt, dt, gauss, time_shift, water, rf_type, method);
+  int rc = make_rf_cfg(ctx, cfg, nlayer, nt, dt, gauss[0], time_shift, water, rf_type, method, ngauss);
   if (rc) return rc;
   ctx->rf = cfg;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
+  ctx->gauss.n = ngauss;
+  for (int i = 0; i < ngauss; i++) ctx->gauss.a[i] = gauss[i];
   ctx->has_rf = true;
-  drop_tables(ctx, TAB_RAYS | TAB_RF);  // both are laid out by the previous ray list and nt
+  drop_tables(ctx, TAB_RAYS | TAB_RF);  // both are laid out by the previous ray and width lists and nt
   return RFS_OK;
+}
+
+int rfs_config_rf_gauss(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int ngauss,
+                        const double *gauss, int nt, double dt, double time_shift, double water,
+                        int rf_type, int method) {
+  if (!ctx) return RFS_E_ARG;
+  if (ngauss < 1 || ngauss > RFS_MAX_GAUSS || !gauss)
+    return fail(ctx, RFS_E_ARG, "bad Gaussian-width list (1 to " + std::to_string(RFS_MAX_GAUSS) + " widths)");
+  for (int i = 0; i < ngauss; i++)
+    if (!(isfinite(gauss[i]) && gauss[i] > 0.0)) return fail(ctx, RFS_E_ARG, "Gaussian widths must be finite and > 0");
+  return config_rf(ctx, nlayer, nray, ray_p, ngauss, gauss, nt, dt, time_shift, water, rf_type, method);
+}
+
+int rfs_config_rf_rays(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int nt, double dt,
+                       double gauss, double time_shift, double water, int rf_type, int method) {
+  if (!ctx) return RFS_E_ARG;
+  return config_rf(ctx, nlayer, nray, ray_p, 1, &gauss, nt, dt, time_shift, water, rf_type, method);
 }
 
 int rfs_config_rf(rfs_ctx *ctx, int nlayer, double ray_p, int nt, double dt, double gauss,
@@ -1083,7 +1121,9 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
       unsigned char *fo = (which == 1) ? flag + off : nullptr;
       if (fo) CK(cudaMemsetAsync(fo, 1, Bc, sr));
       // one pass per ray parameter; misfit and gradient accumulate over the passes (the reference's
-      // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3)
+      // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3).  A ray
+      // pass covers every Gaussian width: its traces are [gauss][nt] of the data vector.
+      const int G = ctx->gauss.n;
       for (int ir = 0; ir < nray; ir++) {
         // obs_k.set: this chunk's rows, as the residual kernels read them
         const RayView ray{ot.has_rays ? (const double *)ot.d_rays.p : nullptr, obs_k.set, ctx->nsets, nray, ir,
@@ -1092,19 +1132,27 @@ int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const i
                                  (const double *)F.w_chain.p, nullptr, nullptr, Bc, n, rf_time ? 4 : 2, sigma,
                                  sr, rf_time ? RFS_PI64 : RFS_PI32)))
           return rc;
-        double *dsyn_r = dsyn + off * ndata + (size_t)ir * rf.nt;
+        double *dsyn_r = dsyn + off * ndata + (size_t)ir * G * rf.nt;
         ObsSets obs_r = obs_k;
-        obs_r.dobs += (size_t)ir * rf.nt;
-        if (obs_r.use) obs_r.use += (size_t)ir * rf.nt;
+        obs_r.dobs += (size_t)ir * G * rf.nt;
+        if (obs_r.use) obs_r.use += (size_t)ir * G * rf.nt;
         if (!rf_time) {
-          if ((rc = run_rf_decon(ctx, rf, Bc, 2 * n, obs_r, dsyn_r, ndata, Uo, go, fo, sigma, tshift, sr, ir > 0)))
+          if ((rc = run_rf_decon(ctx, rf, ctx->gauss, Bc, 2 * n, obs_r, dsyn_r, ndata, Uo, go, fo, sigma, tshift,
+                                 sr, ir > 0)))
             return rc;
         } else {
-          // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces
-          if ((rc = run_rf_time(ctx, rf, Bc, 4 * n, dsyn_r, ndata, tshift, sr))) return rc;
-          LAUNCH(rf_trace_grad_kernel, gridFor(Bc * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
-                 (const double *)F.w_chain.p, dsyn_r, (long long)ndata, obs_r, Bc, n, rf.nt, Uo, go, fo,
-                 ir > 0);
+          // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces of
+          // each width in turn from the same spectra
+          for (int ig = 0; ig < G; ig++) {
+            ObsSets obs_g = obs_r;
+            obs_g.dobs += (size_t)ig * rf.nt;
+            if (obs_g.use) obs_g.use += (size_t)ig * rf.nt;
+            double *dsyn_g = dsyn_r + (size_t)ig * rf.nt;
+            if ((rc = run_rf_time(ctx, rf, ctx->gauss.a[ig], Bc, 4 * n, dsyn_g, ndata, tshift, sr))) return rc;
+            LAUNCH(rf_trace_grad_kernel, gridFor(Bc * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
+                   (const double *)F.w_chain.p, dsyn_g, (long long)ndata, obs_g, Bc, n, rf.nt, Uo, go, fo,
+                   ir > 0 || ig > 0);
+          }
         }
       }
       if (sr != st) CK(cudaEventRecord(ctx->ev_join, sr));
@@ -1370,11 +1418,11 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
   if ((rc = ensure(ctx, ctx->io_b, sizeof(double) * B * nt))) return rc;
   const int nrow = 4 * n;
   if (method == 0) {
-    if ((rc = run_rf_time(ctx, cfg, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, tshift, st)))
+    if ((rc = run_rf_time(ctx, cfg, gauss, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, tshift, st)))
       return rc;
   } else {
-    if ((rc = run_rf_decon(ctx, cfg, B, 0, ObsSets{nullptr, nullptr, 1, 0}, (double *)ctx->io_b.p, nt, nullptr,
-                           nullptr, nullptr, sigma, tshift, st)))
+    if ((rc = run_rf_decon(ctx, cfg, GaussList{1, {gauss}}, B, 0, ObsSets{nullptr, nullptr, 1, 0},
+                           (double *)ctx->io_b.p, nt, nullptr, nullptr, nullptr, sigma, tshift, st)))
       return rc;
   }
   CK(cudaMemcpyAsync(rf, ctx->io_b.p, sizeof(double) * B * nt, cudaMemcpyDeviceToHost, st));

@@ -592,30 +592,49 @@ RFS_DEVINL double block_reduce(double v, double *red, bool is_max) {
   return r;
 }
 
-// ---- K4: one block per model: water-level deconvolution, c2r FFT, trace, misfit and (optional)
-// adjoint gradient.   dynamic smem: cd buf[nft] + cd s21[n2] + cd s22[n2] + cd wt[n2] + 32 doubles
-//   rf   : [B][ldrf>=nt]  obs.dobs: [nsets][ld >= nt] or NULL   U: [B]   grad: [B][nrow] (nrow = NQ*n)
-//   the residual is 0 at the samples the row's set does not fit (ObsSets::observed); rf is written whole
+// Gaussian widths of one RF objective (rfs_config_rf_gauss), passed by value: each width is one trace
+// of the data vector's [ray][gauss][nt] block
+#define RFS_MAX_GAUSS 16
+struct GaussList {
+  int n;
+  double a[RFS_MAX_GAUSS];
+};
+
+// ---- K4: one block per (model, ray pass): water-level deconvolution, c2r FFT, trace, misfit and
+// (optional) adjoint gradient, for every Gaussian width of the list on the same staged spectra.
+//   dynamic smem: cd buf[nft] + cd s21[n2] + cd s22[n2] + cd wt[n2] + 64 doubles, + cd acc[n2] for G > 1
+//   rf   : [B][ldrf >= G*nt], the widths' traces one after the other
+//   obs.dobs: [nsets][ld >= G*nt] or NULL   U: [B]   grad: [B][nrow] (nrow = NQ*n)
+//   the residual is 0 at the samples the row's set does not fit (ObsSets::observed, sample g*nt + t of
+//   width g); rf is written whole
 //   flag : [B] or NULL; only written (0) for a row whose observation-set index is out of range
+// The spectra, both water levels and the derivative spectra D do not depend on the width, and the
+// gradient sum_k Re(W_k D_jk) is linear in the adjoint weights W: the widths' weights are summed in acc
+// and contracted with D once.  With one width the weights go straight into wt.
+// MULTI = false runs gauss.a[0] only: without the width loop's state the kernel keeps 54 registers
+// (64 with it), which is the occupancy of the one-width objectives at small nt.
+template <bool MULTI>
 __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 *__restrict__ dspec,
                                 long long B, int nrow, int nt, int nft, int logn, double dt,
-                                double f0, double t0, double water, double sigma, ObsSets obs,
+                                GaussList gauss, double t0, double water, double sigma, ObsSets obs,
                                 double *__restrict__ rf, long long ldrf, double *__restrict__ U,
                                 double *__restrict__ grad, unsigned char *__restrict__ flag,
                                 const double2 *__restrict__ tw, int accumulate) {
   // accumulate != 0: U and grad are added to (second and later ray parameters of one objective)
   extern __shared__ double smem[];
   const int n2 = nft / 2 + 1;
+  const int G = MULTI ? gauss.n : 1;
   cd *buf = reinterpret_cast<cd *>(smem);
   cd *s21 = buf + nft;
   cd *s22 = s21 + n2;
   cd *wt = s22 + n2;
   double *red = reinterpret_cast<double *>(wt + n2);
+  cd *acc = G > 1 ? reinterpret_cast<cd *>(red + 64) : wt;  // adjoint weights summed over the widths
   const long long b = blockIdx.x;
   const int tid = threadIdx.x, nth = blockDim.x;
   const int set = obs.row_set(b);
   if (set < 0) {
-    for (int it = tid; it < nt; it += nth) rf[b * ldrf + it] = nan("");
+    for (int it = tid; it < G * nt; it += nth) rf[b * ldrf + it] = nan("");
     if (grad)
       for (int rr = tid; rr < nrow; rr += nth) grad[b * nrow + rr] = 0.0;
     if (tid == 0) {
@@ -634,73 +653,84 @@ __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 
     lmax = fmax(lmax, a.x * a.x + a.y * a.y);
   }
   const double wmax = block_reduce(lmax, red, true);
-  // spectral division (:393-401) into wt (free until the adjoint pass), then the c2r transform
-  for (int k = tid; k < n2; k += nth) {
-    const double w = 1.0 / nft / dt * k * 2.0 * RFS_PI32;
-    const double gx = w / 2 / f0;
-    const double g = exp(-(gx * gx));
-    const double wa = norm2(s21[k]);
-    const double fai = fmax(wa, water * wmax);
-    wt[k] = conj(s21[k]) * s22[k] * g * cis(-w * t0) / fai;
-  }
-  __syncthreads();
-  const cd *z = block_irfft<false>([&](int k) { return wt[k]; }, buf, nft, logn, tw);
-  // trace, residual, weighted residual (:404-407 and the adjoint source; the real sequence is kept in
-  // the .x of wt[0..nt), the rest of the padded sequence is zero)
-  double lsum = 0.0;
-  double *rsd = reinterpret_cast<double *>(wt);  // nt <= nft doubles fit in n2 complex entries
-  for (int it = tid; it < nft; it += nth) {
-    double rt = 0.0;
-    if (it < nt) {
-      const double e = exp(sigma * (-t0 + it * dt));
-      const double v = irfft_at(z, it) / nft / dt * e;
-      rf[b * ldrf + it] = v;
-      if (dobs) {
-        const double r = obs.observed(set, it) ? v - dobs[it] : 0.0;
-        lsum += r * r;
-        rt = r * e / dt;
-      }
+  // second water level on |R21^2|^2 (:410-413), for the adjoint weights of every width
+  double wmax2 = 0.0;
+  if (dobs && grad) {
+    double lmax2 = 0.0;
+    for (int k = tid; k < n2; k += nth) {
+      const double wa = norm2(s21[k]);
+      lmax2 = fmax(lmax2, wa * wa);
     }
-    rsd[it] = rt;
+    wmax2 = block_reduce(lmax2, red, true);
   }
-  if (dobs == nullptr) return;
-  const double ss = block_reduce(lsum, red, false);
-  if (tid == 0) U[b] = accumulate ? U[b] + 0.5 * ss : 0.5 * ss;
-  if (grad == nullptr) return;
+  for (int ig = 0; ig < G; ig++) {
+    if (ig > 0) __syncthreads();  // the previous width's reads of buf and wt are done
+    const double f0 = gauss.a[ig];
+    // spectral division (:393-401) into wt (free until the adjoint pass), then the c2r transform
+    for (int k = tid; k < n2; k += nth) {
+      const double w = 1.0 / nft / dt * k * 2.0 * RFS_PI32;
+      const double gx = w / 2 / f0;
+      const double g = exp(-(gx * gx));
+      const double wa = norm2(s21[k]);
+      const double fai = fmax(wa, water * wmax);
+      wt[k] = conj(s21[k]) * s22[k] * g * cis(-w * t0) / fai;
+    }
+    __syncthreads();
+    const cd *z = block_irfft<false>([&](int k) { return wt[k]; }, buf, nft, logn, tw);
+    // trace, residual, weighted residual (:404-407 and the adjoint source; the real sequence is kept in
+    // the .x of wt[0..nt), the rest of the padded sequence is zero)
+    double lsum = 0.0;
+    double *rsd = reinterpret_cast<double *>(wt);  // nt <= nft doubles fit in n2 complex entries
+    const int o = ig * nt;                         // this width's trace in rf, dobs and the sample mask
+    for (int it = tid; it < nft; it += nth) {
+      double rt = 0.0;
+      if (it < nt) {
+        const double e = exp(sigma * (-t0 + it * dt));
+        const double v = irfft_at(z, it) / nft / dt * e;
+        rf[b * ldrf + o + it] = v;
+        if (dobs) {
+          const double r = obs.observed(set, o + it) ? v - dobs[o + it] : 0.0;
+          lsum += r * r;
+          rt = r * e / dt;
+        }
+      }
+      rsd[it] = rt;
+    }
+    if (dobs == nullptr) continue;
+    const double ss = block_reduce(lsum, red, false);
+    if (tid == 0) U[b] = (accumulate || ig > 0) ? U[b] + 0.5 * ss : 0.5 * ss;
+    if (grad == nullptr) continue;
+    __syncthreads();
+    const cd *zr = block_rfft<false>([&](int t) { return rsd[t]; }, buf, nft, logn, tw);
+    // adjoint weights of this width
+    for (int k = tid; k < n2; k += nth) {
+      const double w = 1.0 / nft / dt * k * 2.0 * RFS_PI32;
+      const double gx = w / 2 / f0;
+      const double g = exp(-(gx * gx));
+      const cd sq = s21[k] * s21[k];
+      const double wa = norm2(sq);
+      const double fai = fmax(wa, water * wmax2);
+      const cd Mk = conj(sq) * g * cis(-w * t0) / fai;
+      const double ck = (k == 0 || k == nft / 2) ? 1.0 : 2.0;
+      cd rk = rfft_at<false>(zr, k, nft, tw);
+      if (k == 0 || k == nft / 2) rk.y = 0.0;
+      const cd wk = Mk * conj(rk) * (ck / nft);  // the residual sequence kept in wt has been consumed
+      acc[k] = ig > 0 ? acc[k] + wk : wk;
+    }
+  }
+  if (dobs == nullptr || grad == nullptr) return;
   __syncthreads();
-  const cd *zr = block_rfft<false>([&](int t) { return rsd[t]; }, buf, nft, logn, tw);
-  // second water level on |R21^2|^2 (:410-413) and adjoint weights
-  double lmax2 = 0.0;
-  for (int k = tid; k < n2; k += nth) {
-    const double wa = norm2(s21[k]);
-    lmax2 = fmax(lmax2, wa * wa);
-  }
-  const double wmax2 = block_reduce(lmax2, red, true);
-  for (int k = tid; k < n2; k += nth) {
-    const double w = 1.0 / nft / dt * k * 2.0 * RFS_PI32;
-    const double gx = w / 2 / f0;
-    const double g = exp(-(gx * gx));
-    const cd sq = s21[k] * s21[k];
-    const double wa = norm2(sq);
-    const double fai = fmax(wa, water * wmax2);
-    const cd Mk = conj(sq) * g * cis(-w * t0) / fai;
-    const double ck = (k == 0 || k == nft / 2) ? 1.0 : 2.0;
-    cd rk = rfft_at<false>(zr, k, nft, tw);
-    if (k == 0 || k == nft / 2) rk.y = 0.0;
-    wt[k] = Mk * conj(rk) * (ck / nft);  // the residual sequence kept in wt has been consumed by block_rfft
-  }
-  __syncthreads();
-  // grad_row = sum_k Re(wt_k D_row,k): one warp per row
+  // grad_row = sum_k Re(acc_k D_row,k): one warp per row
   const int lane = tid & 31, wid = tid >> 5, nw = nth >> 5;
   for (int rr = wid; rr < nrow; rr += nw) {
     const double2 *dp = dspec + (b * (long long)nrow + rr) * n2;
-    double acc = 0.0;
+    double acc_r = 0.0;
     for (int k = lane; k < n2; k += 32) {
       const double2 d = dp[k];
-      acc += wt[k].x * d.x - wt[k].y * d.y;
+      acc_r += acc[k].x * d.x - acc[k].y * d.y;
     }
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
-    if (lane == 0) grad[b * nrow + rr] = accumulate ? grad[b * nrow + rr] + acc : acc;
+    for (int o = 16; o > 0; o >>= 1) acc_r += __shfl_down_sync(0xffffffffu, acc_r, o);
+    if (lane == 0) grad[b * nrow + rr] = accumulate ? grad[b * nrow + rr] + acc_r : acc_r;
   }
 }
 

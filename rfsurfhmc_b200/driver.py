@@ -6,14 +6,16 @@ write `real_syn.npy`, per-chain result files and `misfit.npy [nchains, nsamples]
     torchrun --nproc-per-node 8 -m rfsurfhmc_b200.driver --sampler da --chains 16384
 
 `mpiexec -n N` of the reference becomes `--chains N`: all chains of a rank run at once on its GPU.
+In the parameter file, rf.ray_p may be a list of ray parameters and rf.gauss a list of Gaussian widths
+(e.g. `gauss: [1.0, 2.5]`): the receiver-function data are then one trace per (ray, width), in that order.
 
     python -m rfsurfhmc_b200.driver --param param.yaml --stations stations.npz --chains K
 
 inverts a station array instead: the observations of S stations come from the file (see
 model/stations.py: load_stations; the optional key ray_p [S] or [S, nray] gives each station its own
 ray parameter(s) in place of rf.ray_p, swd_use [S, nper] the periods of the swd lists it observes and
-rf_use [S, nray*nt] or [S, nray, nt] the receiver-function samples it fits: missing ray bins, fitting
-windows), K chains run per station, all S*K in one device run (sharded
+rf_use [S, nray*ngauss*nt] or [S, nray, ngauss, nt] ([S, nray, nt] with one width) the
+receiver-function samples it fits: missing ray bins, fitting windows), K chains run per station, all S*K in one device run (sharded
 over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
 import argparse
 import os
@@ -115,7 +117,8 @@ def main():
     ap.add_argument("--stations", default=None,
                     help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2], "
                          "ray_p [S] or [S,nray] in place of rf.ray_p, swd_use [S,nper] observed periods of the "
-                         "swd lists, rf_use [S,nray*nt] or [S,nray,nt] fitted RF samples): invert every station "
+                         "swd lists, rf_use [S,nray*ngauss*nt] or [S,nray,ngauss,nt] fitted RF samples): invert every "
+                         "station "
                          "instead of "
                          "observations synthesised from true_model")
     ap.add_argument("--no-chain-files", action="store_true")

@@ -4,9 +4,10 @@ Same constructor / `init(**kargs)` / `set_obsdata` / `set_thk` / `empirical_rela
 `misfit` / `misfit_and_grad` (3-tuple, no flag, as the reference).  `misfit_and_grad` runs the fused
 CUDA path (rfs_misfit_grad_host, which=1): propagator + spectral deconvolution + adjoint gradient.
 
-Extension: `ray_p` may be a list of ray parameters; the data vector is then the concatenation of one
-trace per ray parameter (`nt` counts all of them, `nt_trace` one trace) and misfit / gradient sum over
-them — one objective per chain instead of one model object per ray parameter."""
+Extensions: `ray_p` may be a list of ray parameters and `gauss` a list of Gaussian widths; the data
+vector is then the concatenation of one trace per (ray parameter, width) in the order [ray][gauss]
+(`nt` counts all of them, `nt_trace` one trace) and misfit / gradient sum over them — one objective per
+chain instead of one model object per ray parameter and width."""
 import numpy as np
 from .lib import librf
 from .._lib import Context
@@ -16,8 +17,10 @@ class ReceiverFunc:
     def __init__(self, ray_p, nt, dt, gauss, time_shift, water_level=0.001, type_="p", method="time"):
         self.ray_p = ray_p
         self.nray = int(np.size(ray_p))
+        self.ngauss = int(np.size(gauss))
         self.nt_trace = nt
-        self.nt = nt * self.nray          # data count (== nt for the reference's single ray parameter)
+        # data count (== nt for the reference's single ray parameter and width)
+        self.nt = nt * self.nray * self.ngauss
         self.dt = dt
         self.gauss = gauss
         self.time_shift = time_shift
@@ -59,7 +62,8 @@ class ReceiverFunc:
     def _config_fields(self, n):
         # every field the reference reads on each misfit_and_grad call (model_rf.py:137-197): changing
         # one of them after the first call re-configures the device context
-        return (n, tuple(np.atleast_1d(self.ray_p).tolist()), self.nt_trace, self.dt, self.gauss,
+        gauss = self.gauss if np.ndim(self.gauss) == 0 else tuple(np.asarray(self.gauss, dtype=np.float64).tolist())
+        return (n, tuple(np.atleast_1d(self.ray_p).tolist()), self.nt_trace, self.dt, gauss,
                 self.time_shift, self.water_level, self.rf_type, self.method)
 
     def _config_key(self, n):
@@ -89,10 +93,10 @@ class ReceiverFunc:
         vp, rho = self.empirical_relation(vs, deriv=False)
         qa = thk * 0 + 9999.
         qb = thk * 0 + 9999.
-        out = [librf.forward(thk, rho, vp, vs, qa, qb, float(p), self.nt_trace, self.dt, self.gauss,
+        out = [librf.forward(thk, rho, vp, vs, qa, qb, float(p), self.nt_trace, self.dt, float(g),
                              self.time_shift, self.method, self.water_level, self.rf_type)
-               for p in np.atleast_1d(self.ray_p)]
-        return out[0] if self.nray == 1 else np.hstack(out)
+               for p in np.atleast_1d(self.ray_p) for g in np.atleast_1d(self.gauss)]
+        return out[0] if len(out) == 1 else np.hstack(out)
 
     def misfit(self, x):
         d = self.forward(x)

@@ -15,14 +15,14 @@ With swd_use [S, nper] the template's four period lists are a common grid (nper 
 len(tLc) + len(tLg)) and station s observes the grid periods where swd_use[s] is true: dobs keeps the grid
 layout (its values at unobserved periods are ignored), synthetics are NaN there.
 
-With rf_use [S, nray * nt] (or [S, nray, nt]) station s fits the receiver-function samples where
-rf_use[s] is true: a missing ray-parameter bin is a ray whose trace is all false, a fitting window a run
-of true samples.  dobs keeps the full layout (its values at unobserved samples are never read, NaN is
+With rf_use [S, nray * ngauss * nt] (or [S, nray, ngauss, nt], or [S, nray, nt] with one Gaussian width)
+station s fits the receiver-function samples where rf_use[s] is true: a missing ray-parameter bin is a ray
+whose traces are all false, a fitting window a run of true samples.  dobs keeps the full layout (its values at unobserved samples are never read, NaN is
 fine) and the synthetics keep the full traces.  rf_time_window builds the mask from bounds in seconds.
 
 A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
 keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray], swd_use [S, nper] and
-rf_use [S, nray * nt] or [S, nray, nt].
+rf_use in one of the shapes above.
 """
 import copy
 import numpy as np
@@ -51,9 +51,9 @@ class StationArray:
         [S, nray] with the template's ray count; not for a SurfWD template.
         swd_use: None (every station observes every period) or [S, nper] bool / 0-1, the grid periods
         each station observes; for a Joint_RF_SWD or SurfWD template.
-        rf_use: None (every station fits every RF sample) or [S, nray * nt] / [S, nray, nt] bool / 0-1,
-        the receiver-function samples each station fits (see rf_time_window); for a Joint_RF_SWD or
-        ReceiverFunc template."""
+        rf_use: None (every station fits every RF sample) or [S, nray * ngauss * nt] / [S, nray, ngauss, nt]
+        ([S, nray, nt] with one width) bool / 0-1, the receiver-function samples each station fits (see
+        rf_time_window); for a Joint_RF_SWD or ReceiverFunc template."""
         if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
             raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
         self.template = model
@@ -131,8 +131,9 @@ class StationArray:
         """Single-station copy of the template holding station s's observations (and sigmas, and ray
         parameter(s): a scalar for one ray, a list otherwise).  With swd_use its SurfWD holds the
         station's subset period lists and its dispersion data only the observed values.  With rf_use its
-        ReceiverFunc holds only the station's observed rays (ray parameters and traces); a station that
-        fits part of a trace has no single-station model (ValueError)."""
+        ReceiverFunc holds only the station's observed rays and widths (ray parameters, widths and
+        traces); a station that fits part of a trace, or whose observed traces are not every observed
+        width of every observed ray, has no single-station model (ValueError)."""
         s = int(s)
         if not 0 <= s < self.nstations:
             raise IndexError(f"station {s} outside [0, {self.nstations})")
@@ -184,20 +185,28 @@ class StationArray:
         return c
 
     def _station_rf(self, rf, s):
-        """Station s's ReceiverFunc and the data positions of its observed rays' traces."""
+        """Station s's ReceiverFunc and the data positions of its observed traces."""
         c = _fresh_copy(rf)
         r = self.ray_p[s] if self.ray_p is not None else np.atleast_1d(np.asarray(rf.ray_p, dtype=np.float64))
         keep = np.ones(rf.nt, dtype=bool)
         if self.rf_use is not None:
-            u = self.rf_use[s].reshape(rf.nray, rf.nt_trace)
-            obs = u.all(axis=1)
-            if not np.array_equal(obs, u.any(axis=1)):
+            u = self.rf_use[s].reshape(rf.nray, rf.ngauss, rf.nt_trace)
+            obs = u.all(axis=2)
+            if not np.array_equal(obs, u.any(axis=2)):
                 raise ValueError(f"station {s} ({self.names[s]}) fits part of a receiver-function trace: no "
                                  "single-station ReceiverFunc fits a window, use station_view")
-            r = r[obs]
+            # a ReceiverFunc evaluates every width of every ray: the observed traces must be such a product
+            rays, widths = obs.any(axis=1), obs.any(axis=0)
+            if not np.array_equal(obs, np.outer(rays, widths)):
+                raise ValueError(f"station {s} ({self.names[s]}) observes different Gaussian widths on different "
+                                 "rays: no single-station ReceiverFunc fits that, use station_view")
+            r = r[rays]
             keep = u.reshape(-1)
             c.nray = int(r.size)
-            c.nt = c.nt_trace * c.nray
+            if np.ndim(rf.gauss) > 0:
+                c.gauss = np.asarray(rf.gauss, dtype=np.float64)[widths].tolist()
+            c.ngauss = int(widths.sum())
+            c.nt = c.nt_trace * c.nray * c.ngauss
         if self.ray_p is not None or self.rf_use is not None:
             c.ray_p = float(r[0]) if r.size == 1 else r.tolist()
         return c, keep
@@ -240,12 +249,16 @@ def station_periods(use, S, swd, where=""):
 
 
 def station_rf_samples(use, S, rf, where=""):
-    """rf_use [S, nray * nt] or [S, nray, nt] (bool or 0/1) of a ReceiverFunc template's data vector ->
-    bool [S, nray * nt]; the ValueError names the key 'rf_use' (after `where`)."""
+    """rf_use [S, nray * ngauss * nt], [S, nray, ngauss, nt] or, with one Gaussian width, [S, nray, nt]
+    (bool or 0/1) of a ReceiverFunc template's data vector -> bool [S, nray * ngauss * nt]; the ValueError
+    names the key 'rf_use' (after `where`)."""
     u = np.asarray(use)
-    if u.shape not in ((S, rf.nt), (S, rf.nray, rf.nt_trace)):
-        raise ValueError(f"{where}'rf_use' must have shape [{S}, {rf.nt}] or [{S}, {rf.nray}, {rf.nt_trace}], "
-                         f"got {u.shape}")
+    shapes = [(S, rf.nt), (S, rf.nray, rf.ngauss, rf.nt_trace)]
+    if rf.ngauss == 1:
+        shapes.append((S, rf.nray, rf.nt_trace))
+    if u.shape not in shapes:
+        raise ValueError(f"{where}'rf_use' must have shape " + " or ".join(
+            "[" + ", ".join(map(str, sh)) + "]" for sh in shapes) + f", got {u.shape}")
     if u.dtype != np.bool_ and not np.all((u == 0) | (u == 1)):
         raise ValueError(f"{where}'rf_use' must hold booleans or 0/1")
     u = np.ascontiguousarray(u.reshape(S, rf.nt), dtype=bool)
@@ -259,8 +272,9 @@ def station_rf_samples(use, S, rf, where=""):
 def rf_time_window(rf, lo, hi):
     """RF sample mask (rf_use) of the time windows lo <= t <= hi on a ReceiverFunc's trace axis
     t = arange(nt) * dt - time_shift (rf.t), in seconds.  lo, hi: [S] (every ray) or [S, nray]; a NaN
-    bound marks a ray the station does not observe.  A bound equal to a sample time, up to rounding
-    (1e-9 of dt), includes that sample.  Returns bool [S, nray * nt]."""
+    bound marks a ray the station does not observe.  A ray's bounds apply to every Gaussian width of
+    that ray.  A bound equal to a sample time, up to rounding (1e-9 of dt), includes that sample.
+    Returns bool [S, nray * ngauss * nt]."""
     lo = np.asarray(lo, dtype=np.float64)
     hi = np.asarray(hi, dtype=np.float64)
     if lo.shape != hi.shape or lo.ndim not in (1, 2) or (lo.ndim == 2 and lo.shape[1] != rf.nray):
@@ -272,7 +286,8 @@ def rf_time_window(rf, lo, hi):
     t = np.asarray(rf.t, dtype=np.float64)
     # comparisons with NaN are false: a NaN bound leaves its ray without samples
     u = (t >= lo[..., None] - eps) & (t <= hi[..., None] + eps)
-    return u.reshape(S, rf.nray * rf.nt_trace)
+    u = np.broadcast_to(u[:, :, None, :], (S, rf.nray, rf.ngauss, rf.nt_trace))
+    return np.ascontiguousarray(u.reshape(S, rf.nt))
 
 
 def station_rays(ray_p, S, nray, where=""):
@@ -292,8 +307,9 @@ def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None, rf=None)
     dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0), bounds [S, nparam, 2]
     (default: default_bounds [nparam, 2] for every station), ray_p [S] or [S, nray] (default None: the
     ray parameter(s) of the forward configuration), swd_use [S, nper] (default None: every period;
-    swd = the SurfWD whose period grid it marks) and rf_use [S, nray * nt] or [S, nray, nt] (default
-    None: every RF sample; rf = the ReceiverFunc whose data it marks).  Raises ValueError naming the
+    swd = the SurfWD whose period grid it marks) and rf_use [S, nray * ngauss * nt] or
+    [S, nray, ngauss, nt] ([S, nray, nt] with one width; default None: every RF sample; rf = the
+    ReceiverFunc whose data it marks).  Raises ValueError naming the
     bad key."""
     if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
         with np.load(src, allow_pickle=False) as f:
