@@ -38,12 +38,14 @@ struct Buf {
   }
 };
 
-// settings of one receiver-function run: the fused objective's (rfs_config_rf*) or one drop-in call's.
-// The ray parameter is passed on its own (RayView): the fused objective has a list of them, and may have
-// one list per observation set.
+// settings of one receiver-function run: the fused objective's (rfs_config_rf*) or one drop-in call's
+// (one Gaussian width).  t0: the time shift, negated for S receiver functions (src/RF/main.cpp:35);
+// sigma: the damping of the frequency method, 0 for the time method.  The ray parameter is passed on
+// its own (RayView): the fused objective has a list of them, and may have one list per observation set.
 struct RfCfg {
   int n = 0, nt = 0, nft = 0, logn = 0, n2 = 0, rf_type = 1, method = 1;
-  double dt = 0, gauss = 0, tshift = 0, water = 0.001;
+  double dt = 0, water = 0.001, t0 = 0, sigma = 0;
+  GaussList gauss{1, {0.0}};
 };
 
 // Per-set observation tables of the sets held (rfs_config_obs_rays / _periods / _rf_samples).  Each one
@@ -93,7 +95,6 @@ struct rfs_ctx {
   cudaStream_t stream = nullptr;  // used by the *_host entry points
   cudaStream_t stream2 = nullptr; // RF branch of the joint evaluation runs concurrently with SWD
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_asm = nullptr;
-  bool overlap = true;  // false only inside rfs_profile_eval, which serialises the RF branch
   // ---- SWD configuration
   bool has_swd = false;
   int n_swd = 0, mode = 0, stale = 1, sphere = 0;
@@ -106,9 +107,8 @@ struct rfs_ctx {
   int swd_nts[4] = {0, 0, 0, 0};
   // ---- RF configuration
   bool has_rf = false;
-  RfCfg rf;
+  RfCfg rf;                    // its Gaussian widths: rf.gauss (reference: one)
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
-  GaussList gauss{1, {0.0}};   // its Gaussian widths (reference: one, rf.gauss)
   // ---- observations: nsets data vectors ("stations") of ndobs values each, and their per-set tables
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
@@ -256,7 +256,7 @@ int check_mask(rfs_ctx *ctx, const std::string &name, const char *what, const un
 // Length of one set's data vector for `which` (0 joint, 1 RF, 2 SWD): the RF block [ray][gauss][nt],
 // then the SWD block [mode][grid periods].
 int ndata_of(const rfs_ctx *ctx, int which) {
-  return (which != 2 ? ctx->rf.nt * (int)ctx->ray_ps.size() * ctx->gauss.n : 0) +
+  return (which != 2 ? ctx->rf.nt * (int)ctx->ray_ps.size() * ctx->rf.gauss.n : 0) +
          (which != 1 ? ctx->plan.ndata * (int)ctx->modes.size() : 0);
 }
 
@@ -536,7 +536,7 @@ int run_swd(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, c
 // FFTs of run_rf_decon / run_rf_time read to cfg.nft, in order on `st`.
 int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const double *d_rfm,
                    const double *d_chain, const double *d_qa, const double *d_qb, long long B, int n,
-                   int nq, double sigma, cudaStream_t st, double pi_used = RFS_PI32) {
+                   int nq, cudaStream_t st, double pi_used = RFS_PI32) {
   int rc;
   if (ctx->tw_nft != cfg.nft) {  // not counted in rfs_launch_count
     fft_twiddle_kernel<<<(cfg.nft / 2 + 127) / 128, 128, 0, st>>>(cfg.nft, (double2 *)ctx->d_tw.p);
@@ -555,7 +555,7 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const dou
   const long long tot = B * n2;
 #define PROP(NM, NQ)                                                                             \
   LAUNCH((rf_propagate_kernel<NM, NQ>), gridFor(tot, 128), 128, 0, st,                           \
-         (const RfLayer *)ctx->w_rfl.p, d_chain, B, n, n2, cfg.nft, cfg.dt, ray, sigma,          \
+         (const RfLayer *)ctx->w_rfl.p, d_chain, B, n, n2, cfg.nft, cfg.dt, ray, cfg.sigma,      \
          pi_used, cfg.rf_type, (double2 *)ctx->w_spec.p, dsp)
 #define PROPQ(NM)    \
   if (nq == 2) {     \
@@ -575,6 +575,17 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const dou
   return RFS_OK;
 }
 
+// Dynamic shared memory above the default 48 KB needs an opt-in per kernel.  It also asks for the full
+// shared-memory carve-out (rf_time_kernel at nft = 2048: two ~100 KB blocks per SM instead of one).
+template <class K>
+int allow_smem(rfs_ctx *ctx, K kernel, size_t bytes) {
+  if (bytes > 48 * 1024) {
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+  }
+  return RFS_OK;
+}
+
 // rf_decon_kernel's layout; more than one Gaussian width adds the weight accumulator (n2 complex)
 size_t decon_smem(int nft, int n2, int ngauss = 1) {
   return sizeof(double) * (2 * (size_t)nft + (ngauss > 1 ? 8 : 6) * (size_t)n2 + 64);
@@ -582,30 +593,25 @@ size_t decon_smem(int nft, int n2, int ngauss = 1) {
 int decon_threads(int nft) { return std::max(64, std::min(512, nft / 2)); }
 
 template <bool MULTI>
-int launch_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussList &gauss, long long B, int nrow,
-                    const ObsSets &obs, double *d_rf, long long ldrf, double *d_U, double *d_grad,
-                    unsigned char *d_flag, double sigma, double tshift, cudaStream_t st, int accumulate) {
-  const size_t sm = decon_smem(cfg.nft, cfg.n2, gauss.n);
-  if (sm > 48 * 1024) {
-    CK(cudaFuncSetAttribute(rf_decon_kernel<MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    CK(cudaFuncSetAttribute(rf_decon_kernel<MULTI>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                            cudaSharedmemCarveoutMaxShared));
-  }
+int launch_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs, double *d_rf,
+                    long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
+                    int accumulate) {
+  const size_t sm = decon_smem(cfg.nft, cfg.n2, cfg.gauss.n);
+  int rc;
+  if ((rc = allow_smem(ctx, rf_decon_kernel<MULTI>, sm))) return rc;
   LAUNCH(rf_decon_kernel<MULTI>, (unsigned)B, decon_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, gauss, tshift, cfg.water, sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
+         cfg.logn, cfg.dt, cfg.gauss, cfg.t0, cfg.water, cfg.sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
          (const double2 *)ctx->d_tw.p, accumulate);
   return RFS_OK;
 }
-// gauss: the widths, each one trace of d_rf / obs (cfg.gauss is not read)
-int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussList &gauss, long long B, int nrow,
-                 const ObsSets &obs, double *d_rf, long long ldrf, double *d_U, double *d_grad,
-                 unsigned char *d_flag, double sigma, double tshift, cudaStream_t st, int accumulate = 0) {
-  if (gauss.n > 1)
-    return launch_rf_decon<true>(ctx, cfg, gauss, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, sigma, tshift,
-                                 st, accumulate);
-  return launch_rf_decon<false>(ctx, cfg, gauss, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, sigma, tshift,
-                                st, accumulate);
+// every width of cfg.gauss, each one trace of d_rf / obs
+int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs, double *d_rf,
+                 long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
+                 int accumulate = 0) {
+  if (cfg.gauss.n > 1)
+    return launch_rf_decon<true>(ctx, cfg, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
+  return launch_rf_decon<false>(ctx, cfg, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
 }
 
 size_t time_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 5 * (size_t)n2 + 64); }
@@ -614,83 +620,299 @@ size_t time_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 5
 int time_threads(int nft) { return std::max(64, std::min(256, nft / 8)); }
 
 // time-domain method: iterative deconvolution of the spectra in w_spec / w_dspec (sigma = 0)
-// nrow = 0 (receiver function only) or 4n (plus all Frechet traces -> w_rftr [B][4n][nt]); gauss: the
-// Gaussian width of this pass (cfg.gauss is not read)
-int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, double gauss, long long B, int nrow, double *d_rf,
-                long long ldrf, double tshift, cudaStream_t st) {
+// nrow = 0 (receiver function only) or 4n (plus all Frechet traces -> w_rftr [B][4n][nt]); ig: the
+// Gaussian width of this pass (cfg.gauss.a[ig])
+int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, int ig, long long B, int nrow, double *d_rf, long long ldrf,
+                cudaStream_t st) {
   int rc;
   if (nrow > 0)
     if ((rc = ensure(ctx, ctx->w_rftr, sizeof(double) * (size_t)B * nrow * cfg.nt))) return rc;
   const size_t sm = time_smem(cfg.nft, cfg.n2);
-  if (sm > 48 * 1024) {
-    CK(cudaFuncSetAttribute(rf_time_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-    // ask for the full shared-memory carve-out: two ~100 KB blocks per SM instead of one
-    CK(cudaFuncSetAttribute(rf_time_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                            cudaSharedmemCarveoutMaxShared));
-  }
+  if ((rc = allow_smem(ctx, rf_time_kernel, sm))) return rc;
   LAUNCH(rf_time_kernel, (unsigned)(B * (nrow + 1)), time_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, gauss, tshift, d_rf, ldrf, (double *)ctx->w_rftr.p,
+         cfg.logn, cfg.dt, cfg.gauss.a[ig], cfg.t0, d_rf, ldrf, (double *)ctx->w_rftr.p,
          (const double2 *)ctx->d_tw.p);
   return RFS_OK;
 }
 
-// validated RF settings with the transform length derived from nt; ctx only receives the error message.
-// ngauss: the number of Gaussian widths the frequency method deconvolves per block
-int make_rf_cfg(rfs_ctx *ctx, RfCfg &cfg, int n, int nt, double dt, double gauss, double time_shift,
-                double water, int rf_type, int method, int ngauss = 1) {
+// validated RF settings with the transform length, the signed time shift and the damping derived;
+// ctx only receives the error message.  The frequency method deconvolves every width of `gauss` per block.
+int make_rf_cfg(rfs_ctx *ctx, RfCfg &cfg, int n, int nt, double dt, const GaussList &gauss, double time_shift,
+                double water, int rf_type, int method) {
   if (rf_type != 1 && rf_type != 2) return fail(ctx, RFS_E_ARG, "rf_type should be one of [P,p,S,s]");
   if (method != 0 && method != 1) return fail(ctx, RFS_E_ARG, "method should be time or freq");
   if (nt < 1 || !(dt > 0.0) || n < 2) return fail(ctx, RFS_E_ARG, "bad nt/dt/nlayer");
   if (nmax_for(n) < 0) return fail(ctx, RFS_E_ARG, "too many layers (max 208)");
-  int nft = 1, lg = 0;
-  while (nft < nt) {
-    nft *= 2;
-    lg++;
-  }
-  if (nft < 2) {
-    nft = 2;
-    lg = 1;
-  }
-  const int n2 = nft / 2 + 1;
+  int lg = 1;  // nft: the smallest power of two >= max(nt, 2)
+  while ((1 << lg) < nt) lg++;
+  const int nft = 1 << lg, n2 = nft / 2 + 1;
   // this cap also bounds the twiddle table allocated in rfs_create (nft / 2 <= 2048 entries); at nft = 4096
   // rf_decon_kernel takes 197 184 bytes with several widths, so the cap is the same for every width count
-  if (std::max(decon_smem(nft, n2, ngauss), time_smem(nft, n2)) > 220 * 1024)
+  if (std::max(decon_smem(nft, n2, gauss.n), time_smem(nft, n2)) > 220 * 1024)
     return fail(ctx, RFS_E_ARG, "nt too large (max 4096 samples after padding)");
-  cfg = RfCfg{n, nt, nft, lg, n2, rf_type, method, dt, gauss, time_shift, water};
+  const double t0 = rf_type == 2 ? -time_shift : time_shift;  // src/RF/main.cpp:35
+  const double sigma = method == 0 ? 0.0 : 1.0 / dt / nft * 4.;
+  cfg = RfCfg{n, nt, nft, lg, n2, rf_type, method, dt, water, t0, sigma, gauss};
   return RFS_OK;
 }
 
-// bytes of workspace one model needs in the fused path (used to size chunks)
-// bytes of workspace one model needs in the fused path: front = model blocks + root-search results
-// (kept for the whole batch), back = eigen / RF workspaces (sized per chunk)
-size_t per_model_front_bytes(const rfs_ctx *ctx, int which) {
-  size_t s = 0;
-  const int n = (which != 1) ? ctx->n_swd : ctx->rf.n;
-  if (which != 1 && ctx->has_swd) {
-    const SwdPlan &P = swd_grid(ctx).plan;
-    const size_t nmo = ctx->modes.size() > 1 ? (size_t)P.nmode : 1;
-    s += sizeof(double) * ((size_t)SWD_NF * n * (ctx->sphere ? 5 : 1) + (1 + nmo) * (size_t)P.nsolve) +
-         sizeof(int) * ((size_t)3 * P.nseq + P.nsolve);  // ierr, sched key + perm, rstat
-  }
-  if (which != 2 && ctx->has_rf) s += sizeof(double) * (4 * (size_t)n);
-  return s + sizeof(double) * 2 * (size_t)n;
+// The checks of every evaluation of the objective (rfs_misfit_grad_sets_dev / _host, rfs_hmc_run_sets); entry
+// names the caller in the message about a missing set array.  n: layers, ndata: one set's data length.
+int check_objective(rfs_ctx *ctx, int which, bool has_set, const char *entry, int &n, int &ndata) {
+  if (which < 0 || which > 2) return fail(ctx, RFS_E_ARG, "which must be 0,1,2");
+  const bool use_swd = which != 1, use_rf = which != 2;
+  if ((use_swd && !ctx->has_swd) || (use_rf && !ctx->has_rf) || !ctx->has_obs)
+    return fail(ctx, RFS_E_CONFIG, "objective not configured (rfs_config_swd/rf/obs)");
+  if (!has_set && ctx->nsets > 1)
+    return fail(ctx, RFS_E_CONFIG, "the context holds " + std::to_string(ctx->nsets) +
+                                       " observation sets: call " + entry + " with a set array");
+  if (use_swd && use_rf && ctx->n_swd != ctx->rf.n) return fail(ctx, RFS_E_CONFIG, "SWD and RF layer counts differ");
+  n = use_swd ? ctx->n_swd : ctx->rf.n;
+  ndata = ndata_of(ctx, which);
+  if (ctx->ndobs != ndata) return fail(ctx, RFS_E_CONFIG, "dobs length != ndata");
+  return RFS_OK;
 }
-size_t per_model_bytes(const rfs_ctx *ctx, int which) {
-  size_t s = 0;
-  if (which != 1 && ctx->has_swd) {
-    const SwdPlan &P = swd_grid(ctx).plan;
-    const size_t nmo = ctx->modes.size() > 1 ? (size_t)P.nmode : 1;
-    s += sizeof(double) * (nmo * (size_t)P.nsolve + nmo * (size_t)P.nsolve * 4 * ctx->n_swd);
+
+// Constants of one fused evaluation, shared by its stages.  overlap: the RF branch of a joint evaluation
+// runs on stream2 and root searches on the front streams (false in rfs_profile_eval: every kernel alone).
+struct Eval {
+  long long B;
+  const double *x;
+  int which, n, ndata, n1, nsw, nray;
+  double *U, *grad, *dsyn;
+  unsigned char *flag;
+  cudaStream_t st;
+  bool overlap, use_swd, use_rf;
+  SwdGrid grid;  // the period table's plan when there is one (rfs_config_obs_periods)
+  ObsSets obs;   // the RF sample mask rides along for the RF residual kernels (ld n1: one set's RF block)
+  SwdSetView sv;  // each row's own period lists (rfs_config_obs_periods)
+  // several modes in one objective: solve all modes 0..max in one chained pass and pick the listed ones
+  bool multi_mode;
+  ModeSel msel;
+  int nch = 1;  // chunks of Bch rows (plan_chunks)
+  long long Bch = 0;
+
+  Eval(const rfs_ctx *ctx, long long B, const double *x, const int *set, int which, int n, int ndata, double *U,
+       double *grad, double *dsyn, unsigned char *flag, cudaStream_t st, bool overlap)
+      : B(B), x(x), which(which), n(n), ndata(ndata), U(U), grad(grad), dsyn(dsyn), flag(flag), st(st),
+        overlap(overlap), use_swd(which != 1), use_rf(which != 2), grid(swd_grid(ctx)) {
+    n1 = use_rf ? ndata_of(ctx, 1) : 0;
+    nsw = ndata - n1;
+    nray = use_rf ? (int)ctx->ray_ps.size() : 0;
+    const ObsTables &ot = ctx->tables;
+    obs = ObsSets{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata,
+                  use_rf && ot.has_rf ? (const unsigned char *)ot.d_rf.p : nullptr, n1};
+    sv = SwdSetView{ot.has_periods ? (const int *)ot.d_tab.p : nullptr, set, ctx->nsets, ot.ld};
+    const int nmsel = use_swd ? (int)ctx->modes.size() : 0;
+    multi_mode = nmsel > 1;
+    msel.n = use_swd ? nmsel : 1;
+    for (int i = 0; i < RFS_MAX_MODES; i++) msel.m[i] = multi_mode && i < nmsel ? ctx->modes[i] : 0;
   }
-  if (which != 2 && ctx->has_rf) {
+  // chunk k: rows [off, off + B) of the batch; obs and sv as its rows read them (set indices from off on)
+  struct Chunk {
+    int k;
+    long long off, B;
+    ObsSets obs;
+    SwdSetView sv;
+  };
+  Chunk chunk(int k) const {
+    Chunk c{k, (long long)k * Bch, 0, obs, sv};
+    c.B = std::min(Bch, B - c.off);
+    if (obs.set) c.obs.set = c.sv.set = obs.set + c.off;
+    return c;
+  }
+};
+
+// Trace (ray ir, width ig) of the RF block [ray][gauss][nt]: its observations, sample mask and synthetics
+struct RfTrace {
+  ObsSets obs;
+  double *dsyn;
+};
+RfTrace rf_trace(const RfCfg &rf, ObsSets obs, double *dsyn, int ir, int ig) {
+  const size_t o = ((size_t)ir * rf.gauss.n + ig) * rf.nt;
+  obs.dobs += o;
+  if (obs.use) obs.use += o;
+  return {obs, dsyn + o};
+}
+
+// Chunking.  Bytes of workspace per model: pmf for the front buffers (model blocks and root-search
+// results), kept for the whole batch; pm for the eigen / RF workspaces, sized per chunk against what is
+// left of the budget.  Chunks are balanced.
+void plan_chunks(const rfs_ctx *ctx, Eval &E) {
+  size_t pmf = sizeof(double) * 2 * (size_t)E.n, pm = 64;
+  if (E.use_swd) {
+    const SwdPlan &P = E.grid.plan;
+    const size_t nmo = E.multi_mode ? (size_t)P.nmode : 1;
+    pmf += sizeof(double) * ((size_t)SWD_NF * E.n * (ctx->sphere ? 5 : 1) + (1 + nmo) * (size_t)P.nsolve) +
+           sizeof(int) * ((size_t)3 * P.nseq + P.nsolve);  // ierr, sched key + perm, rstat
+    pm += sizeof(double) * (nmo * (size_t)P.nsolve + nmo * (size_t)P.nsolve * 4 * E.n);
+  }
+  if (E.use_rf) {
     const RfCfg &rf = ctx->rf;
-    s += sizeof(RfLayer) * (size_t)rf.n + sizeof(double2) * ((size_t)2 * rf.n2 + (size_t)2 * rf.n * rf.n2) +
-         sizeof(double) * (1 + 2 * (size_t)rf.n);
+    pmf += sizeof(double) * (4 * (size_t)rf.n);
+    pm += sizeof(RfLayer) * (size_t)rf.n + sizeof(double2) * ((size_t)2 * rf.n2 + (size_t)2 * rf.n * rf.n2) +
+          sizeof(double) * (1 + 2 * (size_t)rf.n);
     if (rf.method == 0)
-      s += sizeof(double2) * ((size_t)2 * rf.n * rf.n2) + sizeof(double) * ((size_t)4 * rf.n * rf.nt);
+      pm += sizeof(double2) * ((size_t)2 * rf.n * rf.n2) + sizeof(double) * ((size_t)4 * rf.n * rf.nt);
   }
-  return s + 64;
+  const size_t front_total = pmf * (size_t)E.B + (pmf * (size_t)E.B) / 8;
+  const size_t budget = std::max(ctx->ws_budget > front_total ? ctx->ws_budget - front_total : (size_t)0,
+                                 ctx->ws_budget / 4);
+  long long Bmax = (long long)std::max<size_t>(32, budget / (pm + pm / 8));
+  Bmax = std::min(Bmax, 2147483647LL / ((long long)SWD_NF * E.n));  // 32-bit offsets in SwdModel::ld
+  E.nch = (int)((E.B + Bmax - 1) / Bmax);
+  E.Bch = (E.B + E.nch - 1) / E.nch;
+}
+
+// the SWD weight of the joint objective per set, uploaded again when the data lengths change
+int upload_weights(rfs_ctx *ctx, const Eval &E) {
+  if (ctx->wt_n1 == E.n1 && ctx->wt_nsw == E.nsw) return RFS_OK;
+  const ObsTables &ot = ctx->tables;
+  ctx->wt.resize(ctx->nsets);
+  for (int k = 0; k < ctx->nsets; k++) {
+    const double q = ctx->sigma1[k] / ctx->sigma2[k];
+    // with per-set period lists: the data count of set k's own lists, as a one-set context has it
+    const int nsw_k = ot.has_periods ? E.msel.n * ot.nobs[k] : E.nsw;
+    // likewise the set's own observed RF samples (rfs_config_obs_rf_samples)
+    const int n1_k = ot.has_rf ? ot.n1[k] : E.n1;
+    ctx->wt[k] = q * q * n1_k / nsw_k;
+  }
+  int rc;
+  if ((rc = ensure(ctx, ctx->d_wt, sizeof(double) * ctx->nsets))) return rc;
+  CK(cudaMemcpyAsync(ctx->d_wt.p, ctx->wt.data(), sizeof(double) * ctx->nsets, cudaMemcpyHostToDevice, E.st));
+  ctx->wt_n1 = E.n1;
+  ctx->wt_nsw = E.nsw;
+  return RFS_OK;
+}
+
+// Pass A of chunk k: model blocks and root search.  The search runs on a (high-priority) front stream
+// for every chunk after the first, and for the first one too when an RF branch competes with it for the SMs.
+int front_pass(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, Front &F, SwdBlocks &blk) {
+  const int n = E.n;
+  const bool side = E.overlap && (E.nch > 1 || (E.use_swd && E.use_rf));
+  cudaStream_t sk = side ? ctx->stream_front[c.k % 3] : E.st;
+  if (sk != E.st) CK(cudaStreamWaitEvent(sk, ctx->ev_fork, 0));
+  int rc;
+  const size_t nB = (size_t)n * c.B;
+  if (E.use_swd && (rc = ensure(ctx, F.w_swd, sizeof(double) * SWD_NF * nB))) return rc;
+  if (E.use_rf && (rc = ensure(ctx, F.w_rfm, sizeof(double) * 4 * nB))) return rc;
+  if ((rc = ensure(ctx, F.w_chain, sizeof(double) * 2 * nB))) return rc;
+  LAUNCH(prep_models_kernel, gridFor(c.B * n, 256), 256, 0, sk, E.x + c.off * 2 * n, c.B, n,
+         E.use_swd ? (double *)F.w_swd.p : nullptr, E.use_rf ? (double *)F.w_rfm.p : nullptr,
+         (double *)F.w_chain.p);
+  if (!F.ev_prep) CK(cudaEventCreateWithFlags(&F.ev_prep, cudaEventDisableTiming));
+  if (!F.ev_ready) CK(cudaEventCreateWithFlags(&F.ev_ready, cudaEventDisableTiming));
+  F.prep_pending = true;  // recorded by launch_roots right before the search kernel, or just below
+  if (E.use_swd) {
+    if ((rc = make_blocks(ctx, F, (const double *)F.w_swd.p, c.B, n, ctx->sphere, blk, sk))) return rc;
+    if ((rc = run_swd_roots(ctx, F, E.grid.plan, c.sv, E.grid.periods, blk, c.B, n, E.multi_mode, sk)))
+      return rc;
+  }
+  release_rf_branch(F, sk);
+  CK(cudaEventRecord(F.ev_ready, sk));
+  return RFS_OK;
+}
+
+// RF branch of chunk k: one pass per ray parameter; misfit and gradient accumulate over the passes (the
+// reference's ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3).
+// A ray pass covers every Gaussian width: its traces are [gauss][nt] of the data vector.
+int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F) {
+  const int n = E.n;
+  const RfCfg &rf = ctx->rf;
+  int rc;
+  // the RF branch only needs the chunk's model blocks: it runs on a second stream, beside the
+  // (latency-bound, < 1 wave) root search and the eigen solves
+  const bool side = E.use_swd && E.overlap;
+  cudaStream_t sr = side ? ctx->stream2 : E.st;
+  // RF workspaces and outputs are shared by the chunks: wait for the previous chunk's assemble
+  if (side) CK(cudaStreamWaitEvent(sr, c.k == 0 ? ctx->ev_fork : ctx->ev_asm, 0));
+  CK(cudaStreamWaitEvent(sr, F.ev_prep, 0));
+  if (side) {
+    // The RF branch starts behind a 25 us hold kernel, so that the root search's blocks are placed on
+    // the SMs before the RF kernels' large grids.  Measured on a B200 in round 2 (tools/gpu_r2_x.sh at
+    // commit d506195; ms per step / e2e / HMC evaluations per s), first chunk's search on the caller's
+    // stream: 7.99-8.13 / 2.19 M / 1.86 M without the hold, 7.98 / 2.20 M / 1.92 M with it; on a front
+    // stream: 10.6 / 2.25 M / 1.87 M without, 8.00 / 2.31 M / 1.92 M with it (the arrangement used).
+    LAUNCH(rf_branch_hold_kernel, 1, 32, 0, sr, 25000u);
+  }
+  if ((rc = ensure(ctx, ctx->w_urf, sizeof(double) * c.B))) return rc;
+  if ((rc = ensure(ctx, ctx->w_grf, sizeof(double) * 2 * (size_t)n * c.B))) return rc;
+  double *Uo = (E.which == 1) ? E.U + c.off : (double *)ctx->w_urf.p;
+  double *go = (E.which == 1) ? E.grad + c.off * 2 * n : (double *)ctx->w_grf.p;
+  // RF only: every row succeeds except one whose set index is out of range (the RF kernels write its 0)
+  unsigned char *fo = (E.which == 1) ? E.flag + c.off : nullptr;
+  if (fo) CK(cudaMemsetAsync(fo, 1, c.B, sr));
+  double *dsyn = E.dsyn + c.off * E.ndata;
+  const bool rf_time = rf.method == 0;
+  for (int ir = 0; ir < E.nray; ir++) {
+    const RayView ray{ctx->tables.has_rays ? (const double *)ctx->tables.d_rays.p : nullptr, c.obs.set, ctx->nsets,
+                      E.nray, ir, ctx->ray_ps[ir]};
+    if ((rc = run_rf_spectra(ctx, rf, ray, (const double *)F.w_rfm.p, (const double *)F.w_chain.p, nullptr,
+                             nullptr, c.B, n, rf_time ? 4 : 2, sr, rf_time ? RFS_PI64 : RFS_PI32)))
+      return rc;
+    if (!rf_time) {
+      const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, 0);
+      if ((rc = run_rf_decon(ctx, rf, c.B, 2 * n, t.obs, t.dsyn, E.ndata, Uo, go, fo, sr, ir > 0))) return rc;
+      continue;
+    }
+    // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces of each
+    // width in turn from the same spectra
+    for (int ig = 0; ig < rf.gauss.n; ig++) {
+      const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, ig);
+      if ((rc = run_rf_time(ctx, rf, ig, c.B, 4 * n, t.dsyn, E.ndata, sr))) return rc;
+      LAUNCH(rf_trace_grad_kernel, gridFor(c.B * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
+             (const double *)F.w_chain.p, t.dsyn, (long long)E.ndata, t.obs, c.B, n, rf.nt, Uo, go, fo,
+             ir > 0 || ig > 0);
+    }
+  }
+  if (sr != E.st) CK(cudaEventRecord(ctx->ev_join, sr));
+  return RFS_OK;
+}
+
+// SWD back pass of chunk k on the caller's stream: the eigen solves, then (after the chunk's RF branch)
+// the assembly of the objective
+int swd_back_pass(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F, const SwdBlocks &blk) {
+  const int n = E.n;
+  CK(cudaStreamWaitEvent(E.st, F.ev_ready, 0));
+  int rc;
+  if ((rc = run_swd_eigen(ctx, F, E.grid.plan, c.sv, E.grid.periods, blk, c.B, n, E.multi_mode, E.st))) return rc;
+  const SwdView V{(const double *)F.w_croot.p, (const double *)ctx->w_ugr.p, (const double *)ctx->w_kern.p,
+                  E.grid.periods, c.B, n, blk, 0};
+  if (E.use_rf && E.overlap) CK(cudaStreamWaitEvent(E.st, ctx->ev_join, 0));
+  LAUNCH(joint_assemble_kernel, dim3(gridFor(c.B, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, E.st, E.grid.plan, V, c.sv,
+         (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, E.which, E.n1, c.obs,
+         (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p, E.U + c.off,
+         E.grad + c.off * 2 * n, E.dsyn + c.off * E.ndata, E.flag + c.off, E.msel);
+  CK(cudaEventRecord(ctx->ev_asm, E.st));
+  return RFS_OK;
+}
+
+// the fused evaluation behind rfs_misfit_grad_sets_dev (overlap) and rfs_profile_eval (no overlap)
+int misfit_grad(rfs_ctx *ctx, long long B, const double *x, const int *set, int which, double *U, double *grad,
+                double *dsyn, unsigned char *flag, cudaStream_t st, bool overlap) {
+  if (B <= 0) return RFS_OK;
+  int n, ndata, rc;
+  if ((rc = check_objective(ctx, which, set != nullptr, "rfs_misfit_grad_sets_dev", n, ndata))) return rc;
+  CK(cudaSetDevice(ctx->device));
+  Eval E(ctx, B, x, set, which, n, ndata, U, grad, dsyn, flag, st, overlap);
+  plan_chunks(ctx, E);
+  if (which == 0 && (rc = upload_weights(ctx, E))) return rc;
+  while ((int)ctx->fronts.size() < E.nch) ctx->fronts.push_back(std::make_unique<Front>());
+  std::vector<SwdBlocks> blks((size_t)E.nch);
+  // ---- pass A: model blocks and root search of EVERY chunk.  A chunk's root search is latency-bound
+  // when the chunk is small against the machine (n = 200: ~290 ms for anything up to ~25 k models), so
+  // the chunks' searches run concurrently instead of one after the other.
+  CK(cudaEventRecord(ctx->ev_fork, st));  // everything this call launches comes after what is on `st`
+  for (int k = 0; k < E.nch; k++)
+    if ((rc = front_pass(ctx, E, E.chunk(k), *ctx->fronts[k], blks[k]))) return rc;
+  // ---- pass B: the memory-hungry stages chunk by chunk (RF branch beside the SWD branch)
+  for (int k = 0; k < E.nch; k++) {
+    const Eval::Chunk c = E.chunk(k);
+    if (E.use_rf && (rc = rf_branch(ctx, E, c, *ctx->fronts[k]))) return rc;
+    if (E.use_swd && (rc = swd_back_pass(ctx, E, c, *ctx->fronts[k], blks[k]))) return rc;
+  }
+  return RFS_OK;
 }
 
 }  // namespace
@@ -828,13 +1050,13 @@ int rfs_config_swd(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, int nt
 static int config_rf(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int ngauss, const double *gauss,
                      int nt, double dt, double time_shift, double water, int rf_type, int method) {
   if (nray < 1 || nray > 64 || !ray_p) return fail(ctx, RFS_E_ARG, "bad ray-parameter list");
+  GaussList widths{ngauss, {}};
+  std::copy(gauss, gauss + ngauss, widths.a);
   RfCfg cfg;
-  int rc = make_rf_cfg(ctx, cfg, nlayer, nt, dt, gauss[0], time_shift, water, rf_type, method, ngauss);
+  int rc = make_rf_cfg(ctx, cfg, nlayer, nt, dt, widths, time_shift, water, rf_type, method);
   if (rc) return rc;
   ctx->rf = cfg;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
-  ctx->gauss.n = ngauss;
-  for (int i = 0; i < ngauss; i++) ctx->gauss.a[i] = gauss[i];
   ctx->has_rf = true;
   drop_tables(ctx, TAB_RAYS | TAB_RF);  // both are laid out by the previous ray and width lists and nt
   return RFS_OK;
@@ -983,204 +1205,7 @@ int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char 
 int rfs_misfit_grad_sets_dev(rfs_ctx *ctx, long long B, const double *x, const int *set, int which,
                              double *U, double *grad, double *dsyn, unsigned char *flag, void *stream) {
   if (!ctx) return RFS_E_ARG;
-  if (B <= 0) return RFS_OK;
-  if (which < 0 || which > 2) return fail(ctx, RFS_E_ARG, "which must be 0,1,2");
-  const bool use_swd = which != 1, use_rf = which != 2;
-  if ((use_swd && !ctx->has_swd) || (use_rf && !ctx->has_rf) || !ctx->has_obs)
-    return fail(ctx, RFS_E_CONFIG, "context not configured (rfs_config_swd/rf/obs)");
-  if (use_swd && use_rf && ctx->n_swd != ctx->rf.n)
-    return fail(ctx, RFS_E_CONFIG, "SWD and RF layer counts differ");
-  if (!set && ctx->nsets > 1)
-    return fail(ctx, RFS_E_CONFIG,
-                "the context holds " + std::to_string(ctx->nsets) +
-                    " observation sets: evaluate with rfs_misfit_grad_sets_dev/_host and a set index per row");
-  const RfCfg &rf = ctx->rf;
-  const int n = use_swd ? ctx->n_swd : rf.n;
-  const int nray = use_rf ? (int)ctx->ray_ps.size() : 0;
-  const int nmsel = use_swd ? (int)ctx->modes.size() : 0;
-  const int n1 = use_rf ? ndata_of(ctx, 1) : 0, nsw = use_swd ? ndata_of(ctx, 2) : 0;
-  const int ndata = n1 + nsw;
-  if (ctx->ndobs != ndata) return fail(ctx, RFS_E_CONFIG, "dobs length != ndata");
-  CK(cudaSetDevice(ctx->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  // chunking: the front buffers (model blocks, roots) are kept for the whole batch, the eigen / RF
-  // workspaces are sized per chunk against what is left of the budget; chunks are balanced
-  const size_t pm = per_model_bytes(ctx, which), pmf = per_model_front_bytes(ctx, which);
-  const size_t front_total = pmf * (size_t)B + (pmf * (size_t)B) / 8;
-  const size_t budget = std::max(ctx->ws_budget > front_total ? ctx->ws_budget - front_total : (size_t)0,
-                                 ctx->ws_budget / 4);
-  long long Bmax = (long long)std::max<size_t>(32, budget / (pm + pm / 8));
-  Bmax = std::min(Bmax, 2147483647LL / ((long long)SWD_NF * n));  // 32-bit offsets in SwdModel::ld
-  const int nch = (int)((B + Bmax - 1) / Bmax);
-  const long long Bch = (B + nch - 1) / nch;
-  const ObsTables &ot = ctx->tables;
-  // the RF sample mask rides along for the RF residual kernels (ld n1: one set's RF block)
-  const ObsSets obs{(const double *)ctx->d_dobs.p, set, ctx->nsets, ndata,
-                    use_rf && ot.has_rf ? (const unsigned char *)ot.d_rf.p : nullptr, n1};
-  // the SWD stage runs the period table's plan when there is one, and each row's own period lists
-  // (rfs_config_obs_periods) for the rows of one chunk
-  const SwdGrid grid = swd_grid(ctx);
-  auto set_view = [&](const int *chunk_set) {
-    return SwdSetView{ot.has_periods ? (const int *)ot.d_tab.p : nullptr, chunk_set, ctx->nsets, ot.ld};
-  };
-  double tshift = rf.tshift;
-  if (rf.rf_type == 2) tshift = -tshift;  // src/RF/main.cpp:35
-  const bool rf_time = use_rf && rf.method == 0;
-  const double sigma = rf_time ? 0.0 : 1.0 / rf.dt / rf.nft * 4.;
-  if (which == 0 && (ctx->wt_n1 != n1 || ctx->wt_nsw != nsw)) {
-    ctx->wt.resize(ctx->nsets);
-    for (int k = 0; k < ctx->nsets; k++) {
-      const double q = ctx->sigma1[k] / ctx->sigma2[k];
-      // with per-set period lists: the data count of set k's own lists, as a one-set context has it
-      const int nsw_k = ot.has_periods ? nmsel * ot.nobs[k] : nsw;
-      // likewise the set's own observed RF samples (rfs_config_obs_rf_samples)
-      const int n1_k = ot.has_rf ? ot.n1[k] : n1;
-      ctx->wt[k] = q * q * n1_k / nsw_k;
-    }
-    int rc;
-    if ((rc = ensure(ctx, ctx->d_wt, sizeof(double) * ctx->nsets))) return rc;
-    CK(cudaMemcpyAsync(ctx->d_wt.p, ctx->wt.data(), sizeof(double) * ctx->nsets, cudaMemcpyHostToDevice, st));
-    ctx->wt_n1 = n1;
-    ctx->wt_nsw = nsw;
-  }
-  // several modes in one objective: solve all modes 0..max in one chained pass and pick the listed ones
-  const bool multi_mode = use_swd && nmsel > 1;
-  ModeSel msel;
-  msel.n = use_swd ? nmsel : 1;
-  for (int i = 0; i < RFS_MAX_MODES; i++) msel.m[i] = 0;
-  if (multi_mode)
-    for (int i = 0; i < nmsel; i++) msel.m[i] = ctx->modes[i];
-  while ((int)ctx->fronts.size() < nch) ctx->fronts.push_back(std::make_unique<Front>());
-  std::vector<SwdBlocks> blks((size_t)nch);
-  // root searches on the (high-priority) front streams: always for chunks after the first, and for the
-  // first one too when an RF branch competes with it for the SMs
-  const bool side = ctx->overlap && (nch > 1 || (use_swd && use_rf));
-
-  // ---- pass A: model blocks and root search of EVERY chunk.  A chunk's root search is latency-bound
-  // when the chunk is small against the machine (n = 200: ~290 ms for anything up to ~25 k models), so
-  // the chunks' searches run concurrently instead of one after the other.
-  CK(cudaEventRecord(ctx->ev_fork, st));  // everything this call launches comes after what is on `st`
-  for (int k = 0; k < nch; k++) {
-    const long long off = (long long)k * Bch, Bc = std::min(Bch, B - off);
-    Front &F = *ctx->fronts[k];
-    cudaStream_t sk = side ? ctx->stream_front[k % 3] : st;
-    if (sk != st) CK(cudaStreamWaitEvent(sk, ctx->ev_fork, 0));
-    int rc;
-    const size_t nB = (size_t)n * Bc;
-    if (use_swd && (rc = ensure(ctx, F.w_swd, sizeof(double) * SWD_NF * nB))) return rc;
-    if (use_rf && (rc = ensure(ctx, F.w_rfm, sizeof(double) * 4 * nB))) return rc;
-    if ((rc = ensure(ctx, F.w_chain, sizeof(double) * 2 * nB))) return rc;
-    LAUNCH(prep_models_kernel, gridFor(Bc * n, 256), 256, 0, sk, x + off * 2 * n, Bc, n,
-           use_swd ? (double *)F.w_swd.p : nullptr, use_rf ? (double *)F.w_rfm.p : nullptr,
-           (double *)F.w_chain.p);
-    if (!F.ev_prep) CK(cudaEventCreateWithFlags(&F.ev_prep, cudaEventDisableTiming));
-    if (!F.ev_ready) CK(cudaEventCreateWithFlags(&F.ev_ready, cudaEventDisableTiming));
-    F.prep_pending = true;  // recorded by launch_roots right before the search kernel
-    if (!use_swd) release_rf_branch(F, sk);
-    if (use_swd) {
-      if ((rc = make_blocks(ctx, F, (const double *)F.w_swd.p, Bc, n, ctx->sphere, blks[k], sk))) return rc;
-      if ((rc = run_swd_roots(ctx, F, grid.plan, set_view(set ? set + off : nullptr), grid.periods, blks[k], Bc,
-                              n, multi_mode, sk)))
-        return rc;
-    }
-    release_rf_branch(F, sk);
-    CK(cudaEventRecord(F.ev_ready, sk));
-  }
-
-  // ---- pass B: the memory-hungry stages chunk by chunk (RF branch beside the SWD branch)
-  for (int k = 0; k < nch; k++) {
-    const long long off = (long long)k * Bch, Bc = std::min(Bch, B - off);
-    Front &F = *ctx->fronts[k];
-    int rc;
-    const size_t nB = (size_t)n * Bc;
-    ObsSets obs_k = obs;  // the set indices of this chunk's rows
-    if (set) obs_k.set = set + off;
-    if (use_rf) {
-      // the RF branch only needs the chunk's model blocks: it runs on a second stream, beside the
-      // (latency-bound, < 1 wave) root search and the eigen solves
-      cudaStream_t sr = st;
-      if (use_swd && ctx->overlap) {
-        sr = ctx->stream2;
-        // RF workspaces and outputs are shared by the chunks: wait for the previous chunk's assemble
-        CK(cudaStreamWaitEvent(sr, k == 0 ? ctx->ev_fork : ctx->ev_asm, 0));
-        CK(cudaStreamWaitEvent(sr, F.ev_prep, 0));
-        // The RF branch starts behind a 25 us hold kernel, so that the root search's blocks are placed on
-        // the SMs before the RF kernels' large grids.  Measured on a B200 in round 2 (tools/gpu_r2_x.sh at
-        // commit d506195; ms per step / e2e / HMC evaluations per s), first chunk's search on the caller's
-        // stream: 7.99-8.13 / 2.19 M / 1.86 M without the hold, 7.98 / 2.20 M / 1.92 M with it; on a front
-        // stream: 10.6 / 2.25 M / 1.87 M without, 8.00 / 2.31 M / 1.92 M with it (the arrangement used).
-        LAUNCH(rf_branch_hold_kernel, 1, 32, 0, sr, 25000u);
-      } else {
-        CK(cudaStreamWaitEvent(sr, F.ev_prep, 0));
-      }
-      if ((rc = ensure(ctx, ctx->w_urf, sizeof(double) * Bc))) return rc;
-      if ((rc = ensure(ctx, ctx->w_grf, sizeof(double) * 2 * nB))) return rc;
-      double *Uo = (which == 1) ? U + off : (double *)ctx->w_urf.p;
-      double *go = (which == 1) ? grad + off * 2 * n : (double *)ctx->w_grf.p;
-      // RF only: every row succeeds except one whose set index is out of range (the RF kernels write its 0)
-      unsigned char *fo = (which == 1) ? flag + off : nullptr;
-      if (fo) CK(cudaMemsetAsync(fo, 1, Bc, sr));
-      // one pass per ray parameter; misfit and gradient accumulate over the passes (the reference's
-      // ReceiverFunc has one ray parameter, model/model_rf.py:5-18; the list is BASELINE config 3).  A ray
-      // pass covers every Gaussian width: its traces are [gauss][nt] of the data vector.
-      const int G = ctx->gauss.n;
-      for (int ir = 0; ir < nray; ir++) {
-        // obs_k.set: this chunk's rows, as the residual kernels read them
-        const RayView ray{ot.has_rays ? (const double *)ot.d_rays.p : nullptr, obs_k.set, ctx->nsets, nray, ir,
-                          ctx->ray_ps[ir]};
-        if ((rc = run_rf_spectra(ctx, rf, ray, (const double *)F.w_rfm.p,
-                                 (const double *)F.w_chain.p, nullptr, nullptr, Bc, n, rf_time ? 4 : 2, sigma,
-                                 sr, rf_time ? RFS_PI64 : RFS_PI32)))
-          return rc;
-        double *dsyn_r = dsyn + off * ndata + (size_t)ir * G * rf.nt;
-        ObsSets obs_r = obs_k;
-        obs_r.dobs += (size_t)ir * G * rf.nt;
-        if (obs_r.use) obs_r.use += (size_t)ir * G * rf.nt;
-        if (!rf_time) {
-          if ((rc = run_rf_decon(ctx, rf, ctx->gauss, Bc, 2 * n, obs_r, dsyn_r, ndata, Uo, go, fo, sigma, tshift,
-                                 sr, ir > 0)))
-            return rc;
-        } else {
-          // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces of
-          // each width in turn from the same spectra
-          for (int ig = 0; ig < G; ig++) {
-            ObsSets obs_g = obs_r;
-            obs_g.dobs += (size_t)ig * rf.nt;
-            if (obs_g.use) obs_g.use += (size_t)ig * rf.nt;
-            double *dsyn_g = dsyn_r + (size_t)ig * rf.nt;
-            if ((rc = run_rf_time(ctx, rf, ctx->gauss.a[ig], Bc, 4 * n, dsyn_g, ndata, tshift, sr))) return rc;
-            LAUNCH(rf_trace_grad_kernel, gridFor(Bc * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
-                   (const double *)F.w_chain.p, dsyn_g, (long long)ndata, obs_g, Bc, n, rf.nt, Uo, go, fo,
-                   ir > 0 || ig > 0);
-          }
-        }
-      }
-      if (sr != st) CK(cudaEventRecord(ctx->ev_join, sr));
-    }
-    if (use_swd) {
-      CK(cudaStreamWaitEvent(st, F.ev_ready, 0));
-      const SwdSetView sv = set_view(obs_k.set);
-      if ((rc = run_swd_eigen(ctx, F, grid.plan, sv, grid.periods, blks[k], Bc, n, multi_mode, st)))
-        return rc;
-      SwdView V;
-      V.blk = blks[k];
-      V.fwd = 0;
-      V.croot = (const double *)F.w_croot.p;
-      V.ugr = (const double *)ctx->w_ugr.p;
-      V.kern = (const double *)ctx->w_kern.p;
-      V.periods = grid.periods;
-      V.B = Bc;
-      V.n = n;
-      if (use_rf && ctx->overlap) CK(cudaStreamWaitEvent(st, ctx->ev_join, 0));
-      LAUNCH(joint_assemble_kernel, dim3(gridFor(Bc, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, st, grid.plan, V, sv,
-             (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, which, n1,
-             obs_k, (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p,
-             U + off,
-             grad + off * 2 * n, dsyn + off * ndata, flag + off, msel);
-      CK(cudaEventRecord(ctx->ev_asm, st));
-    }
-  }
-  return RFS_OK;
+  return misfit_grad(ctx, B, x, set, which, U, grad, dsyn, flag, (cudaStream_t)stream, true);
 }
 
 int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
@@ -1192,19 +1217,14 @@ int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const 
                               double *U, double *grad, double *dsyn, unsigned char *flag) {
   if (!ctx) return RFS_E_ARG;
   if (B <= 0) return RFS_OK;
-  if (which < 0 || which > 2) return fail(ctx, RFS_E_ARG, "which must be 0,1,2");
-  const bool use_swd = which != 1, use_rf = which != 2;
-  if ((use_swd && !ctx->has_swd) || (use_rf && !ctx->has_rf))
-    return fail(ctx, RFS_E_CONFIG, "context not configured (rfs_config_swd/rf/obs)");
+  int n, ndata, rc;
+  if ((rc = check_objective(ctx, which, set != nullptr, "rfs_misfit_grad_sets_host", n, ndata))) return rc;
   if (set)
     for (long long b = 0; b < B; b++)
       if (set[b] < 0 || set[b] >= ctx->nsets)
         return fail(ctx, RFS_E_ARG, "set index " + std::to_string(set[b]) + " of row " + std::to_string(b) +
                                         " outside [0, " + std::to_string(ctx->nsets) + ")");
-  const int n = use_swd ? ctx->n_swd : ctx->rf.n;
-  const int ndata = ndata_of(ctx, which);
   CK(cudaSetDevice(ctx->device));
-  int rc;
   if ((rc = ensure(ctx, ctx->io_x, sizeof(double) * B * 2 * n))) return rc;
   if ((rc = ensure(ctx, ctx->io_U, sizeof(double) * B))) return rc;
   if ((rc = ensure(ctx, ctx->io_grad, sizeof(double) * B * 2 * n))) return rc;
@@ -1386,7 +1406,7 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
                      double water, int rf_type, int par_type, int nq, double *rf, double *drf) {
   if (!ctx) return RFS_E_ARG;
   RfCfg cfg;  // this call's settings; the fused objective's (ctx->rf) stay as they are
-  int rc = make_rf_cfg(ctx, cfg, n, nt, dt, gauss, time_shift, water, rf_type, method);
+  int rc = make_rf_cfg(ctx, cfg, n, nt, dt, GaussList{1, {gauss}}, time_shift, water, rf_type, method);
   if (rc) return rc;
   if (nq == 1 && (par_type < 1 || par_type > 4))
     return fail(ctx, RFS_E_ARG, "par_type should be one of [vp,vs,rho,thick]");
@@ -1408,21 +1428,16 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
   if ((rc = ensure(ctx, F.w_rfm, sizeof(double) * 6 * nB))) return rc;
   CK(cudaMemcpyAsync(F.w_rfm.p, blk.data(), sizeof(double) * 6 * nB, cudaMemcpyHostToDevice, st));
   const double *d_rfm = (const double *)F.w_rfm.p;
-  double tshift = time_shift;
-  if (rf_type == 2) tshift = -tshift;
-  const double sigma = (method == 0) ? 0.0 : 1.0 / dt / cfg.nft * 4.;
   if ((rc = run_rf_spectra(ctx, cfg, RayView{nullptr, nullptr, 0, 1, 0, ray_p}, d_rfm, nullptr, d_rfm + 4 * nB, d_rfm + 5 * nB, B, n,
-                           nq > 0 ? 4 : 0, sigma, st,
-                           (method == 0 && nq == 4) ? RFS_PI64 : RFS_PI32)))
+                           nq > 0 ? 4 : 0, st, (method == 0 && nq == 4) ? RFS_PI64 : RFS_PI32)))
     return rc;
   if ((rc = ensure(ctx, ctx->io_b, sizeof(double) * B * nt))) return rc;
   const int nrow = 4 * n;
   if (method == 0) {
-    if ((rc = run_rf_time(ctx, cfg, gauss, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, tshift, st)))
-      return rc;
+    if ((rc = run_rf_time(ctx, cfg, 0, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, st))) return rc;
   } else {
-    if ((rc = run_rf_decon(ctx, cfg, GaussList{1, {gauss}}, B, 0, ObsSets{nullptr, nullptr, 1, 0},
-                           (double *)ctx->io_b.p, nt, nullptr, nullptr, nullptr, sigma, tshift, st)))
+    if ((rc = run_rf_decon(ctx, cfg, B, 0, ObsSets{nullptr, nullptr, 1, 0}, (double *)ctx->io_b.p, nt, nullptr,
+                           nullptr, nullptr, st)))
       return rc;
   }
   CK(cudaMemcpyAsync(rf, ctx->io_b.p, sizeof(double) * B * nt, cudaMemcpyDeviceToHost, st));
@@ -1430,14 +1445,10 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
     if (method != 0) {
       if ((rc = ensure(ctx, ctx->w_rftr, sizeof(double) * (size_t)B * nrow * nt))) return rc;
       const size_t sm = decon_smem(cfg.nft, cfg.n2);
-      if (sm > 48 * 1024) {
-        CK(cudaFuncSetAttribute(rf_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm));
-        CK(cudaFuncSetAttribute(rf_trace_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                cudaSharedmemCarveoutMaxShared));
-      }
+      if ((rc = allow_smem(ctx, rf_trace_kernel, sm))) return rc;
       LAUNCH(rf_trace_kernel, (unsigned)(B * nrow), decon_threads(cfg.nft), sm, st,
              (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, nt, cfg.nft,
-             cfg.logn, dt, gauss, tshift, water, sigma, (double *)ctx->w_rftr.p,
+             cfg.logn, cfg.dt, cfg.gauss.a[0], cfg.t0, cfg.water, cfg.sigma, (double *)ctx->w_rftr.p,
              (const double2 *)ctx->d_tw.p);
     }
     if (nq == 4) {
@@ -1501,14 +1512,12 @@ int rfs_profile_eval(rfs_ctx *ctx, long long B, const double *x, int which, doub
                      long long *launches) {
   if (!ctx || !ms) return RFS_E_ARG;
   CK(cudaSetDevice(ctx->device));
-  const bool ov = ctx->overlap;
-  ctx->overlap = false;  // serialise the RF branch so that every kernel is timed alone
   ctx->prof = true;
   ctx->prof_recs.clear();
   ctx->prof_used = 0;
-  int rc = rfs_misfit_grad_dev(ctx, B, x, which, U, grad, dsyn, flag, stream);
+  // without overlap: the RF branch serialised, so that every kernel is timed alone
+  int rc = misfit_grad(ctx, B, x, nullptr, which, U, grad, dsyn, flag, (cudaStream_t)stream, false);
   ctx->prof = false;
-  ctx->overlap = ov;
   if (rc) return rc;
   CK(cudaStreamSynchronize((cudaStream_t)stream));
   for (int i = 0; i < RFS_PROF_NK; i++) ms[i] = 0.0;
