@@ -92,15 +92,15 @@ int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dob
  * rfs_hmc_run) returns RFS_E_CONFIG. */
 int rfs_config_obs_sets(rfs_ctx *ctx, int S, const double *sigma1, const double *sigma2,
                         const double *dobs, int ndobs);
-/* Per-set tables.  The three calls below give each of the S observation sets held its own ray
- * parameters, SWD period lists or receiver-function samples.  Each table belongs to the sets held and to
- * the configuration it refines, and its lifetime follows one rule:
- *   - rfs_config_obs_sets and rfs_config_obs drop all three tables;
- *   - a successful rfs_config_rf, rfs_config_rf_rays or rfs_config_rf_gauss drops the ray table and the
- *     RF-sample table, and keeps the period table;
- *   - a successful rfs_config_swd or rfs_config_swd_modes drops the period table, and keeps the other two;
- *   - each of the three calls below drops its own table first, so a call of it that fails leaves no such
- *     table, and it keeps the other two;
+/* Per-set tables.  The four calls below give each of the S observation sets held its own ray
+ * parameters, SWD period lists, receiver-function samples or Gaussian widths.  Each table belongs to the
+ * sets held and to the configuration it refines, and its lifetime follows one rule:
+ *   - rfs_config_obs_sets and rfs_config_obs drop all four tables;
+ *   - a successful rfs_config_rf, rfs_config_rf_rays or rfs_config_rf_gauss drops the ray table, the
+ *     RF-sample table and the width table, and keeps the period table;
+ *   - a successful rfs_config_swd or rfs_config_swd_modes drops the period table, and keeps the other three;
+ *   - each of the four calls below drops its own table first, so a call of it that fails leaves no such
+ *     table, and it keeps the other three;
  *   - a failed rfs_config_swd* or rfs_config_rf* changes nothing: the configuration and every table stay.
  * Without a table the context evaluates every set on the shared configuration.  Each call returns
  * RFS_E_CONFIG without the configuration its table refines or when S differs from the number of
@@ -145,6 +145,20 @@ int rfs_config_obs_periods(rfs_ctx *ctx, int S, int nper, const unsigned char *u
  * Returns RFS_E_ARG when nrf is wrong, use is NULL, a value is not 0 or 1, or a set observes no sample
  * (its joint weight would be zero).  Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char *use);
+/* Per-set Gaussian widths (an observed receiver function can only be fitted by a synthetic filtered with
+ * the Gaussian its data were processed with, and stations from different networks or catalogues come at
+ * different widths): gauss [S][ngauss] (host pointer, copied to the device here), ngauss the width count
+ * of rfs_config_rf*.  Trace (ray ir, width g) of a row of set s is deconvolved with gauss[s][g] in place
+ * of the shared width g, at every ray; the data vector keeps its layout [ray][gauss][nt].  A set that
+ * fits fewer widths drops the others with its RF-sample mask.  Row b of set s gives exactly (bit for bit)
+ * U, grad, dsyn and flag of a one-set context configured with rfs_config_rf_gauss on set s's widths, in
+ * that order, with everything else unchanged (ray table and RF-sample table included).  The joint weight
+ * does not change (n_rf counts samples, not widths).  SWD-only evaluations (which = 2) ignore the table;
+ * the librf drop-ins keep their scalar gauss.  A row with an out-of-range set index reads no width and
+ * is failed as described below.
+ * Returns RFS_E_ARG when ngauss differs from the configured width count, gauss is NULL or a value is not
+ * finite and > 0.  Lifetime: see "Per-set tables" above. */
+int rfs_config_obs_gauss(rfs_ctx *ctx, int S, int ngauss, const double *gauss);
 
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)

@@ -77,6 +77,8 @@ def load_library():
         L.rfs_config_obs_periods.argtypes = [_vp, C.c_int, C.c_int, _u8p]
         L.rfs_config_obs_rf_samples.restype = C.c_int
         L.rfs_config_obs_rf_samples.argtypes = [_vp, C.c_int, C.c_int, _u8p]
+        L.rfs_config_obs_gauss.restype = C.c_int
+        L.rfs_config_obs_gauss.argtypes = [_vp, C.c_int, C.c_int, _dp]
         L.rfs_misfit_grad_sets_dev.restype = C.c_int
         L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_sets_host.restype = C.c_int
@@ -148,7 +150,8 @@ def exported_symbols():
             "rfs_last_roots_sched", "rfs_profile_eval", "rfs_profile_kernel_name",
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
             "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
-            "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples", "rfs_config_rf_gauss"]
+            "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples", "rfs_config_rf_gauss",
+            "rfs_config_obs_gauss"]
 
 
 def _f64(a):
@@ -339,6 +342,17 @@ class Context:
             raise ValueError("use must hold booleans or 0/1")
         u8 = np.ascontiguousarray(u.reshape(u.shape[0], -1), dtype=np.uint8)
         self._ck(self.L.rfs_config_obs_rf_samples(self.h, u8.shape[0], u8.shape[1], u8.ctypes.data_as(_u8p)))
+
+    def config_obs_gauss(self, gauss):
+        """Per-station Gaussian widths: gauss [S] (one width per objective) or [S, ngauss], for the S
+        observation sets held now.  Row b's trace of width g is then deconvolved with gauss[set[b]][g] in
+        place of config_rf's shared width g; the data vector keeps its layout.  config_obs and config_rf
+        drop the table again."""
+        g = _f64(gauss)
+        if g.ndim not in (1, 2) or g.shape[0] == 0:
+            raise ValueError(f"gauss must be [S] or [S, ngauss], got shape {g.shape}")
+        ng = 1 if g.ndim == 1 else g.shape[1]
+        self._ck(self.L.rfs_config_obs_gauss(self.h, g.shape[0], ng, _p(g)))
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)

@@ -11,9 +11,11 @@ class JointEvaluator:
     [ray][gauss][nt].  obs_ray_p [S] or [S, nray]: each set's own ray parameter(s) in place of cfg's
     ray_p (for every width).  obs_swd_use [S, nper]: the periods of cfg's lists (the common grid) each set
     observes.  obs_rf_use [S, nray * ngauss * nt], [S, nray, ngauss, nt] or [S, nray, nt]: the
-    receiver-function samples each set fits."""
+    receiver-function samples each set fits.  obs_gauss [S] or [S, ngauss]: each set's own Gaussian
+    width(s) in place of cfg's gauss (for every ray)."""
 
-    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None, obs_rf_use=None):
+    def __init__(self, cfg, dobs, nlayer, device=0, which=0, obs_ray_p=None, obs_swd_use=None, obs_rf_use=None,
+                 obs_gauss=None):
         self.ctx = Context(device)
         self.which = which
         self.n = nlayer
@@ -31,6 +33,8 @@ class JointEvaluator:
             self.ctx.config_obs_periods(obs_swd_use)
         if obs_rf_use is not None:
             self.ctx.config_obs_rf_samples(obs_rf_use)
+        if obs_gauss is not None:
+            self.ctx.config_obs_gauss(obs_gauss)
         self.device = torch.device("cuda", device)
         self.ndata = self.ctx.ndata(which)
         self._out = None

@@ -48,7 +48,7 @@ struct RfCfg {
   GaussList gauss{1, {0.0}};
 };
 
-// Per-set observation tables of the sets held (rfs_config_obs_rays / _periods / _rf_samples).  Each one
+// Per-set observation tables of the sets held (rfs_config_obs_rays / _periods / _rf_samples / _gauss).  Each one
 // belongs to the sets and to one configuration; drop_tables is the only code that clears one.
 struct ObsTables {
   // ray parameters [nsets][nray], used in place of the shared list
@@ -67,6 +67,9 @@ struct ObsTables {
   bool has_rf = false;
   Buf d_rf;
   std::vector<int> n1;
+  // Gaussian widths [nsets][ngauss], used in place of the shared list (read through GaussView)
+  bool has_gauss = false;
+  Buf d_gauss;
 };
 
 }  // namespace
@@ -211,7 +214,7 @@ int fail(rfs_ctx *ctx, int code, const std::string &msg) {
   return code;
 }
 
-enum { TAB_RAYS = 1, TAB_PERIODS = 2, TAB_RF = 4, TAB_ALL = 7 };
+enum { TAB_RAYS = 1, TAB_PERIODS = 2, TAB_RF = 4, TAB_GAUSS = 8, TAB_ALL = 15 };
 
 // The only code that clears a per-set table.  The joint weights follow the period and RF-sample tables,
 // so their cache goes with any table.
@@ -220,10 +223,11 @@ void drop_tables(rfs_ctx *ctx, int which) {
   if (which & TAB_RAYS) ot.has_rays = false;
   if (which & TAB_PERIODS) ot.has_periods = false;
   if (which & TAB_RF) ot.has_rf = false;
+  if (which & TAB_GAUSS) ot.has_gauss = false;
   ctx->wt_n1 = ctx->wt_nsw = -1;
 }
 
-// Prologue of the three table setters.  It drops the table first, so that a call that fails leaves none.
+// Prologue of the table setters.  It drops the table first, so that a call that fails leaves none.
 int begin_table(rfs_ctx *ctx, int table, const std::string &name, bool configured, const char *config, int S) {
   drop_tables(ctx, table);
   if (!configured) return fail(ctx, RFS_E_CONFIG, name + " needs " + config);
@@ -593,25 +597,25 @@ size_t decon_smem(int nft, int n2, int ngauss = 1) {
 int decon_threads(int nft) { return std::max(64, std::min(512, nft / 2)); }
 
 template <bool MULTI>
-int launch_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs, double *d_rf,
-                    long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
+int launch_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussView &gv, long long B, int nrow, const ObsSets &obs,
+                    double *d_rf, long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
                     int accumulate) {
   const size_t sm = decon_smem(cfg.nft, cfg.n2, cfg.gauss.n);
   int rc;
   if ((rc = allow_smem(ctx, rf_decon_kernel<MULTI>, sm))) return rc;
   LAUNCH(rf_decon_kernel<MULTI>, (unsigned)B, decon_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, cfg.gauss, cfg.t0, cfg.water, cfg.sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
+         cfg.logn, cfg.dt, cfg.gauss, gv, cfg.t0, cfg.water, cfg.sigma, obs, d_rf, ldrf, d_U, d_grad, d_flag,
          (const double2 *)ctx->d_tw.p, accumulate);
   return RFS_OK;
 }
-// every width of cfg.gauss, each one trace of d_rf / obs
-int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, long long B, int nrow, const ObsSets &obs, double *d_rf,
-                 long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
+// every width of cfg.gauss (or of each row's set, gv), each one trace of d_rf / obs
+int run_rf_decon(rfs_ctx *ctx, const RfCfg &cfg, const GaussView &gv, long long B, int nrow, const ObsSets &obs,
+                 double *d_rf, long long ldrf, double *d_U, double *d_grad, unsigned char *d_flag, cudaStream_t st,
                  int accumulate = 0) {
   if (cfg.gauss.n > 1)
-    return launch_rf_decon<true>(ctx, cfg, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
-  return launch_rf_decon<false>(ctx, cfg, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
+    return launch_rf_decon<true>(ctx, cfg, gv, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
+  return launch_rf_decon<false>(ctx, cfg, gv, B, nrow, obs, d_rf, ldrf, d_U, d_grad, d_flag, st, accumulate);
 }
 
 size_t time_smem(int nft, int n2) { return sizeof(double) * (2 * (size_t)nft + 5 * (size_t)n2 + 64); }
@@ -621,9 +625,9 @@ int time_threads(int nft) { return std::max(64, std::min(256, nft / 8)); }
 
 // time-domain method: iterative deconvolution of the spectra in w_spec / w_dspec (sigma = 0)
 // nrow = 0 (receiver function only) or 4n (plus all Frechet traces -> w_rftr [B][4n][nt]); ig: the
-// Gaussian width of this pass (cfg.gauss.a[ig])
-int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, int ig, long long B, int nrow, double *d_rf, long long ldrf,
-                cudaStream_t st) {
+// Gaussian width of this pass (cfg.gauss.a[ig], or each row's set's width ig of gv)
+int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, const GaussView &gv, int ig, long long B, int nrow, double *d_rf,
+                long long ldrf, cudaStream_t st) {
   int rc;
   if (nrow > 0)
     if ((rc = ensure(ctx, ctx->w_rftr, sizeof(double) * (size_t)B * nrow * cfg.nt))) return rc;
@@ -631,7 +635,7 @@ int run_rf_time(rfs_ctx *ctx, const RfCfg &cfg, int ig, long long B, int nrow, d
   if ((rc = allow_smem(ctx, rf_time_kernel, sm))) return rc;
   LAUNCH(rf_time_kernel, (unsigned)(B * (nrow + 1)), time_threads(cfg.nft), sm, st,
          (const double2 *)ctx->w_spec.p, (const double2 *)ctx->w_dspec.p, B, nrow, cfg.nt, cfg.nft,
-         cfg.logn, cfg.dt, cfg.gauss.a[ig], cfg.t0, d_rf, ldrf, (double *)ctx->w_rftr.p,
+         cfg.logn, cfg.dt, gv, ig, cfg.gauss.a[ig], cfg.t0, d_rf, ldrf, (double *)ctx->w_rftr.p,
          (const double2 *)ctx->d_tw.p);
   return RFS_OK;
 }
@@ -845,6 +849,8 @@ int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F)
   if (fo) CK(cudaMemsetAsync(fo, 1, c.B, sr));
   double *dsyn = E.dsyn + c.off * E.ndata;
   const bool rf_time = rf.method == 0;
+  const GaussView gv{ctx->tables.has_gauss ? (const double *)ctx->tables.d_gauss.p : nullptr, c.obs.set, ctx->nsets,
+                     rf.gauss.n};
   for (int ir = 0; ir < E.nray; ir++) {
     const RayView ray{ctx->tables.has_rays ? (const double *)ctx->tables.d_rays.p : nullptr, c.obs.set, ctx->nsets,
                       E.nray, ir, ctx->ray_ps[ir]};
@@ -853,14 +859,14 @@ int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F)
       return rc;
     if (!rf_time) {
       const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, 0);
-      if ((rc = run_rf_decon(ctx, rf, c.B, 2 * n, t.obs, t.dsyn, E.ndata, Uo, go, fo, sr, ir > 0))) return rc;
+      if ((rc = run_rf_decon(ctx, rf, gv, c.B, 2 * n, t.obs, t.dsyn, E.ndata, Uo, go, fo, sr, ir > 0))) return rc;
       continue;
     }
     // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces of each
     // width in turn from the same spectra
     for (int ig = 0; ig < rf.gauss.n; ig++) {
       const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, ig);
-      if ((rc = run_rf_time(ctx, rf, ig, c.B, 4 * n, t.dsyn, E.ndata, sr))) return rc;
+      if ((rc = run_rf_time(ctx, rf, gv, ig, c.B, 4 * n, t.dsyn, E.ndata, sr))) return rc;
       LAUNCH(rf_trace_grad_kernel, gridFor(c.B * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
              (const double *)F.w_chain.p, t.dsyn, (long long)E.ndata, t.obs, c.B, n, rf.nt, Uo, go, fo,
              ir > 0 || ig > 0);
@@ -1045,6 +1051,13 @@ int rfs_config_swd(rfs_ctx *ctx, int nlayer, int ntRc, const double *tRc, int nt
                               sphere, stale);
 }
 
+// Gaussian widths must be finite and > 0 (rfs_config_rf_gauss, rfs_config_obs_gauss)
+static int check_widths(rfs_ctx *ctx, const double *gauss, size_t cnt) {
+  for (size_t i = 0; i < cnt; i++)
+    if (!(isfinite(gauss[i]) && gauss[i] > 0.0)) return fail(ctx, RFS_E_ARG, "Gaussian widths must be finite and > 0");
+  return RFS_OK;
+}
+
 // The one implementation of the rfs_config_rf* calls; the width list is checked by rfs_config_rf_gauss
 // (rfs_config_rf and rfs_config_rf_rays accept any one width, as they always have).
 static int config_rf(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, int ngauss, const double *gauss,
@@ -1058,7 +1071,7 @@ static int config_rf(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p, in
   ctx->rf = cfg;
   ctx->ray_ps.assign(ray_p, ray_p + nray);
   ctx->has_rf = true;
-  drop_tables(ctx, TAB_RAYS | TAB_RF);  // both are laid out by the previous ray and width lists and nt
+  drop_tables(ctx, TAB_RAYS | TAB_RF | TAB_GAUSS);  // laid out by the previous ray and width lists and nt
   return RFS_OK;
 }
 
@@ -1068,8 +1081,8 @@ int rfs_config_rf_gauss(rfs_ctx *ctx, int nlayer, int nray, const double *ray_p,
   if (!ctx) return RFS_E_ARG;
   if (ngauss < 1 || ngauss > RFS_MAX_GAUSS || !gauss)
     return fail(ctx, RFS_E_ARG, "bad Gaussian-width list (1 to " + std::to_string(RFS_MAX_GAUSS) + " widths)");
-  for (int i = 0; i < ngauss; i++)
-    if (!(isfinite(gauss[i]) && gauss[i] > 0.0)) return fail(ctx, RFS_E_ARG, "Gaussian widths must be finite and > 0");
+  int rc = check_widths(ctx, gauss, ngauss);
+  if (rc) return rc;
   return config_rf(ctx, nlayer, nray, ray_p, ngauss, gauss, nt, dt, time_shift, water, rf_type, method);
 }
 
@@ -1199,6 +1212,24 @@ int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char 
   if ((rc = ensure(ctx, ot.d_rf, bytes))) return rc;
   CK(cudaMemcpy(ot.d_rf.p, use, bytes, cudaMemcpyHostToDevice));
   ot.has_rf = true;
+  return RFS_OK;
+}
+
+int rfs_config_obs_gauss(rfs_ctx *ctx, int S, int ngauss, const double *gauss) {
+  if (!ctx) return RFS_E_ARG;
+  int rc = begin_table(ctx, TAB_GAUSS, "Gaussian-width table", ctx->has_rf, "an RF configuration (rfs_config_rf)", S);
+  if (rc) return rc;
+  if (ngauss != ctx->rf.gauss.n)
+    return fail(ctx, RFS_E_ARG, "Gaussian-width table has " + std::to_string(ngauss) + " widths per set, the RF " +
+                                    "objective has " + std::to_string(ctx->rf.gauss.n));
+  if (!gauss) return fail(ctx, RFS_E_ARG, "no Gaussian-width table");
+  const size_t cnt = (size_t)S * ngauss;
+  if ((rc = check_widths(ctx, gauss, cnt))) return rc;
+  CK(cudaSetDevice(ctx->device));
+  ObsTables &ot = ctx->tables;
+  if ((rc = ensure(ctx, ot.d_gauss, sizeof(double) * cnt))) return rc;
+  CK(cudaMemcpy(ot.d_gauss.p, gauss, sizeof(double) * cnt, cudaMemcpyHostToDevice));
+  ot.has_gauss = true;
   return RFS_OK;
 }
 
@@ -1433,10 +1464,11 @@ static int rf_common(rfs_ctx *ctx, long long B, int n, const double *thk, const 
     return rc;
   if ((rc = ensure(ctx, ctx->io_b, sizeof(double) * B * nt))) return rc;
   const int nrow = 4 * n;
+  const GaussView one{nullptr, nullptr, 1, 1};  // the call's one width, gauss
   if (method == 0) {
-    if ((rc = run_rf_time(ctx, cfg, 0, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, st))) return rc;
+    if ((rc = run_rf_time(ctx, cfg, one, 0, B, nq > 0 ? nrow : 0, (double *)ctx->io_b.p, nt, st))) return rc;
   } else {
-    if ((rc = run_rf_decon(ctx, cfg, B, 0, ObsSets{nullptr, nullptr, 1, 0}, (double *)ctx->io_b.p, nt, nullptr,
+    if ((rc = run_rf_decon(ctx, cfg, one, B, 0, ObsSets{nullptr, nullptr, 1, 0}, (double *)ctx->io_b.p, nt, nullptr,
                            nullptr, nullptr, st)))
       return rc;
   }

@@ -599,6 +599,19 @@ struct GaussList {
   int n;
   double a[RFS_MAX_GAUSS];
 };
+// Gaussian width g of each row: gauss[set[b]][g] of a per-set table (rfs_config_obs_gauss), or the shared
+// width.  Like RayView: set points at the rows of this launch (NULL: every row is set 0), and a row whose
+// set index lies outside [0, nsets) reads nothing from the table (the residual kernels fail that row).
+struct GaussView {
+  const double *tab;  // [nsets][G] or NULL (every row uses `shared`)
+  const int *set;     // [B] or NULL
+  int nsets, G;
+  RFS_DEVINL double row_a(long long b, int g, double shared) const {
+    if (!tab) return shared;
+    const int s = set ? set[b] : 0;
+    return (s >= 0 && s < nsets) ? tab[s * G + g] : shared;
+  }
+};
 
 // ---- K4: one block per (model, ray pass): water-level deconvolution, c2r FFT, trace, misfit and
 // (optional) adjoint gradient, for every Gaussian width of the list on the same staged spectra.
@@ -611,13 +624,15 @@ struct GaussList {
 // The spectra, both water levels and the derivative spectra D do not depend on the width, and the
 // gradient sum_k Re(W_k D_jk) is linear in the adjoint weights W: the widths' weights are summed in acc
 // and contracted with D once.  With one width the weights go straight into wt.
-// MULTI = false runs gauss.a[0] only: without the width loop's state the kernel keeps 54 registers
+// MULTI = false runs width 0 only: without the width loop's state the kernel keeps 54 registers
 // (64 with it), which is the occupancy of the one-width objectives at small nt.
+// gv: each set's own widths (rfs_config_obs_gauss) in place of gauss.a; rows of an out-of-range set
+// return above, before any width is read.
 template <bool MULTI>
 __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 *__restrict__ dspec,
                                 long long B, int nrow, int nt, int nft, int logn, double dt,
-                                GaussList gauss, double t0, double water, double sigma, ObsSets obs,
-                                double *__restrict__ rf, long long ldrf, double *__restrict__ U,
+                                GaussList gauss, GaussView gv, double t0, double water, double sigma,
+                                ObsSets obs, double *__restrict__ rf, long long ldrf, double *__restrict__ U,
                                 double *__restrict__ grad, unsigned char *__restrict__ flag,
                                 const double2 *__restrict__ tw, int accumulate) {
   // accumulate != 0: U and grad are added to (second and later ray parameters of one objective)
@@ -665,7 +680,7 @@ __global__ void rf_decon_kernel(const double2 *__restrict__ spec, const double2 
   }
   for (int ig = 0; ig < G; ig++) {
     if (ig > 0) __syncthreads();  // the previous width's reads of buf and wt are done
-    const double f0 = gauss.a[ig];
+    const double f0 = gv.row_a(b, ig, gauss.a[ig]);
     // spectral division (:393-401) into wt (free until the adjoint pass), then the c2r transform
     for (int k = tid; k < n2; k += nth) {
       const double w = 1.0 / nft / dt * k * 2.0 * RFS_PI32;

@@ -22,10 +22,12 @@ namespace rfs {
 //   residual power (Parseval)    sum |R|^2 = sum |U|^2 - 2 dt Re(P conj(UW)) + dt^2 |P|^2 W2
 // dynamic smem: cd buf[nft] + cd UW[n2] + cd P[n2] + double W2[n2] + 64 doubles   (74 KB at nft = 2048:
 // three blocks per SM; the twiddle table stays in global memory / L1)
+// Gaussian width: width ig of the block's row's set (GaussView, rfs_config_obs_gauss) or `shared`; a row of
+// an out-of-range set computes with `shared` and is failed by rf_trace_grad_kernel.
 __global__ void __launch_bounds__(256, 3) rf_time_kernel(const double2 *__restrict__ spec, const double2 *__restrict__ dspec,
                                long long B, int nrow, int nt, int nft, int logn, double dt,
-                               double f0, double tshift, double *__restrict__ rf, long long ldrf,
-                               double *__restrict__ traces, const double2 *__restrict__ tw) {
+                               GaussView gauss, int ig, double shared, double tshift, double *__restrict__ rf,
+                               long long ldrf, double *__restrict__ traces, const double2 *__restrict__ tw) {
   extern __shared__ double smem[];
   const int n2 = nft / 2 + 1;
   cd *buf = reinterpret_cast<cd *>(smem);
@@ -38,6 +40,7 @@ __global__ void __launch_bounds__(256, 3) rf_time_kernel(const double2 *__restri
   const int r = (int)(blockIdx.x % nrow1);
   const int tid = threadIdx.x, nth = blockDim.x;
   const double minderr = (double)0.001f;
+  const double f0 = gauss.row_a(b, ig, shared);
 
   // ---- spectra of u and w (the reference goes through the time domain: c2r drops Im of bins 0, N/2)
   double lpu = 0.0, lpw = 0.0;

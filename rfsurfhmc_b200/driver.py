@@ -13,9 +13,10 @@ In the parameter file, rf.ray_p may be a list of ray parameters and rf.gauss a l
 
 inverts a station array instead: the observations of S stations come from the file (see
 model/stations.py: load_stations; the optional key ray_p [S] or [S, nray] gives each station its own
-ray parameter(s) in place of rf.ray_p, swd_use [S, nper] the periods of the swd lists it observes and
+ray parameter(s) in place of rf.ray_p, swd_use [S, nper] the periods of the swd lists it observes,
 rf_use [S, nray*ngauss*nt] or [S, nray, ngauss, nt] ([S, nray, nt] with one width) the
-receiver-function samples it fits: missing ray bins, fitting windows), K chains run per station, all S*K in one device run (sharded
+receiver-function samples it fits: missing ray bins, fitting windows, and gauss [S] or [S, ngauss] its
+own Gaussian width(s) in place of rf.gauss: the widths its data were processed with), K chains run per station, all S*K in one device run (sharded
 over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
 import argparse
 import os
@@ -69,9 +70,10 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
         npairs = nchains
         ids, sidx = D.shard_chains(nchains), None
     else:
-        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray, model_swd, model_rf)
+        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray, model_swd, model_rf,
+                           model_rf.ngauss)
         model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"], st["ray_p"],
-                             st["swd_use"], st["rf_use"])
+                             st["swd_use"], st["rf_use"], st["gauss"])
         boundaries = st["bounds"]
         npairs = model.nstations * nchains
         sidx, ids = D.shard_station_chains(model.nstations, nchains)
@@ -117,7 +119,8 @@ def main():
     ap.add_argument("--stations", default=None,
                     help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2], "
                          "ray_p [S] or [S,nray] in place of rf.ray_p, swd_use [S,nper] observed periods of the "
-                         "swd lists, rf_use [S,nray*ngauss*nt] or [S,nray,ngauss,nt] fitted RF samples): invert every "
+                         "swd lists, rf_use [S,nray*ngauss*nt] or [S,nray,ngauss,nt] fitted RF samples, gauss [S] or "
+                         "[S,ngauss] in place of rf.gauss): invert every "
                          "station "
                          "instead of "
                          "observations synthesised from true_model")

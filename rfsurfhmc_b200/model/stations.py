@@ -2,11 +2,11 @@
 
 A station array is inverted station by station: each station has its own data vector (receiver
 function and dispersion curves), its own sigma1 / sigma2 and optionally its own ray parameter(s), its
-own subset of the dispersion periods and its own receiver-function samples, while the layer count, the
-period grid, modes and RF sampling are shared.  The reference runs one job per station; here one context holds every station's
+own subset of the dispersion periods, its own receiver-function samples and its own Gaussian width(s),
+while the layer count, the period grid, modes, the width count and RF sampling are shared.  The reference runs one job per station; here one context holds every station's
 observations and each evaluated row, or each HMC chain, names its station, so one device run fills the
 GPU with all of them (include/rfsurfhmc.h: rfs_config_obs_sets, rfs_config_obs_rays,
-rfs_config_obs_periods, rfs_config_obs_rf_samples).
+rfs_config_obs_periods, rfs_config_obs_rf_samples, rfs_config_obs_gauss).
 
     stations = StationArray(joint_model, dobs, ray_p=p)   # dobs [S, ndata], p [S] or [S, nray]
     HamitonianMC(stations, bounds, ...).sample_chains(ids, stations=station_of_each_chain)
@@ -20,9 +20,13 @@ station s fits the receiver-function samples where rf_use[s] is true: a missing 
 whose traces are all false, a fitting window a run of true samples.  dobs keeps the full layout (its values at unobserved samples are never read, NaN is
 fine) and the synthetics keep the full traces.  rf_time_window builds the mask from bounds in seconds.
 
+With gauss [S] or [S, ngauss] station s's receiver functions are computed with its own Gaussian widths
+(those its data were processed with) in place of the template's, one per template width: the width count
+stays shared, and a station that fits fewer widths drops the others with rf_use.
+
 A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
-keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray], swd_use [S, nper] and
-rf_use in one of the shapes above.
+keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray], swd_use [S, nper],
+rf_use in one of the shapes above and gauss [S] or [S, ngauss].
 """
 import copy
 import numpy as np
@@ -42,7 +46,7 @@ def _fresh_copy(m):
 
 class StationArray:
     def __init__(self, model, dobs, sigma1=None, sigma2=None, names=None, ray_p=None, swd_use=None,
-                 rf_use=None):
+                 rf_use=None, gauss=None):
         """model: a configured Joint_RF_SWD, ReceiverFunc or SurfWD; only its forward configuration is
         used (its own observations are ignored).  dobs [S, ndata] in the model's data layout.
         sigma1 / sigma2: scalars or [S] (default: the joint model's own, 1.0 for the others; they only
@@ -53,7 +57,9 @@ class StationArray:
         each station observes; for a Joint_RF_SWD or SurfWD template.
         rf_use: None (every station fits every RF sample) or [S, nray * ngauss * nt] / [S, nray, ngauss, nt]
         ([S, nray, nt] with one width) bool / 0-1, the receiver-function samples each station fits (see
-        rf_time_window); for a Joint_RF_SWD or ReceiverFunc template."""
+        rf_time_window); for a Joint_RF_SWD or ReceiverFunc template.
+        gauss: None (every station uses the template's Gaussian width(s)) or each station's own, [S] or
+        [S, ngauss] with the template's width count; not for a SurfWD template."""
         if not (hasattr(model, "_config_forward") and hasattr(model, "which")):
             raise TypeError("StationArray needs a Joint_RF_SWD, ReceiverFunc or SurfWD template")
         self.template = model
@@ -92,6 +98,12 @@ class StationArray:
             if not isinstance(rf, ReceiverFunc):
                 raise TypeError("rf_use needs a receiver-function template (Joint_RF_SWD or ReceiverFunc)")
             self.rf_use = station_rf_samples(rf_use, S, rf)
+        self.gauss = None
+        if gauss is not None:
+            rf = model.rfmodel if isinstance(model, Joint_RF_SWD) else model
+            if not isinstance(rf, ReceiverFunc):
+                raise TypeError("gauss needs a receiver-function template (Joint_RF_SWD or ReceiverFunc)")
+            self.gauss = station_gauss(gauss, S, rf.ngauss)
         self._ctx = None
         self._ctx_key = None
 
@@ -108,7 +120,8 @@ class StationArray:
         key = (type(self.template), self.template._config_fields(n), self.sigma1.tobytes(),
                self.sigma2.tobytes(), self.dobs.tobytes(), None if self.ray_p is None else self.ray_p.tobytes(),
                None if self.swd_use is None else self.swd_use.tobytes(),
-               None if self.rf_use is None else self.rf_use.tobytes())
+               None if self.rf_use is None else self.rf_use.tobytes(),
+               None if self.gauss is None else self.gauss.tobytes())
         if self._ctx_key != key:
             self.template._config_forward(self._ctx, n)
             self._ctx.config_obs(self.dobs, self.sigma1, self.sigma2)
@@ -118,6 +131,8 @@ class StationArray:
                 self._ctx.config_obs_periods(self.swd_use)
             if self.rf_use is not None:
                 self._ctx.config_obs_rf_samples(self.rf_use)
+            if self.gauss is not None:
+                self._ctx.config_obs_gauss(self.gauss)
             self._ctx_key = key
         return self._ctx
 
@@ -128,8 +143,9 @@ class StationArray:
         return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=self.which, sets=stations)
 
     def station_model(self, s):
-        """Single-station copy of the template holding station s's observations (and sigmas, and ray
-        parameter(s): a scalar for one ray, a list otherwise).  With swd_use its SurfWD holds the
+        """Single-station copy of the template holding station s's observations (and sigmas, ray
+        parameter(s): a scalar for one ray, a list otherwise, and Gaussian width(s): a scalar when the
+        template's gauss is one, a list otherwise).  With swd_use its SurfWD holds the
         station's subset period lists and its dispersion data only the observed values.  With rf_use its
         ReceiverFunc holds only the station's observed rays and widths (ray parameters, widths and
         traces); a station that fits part of a trace, or whose observed traces are not every observed
@@ -189,6 +205,7 @@ class StationArray:
         c = _fresh_copy(rf)
         r = self.ray_p[s] if self.ray_p is not None else np.atleast_1d(np.asarray(rf.ray_p, dtype=np.float64))
         keep = np.ones(rf.nt, dtype=bool)
+        widths = np.ones(rf.ngauss, dtype=bool)
         if self.rf_use is not None:
             u = self.rf_use[s].reshape(rf.nray, rf.ngauss, rf.nt_trace)
             obs = u.all(axis=2)
@@ -203,12 +220,14 @@ class StationArray:
             r = r[rays]
             keep = u.reshape(-1)
             c.nray = int(r.size)
-            if np.ndim(rf.gauss) > 0:
-                c.gauss = np.asarray(rf.gauss, dtype=np.float64)[widths].tolist()
             c.ngauss = int(widths.sum())
             c.nt = c.nt_trace * c.nray * c.ngauss
         if self.ray_p is not None or self.rf_use is not None:
             c.ray_p = float(r[0]) if r.size == 1 else r.tolist()
+        # the station's own widths, or the template's observed ones; a template scalar stays a scalar
+        if self.gauss is not None or (self.rf_use is not None and np.ndim(rf.gauss) > 0):
+            g = (self.gauss[s] if self.gauss is not None else np.asarray(rf.gauss, dtype=np.float64))[widths]
+            c.gauss = float(g[0]) if np.ndim(rf.gauss) == 0 else g.tolist()
         return c, keep
 
 
@@ -302,15 +321,27 @@ def station_rays(ray_p, S, nray, where=""):
     return np.ascontiguousarray(r.reshape(S, nray))
 
 
-def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None, rf=None):
+def station_gauss(gauss, S, ngauss, where=""):
+    """gauss [S] (ngauss = 1) or [S, ngauss] -> float64 [S, ngauss], finite and > 0; the ValueError names
+    the key 'gauss' (after `where`)."""
+    g = np.asarray(gauss, dtype=np.float64)
+    if not (g.shape == (S, ngauss) or (ngauss == 1 and g.shape == (S,))):
+        want = f"[{S}] or [{S}, 1]" if ngauss == 1 else f"[{S}, {ngauss}]"
+        raise ValueError(f"{where}'gauss' must have shape {want}, got {g.shape}")
+    if not np.all(np.isfinite(g) & (g > 0)):
+        raise ValueError(f"{where}'gauss' must be finite and positive")
+    return np.ascontiguousarray(g.reshape(S, ngauss))
+
+
+def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None, rf=None, ngauss=1):
     """Validated content of a stations file (.npz path or a mapping with the same keys):
     dobs [S, ndata] (required), names [S], sigma1 / sigma2 [S] (default 1.0), bounds [S, nparam, 2]
     (default: default_bounds [nparam, 2] for every station), ray_p [S] or [S, nray] (default None: the
     ray parameter(s) of the forward configuration), swd_use [S, nper] (default None: every period;
     swd = the SurfWD whose period grid it marks) and rf_use [S, nray * ngauss * nt] or
     [S, nray, ngauss, nt] ([S, nray, nt] with one width; default None: every RF sample; rf = the
-    ReceiverFunc whose data it marks).  Raises ValueError naming the
-    bad key."""
+    ReceiverFunc whose data it marks) and gauss [S] or [S, ngauss] (default None: the Gaussian width(s)
+    of the forward configuration).  Raises ValueError naming the bad key."""
     if isinstance(src, (str, bytes)) or hasattr(src, "__fspath__"):
         with np.load(src, allow_pickle=False) as f:
             src = {k: f[k] for k in f.files}
@@ -354,4 +385,5 @@ def load_stations(src, ndata, nparam, default_bounds, nray=1, swd=None, rf=None)
         if rf is None:
             raise ValueError("stations file: 'rf_use' needs a receiver-function configuration")
         out["rf_use"] = station_rf_samples(src["rf_use"], S, rf, "stations file: ")
+    out["gauss"] = station_gauss(src["gauss"], S, ngauss, "stations file: ") if "gauss" in src else None
     return out

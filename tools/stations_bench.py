@@ -37,7 +37,18 @@ parameters 0.045, 0.06, 0.075 in place of F1's one, so that a bin can be missing
   (l) RF only, time method, F1 layers and sampling, 64 stations x 16 models: the same two;
   (m) HMC, 16 stations x 64 chains with whole-trace masks (missing bins only): one grouped run vs 16
       single-station runs, each in a context configured on its station's observed rays.
---legs sets,rays,periods,rfwin selects the legs (default sets,rays); the legs run replace their keys in
+Leg "gauss" (per-station Gaussian widths, rfs_config_obs_gauss), every station with its own widths:
+  (n) F1 joint, one width per station drawn from {1.0, 1.5, 2.0, 2.5, 3.0}, (S, K) = (256, 64), (1024, 16):
+      the grouped call with the width table vs the same grouped call on the shared width (two contexts,
+      timed alternately, --inner calls per timing) vs one context reconfigured for each station in turn
+      (config_rf on its width, config_obs, its K rows);
+  (o) RF only, frequency method, n = 40, nt = 2048, three rays, two widths per station, 256 stations x 256
+      models: the table vs the shared widths (48 GB workspace budget each, as in (e));
+  (p) RF only, time method, F1 layers and sampling, two widths per station, 64 stations x 16 models: the
+      same two;
+  (q) HMC, 16 stations x 64 chains: one grouped run vs 16 single-station runs, each in a context configured
+      with its station's width.
+--legs sets,rays,periods,rfwin,gauss selects the legs (default sets,rays); the legs run replace their keys in
 --out and keep the others.
 Every shape is warmed up first; each timing is repeated --reps times (median, min, max reported), with a
 host clock around work that ends in a device synchronise.  Station observations are the forward model
@@ -132,6 +143,8 @@ def main():
         res["periods"] = periods_leg(a, torch, X)
     if "rfwin" in legs:
         res["rfwin"] = rfwin_leg(a, torch, X)
+    if "gauss" in legs:
+        res["gauss"] = gauss_leg(a, torch, X)
     if "sets" not in legs:
         c.close()
         return write(a, res)
@@ -598,6 +611,167 @@ def rfwin_leg(a, torch, X):
     runs = {"grouped": lambda: grouped.hmc_run(0, ids, bounds, sets=hsets, **kw)["evals"],
             "per_station": lambda: sum(single[s].hmc_run(0, np.arange(Kh), bounds, **kw)["evals"] for s in range(Sh))}
     hmc = {"S": Sh, "K": Kh, "max_iters": a.hmc_iters, "stations_missing_a_bin": int((~use.all(axis=1)).sum())}
+    for name, fn in runs.items():
+        fn()
+        ts, evs = [], 0
+        for _ in range(max(1, a.reps // 2)):
+            t0 = time.perf_counter()
+            evs = fn()
+            ts.append(time.perf_counter() - t0)
+        hmc[name] = {**spread(ts), "evals": int(evs), "evals_per_s": float(evs / np.median(ts))}
+    hmc["speedup_per_station_over_grouped"] = hmc["per_station"]["median_ms"] / hmc["grouped"]["median_ms"]
+    out["hmc"] = hmc
+    grouped.close()
+    for c in single:
+        c.close()
+    return out
+
+
+def gauss_leg(a, torch, X):
+    """Per-station Gaussian widths against the same grouped call on the shared widths, and against one
+    context reconfigured per station (see the module docstring)."""
+    from rfsurfhmc_b200._lib import Context
+    from rfsurfhmc_b200.fixtures import f1_config, f1_true_model, driver_bounds, perturbed_models
+    from bench import layered_models
+    cfg, x0 = f1_config(), f1_true_model()
+    dev = torch.device("cuda", 0)
+    st = torch.cuda.current_stream(dev)
+    widths = np.array([1.0, 1.5, 2.0, 2.5, 3.0])
+    out = {**gpu_info(), "inner_calls": a.inner, "widths": widths.tolist(), "eval": []}
+    rng = np.random.default_rng(31)
+
+    def configure(c, which, n, rays, nt, dt, gauss, method):
+        if which != 1:
+            c.config_swd(n, tRc=cfg["tRc"], tRg=cfg["tRg"])
+        c.config_rf(n, rays, nt, dt, gauss, cfg["time_shift"], cfg["water"], "P", method)
+
+    def observations(which, shape, table, Xs):
+        c = Context(0)
+        configure(c, which, *shape)
+        S = Xs.shape[0]
+        c.config_obs(np.zeros((S, c.ndata(which))))
+        c.config_obs_gauss(table)
+        _, _, d, _ = c.misfit_grad_host(Xs, which, sets=np.arange(S))
+        c.close()
+        d = np.where(np.isfinite(d), d, 0.0)
+        return d + 0.01 * np.random.default_rng(S).standard_normal(d.shape)
+
+    def compare(which, shape, Xd, S, K, dobs, table, per_station=False):
+        B = Xd.shape[0]
+        sets = torch.from_numpy(np.repeat(np.arange(S, dtype=np.int32), K)).to(dev)
+        cs = []
+        for with_table in (True, False):
+            c = Context(0)
+            configure(c, which, *shape)
+            c.config_obs(dobs)
+            if with_table:
+                c.config_obs_gauss(table)
+            cs.append(c)
+        U = torch.empty(B, dtype=torch.float64, device=dev)
+        G = torch.empty(Xd.shape, dtype=torch.float64, device=dev)
+        D = torch.empty(B, cs[0].ndata(which), dtype=torch.float64, device=dev)
+        F = torch.empty(B, dtype=torch.uint8, device=dev)
+
+        def call(c):
+            for _ in range(a.inner):
+                c.misfit_grad_dev(B, Xd.data_ptr(), which, U.data_ptr(), G.data_ptr(), D.data_ptr(), F.data_ptr(),
+                                  st.cuda_stream, sets_ptr=sets.data_ptr())
+        ts = ([], [])
+        for c in cs:
+            call(c)
+        torch.cuda.synchronize()
+        for _ in range(a.reps):
+            for k, c in enumerate(cs):
+                t0 = time.perf_counter()
+                call(c)
+                torch.cuda.synchronize()
+                ts[k].append((time.perf_counter() - t0) / a.inner)
+        for c in cs:
+            c.close()
+        tab, shared = spread(ts[0]), spread(ts[1])
+        r = {"width_table": tab, "shared_width": shared, "table_cost": tab["median_ms"] / shared["median_ms"] - 1.0}
+        if not per_station:
+            return r
+        # what a user does without the table: one context, reconfigured for each station in turn
+        one = Context(0)
+        n, rays, nt, dt = shape[:4]
+
+        def seq():
+            for s in range(S):
+                one.config_rf(n, rays, nt, dt, float(table[s]), cfg["time_shift"], cfg["water"], "P", shape[-1])
+                one.config_obs(dobs[s])
+                one.misfit_grad_dev(K, Xd[s * K].data_ptr(), which, U[s * K].data_ptr(), G[s * K].data_ptr(),
+                                    D[s * K].data_ptr(), F[s * K].data_ptr(), st.cuda_stream)
+        configure(one, which, *shape)
+        seq()
+        torch.cuda.synchronize()
+        tp = []
+        for _ in range(a.reps):
+            t0 = time.perf_counter()
+            seq()
+            torch.cuda.synchronize()
+            tp.append(time.perf_counter() - t0)
+        one.close()
+        r["per_station"] = spread(tp)
+        r["speedup_per_station_over_table"] = r["per_station"]["median_ms"] / tab["median_ms"]
+        return r
+
+    n = x0.size // 2
+    f1 = (n, cfg["ray_p"], cfg["nt"], cfg["dt"], cfg["gauss"], "freq")
+    for S, K in ((256, 64), (1024, 16)):
+        table = rng.choice(widths, S)
+        dobs = observations(0, f1, table, perturbed_models(x0, S, seed=100 + S, rel=0.05))
+        out["eval"].append({"workload": "F1 joint, one width per station, %d stations x %d models" % (S, K),
+                            "S": S, "K": K, **compare(0, f1, X[:S * K], S, K, dobs, table, per_station=True)})
+        progress(out["eval"][-1])
+    # RF only, frequency method, C3-like, two widths per station
+    nc, ntc, S, K = 40, 2048, 256, 256
+    c3 = (nc, [0.04, 0.06, 0.08], ntc, 0.05, [1.0, 2.5], "freq")
+    Xc = torch.from_numpy(layered_models(S * K, nc, 2)).to(dev)
+    table = np.sort(rng.choice(widths, (S, 2)), axis=1)
+    dobs = 0.01 * np.random.default_rng(3).standard_normal((S, 3 * 2 * ntc))
+    old = os.environ.get("RFS_WS_BUDGET_MB")
+    os.environ["RFS_WS_BUDGET_MB"] = "48000"
+    try:
+        out["rf_c3"] = {"workload": "RF only (freq), n=40, nt=2048, dt=0.05, three rays, two widths per station, "
+                                    "%d stations x %d models" % (S, K), "S": S, "K": K,
+                        **compare(1, c3, Xc, S, K, dobs, table)}
+    finally:
+        if old is None:
+            del os.environ["RFS_WS_BUDGET_MB"]
+        else:
+            os.environ["RFS_WS_BUDGET_MB"] = old
+    progress(out["rf_c3"])
+    # RF only, time method, two widths per station
+    S, K = 64, 16
+    ft = (n, cfg["ray_p"], cfg["nt"], cfg["dt"], [1.0, 2.5], "time")
+    table = np.sort(rng.choice(widths, (S, 2)), axis=1)
+    dobs = observations(1, ft, table, perturbed_models(x0, S, seed=43, rel=0.05))
+    out["rf_time"] = {"workload": "RF only (time), F1 layers and sampling, two widths per station, "
+                                  "%d stations x %d models" % (S, K), "S": S, "K": K,
+                      **compare(1, ft, X[:S * K], S, K, dobs, table)}
+    progress(out["rf_time"])
+    # HMC, 16 stations x 64 chains, base sampler
+    Sh, Kh = 16, 64
+    table = rng.choice(widths, Sh)
+    dobs = observations(0, f1, table, perturbed_models(x0, Sh, seed=7, rel=0.05))
+    bounds = driver_bounds(x0)
+    kw = dict(dt=0.1, Lrange=(5, 20), seed=991206, nsamples=a.hmc_iters + 1, ndraws=0, max_iters=a.hmc_iters,
+              want_samples=False)
+    grouped = Context(0)
+    configure(grouped, 0, *f1)
+    grouped.config_obs(dobs)
+    grouped.config_obs_gauss(table)
+    single = []
+    for s in range(Sh):
+        c = Context(0)
+        configure(c, 0, n, cfg["ray_p"], cfg["nt"], cfg["dt"], float(table[s]), "freq")
+        c.config_obs(dobs[s])
+        single.append(c)
+    ids, hsets = np.tile(np.arange(Kh), Sh), np.repeat(np.arange(Sh), Kh)
+    runs = {"grouped": lambda: grouped.hmc_run(0, ids, bounds, sets=hsets, **kw)["evals"],
+            "per_station": lambda: sum(single[s].hmc_run(0, np.arange(Kh), bounds, **kw)["evals"] for s in range(Sh))}
+    hmc = {"S": Sh, "K": Kh, "max_iters": a.hmc_iters}
     for name, fn in runs.items():
         fn()
         ts, evs = [], 0
