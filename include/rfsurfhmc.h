@@ -160,8 +160,29 @@ int rfs_config_obs_rf_samples(rfs_ctx *ctx, int S, int nrf, const unsigned char 
  * finite and > 0.  Lifetime: see "Per-set tables" above. */
 int rfs_config_obs_gauss(rfs_ctx *ctx, int S, int ngauss, const double *gauss);
 
+/* Parameterisation of the model vector (no reference counterpart: model_rf_swd_vs_thk.py fixes
+ * [vs, thk]).  Receiver functions constrain Vp through the Ps delays, which trade thickness against
+ * Vp/Vs (the H-kappa trade-off); with Vp tied to vs by Brocher's curve that trade-off cannot be sampled.
+ *   RFS_PARAM_VS_THK      (0, the default at rfs_create): x = [vs(n), thk(n)], vp and rho from Brocher's
+ *                         polynomials of vs.
+ *   RFS_PARAM_VS_THK_VPVS (1): x = [vs(n), thk(n), k(n)], k the Vp/Vs ratio of each layer (half-space
+ *                         included): vp = k vs, rho = Brocher's density polynomial of that vp.  grad is
+ *                         [dU/dvs | dU/dthk | dU/dk] with, per layer, g_vs = K_b + k (K_a + drho/dvp K_r)
+ *                         and g_k = vs (K_a + drho/dvp K_r).
+ * With param 1 every x, grad, samples and initmodel row below has P n = 3n columns instead of 2n, and the
+ * HMC bounds are [nb][3n][2]; the failure convention writes grad zeros of width 3n.  This covers
+ * rfs_misfit_grad_{dev,host}, rfs_misfit_grad_sets_{dev,host} (every which), rfs_profile_eval,
+ * rfs_hmc_run and rfs_hmc_run_sets; the libsurf/librf drop-ins are not affected.  The setting belongs to
+ * the context and is shared by every observation set: no other rfs_config_* call changes it and it
+ * changes no per-set table.  It copies nothing to the device, but like every rfs_config_* call it must
+ * not be made while an evaluation on the context is in flight.  Any other value returns RFS_E_ARG. */
+#define RFS_PARAM_VS_THK 0
+#define RFS_PARAM_VS_THK_VPVS 1
+int rfs_config_param(rfs_ctx *ctx, int param);
+
 /* ---- the hot path: batched misfit + gradient ------------------------------------------------
  * x [B][2n] = [vs(n), thk(n)];  U [B];  grad [B][2n];  dsyn [B][ndata];  flag [B] (1 ok / 0 fail)
+ * (P n = 3n columns for x and grad under RFS_PARAM_VS_THK_VPVS, see rfs_config_param)
  * which: 0 Joint_RF_SWD.misfit_and_grad, 1 ReceiverFunc.misfit_and_grad, 2 SurfWD.misfit_and_grad */
 int rfs_misfit_grad_dev(rfs_ctx *ctx, long long B, const double *x, int which, double *U,
                         double *grad, double *dsyn, unsigned char *flag, void *stream);

@@ -79,6 +79,8 @@ def load_library():
         L.rfs_config_obs_rf_samples.argtypes = [_vp, C.c_int, C.c_int, _u8p]
         L.rfs_config_obs_gauss.restype = C.c_int
         L.rfs_config_obs_gauss.argtypes = [_vp, C.c_int, C.c_int, _dp]
+        L.rfs_config_param.restype = C.c_int
+        L.rfs_config_param.argtypes = [_vp, C.c_int]
         L.rfs_misfit_grad_sets_dev.restype = C.c_int
         L.rfs_misfit_grad_sets_dev.argtypes = [_vp, C.c_longlong, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp]
         L.rfs_misfit_grad_sets_host.restype = C.c_int
@@ -151,7 +153,7 @@ def exported_symbols():
             "rfs_config_swd_modes", "rfs_config_rf_rays", "rfs_hmc_last_steps", "rfs_set_hmc_options",
             "rfs_config_obs_sets", "rfs_misfit_grad_sets_dev", "rfs_misfit_grad_sets_host", "rfs_hmc_run_sets",
             "rfs_config_obs_rays", "rfs_config_obs_periods", "rfs_config_obs_rf_samples", "rfs_config_rf_gauss",
-            "rfs_config_obs_gauss"]
+            "rfs_config_obs_gauss", "rfs_config_param"]
 
 
 def _f64(a):
@@ -353,6 +355,13 @@ class Context:
             raise ValueError(f"gauss must be [S] or [S, ngauss], got shape {g.shape}")
         ng = 1 if g.ndim == 1 else g.shape[1]
         self._ck(self.L.rfs_config_obs_gauss(self.h, g.shape[0], ng, _p(g)))
+
+    def config_param(self, vpvs):
+        """Model-vector layout of every evaluation and HMC run on this context: vpvs False (default)
+        x = [vs, thk] with Brocher vp and rho, True x = [vs, thk, vpvs] with vp = vpvs * vs and Brocher rho
+        of that vp.  Accepts a bool or the RFS_PARAM_* code (0, 1)."""
+        code = int(vpvs) if not isinstance(vpvs, bool) else (1 if vpvs else 0)
+        self._ck(self.L.rfs_config_param(self.h, code))
 
     def ndata(self, which=0):
         return (self.nt_rf if which != 2 else 0) + (self.n_swd_data if which != 1 else 0)

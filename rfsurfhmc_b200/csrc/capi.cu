@@ -112,6 +112,9 @@ struct rfs_ctx {
   bool has_rf = false;
   RfCfg rf;                    // its Gaussian widths: rf.gauss (reference: one)
   std::vector<double> ray_ps;  // ray parameters of the fused RF objective (reference: one)
+  // ---- parameterisation (rfs_config_param): npar blocks of n per model, [vs, thk] with Brocher vp and
+  // rho (2) or [vs, thk, Vp/Vs] with vp = k vs and Brocher rho (3).  Shared by every set.
+  int npar = 2;
   // ---- observations: nsets data vectors ("stations") of ndobs values each, and their per-set tables
   bool has_obs = false;
   int nsets = 0, ndobs = 0;
@@ -536,7 +539,7 @@ int run_swd(rfs_ctx *ctx, Front &F, const SwdPlan &P, const double *d_periods, c
 }
 
 // ---- RF pipeline on a prepared model block (freq method)
-// nq: 0 forward only, 2 chain-rule rows (vs, thk), 4 all parameters.  Brings the twiddle table that the
+// nq: 0 forward only, 2 chain-rule rows (vs, thk), 3 (vs, thk, Vp/Vs), 4 all parameters.  Brings the twiddle table that the
 // FFTs of run_rf_decon / run_rf_time read to cfg.nft, in order on `st`.
 int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const double *d_rfm,
                    const double *d_chain, const double *d_qa, const double *d_qb, long long B, int n,
@@ -564,6 +567,8 @@ int run_rf_spectra(rfs_ctx *ctx, const RfCfg &cfg, const RayView &ray, const dou
 #define PROPQ(NM)    \
   if (nq == 2) {     \
     PROP(NM, 2);     \
+  } else if (nq == 3) { \
+    PROP(NM, 3);     \
   } else {           \
     PROP(NM, 4);     \
   }
@@ -683,7 +688,7 @@ int check_objective(rfs_ctx *ctx, int which, bool has_set, const char *entry, in
 struct Eval {
   long long B;
   const double *x;
-  int which, n, ndata, n1, nsw, nray;
+  int which, n, P, ndata, n1, nsw, nray;  // P: parameter blocks per model (rfs_ctx::npar)
   double *U, *grad, *dsyn;
   unsigned char *flag;
   cudaStream_t st;
@@ -699,7 +704,7 @@ struct Eval {
 
   Eval(const rfs_ctx *ctx, long long B, const double *x, const int *set, int which, int n, int ndata, double *U,
        double *grad, double *dsyn, unsigned char *flag, cudaStream_t st, bool overlap)
-      : B(B), x(x), which(which), n(n), ndata(ndata), U(U), grad(grad), dsyn(dsyn), flag(flag), st(st),
+      : B(B), x(x), which(which), n(n), P(ctx->npar), ndata(ndata), U(U), grad(grad), dsyn(dsyn), flag(flag), st(st),
         overlap(overlap), use_swd(which != 1), use_rf(which != 2), grid(swd_grid(ctx)) {
     n1 = use_rf ? ndata_of(ctx, 1) : 0;
     nsw = ndata - n1;
@@ -744,7 +749,7 @@ RfTrace rf_trace(const RfCfg &rf, ObsSets obs, double *dsyn, int ir, int ig) {
 // results), kept for the whole batch; pm for the eigen / RF workspaces, sized per chunk against what is
 // left of the budget.  Chunks are balanced.
 void plan_chunks(const rfs_ctx *ctx, Eval &E) {
-  size_t pmf = sizeof(double) * 2 * (size_t)E.n, pm = 64;
+  size_t pmf = sizeof(double) * E.P * (size_t)E.n, pm = 64;
   if (E.use_swd) {
     const SwdPlan &P = E.grid.plan;
     const size_t nmo = E.multi_mode ? (size_t)P.nmode : 1;
@@ -755,10 +760,10 @@ void plan_chunks(const rfs_ctx *ctx, Eval &E) {
   if (E.use_rf) {
     const RfCfg &rf = ctx->rf;
     pmf += sizeof(double) * (4 * (size_t)rf.n);
-    pm += sizeof(RfLayer) * (size_t)rf.n + sizeof(double2) * ((size_t)2 * rf.n2 + (size_t)2 * rf.n * rf.n2) +
-          sizeof(double) * (1 + 2 * (size_t)rf.n);
-    if (rf.method == 0)
-      pm += sizeof(double2) * ((size_t)2 * rf.n * rf.n2) + sizeof(double) * ((size_t)4 * rf.n * rf.nt);
+    pm += sizeof(RfLayer) * (size_t)rf.n + sizeof(double2) * ((size_t)2 * rf.n2 + (size_t)E.P * rf.n * rf.n2) +
+          sizeof(double) * (1 + E.P * (size_t)rf.n);
+    if (rf.method == 0)  // all four derivative rows, and the Frechet traces
+      pm += sizeof(double2) * ((size_t)(4 - E.P) * rf.n * rf.n2) + sizeof(double) * ((size_t)4 * rf.n * rf.nt);
   }
   const size_t front_total = pmf * (size_t)E.B + (pmf * (size_t)E.B) / 8;
   const size_t budget = std::max(ctx->ws_budget > front_total ? ctx->ws_budget - front_total : (size_t)0,
@@ -801,10 +806,16 @@ int front_pass(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, Front &F, SwdB
   const size_t nB = (size_t)n * c.B;
   if (E.use_swd && (rc = ensure(ctx, F.w_swd, sizeof(double) * SWD_NF * nB))) return rc;
   if (E.use_rf && (rc = ensure(ctx, F.w_rfm, sizeof(double) * 4 * nB))) return rc;
-  if ((rc = ensure(ctx, F.w_chain, sizeof(double) * 2 * nB))) return rc;
-  LAUNCH(prep_models_kernel, gridFor(c.B * n, 256), 256, 0, sk, E.x + c.off * 2 * n, c.B, n,
-         E.use_swd ? (double *)F.w_swd.p : nullptr, E.use_rf ? (double *)F.w_rfm.p : nullptr,
-         (double *)F.w_chain.p);
+  if ((rc = ensure(ctx, F.w_chain, sizeof(double) * E.P * nB))) return rc;
+#define PREP(P)                                                                                        \
+  LAUNCH(prep_models_kernel<P>, gridFor(c.B * n, 256), 256, 0, sk, E.x + c.off * P * n, c.B, n,         \
+         E.use_swd ? (double *)F.w_swd.p : nullptr, E.use_rf ? (double *)F.w_rfm.p : nullptr,           \
+         (double *)F.w_chain.p)
+  if (E.P == 3)
+    PREP(3);
+  else
+    PREP(2);
+#undef PREP
   if (!F.ev_prep) CK(cudaEventCreateWithFlags(&F.ev_prep, cudaEventDisableTiming));
   if (!F.ev_ready) CK(cudaEventCreateWithFlags(&F.ev_ready, cudaEventDisableTiming));
   F.prep_pending = true;  // recorded by launch_roots right before the search kernel, or just below
@@ -841,9 +852,9 @@ int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F)
     LAUNCH(rf_branch_hold_kernel, 1, 32, 0, sr, 25000u);
   }
   if ((rc = ensure(ctx, ctx->w_urf, sizeof(double) * c.B))) return rc;
-  if ((rc = ensure(ctx, ctx->w_grf, sizeof(double) * 2 * (size_t)n * c.B))) return rc;
+  if ((rc = ensure(ctx, ctx->w_grf, sizeof(double) * E.P * (size_t)n * c.B))) return rc;
   double *Uo = (E.which == 1) ? E.U + c.off : (double *)ctx->w_urf.p;
-  double *go = (E.which == 1) ? E.grad + c.off * 2 * n : (double *)ctx->w_grf.p;
+  double *go = (E.which == 1) ? E.grad + c.off * E.P * n : (double *)ctx->w_grf.p;
   // RF only: every row succeeds except one whose set index is out of range (the RF kernels write its 0)
   unsigned char *fo = (E.which == 1) ? E.flag + c.off : nullptr;
   if (fo) CK(cudaMemsetAsync(fo, 1, c.B, sr));
@@ -855,11 +866,11 @@ int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F)
     const RayView ray{ctx->tables.has_rays ? (const double *)ctx->tables.d_rays.p : nullptr, c.obs.set, ctx->nsets,
                       E.nray, ir, ctx->ray_ps[ir]};
     if ((rc = run_rf_spectra(ctx, rf, ray, (const double *)F.w_rfm.p, (const double *)F.w_chain.p, nullptr,
-                             nullptr, c.B, n, rf_time ? 4 : 2, sr, rf_time ? RFS_PI64 : RFS_PI32)))
+                             nullptr, c.B, n, rf_time ? 4 : E.P, sr, rf_time ? RFS_PI64 : RFS_PI32)))
       return rc;
     if (!rf_time) {
       const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, 0);
-      if ((rc = run_rf_decon(ctx, rf, gv, c.B, 2 * n, t.obs, t.dsyn, E.ndata, Uo, go, fo, sr, ir > 0))) return rc;
+      if ((rc = run_rf_decon(ctx, rf, gv, c.B, E.P * n, t.obs, t.dsyn, E.ndata, Uo, go, fo, sr, ir > 0))) return rc;
       continue;
     }
     // deconit is nonlinear (argmax spike picking): no adjoint shortcut, materialise the traces of each
@@ -867,9 +878,15 @@ int rf_branch(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front &F)
     for (int ig = 0; ig < rf.gauss.n; ig++) {
       const RfTrace t = rf_trace(rf, c.obs, dsyn, ir, ig);
       if ((rc = run_rf_time(ctx, rf, gv, ig, c.B, 4 * n, t.dsyn, E.ndata, sr))) return rc;
-      LAUNCH(rf_trace_grad_kernel, gridFor(c.B * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,
-             (const double *)F.w_chain.p, t.dsyn, (long long)E.ndata, t.obs, c.B, n, rf.nt, Uo, go, fo,
-             ir > 0 || ig > 0);
+#define TGRAD(P)                                                                                         \
+  LAUNCH(rf_trace_grad_kernel<P>, gridFor(c.B * n, 128), 128, 0, sr, (const double *)ctx->w_rftr.p,        \
+         (const double *)F.w_chain.p, t.dsyn, (long long)E.ndata, t.obs, c.B, n, rf.nt, Uo, go, fo, \
+         ir > 0 || ig > 0)
+      if (E.P == 3)
+        TGRAD(3);
+      else
+        TGRAD(2);
+#undef TGRAD
     }
   }
   if (sr != E.st) CK(cudaEventRecord(ctx->ev_join, sr));
@@ -886,10 +903,16 @@ int swd_back_pass(rfs_ctx *ctx, const Eval &E, const Eval::Chunk &c, const Front
   const SwdView V{(const double *)F.w_croot.p, (const double *)ctx->w_ugr.p, (const double *)ctx->w_kern.p,
                   E.grid.periods, c.B, n, blk, 0};
   if (E.use_rf && E.overlap) CK(cudaStreamWaitEvent(E.st, ctx->ev_join, 0));
-  LAUNCH(joint_assemble_kernel, dim3(gridFor(c.B, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, E.st, E.grid.plan, V, c.sv,
-         (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, E.which, E.n1, c.obs,
-         (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p, E.U + c.off,
-         E.grad + c.off * 2 * n, E.dsyn + c.off * E.ndata, E.flag + c.off, E.msel);
+#define ASM(P)                                                                                                  \
+  LAUNCH(joint_assemble_kernel<P>, dim3(gridFor(c.B, 32), (unsigned)n), 32 * RFS_ASM_Q, 0, E.st, E.grid.plan, V, \
+         c.sv, (const int *)F.w_ierr.p, (const double *)F.w_chain.p, ctx->stale, E.which, E.n1, c.obs,          \
+         (const double *)ctx->w_urf.p, (const double *)ctx->w_grf.p, (const double *)ctx->d_wt.p, E.U + c.off,  \
+         E.grad + c.off * P * n, E.dsyn + c.off * E.ndata, E.flag + c.off, E.msel)
+  if (E.P == 3)
+    ASM(3);
+  else
+    ASM(2);
+#undef ASM
   CK(cudaEventRecord(ctx->ev_asm, E.st));
   return RFS_OK;
 }
@@ -1119,6 +1142,14 @@ int rfs_config_obs(rfs_ctx *ctx, double sigma1, double sigma2, const double *dob
   return rfs_config_obs_sets(ctx, 1, &sigma1, &sigma2, dobs, ndobs);
 }
 
+int rfs_config_param(rfs_ctx *ctx, int param) {
+  if (!ctx) return RFS_E_ARG;
+  if (param != RFS_PARAM_VS_THK && param != RFS_PARAM_VS_THK_VPVS)
+    return fail(ctx, RFS_E_ARG, "param must be RFS_PARAM_VS_THK (0) or RFS_PARAM_VS_THK_VPVS (1)");
+  ctx->npar = param == RFS_PARAM_VS_THK_VPVS ? 3 : 2;
+  return RFS_OK;
+}
+
 int rfs_config_obs_rays(rfs_ctx *ctx, int S, int nray, const double *ray_p) {
   if (!ctx) return RFS_E_ARG;
   int rc = begin_table(ctx, TAB_RAYS, "ray-parameter table", ctx->has_rf, "an RF configuration (rfs_config_rf)", S);
@@ -1256,14 +1287,15 @@ int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const 
         return fail(ctx, RFS_E_ARG, "set index " + std::to_string(set[b]) + " of row " + std::to_string(b) +
                                         " outside [0, " + std::to_string(ctx->nsets) + ")");
   CK(cudaSetDevice(ctx->device));
-  if ((rc = ensure(ctx, ctx->io_x, sizeof(double) * B * 2 * n))) return rc;
+  const int np = ctx->npar * n;  // x and grad columns
+  if ((rc = ensure(ctx, ctx->io_x, sizeof(double) * B * np))) return rc;
   if ((rc = ensure(ctx, ctx->io_U, sizeof(double) * B))) return rc;
-  if ((rc = ensure(ctx, ctx->io_grad, sizeof(double) * B * 2 * n))) return rc;
+  if ((rc = ensure(ctx, ctx->io_grad, sizeof(double) * B * np))) return rc;
   if ((rc = ensure(ctx, ctx->io_dsyn, sizeof(double) * B * ndata))) return rc;
   if ((rc = ensure(ctx, ctx->io_flag, B))) return rc;
   if (set && (rc = ensure(ctx, ctx->io_set, sizeof(int) * B))) return rc;
   cudaStream_t st = ctx->stream;
-  CK(cudaMemcpyAsync(ctx->io_x.p, x, sizeof(double) * B * 2 * n, cudaMemcpyHostToDevice, st));
+  CK(cudaMemcpyAsync(ctx->io_x.p, x, sizeof(double) * B * np, cudaMemcpyHostToDevice, st));
   if (set) CK(cudaMemcpyAsync(ctx->io_set.p, set, sizeof(int) * B, cudaMemcpyHostToDevice, st));
   rc = rfs_misfit_grad_sets_dev(ctx, B, (const double *)ctx->io_x.p, set ? (const int *)ctx->io_set.p : nullptr,
                                 which, (double *)ctx->io_U.p, (double *)ctx->io_grad.p, (double *)ctx->io_dsyn.p,
@@ -1271,7 +1303,7 @@ int rfs_misfit_grad_sets_host(rfs_ctx *ctx, long long B, const double *x, const 
   if (rc) return rc;
   if (U) CK(cudaMemcpyAsync(U, ctx->io_U.p, sizeof(double) * B, cudaMemcpyDeviceToHost, st));
   if (grad)
-    CK(cudaMemcpyAsync(grad, ctx->io_grad.p, sizeof(double) * B * 2 * n, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(grad, ctx->io_grad.p, sizeof(double) * B * np, cudaMemcpyDeviceToHost, st));
   if (dsyn)
     CK(cudaMemcpyAsync(dsyn, ctx->io_dsyn.p, sizeof(double) * B * ndata, cudaMemcpyDeviceToHost, st));
   if (flag) CK(cudaMemcpyAsync(flag, ctx->io_flag.p, B, cudaMemcpyDeviceToHost, st));

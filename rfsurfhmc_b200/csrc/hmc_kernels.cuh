@@ -24,8 +24,9 @@ enum { HP_INIT = 0, HP_FD = 1, HP_LEAP = 2, HP_DONE = 3 };
 // (the reference would loop forever), 4 failure inside _find_initial_dt (reference: exit(1)),
 // 5 stopped by the wall-clock budget of rfs_set_hmc_options
 
+// n2: columns of x, P n for P parameter blocks of n layers ([vs, thk] or [vs, thk, Vp/Vs])
 struct HmcCfg {
-  int n2, ndata, sampler, Lmin, Lmax, L0, nsamples, ndraws;
+  int n2, n, ndata, sampler, Lmin, Lmax, L0, nsamples, ndraws;
   double dt0, target, lambda, mu;
   long long max_iters, max_log;
 };
@@ -242,28 +243,32 @@ RFS_DEVINL void hmc_chain_start(const HmcDev &D, const HmcCfg &cfg, long long R,
   r.C = R;
   r.c = c;
   r.seed((unsigned int)((D.seed + D.chain_id[ch]) & 0xffffffffLL));
-  const int n2 = cfg.n2, n = n2 / 2;
+  const int n2 = cfg.n2, n = cfg.n;
+  const bool vpvs = n2 == 3 * n;
   double *x = D.xcur + c * n2;
   for (;;) {
     for (int i = 0; i < n2; i++) {
       const double lo = box[2 * i], hi = box[2 * i + 1];
       x[i] = lo + (hi - lo) * r.rand();
     }
-    // sort vs ascending, permute thk alike (insertion sort; values are distinct a.s.)
+    // sort vs ascending, permute thk (and Vp/Vs) alike (insertion sort; values are distinct a.s.)
     for (int i = 1; i < n; i++) {
-      const double v = x[i], h = x[n + i];
+      const double v = x[i], h = x[n + i], k = vpvs ? x[2 * n + i] : 0.0;
       int j = i - 1;
       while (j >= 0 && x[j] > v) {
         x[j + 1] = x[j];
         x[n + j + 1] = x[n + j];
+        if (vpvs) x[2 * n + j + 1] = x[2 * n + j];
         j--;
       }
       x[j + 1] = v;
       x[n + j + 1] = h;
+      if (vpvs) x[2 * n + j + 1] = k;
     }
+    // every entry in its box except the half-space thickness (index 2n - 1)
     bool ok = true;
-    for (int i = 0; i < n2 - 1; i++)
-      if (x[i] < box[2 * i] || x[i] > box[2 * i + 1]) ok = false;
+    for (int i = 0; i < n2; i++)
+      if (i != 2 * n - 1 && (x[i] < box[2 * i] || x[i] > box[2 * i + 1])) ok = false;
     if (ok) break;
   }
   for (int i = 0; i < n2; i++) {

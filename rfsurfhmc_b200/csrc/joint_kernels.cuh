@@ -26,13 +26,15 @@ struct ModeSel {
 // order through shared memory (deterministic).  The loop over the Jacobian rows is a chain of dependent
 // global loads: four times the threads cut its latency (0.30 -> ~0.1 ms at C1).
 // Layout of outputs (row-major per model, as the Python API):
-//   U[B], grad[B][2n] (vs then thk), dsyn[B][ndata] with ndata = nt_rf + nsw (joint),
+//   U[B], grad[B][P n] (vs, thk, then Vp/Vs when P = 3), dsyn[B][ndata] with ndata = nt_rf + nsw (joint),
 //   flag[B] (1 ok, 0 failed SWD root search or observation-set index out of range)
 // Row b is compared with observation set obs.row_set(b); wt[S] is each set's SWD weight
 // (sigma1/sigma2)^2 n1/nsw of the joint objective.  With per-set period lists (sv) slice q contracts the
 // set's compact periods k = q, q + Q, ... (the sums of a one-set context on those lists), dsyn holds
 // them at their grid positions and NaN at the grid positions the set does not observe.
+// chain [P][n][B]: dadb, drda (P = 3: dadb = k, then dadk = vs; g_k = dadk*(K_a + drda*K_r)).
 #define RFS_ASM_Q 4
+template <int P>
 __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, const int *__restrict__ ierr,
                                       const double *__restrict__ chain, int stale, int which,
                                       int nt_rf, ObsSets obs, const double *__restrict__ U_rf,
@@ -40,7 +42,7 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, co
                                       double *__restrict__ U, double *__restrict__ grad,
                                       double *__restrict__ dsyn, unsigned char *__restrict__ flag,
                                       ModeSel ms) {
-  __shared__ double red[3][RFS_ASM_Q][32];
+  __shared__ double red[P + 1][RFS_ASM_Q][32];
   const int bl = threadIdx.x & 31, q = threadIdx.x >> 5;
   const long long B = V.B;
   const int n = V.n;
@@ -56,9 +58,10 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, co
   bool ok = set >= 0;
   if (which != 1 && live)
     for (int s = 0; s < plan.nseq; s++) ok = ok && (ierr[(long long)s * B + b] == 0);
-  double gv = 0.0, gh = 0.0, us = 0.0;
+  double gv = 0.0, gh = 0.0, gk = 0.0, us = 0.0;
   if (which != 1 && ok && live) {
     const double dadb = chain[0 * nB + m * B + b], drda = chain[1 * nB + m * B + b];
+    const double dadk = P == 3 ? chain[2 * nB + m * B + b] : 0.0;
     for (int im = 0; im < ms.n; im++) {
       // view of mode ms.m[im]: results are laid out [mode][solve]...
       SwdView Vm = V;
@@ -79,6 +82,7 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, co
           const double kv = K[1] + K[0] * dadb + K[2] * drda * dadb;
           gv += res * kv;
           gh += res * K[3];
+          if (P == 3) gk += res * (K[0] * dadk + K[2] * drda * dadk);
           if (m == 0) {
             us += res * res;
             dsyn[b * ndata + j] = d;
@@ -97,24 +101,28 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, co
   red[0][q][bl] = gv;
   red[1][q][bl] = gh;
   red[2][q][bl] = us;
+  if (P == 3) red[3][q][bl] = gk;
   __syncthreads();
   if (q != 0 || !live) return;
-  gv = gh = us = 0.0;
+  gv = gh = gk = us = 0.0;
 #pragma unroll
   for (int j = 0; j < RFS_ASM_Q; j++) {
     gv += red[0][j][bl];
     gh += red[1][j][bl];
     us += red[2][j][bl];
+    if (P == 3) gk += red[3][j][bl];
   }
   if (ok) {
     const double w = (which == 0) ? wt[set] : 1.0;
-    double g0 = w * gv, g1 = w * gh;
+    double g0 = w * gv, g1 = w * gh, g2 = w * gk;
     if (which != 2) {
-      g0 += g_rf[b * 2 * n + m];
-      g1 += g_rf[b * 2 * n + n + m];
+      g0 += g_rf[b * P * n + m];
+      g1 += g_rf[b * P * n + n + m];
+      if (P == 3) g2 += g_rf[b * P * n + 2 * n + m];
     }
-    grad[b * 2 * n + m] = g0;
-    grad[b * 2 * n + n + m] = g1;
+    grad[b * P * n + m] = g0;
+    grad[b * P * n + n + m] = g1;
+    if (P == 3) grad[b * P * n + 2 * n + m] = g2;
     if (m == 0) {
       double u = w * 0.5 * us;
       if (which != 2) u += U_rf[b];
@@ -123,8 +131,9 @@ __global__ void joint_assemble_kernel(SwdPlan plan, SwdView V, SwdSetView sv, co
     }
   } else {
     // model_rf_swd_vs_thk.py:73-74: (0.0, zeros, dobs, False), dobs of the row's own set
-    grad[b * 2 * n + m] = 0.0;
-    grad[b * 2 * n + n + m] = 0.0;
+    grad[b * P * n + m] = 0.0;
+    grad[b * P * n + n + m] = 0.0;
+    if (P == 3) grad[b * P * n + 2 * n + m] = 0.0;
     const double fill = (set < 0) ? nan("") : 0.0;
     for (int j = m; j < ndata; j += n) dsyn[b * ndata + j] = (which == 2 || set < 0) ? fill : dobs[j];
     if (m == 0) {

@@ -267,11 +267,12 @@ RFS_DEVINL void rf_mat_a_par(const RfLayer &L, const RfTrig &t, cd k, cd v_alpha
 RFS_DEVINL cd nan0(cd z) { return (isnan(z.x) || isnan(z.y)) ? cd(0.0, 0.0) : z; }
 
 // ---- K3: one thread per (model, frequency bin)
-//  rfm  : [4][n][B] thk, rho, vp, vs (float64)     chain: [2][n][B] dadb, drda (NQ==2 only)
+//  rfm  : [4][n][B] thk, rho, vp, vs (float64)     chain: [NQ][n][B] dadb, drda, dadk (NQ==2,3 only)
 //  qa,qb: [n][B] or NULL (=> 9999)
 //  spec : [B][2][n2] complex  (R21, R22)
 //  dspec: [B][NQ*n][n2] complex  D = R22_m R21 - R21_m R22
-//         NQ==4: rows rho,vp,vs,h (kernel_all order);  NQ==2: rows vs-chain, thk
+//         NQ==4: rows rho,vp,vs,h (kernel_all order);  NQ==2: rows vs-chain, thk;
+//         NQ==3: rows vs-chain, thk, k-chain (x = [vs, thk, Vp/Vs])
 //  sigma: imaginary part of omega is -sigma (freq method) or 0 (time method)
 #ifndef RFS_RF_MINBLOCKS
 #define RFS_RF_MINBLOCKS 2
@@ -448,6 +449,12 @@ __global__ void __launch_bounds__(128, RFS_RF_MINBLOCKS)
       const cd Dv = Dq[2] + dadb * Dq[1] + (drda * dadb) * Dq[0];
       dout[((long long)0 * n + m) * n2] = make_double2(Dv.x, Dv.y);
       dout[((long long)1 * n + m) * n2] = make_double2(Dq[3].x, Dq[3].y);
+      if (NQ == 3) {
+        // Vp/Vs row (vp = k vs): dadk*kvp + drda*dadk*krho, dadk = vs
+        const double dadk = chain[2 * nB + m * B + b];
+        const cd Dk = dadk * Dq[1] + (drda * dadk) * Dq[0];
+        dout[((long long)2 * n + m) * n2] = make_double2(Dk.x, Dk.y);
+      }
     }
   }
 }

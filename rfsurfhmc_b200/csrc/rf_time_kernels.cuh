@@ -159,10 +159,12 @@ __global__ void __launch_bounds__(256, 3) rf_time_kernel(const double2 *__restri
 
 // misfit and gradient from materialised Frechet traces (time-domain method, where the adjoint
 // shortcut does not apply because deconit is nonlinear).  One thread per (model, layer).
-//   traces [B][4][n][nt] (rho, vp, vs, h);  chain [2][n][B];  rf [B][ldrf];  grad [B][2n]
+//   traces [B][4][n][nt] (rho, vp, vs, h);  chain [P][n][B];  rf [B][ldrf];  grad [B][P n]
+//   P = 3: the third block is the Vp/Vs gradient dadk*kvp + drda*dadk*krho (dadk = vs)
 //   flag [B] or NULL: only written (0) for a row whose observation-set index is out of range; such a
 //   row gets U 0, grad 0 and a NaN trace.  The residual is 0 at the samples the row's set does not fit
 //   (ObsSets::observed).
+template <int P>
 __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const double *__restrict__ chain,
                                      double *__restrict__ rf, long long ldrf, ObsSets obs, long long B,
                                      int n, int nt, double *__restrict__ U, double *__restrict__ grad,
@@ -173,8 +175,9 @@ __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const do
   const int m = (int)(i / B);
   const int set = obs.row_set(b);
   if (set < 0) {
-    grad[b * 2 * n + m] = 0.0;
-    grad[b * 2 * n + n + m] = 0.0;
+    grad[b * P * n + m] = 0.0;
+    grad[b * P * n + n + m] = 0.0;
+    if (P == 3) grad[b * P * n + 2 * n + m] = 0.0;
     if (m == 0) {
       for (int t = 0; t < nt; t++) rf[b * ldrf + t] = nan("");
       U[b] = 0.0;
@@ -185,23 +188,27 @@ __global__ void rf_trace_grad_kernel(const double *__restrict__ traces, const do
   const double *dobs = obs.row(set);
   const long long nB = (long long)n * B;
   const double dadb = chain[0 * nB + m * B + b], drda = chain[1 * nB + m * B + b];
+  const double dadk = P == 3 ? chain[2 * nB + m * B + b] : 0.0;
   const double *kr = traces + ((b * 4 + 0) * n + m) * (long long)nt;
   const double *ka = traces + ((b * 4 + 1) * n + m) * (long long)nt;
   const double *kb = traces + ((b * 4 + 2) * n + m) * (long long)nt;
   const double *kh = traces + ((b * 4 + 3) * n + m) * (long long)nt;
-  double g0 = 0.0, g1 = 0.0, us = 0.0;
+  double g0 = 0.0, g1 = 0.0, g2 = 0.0, us = 0.0;
   for (int t = 0; t < nt; t++) {
     const double res = obs.observed(set, t) ? rf[b * ldrf + t] - dobs[t] : 0.0;
     g0 += (kb[t] + dadb * ka[t] + drda * dadb * kr[t]) * res;
     g1 += kh[t] * res;
+    if (P == 3) g2 += (dadk * ka[t] + drda * dadk * kr[t]) * res;
     us += res * res;
   }
   if (accumulate) {
-    g0 += grad[b * 2 * n + m];
-    g1 += grad[b * 2 * n + n + m];
+    g0 += grad[b * P * n + m];
+    g1 += grad[b * P * n + n + m];
+    if (P == 3) g2 += grad[b * P * n + 2 * n + m];
   }
-  grad[b * 2 * n + m] = g0;
-  grad[b * 2 * n + n + m] = g1;
+  grad[b * P * n + m] = g0;
+  grad[b * P * n + n + m] = g1;
+  if (P == 3) grad[b * P * n + 2 * n + m] = g2;
   if (m == 0) U[b] = accumulate ? U[b] + 0.5 * us : 0.5 * us;
 }
 

@@ -12,9 +12,11 @@ namespace rfs {
 // ---- model preparation: x=[vs(n),thk(n)] -> Brocher vp/rho (+derivatives) and the two model
 // blocks.  Follows model/model_surf.py:47-79 and model/model_rf.py:52-77 (same polynomials) and
 // the float32 cast at the SWD boundary (src/SWD/main.cpp:7-9).
+// P = 3 (rfs_config_param RFS_PARAM_VS_THK_VPVS): x=[vs(n),thk(n),k(n)] with vp = k vs, rho = Brocher(vp).
 // swd  : [SWD_NF][n][B]  float32-rounded values stored as double
 // rfm  : [4][n][B]       thk, rho, vp, vs in float64 (RF argument order)
-// chain: [2][n][B]       dadb, drda
+// chain: [P][n][B]       dadb, drda (P = 3: dadb = k, then dadk = vs)
+template <int P>
 __global__ void prep_models_kernel(const double *__restrict__ x, long long B, int n,
                                    double *__restrict__ swd, double *__restrict__ rfm,
                                    double *__restrict__ chain) {
@@ -22,14 +24,19 @@ __global__ void prep_models_kernel(const double *__restrict__ x, long long B, in
   if (i >= B * n) return;
   const long long b = i % B;
   const int m = (int)(i / B);
-  const double vs = x[b * 2 * n + m], thk = x[b * 2 * n + n + m];
-  const double vp = 0.9409 + 2.0947 * vs - 0.8206 * (vs * vs) + 0.2683 * (vs * vs * vs) -
-                    0.0251 * (vs * vs * vs * vs);
+  const double vs = x[b * P * n + m], thk = x[b * P * n + n + m];
+  double vp, dadb;
+  if (P == 3) {
+    dadb = x[b * P * n + 2 * n + m];
+    vp = dadb * vs;
+  } else {
+    vp = 0.9409 + 2.0947 * vs - 0.8206 * (vs * vs) + 0.2683 * (vs * vs * vs) - 0.0251 * (vs * vs * vs * vs);
+    dadb = 2.0947 - 0.8206 * 2 * vs + 0.2683 * 3 * (vs * vs) - 0.0251 * 4 * (vs * vs * vs);
+  }
   const double rho = 1.6612 * vp - 0.4721 * (vp * vp) + 0.0671 * (vp * vp * vp) -
                      0.0043 * (vp * vp * vp * vp) + 0.000106 * (vp * vp * vp * vp * vp);
   const double drda = 1.6612 - 0.4721 * 2 * vp + 0.0671 * 3 * (vp * vp) -
                       0.0043 * 4 * (vp * vp * vp) + 0.000106 * 5 * (vp * vp * vp * vp);
-  const double dadb = 2.0947 - 0.8206 * 2 * vs + 0.2683 * 3 * (vs * vs) - 0.0251 * 4 * (vs * vs * vs);
   const long long nb = (long long)n * B;
   if (swd) {
     const double d32 = (double)(float)thk, a32 = (double)(float)vp, b32 = (double)(float)vs,
@@ -54,6 +61,7 @@ __global__ void prep_models_kernel(const double *__restrict__ x, long long B, in
   if (chain) {
     chain[0 * nb + m * B + b] = dadb;
     chain[1 * nb + m * B + b] = drda;
+    if (P == 3) chain[2 * nb + m * B + b] = vs;
   }
 }
 

@@ -8,6 +8,9 @@ write `real_syn.npy`, per-chain result files and `misfit.npy [nchains, nsamples]
 `mpiexec -n N` of the reference becomes `--chains N`: all chains of a rank run at once on its GPU.
 In the parameter file, rf.ray_p may be a list of ray parameters and rf.gauss a list of Gaussian widths
 (e.g. `gauss: [1.0, 2.5]`): the receiver-function data are then one trace per (ray, width), in that order.
+An optional `true_model.vpvs: [n values]` samples each layer's Vp/Vs ratio as a third parameter block:
+models are [vs, thk, vpvs] (vp = vpvs * vs, density from Brocher's polynomial of vp), the observations are
+synthesised from [vs, thk, vpvs] and the Vp/Vs box is +-10 % of the true values (fixtures.driver_bounds_vpvs).
 
     python -m rfsurfhmc_b200.driver --param param.yaml --stations stations.npz --chains K
 
@@ -17,7 +20,8 @@ ray parameter(s) in place of rf.ray_p, swd_use [S, nper] the periods of the swd 
 rf_use [S, nray*ngauss*nt] or [S, nray, ngauss, nt] ([S, nray, nt] with one width) the
 receiver-function samples it fits: missing ray bins, fitting windows, and gauss [S] or [S, ngauss] its
 own Gaussian width(s) in place of rf.gauss: the widths its data were processed with), K chains run per station, all S*K in one device run (sharded
-over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station."""
+over ranks under torchrun), and {outdir}/{name}/misfit.npy [K, nsamples] is written per station.  With
+true_model.vpvs the file's bounds are [S, 3n, 2]."""
 import argparse
 import os
 import time
@@ -30,7 +34,7 @@ from .model.model_rf_swd_vs_thk import Joint_RF_SWD
 from .model.stations import StationArray, load_stations
 from .pyhmc.hmc import HamitonianMC
 from .pyhmc.hmcda import HMCDualAveraging
-from .fixtures import driver_bounds
+from .fixtures import driver_bounds, driver_bounds_vpvs
 from . import distributed as D
 
 
@@ -45,8 +49,9 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
     torch.cuda.set_device(local)
     if ws > 1 and not dist.is_initialized():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    model_swd = SurfWD.init(**param['swd'])
-    model_rf = ReceiverFunc.init(**param['rf'])
+    vpvs = param['true_model'].get('vpvs')
+    model_swd = SurfWD.init(**param['swd'], vpvs=vpvs is not None)
+    model_rf = ReceiverFunc.init(**param['rf'], vpvs=vpvs is not None)
     thk = np.asarray(param['true_model']['thk'], dtype=np.float64)
     vs = np.asarray(param['true_model']['vs'], dtype=np.float64)
     model_swd.set_thk(thk)
@@ -56,6 +61,13 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
     outdir = param['hmc']['OUTPUT_DIR']
     os.makedirs(outdir, exist_ok=True)
     x = np.hstack((vs, thk))
+    bounds_of = driver_bounds
+    if vpvs is not None:
+        k = np.asarray(vpvs, dtype=np.float64)
+        if k.shape != vs.shape:
+            raise ValueError(f"true_model.vpvs has {k.size} values for {vs.size} layers")
+        x = np.hstack((vs, thk, k))
+        bounds_of = driver_bounds_vpvs
     if stations is None:
         dobs = np.zeros(model.ndata)
         if rank == 0:
@@ -66,11 +78,11 @@ def run(param, sampler="base", nchains=4, save_chains=True, max_iters=0, max_L=0
         dobs = D.bcast_array(dobs)
         nt = model.rfmodel.nt
         model.set_obsdata(dobs[:nt], dobs[nt:])
-        boundaries = driver_bounds(x)
+        boundaries = bounds_of(x)
         npairs = nchains
         ids, sidx = D.shard_chains(nchains), None
     else:
-        st = load_stations(stations, model.ndata, x.size, driver_bounds(x), model_rf.nray, model_swd, model_rf,
+        st = load_stations(stations, model.ndata, x.size, bounds_of(x), model_rf.nray, model_swd, model_rf,
                            model_rf.ngauss)
         model = StationArray(model, st["dobs"], st["sigma1"], st["sigma2"], st["names"], st["ray_p"],
                              st["swd_use"], st["rf_use"], st["gauss"])
@@ -117,7 +129,8 @@ def main():
     ap.add_argument("--sampler", default="base", choices=["base", "da"])
     ap.add_argument("--chains", type=int, default=4, help="chains (per station with --stations)")
     ap.add_argument("--stations", default=None,
-                    help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2], "
+                    help="stations .npz (dobs [S,ndata]; optional names, sigma1, sigma2 [S], bounds [S,2n,2] "
+                         "([S,3n,2] with true_model.vpvs), "
                          "ray_p [S] or [S,nray] in place of rf.ray_p, swd_use [S,nper] observed periods of the "
                          "swd lists, rf_use [S,nray*ngauss*nt] or [S,nray,ngauss,nt] fitted RF samples, gauss [S] or "
                          "[S,ngauss] in place of rf.gauss): invert every "

@@ -31,6 +31,26 @@ def driver_bounds(x_true):
     return b
 
 
+def driver_bounds_vpvs(x_true):
+    """Box of the [vs, thk, vpvs] parameterisation: driver_bounds for vs and thk, Vp/Vs +-10 % of the
+    true value."""
+    n = x_true.size // 3
+    k = x_true[2 * n:]
+    return np.vstack((driver_bounds(x_true[:2 * n]), np.stack((k * 0.9, k * 1.1), axis=1)))
+
+
+def sorted_uniform_models_vpvs(bounds, B, seed):
+    """sorted_uniform_models for [vs, thk, vpvs] boxes [3n, 2]: vs sorted ascending, thk and Vp/Vs
+    permuted alike (the rule of the device HMC's initial models)."""
+    rng = np.random.default_rng(seed)
+    n = bounds.shape[0] // 3
+    X = bounds[:, 0] + (bounds[:, 1] - bounds[:, 0]) * rng.random((B, 3 * n))
+    idx = np.argsort(X[:, :n], axis=1)
+    for j in range(3):
+        X[:, j * n:(j + 1) * n] = np.take_along_axis(X[:, j * n:(j + 1) * n], idx, axis=1)
+    return X
+
+
 def sorted_uniform_models(bounds, B, seed):
     """Uniform draws in the box, vs sorted ascending with thk permuted alike — the distribution of
     HamitonianMC.set_initial_model (pyhmc/hmc.py:74-93), without the in-bounds redraw."""

@@ -7,14 +7,18 @@ CUDA path (rfs_misfit_grad_host, which=1): propagator + spectral deconvolution +
 Extensions: `ray_p` may be a list of ray parameters and `gauss` a list of Gaussian widths; the data
 vector is then the concatenation of one trace per (ray parameter, width) in the order [ray][gauss]
 (`nt` counts all of them, `nt_trace` one trace) and misfit / gradient sum over them — one objective per
-chain instead of one model object per ray parameter and width."""
+chain instead of one model object per ray parameter and width.  With `vpvs=True` the model vector is
+[vs, thk, vpvs] (model/param.py): each layer's Vp/Vs ratio is sampled instead of following Brocher's curve."""
 import numpy as np
 from .lib import librf
 from .._lib import Context
+from . import param
 
 
 class ReceiverFunc:
-    def __init__(self, ray_p, nt, dt, gauss, time_shift, water_level=0.001, type_="p", method="time"):
+    def __init__(self, ray_p, nt, dt, gauss, time_shift, water_level=0.001, type_="p", method="time", *,
+                 vpvs=False):
+        self.vpvs = bool(vpvs)
         self.ray_p = ray_p
         self.nray = int(np.size(ray_p))
         self.ngauss = int(np.size(gauss))
@@ -36,7 +40,7 @@ class ReceiverFunc:
     @classmethod
     def init(self, **kargs):
         return ReceiverFunc(kargs['ray_p'], kargs['nt'], kargs['dt'], kargs['gauss'], kargs['time_shift'],
-                            kargs['water_level'], kargs['type'], kargs['method'])
+                            kargs['water_level'], kargs['type'], kargs['method'], vpvs=kargs.get('vpvs', False))
 
     def set_obsdata(self, dobs):
         self.dobs = dobs
@@ -50,7 +54,14 @@ class ReceiverFunc:
     def set_thk(self, thk):
         self.thk = thk * 1.0
 
-    def empirical_relation(self, vs, deriv=False):
+    @property
+    def npar(self):
+        return param.npar(self.vpvs)
+
+    def empirical_relation(self, vs, deriv=False, k=None):
+        """Brocher vp and rho of vs; with k (Vp/Vs per layer) vp = k vs and dadb = k."""
+        if k is not None:
+            return param.brocher(vs, k, deriv)
         vp = 0.9409 + 2.0947 * vs - 0.8206 * vs**2 + 0.2683 * vs**3 - 0.0251 * vs**4
         rho = 1.6612 * vp - 0.4721 * vp**2 + 0.0671 * vp**3 - 0.0043 * vp**4 + 0.000106 * vp**5
         if deriv:
@@ -64,7 +75,7 @@ class ReceiverFunc:
         # one of them after the first call re-configures the device context
         gauss = self.gauss if np.ndim(self.gauss) == 0 else tuple(np.asarray(self.gauss, dtype=np.float64).tolist())
         return (n, tuple(np.atleast_1d(self.ray_p).tolist()), self.nt_trace, self.dt, gauss,
-                self.time_shift, self.water_level, self.rf_type, self.method)
+                self.time_shift, self.water_level, self.rf_type, self.method, self.vpvs)
 
     def _config_key(self, n):
         return self._config_fields(n) + (np.asarray(self.dobs, dtype=np.float64).tobytes(),)
@@ -81,16 +92,21 @@ class ReceiverFunc:
         return self._ctx
 
     def _config_forward(self, ctx, n):
+        ctx.config_param(self.vpvs)
         ctx.config_rf(n, self.ray_p, self.nt_trace, self.dt, self.gauss, self.time_shift, self.water_level,
                       self.rf_type, self.method)
 
     _context = device_context
 
     def forward(self, x: np.ndarray):
-        layers = int(len(x) / 2)
-        vs = x[:layers]
-        thk = x[layers:]
-        vp, rho = self.empirical_relation(vs, deriv=False)
+        if self.vpvs:
+            vs, thk, k = param.split(x, True)
+            vp, rho = self.empirical_relation(vs, k=k)
+        else:
+            layers = int(len(x) / 2)
+            vs = x[:layers]
+            thk = x[layers:]
+            vp, rho = self.empirical_relation(vs, deriv=False)
         qa = thk * 0 + 9999.
         qb = thk * 0 + 9999.
         out = [librf.forward(thk, rho, vp, vs, qa, qb, float(p), self.nt_trace, self.dt, float(g),
@@ -104,11 +120,11 @@ class ReceiverFunc:
 
     def misfit_and_grad(self, x):
         x = np.asarray(x, dtype=np.float64)
-        n = int(x.shape[0] / 2)
+        n = param.layer_count(x.shape[0], self.vpvs)
         U, g, d, _ = self.device_context(n).misfit_grad_host(x[None, :], which=1)
         return float(U[0]), g[0], d[0]
 
     def misfit_and_grad_batch(self, X):
-        """X [B, 2n] -> (U[B], grad[B,2n], dsyn[B,nt], flag[B]) in one fused GPU evaluation."""
+        """X [B, P n] -> (U[B], grad[B,P n], dsyn[B,nt], flag[B]) in one fused GPU evaluation."""
         X = np.atleast_2d(np.asarray(X, dtype=np.float64))
-        return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=1)
+        return self.device_context(param.layer_count(X.shape[1], self.vpvs)).misfit_grad_host(X, which=1)

@@ -2,15 +2,20 @@
 
 `misfit_and_grad(x)` keeps the reference contract `(misfit, grad[2n], dsyn[ndata], flag)` with the
 failure convention `(0.0, zeros, dobs, False)` (:73-74), and adds `misfit_and_grad_batch(X)` /
-`device_context()` for the many-chains path (one fused CUDA evaluation for all rows of X)."""
+`device_context()` for the many-chains path (one fused CUDA evaluation for all rows of X).  The
+parameterisation (`vpvs`, model/param.py) is the two sub-models' own: they must agree."""
 import numpy as np
 from .model_rf import ReceiverFunc
 from .model_surf import SurfWD
 from .._lib import Context
+from . import param
 
 
 class Joint_RF_SWD:
     def __init__(self, sigma1, sigma2, rfmodel: ReceiverFunc, swdmodel: SurfWD) -> None:
+        if getattr(rfmodel, "vpvs", False) != getattr(swdmodel, "vpvs", False):
+            raise ValueError(f"the receiver-function model has vpvs={rfmodel.vpvs} and the dispersion model "
+                             f"vpvs={swdmodel.vpvs}: a joint model needs one parameterisation")
         self.sigma1 = sigma1
         self.sigma2 = sigma2
         self.rfmodel = rfmodel
@@ -20,6 +25,14 @@ class Joint_RF_SWD:
         self._ctx = None
         self._ctx_key = None
         self._device = 0
+
+    @property
+    def vpvs(self):
+        return self.rfmodel.vpvs
+
+    @property
+    def npar(self):
+        return param.npar(self.vpvs)
 
     def set_obsdata(self, rfobs: np.ndarray, swdobs: np.ndarray):
         self.dobs = np.zeros((self.ndata))
@@ -76,9 +89,9 @@ class Joint_RF_SWD:
         return 0.0, flag
 
     def misfit_and_grad_batch(self, X):
-        """X [B, 2n] -> (U[B], grad[B,2n], dsyn[B,ndata], flag[B]) in one fused GPU evaluation."""
+        """X [B, P n] -> (U[B], grad[B,P n], dsyn[B,ndata], flag[B]) in one fused GPU evaluation."""
         X = np.atleast_2d(np.asarray(X, dtype=np.float64))
-        return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=0)
+        return self.device_context(param.layer_count(X.shape[1], self.vpvs)).misfit_grad_host(X, which=0)
 
     def misfit_and_grad(self, x: np.ndarray):
         x = np.asarray(x, dtype=np.float64)

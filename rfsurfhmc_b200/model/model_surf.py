@@ -8,14 +8,17 @@ goes through the libsurf drop-in.  Reference quirks kept: Lc/Lg are evaluated on
 root search the gradient has length n, not 2n (:179-180).
 
 Extension: `mode` may be an ascending list of modes; the data vector is then [mode][Rc,Rg,Lc,Lg]
-(`nt` counts all of them) and all modes come out of ONE chained root-search pass."""
+(`nt` counts all of them) and all modes come out of ONE chained root-search pass.  With `vpvs=True` the model vector is
+[vs, thk, vpvs] (model/param.py): each layer's Vp/Vs ratio is sampled instead of following Brocher's curve."""
 import numpy as np
 from .lib import libsurf
 from .._lib import Context
+from . import param
 
 
 class SurfWD:
-    def __init__(self, mode=0, sphere=False, tRc=None, tRg=None, tLc=None, tLg=None):
+    def __init__(self, mode=0, sphere=False, tRc=None, tRg=None, tLc=None, tLg=None, *, vpvs=False):
+        self.vpvs = bool(vpvs)
         self.mode = mode
         self.nmode = int(np.size(mode))
         self.sphere = sphere
@@ -46,7 +49,8 @@ class SurfWD:
 
     @classmethod
     def init(self, **kargs):
-        return SurfWD(tRc=kargs['tRc'], tRg=kargs['tRg'], tLc=kargs['tLc'], tLg=kargs['tLg'])
+        return SurfWD(tRc=kargs['tRc'], tRg=kargs['tRg'], tLc=kargs['tLc'], tLg=kargs['tLg'],
+                      vpvs=kargs.get('vpvs', False))
 
     def set_obsdata(self, dobs):
         self.dobs = dobs
@@ -60,7 +64,15 @@ class SurfWD:
     def set_thk(self, thk):
         self.thk = thk * 1.0
 
-    def empirical_relation(self, vs: np.ndarray, deriv=False):
+    @property
+    def npar(self):
+        return param.npar(self.vpvs)
+
+    def empirical_relation(self, vs: np.ndarray, deriv=False, k=None):
+        """Brocher vp and rho of vs (and dadb, drda); with k (Vp/Vs per layer) vp = k vs and dadb = k."""
+        if k is not None:
+            vp, rho, drda, dadb = param.brocher(vs, k, True)
+            return (vp, rho, dadb, drda) if deriv else (vp, rho)
         vp = 0.9409 + 2.0947 * vs - 0.8206 * vs**2 + 0.2683 * vs**3 - 0.0251 * vs**4
         rho = 1.6612 * vp - 0.4721 * vp**2 + 0.0671 * vp**3 - 0.0043 * vp**4 + 0.000106 * vp**5
         dadb = np.zeros(vp.shape)
@@ -85,7 +97,7 @@ class SurfWD:
         # every field the reference reads on each misfit_and_grad call (model_surf.py:155-228)
         per = tuple(None if t is None else np.asarray(t, dtype=np.float64).tobytes()
                     for t in self._grad_periods())
-        return (n, tuple(np.atleast_1d(self.mode).tolist()), bool(self.sphere), per)
+        return (n, tuple(np.atleast_1d(self.mode).tolist()), bool(self.sphere), per, self.vpvs)
 
     def _config_key(self, n):
         return self._config_fields(n) + (np.asarray(self.dobs, dtype=np.float64).tobytes(),)
@@ -102,6 +114,7 @@ class SurfWD:
         return self._ctx
 
     def _config_forward(self, ctx, n):
+        ctx.config_param(self.vpvs)
         tRc, tRg, tLc, tLg = self._grad_periods()
         ctx.config_swd(n, tRc, tRg, tLc, tLg, mode=self.mode, sphere=self.sphere)
 
@@ -109,10 +122,14 @@ class SurfWD:
 
     def forward(self, x: np.ndarray):
         d = np.zeros((self.nt))
-        layers = int(len(x) / 2)
-        vs = x[:layers]
-        thk = x[layers:]
-        vp, rho = self.empirical_relation(vs)
+        if self.vpvs:
+            vs, thk, k = param.split(x, True)
+            vp, rho = self.empirical_relation(vs, k=k)
+        else:
+            layers = int(len(x) / 2)
+            vs = x[:layers]
+            thk = x[layers:]
+            vp, rho = self.empirical_relation(vs)
         k1 = 0
         for mode in np.atleast_1d(self.mode):
             for nt_w, wt in ((self.ntRc, "Rc"), (self.ntRg, "Rg"), (self.ntLc, "Lc"), (self.ntLg, "Lg")):
@@ -132,13 +149,13 @@ class SurfWD:
 
     def misfit_and_grad(self, x):
         x = np.asarray(x, dtype=np.float64)
-        n = int(x.shape[0] / 2)
+        n = param.layer_count(x.shape[0], self.vpvs)
         U, g, d, f = self.device_context(n).misfit_grad_host(x[None, :], which=2)
         if not f[0]:
             return 0.0, np.zeros((n)), d[0], False
         return float(U[0]), g[0], d[0], True
 
     def misfit_and_grad_batch(self, X):
-        """X [B, 2n] -> (U[B], grad[B,2n], dsyn[B,nt], flag[B]) in one fused GPU evaluation."""
+        """X [B, P n] -> (U[B], grad[B,P n], dsyn[B,nt], flag[B]) in one fused GPU evaluation."""
         X = np.atleast_2d(np.asarray(X, dtype=np.float64))
-        return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=2)
+        return self.device_context(param.layer_count(X.shape[1], self.vpvs)).misfit_grad_host(X, which=2)

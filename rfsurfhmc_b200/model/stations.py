@@ -25,8 +25,11 @@ With gauss [S] or [S, ngauss] station s's receiver functions are computed with i
 stays shared, and a station that fits fewer widths drops the others with rf_use.
 
 A stations file (load_stations, `driver --stations`) is an .npz with dobs [S, ndata] and the optional
-keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2], ray_p [S] or [S, nray], swd_use [S, nper],
-rf_use in one of the shapes above and gauss [S] or [S, ngauss].
+keys names [S], sigma1 / sigma2 [S], bounds [S, 2n, 2] ([S, 3n, 2] for a template with vpvs=True),
+ray_p [S] or [S, nray], swd_use [S, nper], rf_use in one of the shapes above and gauss [S] or [S, ngauss].
+
+The array inherits the template's parameterisation (model/param.py): with vpvs=True every row is
+[vs, thk, vpvs] and station_model(s) keeps the flag.
 """
 import copy
 import numpy as np
@@ -34,6 +37,7 @@ from .._lib import Context
 from .model_rf_swd_vs_thk import Joint_RF_SWD
 from .model_rf import ReceiverFunc
 from .model_surf import SurfWD
+from . import param
 
 
 def _fresh_copy(m):
@@ -111,6 +115,14 @@ class StationArray:
     def _device(self):
         return self.template._device
 
+    @property
+    def vpvs(self):
+        return self.template.vpvs
+
+    @property
+    def npar(self):
+        return param.npar(self.vpvs)
+
     def device_context(self, n):
         """Configured rfs context (the template's forward configuration + every station's observations)
         for n layers; re-configured whenever a template field, a sigma or an observation has changed."""
@@ -137,10 +149,11 @@ class StationArray:
         return self._ctx
 
     def misfit_and_grad_batch(self, X, stations):
-        """X [B, 2n], stations [B] -> (U[B], grad[B,2n], dsyn[B,ndata], flag[B]): row b against station
+        """X [B, P n], stations [B] -> (U[B], grad[B,P n], dsyn[B,ndata], flag[B]): row b against station
         stations[b], all rows in one fused GPU evaluation."""
         X = np.atleast_2d(np.asarray(X, dtype=np.float64))
-        return self.device_context(X.shape[1] // 2).misfit_grad_host(X, which=self.which, sets=stations)
+        return self.device_context(param.layer_count(X.shape[1], self.vpvs)).misfit_grad_host(
+            X, which=self.which, sets=stations)
 
     def station_model(self, s):
         """Single-station copy of the template holding station s's observations (and sigmas, ray

@@ -26,13 +26,18 @@ def finish_run(out, nsamples, ndraws):
 
 
 def station_run_args(model, boundaries, chain_ids, stations):
-    """(n, sets) for Context.hmc_run: the layer count from `boundaries` ([2n,2] or [S,2n,2]) and the
-    station of each chain (None without a StationArray).  Chain i samples station stations[i]."""
+    """(n, sets) for Context.hmc_run: the layer count from `boundaries` ([P n,2] or [S,P n,2], P = 3 for
+    a model with vpvs=True, else 2) and the station of each chain (None without a StationArray).  Chain i
+    samples station stations[i]."""
+    from ..model import param
     b = np.asarray(boundaries)
     if b.ndim not in (2, 3) or b.shape[-1] != 2:
         raise ValueError(f"boundaries must be [2n, 2] or [S, 2n, 2], got shape {b.shape}")
+    vpvs = bool(getattr(model, "vpvs", False))
+    n = param.layer_count(b.shape[-2], vpvs)
+    param.check_vpvs_box(b, vpvs)
     if stations is None:
-        return b.shape[-2] // 2, None
+        return n, None
     if not hasattr(model, "station_model"):
         raise ValueError("stations= needs a StationArray model")
     st = np.asarray(stations, dtype=np.int64)
@@ -40,7 +45,7 @@ def station_run_args(model, boundaries, chain_ids, stations):
         raise ValueError("stations must give one station per chain id")
     if b.ndim == 3 and b.shape[0] != model.nstations:
         raise ValueError(f"boundaries has {b.shape[0]} boxes for {model.nstations} stations")
-    return b.shape[-2] // 2, st
+    return n, st
 
 
 def save_chains(model, out, chain_ids, stations, outdir, name, nbest, nsamples):
